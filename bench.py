@@ -86,7 +86,28 @@ def parse_args():
     ap.add_argument("--no-regimes", action="store_true", help="skip the mean-zero regime")
     ap.add_argument("--no-reduction", action="store_true", help="skip the build with the pre-graph reduction (SURVEY.md 8(f)-1)")
     ap.add_argument("--no-hybrid", action="store_true", help="skip the hybrid-search leg (SURVEY.md 8(f)-2; N = 1 only, separate process)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's search results (top-k indices and scores) as DIR/<name>.npy, float64")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, idx, score):
+    """--dump-outputs: the result arrays of the last timed step, so that two builds run with the same arguments (same seeded
+    inputs) can be compared output for output.  float64 holds the int64 indices exactly (-1 = no hit).  A batch whose results
+    exceed 64 MB is written as a fixed, seeded sample of its queries; query_rows.npy names the rows written."""
+    rows = np.arange(idx.shape[0])
+    keep = (DUMP_BYTES - 4096) // (8 + 16 * idx.shape[1])              # bytes per query: its row number + topk (index, score)
+    if len(rows) > keep:
+        rows = np.sort(np.random.default_rng(0).choice(len(rows), keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in (("query_rows", rows), ("search_idx", idx[rows]), ("search_scores", score[rows])):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 # --------------------------------------------------------------------------- clocks
@@ -158,9 +179,10 @@ def cpu_oracle_run(cfg, n_items, nq, reps, label):
     ts = []
     for _ in range(reps):
         t0 = time.perf_counter()
-        s.search_batch(q, g, cfg["tau"])
+        idx, sc, _ = s.search_batch(q, g, cfg["tau"])
         ts.append(time.perf_counter() - t0)
-    return {"build_s": t_build, "search_s": ts, "threads": oracle.num_threads(), "n_items": n_items, "nq": nq}
+    return {"build_s": t_build, "search_s": ts, "threads": oracle.num_threads(), "n_items": n_items, "nq": nq,
+            "idx": idx, "sc": sc}
 
 
 def run_reference(args, cfg):
@@ -172,6 +194,8 @@ def run_reference(args, cfg):
     cfg = dict(cfg, n=n)
     nq = args.ref_queries
     r = cpu_oracle_run(cfg, n, nq, args.warmup + args.steps, "reference")
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, r["idx"], r["sc"])
     ts = r["search_s"][args.warmup:]
     total = sum(ts)
     val = nq * len(ts) / total
@@ -409,6 +433,8 @@ def main():
 
     # ---- search: W warm-up steps, then exactly K timed steps (+ the end-to-end loop)
     main_run = search_regime(aspace, gl, q_dev, q_host, args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:                               # N > 1: every rank holds the whole merged result
+        dump_outputs(args.dump_outputs, main_run["idx"], main_run["sc"])
     step_ms, e2e_ms, launches, stage1_ms, sstat, clk = (main_run[k] for k in ("step_ms", "e2e_ms", "launches", "stage1_ms", "stats", "clocks"))
     slow = sstat["search_slow_queries"]
     stage1_is_tc = sstat["search_stage1_is_tc"] == 1.0

@@ -1106,3 +1106,28 @@ def test_wide_band_one_term_first_then_three_term_retry(oracle_mod):
         _force_stage1(None)
         for k in ("ASP_TC_CAPB", "ASP_TC_FIRST_TERMS"):
             os.environ.pop(k, None)
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(oracle_mod, tmp_path):
+    """`bench.py --dump-outputs` on the CUDA path at a reduced size: the dumped arrays are the results of the last timed step
+    (query batch (steps - 1) % 2 of the bench's two seeded batches), equal to the oracle's full scan of that batch."""
+    import json
+    from pyarrowspace_b200 import synth
+    n, nq, steps = 20000, 1000, 2
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "1", "--items", str(n),
+                        "--queries", str(nq), "--build-reps", "1", "--parity-queries", "0", "--no-cpu-baseline", "--no-item-graph",
+                        "--no-regimes", "--no-reduction", "--no-hybrid", "--dump-outputs", str(tmp_path / "out")],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    lines = [l for l in r.stdout.splitlines() if l.strip()]
+    assert len(lines) == 1 and json.loads(lines[0])["steps"] == steps
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").iterdir()}
+    assert sorted(got) == ["query_rows", "search_idx", "search_scores"]
+    assert all(a.dtype == np.float64 for a in got.values())
+    cfg = synth.config("C4")
+    x = synth.make_items(n, cfg["f"], cfg["seed"], cfg["scale"])
+    q, _ = synth.make_queries(x, nq, cfg["seed"] + (steps - 1) % 2, cfg["scale"])
+    s, g = oracle_mod.build(cfg["graph_params"], x)
+    oidx, osc, _ = s.search_batch(q, g, cfg["tau"])
+    np.testing.assert_array_equal(got["query_rows"], np.arange(nq))
+    _assert_hits_equal(got["search_idx"].astype(np.int64), got["search_scores"], oidx, osc)

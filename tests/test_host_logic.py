@@ -280,6 +280,45 @@ def test_bench_reference_arm_contract():
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_bench_dump_outputs_reference_arm(tmp_path, oracle_mod):
+    """`bench.py --dump-outputs DIR` writes the last timed step's results as float64 .npy files; on the reference arm they
+    equal the oracle's search of the same seeded queries."""
+    from pyarrowspace_b200 import synth
+    n, nq = 20000, 4
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "1",
+                        "--ref-queries", str(nq), "--items", str(n), "--dump-outputs", str(tmp_path / "out")],
+                       capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0, r.stderr[-2000:]
+    got = {p.stem: np.load(p) for p in (tmp_path / "out").iterdir()}
+    assert sorted(got) == ["query_rows", "search_idx", "search_scores"]
+    assert all(a.dtype == np.float64 for a in got.values())
+    cfg = synth.config("C4")
+    x = synth.make_items(n, cfg["f"], cfg["seed"], cfg["scale"])
+    q, _ = synth.make_queries(x, nq, cfg["seed"], cfg["scale"])
+    s, g = oracle_mod.build(cfg["graph_params"], x)
+    oidx, osc, _ = s.search_batch(q, g, cfg["tau"])
+    np.testing.assert_array_equal(got["query_rows"], np.arange(nq))
+    np.testing.assert_array_equal(got["search_idx"], oidx)
+    np.testing.assert_array_equal(got["search_scores"], osc)
+
+
+def test_bench_dump_outputs_sample_large_results(tmp_path, monkeypatch):
+    """Results above the dump budget are written as a fixed, seeded, sorted sample of the queries, within the budget."""
+    import bench
+    monkeypatch.setattr(bench, "DUMP_BYTES", 4096 + 100 * (8 + 16 * 10))
+    idx = np.arange(1000 * 10, dtype=np.int64).reshape(1000, 10)
+    sc = idx / 7.0
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), idx, sc)
+    rows = np.load(tmp_path / "a" / "query_rows.npy")
+    assert len(rows) == 100 and np.all(np.diff(rows) > 0)
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "search_idx.npy"), idx[rows.astype(np.int64)])
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "search_scores.npy"), sc[rows.astype(np.int64)])
+    for name in ("query_rows", "search_idx", "search_scores"):
+        np.testing.assert_array_equal(np.load(tmp_path / "a" / (name + ".npy")), np.load(tmp_path / "b" / (name + ".npy")))
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES
+
+
 def test_peer_exchange_buffer_size():
     """asp_peer_exchange_bytes (pure host arithmetic, no GPU): 4 KB of flags + two parities of `world` slots of
     cap x topk (int64 index, f64 score) pairs; unsupported shapes give 0."""
