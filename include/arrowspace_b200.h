@@ -79,7 +79,7 @@ typedef struct {
     int32_t laplacian;     /* ASP_LAPLACIAN_* : D - W | I - D^-1/2 W D^-1/2 | I - D^-1 W   (D = row sums of W)   */
     int32_t k_counts_self; /* 1: a node is its own first neighbour, so k keeps k - 1 others                      */
     int32_t topk_prunes;   /* 1: the neighbour cap is min(k, topk) (graph_params.topk also prunes the graph)     */
-    int32_t distance;      /* ASP_DISTANCE_*  : 1 - max(0,cos) | sqrt(|a|^2+|b|^2-2<a,b>) | its square (feature graph only) */
+    int32_t distance;      /* ASP_DISTANCE_*  : 1 - max(0,cos) | sqrt(|a|^2+|b|^2-2<a,b>) | its square (feature and item graph) */
 } asp_switches;
 
 typedef struct asp_ctx   asp_ctx;    /* device, streams, scratch */
@@ -250,12 +250,15 @@ int asp_peer_merge(asp_ctx *ctx, int world, int rank, const uint64_t *peer_bases
 /* ---- item graph (nodes = items; the graph-build workload of configs C4/C5) ------------------ */
 
 /* K1 (item orientation) + K2 for the shard's rows against `all_items` (n_total x f, host or
- * device; NULL = the shard itself, single GPU): eps / k-NN graph on rectified-cosine distance,
+ * device; NULL = the shard itself, single GPU): eps / k-NN graph on the distance of sw->distance (rectified cosine by
+ * default; l2 / l2sq: the oracle's Gram form (<a,a> + <b,b>) - 2<a,b> from left-to-right sums, clamped at 0),
  * weights, symmetrised Laplacian CSR over n_total nodes.  Single GPU; candidates on the tensor cores (tcgen05) for
- * n >= 8192 and k <= 30, FP64 DMMA otherwise; same exact stage 2 and answers. */
+ * n >= 8192, k <= 30 and <= 6144 features; below that FP64 DMMA (cosine) or the exact scan of every row (l2 / l2sq);
+ * same exact stage 2 and answers.  l2 / l2sq: k > 30, more than 6144 features at n >= 8192, or norms above 1e18 on the
+ * tensor-core route fail with ASP_ERR_UNSUPPORTED. */
 int asp_item_graph(asp_space *s, const asp_graph_params *gp, const asp_switches *sw, asp_graph **out_graph);
 
-/* Multi-GPU item graph (BASELINE.json configs C4/C5: "items sharded over 8 GPUs, NCCL halo exchange"): every rank
+/* Multi-GPU item graph (BASELINE.json configs C4/C5: "items sharded over 8 GPUs, NCCL halo exchange"; any distance): every rank
  * holds ALL items (the halo rows arrive by all-gather) in a world-1 space and resolves the eps / k-NN lists of ITS rows
  * [row_begin, row_end) on the tensor cores; the lists are all-gathered and the Laplacian is assembled from them.
  *   asp_item_knn_rows: out_idx / out_dist [rows][*out_kk] (only the first out_cnt[r] entries of a row are valid,

@@ -348,6 +348,7 @@ void asp_free_space(asp_space *s)
     if (s->items && s->owns_items) cudaFreeAsync(s->items, st);
     if (s->norms) cudaFreeAsync(s->norms, st);
     if (s->inv_norms) cudaFreeAsync(s->inv_norms, st);
+    if (s->nsq) cudaFreeAsync(s->nsq, st);
     if (s->lambdas) cudaFreeAsync(s->lambdas, st);
     delete s;
 }
@@ -1081,12 +1082,10 @@ int asp_item_graph(asp_space *s, const asp_graph_params *gp, const asp_switches 
     asp_switches sw;
     if (sw_in) sw = *sw_in; else asp_default_switches(&sw);
     ASP_CHECK(check_switches(&sw));
-    if (sw.distance != ASP_DISTANCE_COSINE)
-        ASP_FAIL(ASP_ERR_UNSUPPORTED, "the item graph (tensor-core candidates) supports the rectified-cosine distance only");
     asp_knn_lists lists;
     asp_graph_params gpe = *gp;
     gpe.k = asp_neighbour_cap(gp, &sw, s->n_total);               // k convention switches (k_counts_self, topk_prunes)
-    ASP_CHECK(asp_item_knn(s, &gpe, &lists));
+    ASP_CHECK(asp_item_knn(s, &gpe, sw.distance, &lists));
     asp_graph *g = new asp_graph();
     g->ctx = ctx;
     g->gp = *gp;
@@ -1111,12 +1110,10 @@ int asp_item_knn_rows(asp_space *s, const asp_graph_params *gp, const asp_switch
     asp_switches sw;
     if (sw_in) sw = *sw_in; else asp_default_switches(&sw);
     ASP_CHECK(check_switches(&sw));
-    if (sw.distance != ASP_DISTANCE_COSINE)
-        ASP_FAIL(ASP_ERR_UNSUPPORTED, "the item graph (tensor-core candidates) supports the rectified-cosine distance only");
     asp_knn_lists lists;
     asp_graph_params gpe = *gp;
     gpe.k = asp_neighbour_cap(gp, &sw, s->n_total);
-    int rc = asp_item_knn_rows_impl(s, &gpe, row_begin, row_end, &lists);
+    int rc = asp_item_knn_rows_impl(s, &gpe, sw.distance, row_begin, row_end, &lists);
     if (rc == ASP_OK) {
         const size_t rows = (size_t)lists.m;
         *out_kk = lists.kk;

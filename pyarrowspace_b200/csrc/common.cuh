@@ -61,6 +61,7 @@ struct asp_space {
     bool owns_items = true;              // false: adopted from the caller (asp_space_adopt)
     double *norms = nullptr;             // device, n_local: sqrt(sum x^2), left-to-right
     double *inv_norms = nullptr;         // device, n_local: 1/norm (0 for zero rows)
+    double *nsq = nullptr;               // device, n_local: sum x^2, left-to-right (Euclidean item graph; allocated on first use)
     double *lambdas = nullptr;           // device, n_local
     bool have_lambdas = false;
     CUtensorMap tmap_gram;               // (4, n_local, fp/4), box (4, 32 rows, 32 quads): Gram kernel
@@ -164,9 +165,11 @@ struct asp_tc_batch {                     // device buffers of one batch of quer
     int32_t *emit_ix = nullptr, *emit_cnt = nullptr; // local item indices; [nq][nsub] counts (> capb: overflow)
     uint32_t *theta_glob = nullptr;
 };
+enum { ASP_TC_ORDER_IDENTITY = 0, ASP_TC_ORDER_LAMBDA = 1, ASP_TC_ORDER_NORM = 2 };   // item order of the operand cache
 int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                   const double *qnorm_dev, double tau, int64_t topk, double score_floor, int force_terms, int capb_override,
-                  float *dump_dev, asp_tc_batch *b);
+                  float *dump_dev, asp_tc_batch *b, bool l2 = false);
+int asp_device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out);   // max(0, max v), synchronises
 void asp_tc_batch_free(asp_ctx *ctx, asp_tc_batch *b);
 bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, double tau);
 int asp_search_tc_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
@@ -181,5 +184,7 @@ int asp_make_f16_tmap(CUtensorMap *out, const void *base, int64_t rows, int32_t 
 int asp_make_f16_tmap_narrow(CUtensorMap *out, const void *base, int64_t rows, int32_t kp, int box_rows, int nw);
 
 // knn.cu
-int asp_item_knn(asp_space *s, const asp_graph_params *gp, asp_knn_lists *lists);
-int asp_item_knn_rows_impl(asp_space *s, const asp_graph_params *gp, int64_t row_begin, int64_t row_end, asp_knn_lists *lists);
+// distance: ASP_DISTANCE_COSINE | L2 | L2SQ
+int asp_item_knn(asp_space *s, const asp_graph_params *gp, int distance, asp_knn_lists *lists);
+int asp_item_knn_rows_impl(asp_space *s, const asp_graph_params *gp, int distance, int64_t row_begin, int64_t row_end,
+                           asp_knn_lists *lists);

@@ -1,5 +1,5 @@
-// knn.cu -- K1, item orientation (nodes = items): eps-radius / k-NN lists on rectified-cosine distance
-// for every item against every item (GRAPH_VARIABLES.md:7-8; SURVEY.md Appendix A2 `nodes = items`,
+// knn.cu -- K1, item orientation (nodes = items): eps-radius / k-NN lists on the rectified-cosine distance (default) or the
+// Euclidean one (l2 / l2sq, the Gram form of oracle.c node_distance) for every item against every item (GRAPH_VARIABLES.md:7-8; SURVEY.md Appendix A2 `nodes = items`,
 // A3-A4; the graph-build workload of BASELINE.json configs C4/C5).
 //
 // Bound: FP64 tensor pipe, 2*M^2*D FLOP (every ordered pair, as the reference's per-row scan does).
@@ -20,9 +20,10 @@ namespace {
 using namespace asp_gemm;
 using asp::Cand;
 
-// left-to-right norms (the oracle's: sqrt of the sequential sum of squares), one thread per row
+// left-to-right norms (the oracle's: sqrt of the sequential sum of squares), one thread per row; nsq (if given) keeps the
+// sum of squares itself, which the Euclidean distance uses (it is not norm^2: the two differ in the last bits)
 __global__ void row_norms_kernel(const double *__restrict__ items, int64_t n, int f, int pitch, double *__restrict__ norms,
-                                 double *__restrict__ inv_norms)
+                                 double *__restrict__ inv_norms, double *__restrict__ nsq)
 {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         const double *row = items + i * pitch;
@@ -30,7 +31,13 @@ __global__ void row_norms_kernel(const double *__restrict__ items, int64_t n, in
         const double nr = sqrt(n2);
         norms[i] = nr;
         inv_norms[i] = nr > 0.0 ? 1.0 / nr : 0.0;
+        if (nsq) nsq[i] = n2;
     }
+}
+
+__global__ void iota_rows_kernel(int32_t *__restrict__ p, int64_t n)
+{
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) p[i] = (int32_t)i;
 }
 
 // the oracle's distance expression (oracle.c select_neighbours)
@@ -39,6 +46,16 @@ __device__ __forceinline__ double exact_dist(double dot, double na, double nb)
     double c = 0.0;
     if (na != 0.0 && nb != 0.0) c = __ddiv_rn(dot, __dmul_rn(na, nb));
     return __dsub_rn(1.0, c > 0.0 ? c : 0.0);
+}
+
+// oracle.c node_distance for every distance kind: cosine as above; l2 / l2sq from the left-to-right sums
+// saa = <a,a>, sbb = <b,b>, dot = <a,b>:  d2 = (saa + sbb) - 2 dot clamped at 0, and its square root for l2
+__device__ __forceinline__ double exact_node_dist(int distance, double dot, double na, double nb, double saa, double sbb)
+{
+    if (distance == ASP_DISTANCE_COSINE) return exact_dist(dot, na, nb);
+    double d2 = __dsub_rn(__dadd_rn(saa, sbb), __dmul_rn(2.0, dot));
+    if (!(d2 > 0.0)) d2 = 0.0;
+    return distance == ASP_DISTANCE_L2 ? __dsqrt_rn(d2) : d2;
 }
 
 constexpr int KR_WARPS = 4;
@@ -108,18 +125,24 @@ knn_rescore_kernel(const double *__restrict__ items, int64_t n, int f, int pitch
     if (lane == 0) out_cnt[i] = keep;
 }
 
-// slow path (exact_scan.cuh): value = -d(i, j), admissible = another item within eps; the k best by (d asc, index asc)
+// slow path (exact_scan.cuh): value = -d(i, j), admissible = another item within eps; the k best by (d asc, index asc).
+// Also the whole route of a Euclidean graph below the tensor-core size (every row takes it).
 struct KnnScanPolicy {
     const double *items; int pitch; const double *norms; double eps; const int32_t *slow_list;
     int kk; int32_t *out_idx; double *out_dist; int32_t *out_cnt;
-    struct Row { double ni; int64_t self; };
-    struct Item { double nj; };
+    const double *nsq; int distance;                                            // nsq: l2 / l2sq only
+    struct Row { double ni, si; int64_t self; };
+    struct Item { double nj, sj; };
     __device__ const double *query(int slot) const { return items + (int64_t)slow_list[slot] * pitch; }
-    __device__ Row row(int slot) const { const int64_t i = slow_list[slot]; return Row{norms[i], i}; }
-    __device__ Item item(int64_t j) const { return Item{norms[j]}; }
+    __device__ Row row(int slot) const
+    {
+        const int64_t i = slow_list[slot];
+        return Row{norms[i], distance != ASP_DISTANCE_COSINE ? nsq[i] : 0.0, i};
+    }
+    __device__ Item item(int64_t j) const { return Item{norms[j], distance != ASP_DISTANCE_COSINE ? nsq[j] : 0.0}; }
     __device__ double value(const Row &r, const Item &it, double dot, int64_t j, bool &valid) const
     {
-        const double d = exact_dist(dot, r.ni, it.nj);
+        const double d = exact_node_dist(distance, dot, r.ni, it.nj, r.si, it.sj);
         valid = (j != r.self) && (d <= eps);                                    // GRAPH_VARIABLES.md:7
         return -d;
     }
@@ -134,14 +157,17 @@ struct KnnScanPolicy {
 };
 
 // ---------------------------------------------------------------- tcgen05 candidate pass (search_tc.cu) + exact stage 2
-// Stage 1 is the search's tensor-core kernel with tau = 1 (score = cosine), the items themselves as queries, lists of
-// k + 1 (the item finds itself) and an emission floor at 1 - eps; this kernel is the item-graph stage 2, one warp per row:
-//   cut    (k+1)-th largest approximate cosine over all emitted candidates, minus 2 x the row's band
-//   (A)    survivors re-scored in f64 with a coalesced warp-cooperative dot product, best 32 kept
+// Stage 1 is the search's tensor-core kernel with tau = 1 (score = cosine; DIST = l2 / l2sq: the score kind -d^2~), the
+// items themselves as queries, lists of k + 1 (the item finds itself) and an emission floor at 1 - eps (-eps^2 | -eps); this
+// kernel is the item-graph stage 2, one warp per row:
+//   cut    (k+1)-th largest approximate score over all emitted candidates, minus 2 x the row's band
+//   (A)    survivors re-scored in f64 with a coalesced warp-cooperative dot product (cosine, or -(|a|^2 + |b|^2 - 2 dot)
+//          from the left-to-right sums of squares), best 32 kept
 //   (B)    the candidates within 2 eps_fast of the (k+1)-th best get the oracle's distance (left-to-right dot,
-//          d = 1 - max(0, dot/(|a||b|))); self dropped, d <= eps decided on those values, k smallest by (d, index).
-// A band that may extend beyond the 32 kept, a k-th neighbour whose cosine is not clearly positive (rectification ties
-// at d = 1 are ordered by index over ALL such items) or a full emission buffer send the row to the exact scan.
+//          exact_node_dist); self dropped, d <= eps decided on those values, k smallest by (d, index).
+// A band that may extend beyond the 32 kept, a k-th neighbour whose cosine is not clearly positive (cosine only:
+// rectification ties at d = 1 are ordered by index over ALL such items) or a full emission buffer send the row to the
+// exact scan.  For l2 / l2sq eps_fast scales with |a|^2 + max |b|^2 (the dot's rounding is relative to the norms).
 constexpr int KT_QUEUE = 96;
 
 // Sums of FOUR per-lane values over the warp with 12 shuffles instead of 40: the halves of the warp first trade two values,
@@ -159,9 +185,10 @@ __device__ __forceinline__ double warp_sum4_transposed(const double (&d)[4], int
     return f;
 }
 
+template <int DIST>
 __global__ void __launch_bounds__(KR_WARPS * 32)
 knn_tc_rescore_kernel(const double *__restrict__ items, int64_t n, int f, int pitch, const double *__restrict__ norms,
-                      double eps, int kk, int64_t b0, int64_t nq, int nsub, int capb, const float *__restrict__ delta_q,
+                      const double *__restrict__ nsq, double nsq_max, double eps, int kk, int64_t b0, int64_t nq, int nsub, int capb, const float *__restrict__ delta_q,
                       double eps_fast, const float *__restrict__ emit_sc, const int32_t *__restrict__ emit_ix,
                       const int32_t *__restrict__ emit_cnt, const int32_t *__restrict__ qperm, const int32_t *__restrict__ row_map,
                       int64_t out_row0,
@@ -205,6 +232,8 @@ knn_tc_rescore_kernel(const double *__restrict__ items, int64_t n, int f, int pi
         cutoff = kth - 2.0f * delta_q[qi];
     }
     const double ni = norms[i];
+    const double si = (DIST != ASP_DISTANCE_COSINE) ? nsq[i] : 0.0;
+    const double eps_row = (DIST != ASP_DISTANCE_COSINE) ? eps_fast * (si + nsq_max) : eps_fast;
     __syncwarp();
 
     Cand best[2];
@@ -240,8 +269,12 @@ knn_tc_rescore_kernel(const double *__restrict__ items, int64_t n, int f, int pi
             }
         }
         if (my_item >= 0) {
-            const double den = ni * norms[my_item];
-            mine.s = (den != 0.0) ? my_dot / den : 0.0;                          // fast cosine
+            if (DIST != ASP_DISTANCE_COSINE) {
+                mine.s = -((si + nsq[my_item]) - 2.0 * my_dot);                  // fast -d^2
+            } else {
+                const double den = ni * norms[my_item];
+                mine.s = (den != 0.0) ? my_dot / den : 0.0;                      // fast cosine
+            }
             mine.i = my_item;
         }
         best[1] = mine;
@@ -271,9 +304,9 @@ knn_tc_rescore_kernel(const double *__restrict__ items, int64_t n, int f, int pi
 
     const double kth = __shfl_sync(0xffffffffu, best[0].s, kq - 1);              // -inf when fewer than k+1 survivors
     const bool valid = best[0].i != 0x7fffffff;
-    const bool in_band = valid && (best[0].s >= kth - 2.0 * eps_fast);
+    const bool in_band = valid && (best[0].s >= kth - 2.0 * eps_row);
     const unsigned band = __ballot_sync(0xffffffffu, in_band);
-    if (band == 0xffffffffu || (kth != -INFINITY && kth <= 4.0 * eps_fast)) {
+    if (band == 0xffffffffu || (DIST == ASP_DISTANCE_COSINE && kth != -INFINITY && kth <= 4.0 * eps_fast)) {
         if (lane == 0) slow_list[atomicAdd(slow_count, 1)] = (int32_t)i;
         return;
     }
@@ -281,7 +314,8 @@ knn_tc_rescore_kernel(const double *__restrict__ items, int64_t n, int f, int pi
     fin[0] = asp::cand_empty();
     if (in_band && best[0].i != (int32_t)i) {
         const int64_t j = best[0].i;
-        const double d = exact_dist(seq_dot_row(xs, items + j * pitch, f), ni, norms[j]);
+        const double d = exact_node_dist(DIST, seq_dot_row(xs, items + j * pitch, f), ni, norms[j], si,
+                                         (DIST != ASP_DISTANCE_COSINE) ? nsq[j] : 0.0);
         if (d <= eps) { fin[0].s = -d; fin[0].i = (int32_t)j; }                   // GRAPH_VARIABLES.md:7
     }
     asp::warp_sort_best_first<1>(fin, lane);                                     // (-d desc, index asc) == (d asc, index asc)
@@ -295,10 +329,11 @@ knn_tc_rescore_kernel(const double *__restrict__ items, int64_t n, int f, int pi
 }  // namespace
 
 // exact scan of the rows listed in slow_list (device)
-static int knn_slow_rows(asp_space *s, const asp_graph_params *gp, int64_t kk, const int32_t *slow_list, int nslow, asp_knn_lists *lists)
+static int knn_slow_rows(asp_space *s, const asp_graph_params *gp, int distance, int64_t kk, const int32_t *slow_list, int nslow,
+                         asp_knn_lists *lists)
 {
     asp_ctx *ctx = s->ctx;
-    const KnnScanPolicy pol{s->items, s->fp, s->norms, gp->eps, slow_list, (int)kk, lists->idx, lists->dist, lists->cnt};
+    const KnnScanPolicy pol{s->items, s->fp, s->norms, gp->eps, slow_list, (int)kk, lists->idx, lists->dist, lists->cnt, s->nsq, distance};
     const int rc = asp_xs::run(ctx->stream, ctx->num_sms, pol, nslow, s->items, s->n_local, s->f, s->fp, kk,
                                [&](int k) { ctx->launches += k; });
     if (rc == 3) ASP_FAIL(ASP_ERR_NOMEM, "out of device memory in the exact scan of the item graph");
@@ -329,7 +364,7 @@ static int item_knn_fp64(asp_space *s, const asp_graph_params *gp, asp_knn_lists
     if (kk == 0) return ASP_OK;
 
     row_norms_kernel<<<(unsigned)(asp_ceil_div(n, 128) < 65535 ? asp_ceil_div(n, 128) : 65535), 128, 0, st>>>(
-        s->items, n, f, s->fp, s->norms, s->inv_norms);
+        s->items, n, f, s->fp, s->norms, s->inv_norms, nullptr);
     ASP_CUDA(cudaGetLastError());
     ASP_LAUNCHED(ctx);
 
@@ -397,7 +432,7 @@ static int item_knn_fp64(asp_space *s, const asp_graph_params *gp, asp_knn_lists
     ctx->stats["knn_stage1_ms"] = ms;
     ctx->stats["knn_slow_rows"] = nslow;
     ctx->stats["knn_stage1_is_tc"] = 0.0;
-    if (nslow > 0) ASP_CHECK(knn_slow_rows(s, gp, kk, slow_list, nslow, lists));
+    if (nslow > 0) ASP_CHECK(knn_slow_rows(s, gp, ASP_DISTANCE_COSINE, kk, slow_list, nslow, lists));
     ASP_CUDA(cudaFreeAsync(cand_score, st));
     ASP_CUDA(cudaFreeAsync(cand_idx, st));
     ASP_CUDA(cudaFreeAsync(slow_list, st));
@@ -423,7 +458,8 @@ __global__ void gather_rows_kernel(const double *__restrict__ items, int pitch, 
 //   pass 2  the rows whose emission lists or bands overflowed (dense neighbourhoods: the 1-term band of ~1e-4 in cosine
 //           can hold hundreds of neighbours) are gathered and redone with the two-term split (band ~1e-6)
 //   pass 3  what is still unresolved (long runs of exact ties around the k-th neighbour) takes the exact scan
-static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int64_t kk, int64_t row_begin, int64_t row_end, asp_knn_lists *lists)
+static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int distance, int64_t kk, int64_t row_begin, int64_t row_end,
+                       asp_knn_lists *lists)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
@@ -431,7 +467,20 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int64_t kk, int
     const int f = s->f;
     const double u = 1.1102230246251565e-16;
     const double eps_fast = (4.0 * f + 64.0) * u * 2.0;
-    const double floor = (gp->eps < 2.0) ? 1.0 - gp->eps - eps_fast : -INFINITY;   // cos < 1 - eps can never be a neighbour
+    const bool l2 = distance != ASP_DISTANCE_COSINE;
+    double floor = (gp->eps < 2.0) ? 1.0 - gp->eps - eps_fast : -INFINITY;         // cos < 1 - eps can never be a neighbour
+    double nsq_max = 0.0;
+    if (l2) {
+        // score -d^2: d <= eps needs -d^2 >= -eps^2 (l2) | -eps (l2sq); the stage-1 score is f32, so the norms must square
+        // well inside its range
+        double norm_max = 0.0;
+        ASP_CHECK(asp_device_max(ctx, s->norms, n, &norm_max));
+        ASP_CHECK(asp_device_max(ctx, s->nsq, n, &nsq_max));
+        if (!(norm_max <= 1e18))
+            ASP_FAIL(ASP_ERR_UNSUPPORTED, "Euclidean item graph: norms up to %g exceed the f32 range of the tensor-core pass (limit 1e18)", norm_max);
+        const double e2 = (distance == ASP_DISTANCE_L2) ? gp->eps * gp->eps : gp->eps;
+        floor = (gp->eps >= 0.0 && e2 < 1e300) ? -(e2 * (1.0 + 1e-12)) : -INFINITY;
+    }
     const int64_t rows = row_end - row_begin;
     int32_t *slow1 = nullptr, *slow2 = nullptr, *counts = nullptr;                  // counts[0], counts[1]
     unsigned long long *counter = nullptr;
@@ -442,7 +491,9 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int64_t kk, int
     ASP_CUDA(cudaMemsetAsync(counts, 0, sizeof(int32_t) * 2, st));
     ASP_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
     const size_t rsmem = (size_t)KR_WARPS * s->fp * 8 + KR_WARPS * KT_QUEUE * 4;
-    ASP_CUDA(cudaFuncSetAttribute(knn_tc_rescore_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rsmem));
+    auto rescore = (distance == ASP_DISTANCE_L2) ? knn_tc_rescore_kernel<ASP_DISTANCE_L2>
+                 : (distance == ASP_DISTANCE_L2SQ) ? knn_tc_rescore_kernel<ASP_DISTANCE_L2SQ> : knn_tc_rescore_kernel<ASP_DISTANCE_COSINE>;
+    ASP_CUDA(cudaFuncSetAttribute(rescore, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rsmem));
     int64_t batch = 65536;
     if (const char *e = getenv("ASP_KNN_BATCH")) { const long v = atol(e); if (v >= 128) batch = v; }
     double stage1_ms = 0.0, stage2_ms = 0.0;
@@ -452,10 +503,10 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int64_t kk, int
     auto run_batch = [&](const double *q, const double *qn, int64_t nq, int64_t b0, const int32_t *row_map, int terms,
                          int32_t *slow_list, int32_t *slow_count, int *terms_used) -> int {
         asp_tc_batch b;
-        int r = asp_tc_stage1(s, q, nq, s->fp, nullptr, qn, 1.0, kk + 1, floor, terms, 2048, nullptr, &b);
+        int r = asp_tc_stage1(s, q, nq, s->fp, nullptr, qn, 1.0, kk + 1, floor, terms, 2048, nullptr, &b, l2);
         if (r == ASP_OK) {
-            knn_tc_rescore_kernel<<<(unsigned)asp_ceil_div(nq, KR_WARPS), KR_WARPS * 32, rsmem, st>>>(
-                s->items, n, f, s->fp, s->norms, gp->eps, (int)kk, b0, nq, b.nsub, b.capb, b.delta_q, eps_fast, b.emit_sc, b.emit_ix,
+            rescore<<<(unsigned)asp_ceil_div(nq, KR_WARPS), KR_WARPS * 32, rsmem, st>>>(
+                s->items, n, f, s->fp, s->norms, s->nsq, nsq_max, gp->eps, (int)kk, b0, nq, b.nsub, b.capb, b.delta_q, eps_fast, b.emit_sc, b.emit_ix,
                 b.emit_cnt, b.qperm, row_map, row_begin, lists->idx, lists->dist, lists->cnt, slow_list, slow_count, counter);
             if (cudaGetLastError() != cudaSuccess) { asp_set_error("knn_tc_rescore_kernel launch failed"); r = ASP_ERR_CUDA; }
             ASP_LAUNCHED(ctx);
@@ -540,14 +591,47 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int64_t kk, int
         } else if (n_final > 0) {                                     // the exact kernels index the lists by GLOBAL row
             asp_knn_lists shifted = *lists;
             shifted.idx = lists->idx - row_begin * kk; shifted.dist = lists->dist - row_begin * kk; shifted.cnt = lists->cnt - row_begin;
-            rc = knn_slow_rows(s, gp, kk, final_list, n_final, &shifted);
+            rc = knn_slow_rows(s, gp, distance, kk, final_list, n_final, &shifted);
         }
     }
     cudaFreeAsync(slow1, st); cudaFreeAsync(slow2, st); cudaFreeAsync(counts, st); cudaFreeAsync(counter, st);
     return rc;
 }
 
-int asp_item_knn(asp_space *s, const asp_graph_params *gp, asp_knn_lists *lists)
+// norms (and, for the Euclidean distances, the sums of squares) of every item
+static int knn_row_norms(asp_space *s, int distance)
+{
+    asp_ctx *ctx = s->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = s->n_local;
+    if (distance != ASP_DISTANCE_COSINE && !s->nsq) ASP_CUDA(cudaMallocAsync(&s->nsq, sizeof(double) * (size_t)(n > 0 ? n : 1), st));
+    row_norms_kernel<<<(unsigned)(asp_ceil_div(n, 128) < 65535 ? asp_ceil_div(n, 128) : 65535), 128, 0, st>>>(
+        s->items, n, s->f, s->fp, s->norms, s->inv_norms, distance != ASP_DISTANCE_COSINE ? s->nsq : nullptr);
+    ASP_CUDA(cudaGetLastError());
+    ASP_LAUNCHED(ctx);
+    return ASP_OK;
+}
+
+// Euclidean graph below the tensor-core size (or ASP_KNN_STAGE1=fp64): every row takes the batched exact scan
+static int item_knn_scan_all(asp_space *s, const asp_graph_params *gp, int distance, int64_t kk, asp_knn_lists *lists)
+{
+    asp_ctx *ctx = s->ctx;
+    cudaStream_t st = ctx->stream;
+    const int64_t n = s->n_local;
+    int32_t *rows = nullptr;
+    ASP_CUDA(cudaMallocAsync(&rows, sizeof(int32_t) * (size_t)(n > 0 ? n : 1), st));
+    iota_rows_kernel<<<ctx->num_sms * 4, 256, 0, st>>>(rows, n);
+    ASP_CUDA(cudaGetLastError());
+    ASP_LAUNCHED(ctx);
+    const int rc = knn_slow_rows(s, gp, distance, kk, rows, (int)n, lists);
+    cudaFreeAsync(rows, st);
+    ctx->stats["knn_stage1_ms"] = 0.0;
+    ctx->stats["knn_slow_rows"] = (double)n;
+    ctx->stats["knn_stage1_is_tc"] = 0.0;
+    return rc;
+}
+
+int asp_item_knn(asp_space *s, const asp_graph_params *gp, int distance, asp_knn_lists *lists)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
@@ -558,24 +642,29 @@ int asp_item_knn(asp_space *s, const asp_graph_params *gp, asp_knn_lists *lists)
     const char *force = getenv("ASP_KNN_STAGE1");
     const bool want_fp64 = force && force[0] == 'f', want_tc = force && force[0] == 't';
     const bool tc_ok = kk >= 1 && kk + 1 <= 31 && n < 2147483647LL && s->fp <= 6144;
-    if (!tc_ok || want_fp64 || (!want_tc && n < 8192)) return item_knn_fp64(s, gp, lists);
+    const bool l2 = distance != ASP_DISTANCE_COSINE;
+    const bool small = want_fp64 || (!want_tc && n < 8192);
+    if (!l2 && (!tc_ok || small)) return item_knn_fp64(s, gp, lists);
+    if (l2 && kk > 30) ASP_FAIL(ASP_ERR_UNSUPPORTED, "the Euclidean item graph supports k <= 30 (got %lld)", (long long)gp->k);
+    if (l2 && !small && !tc_ok)
+        ASP_FAIL(ASP_ERR_UNSUPPORTED, "the Euclidean item graph on the tensor cores supports at most 6144 features (got %d)", s->f);
 
     lists->m = n;
-    lists->kk = (int32_t)kk;
+    lists->kk = (int32_t)(kk > 0 ? kk : 1);
     ASP_CUDA(cudaMallocAsync(&lists->idx, sizeof(int32_t) * (size_t)n * lists->kk, st));
     ASP_CUDA(cudaMallocAsync(&lists->dist, sizeof(double) * (size_t)n * lists->kk, st));
     ASP_CUDA(cudaMallocAsync(&lists->cnt, sizeof(int32_t) * (size_t)n, st));
     ASP_CUDA(cudaMemsetAsync(lists->cnt, 0, sizeof(int32_t) * (size_t)n, st));
-    row_norms_kernel<<<(unsigned)(asp_ceil_div(n, 128) < 65535 ? asp_ceil_div(n, 128) : 65535), 128, 0, st>>>(
-        s->items, n, s->f, s->fp, s->norms, s->inv_norms);
-    ASP_CUDA(cudaGetLastError());
-    ASP_LAUNCHED(ctx);
-    return item_knn_tc(s, gp, kk, 0, n, lists);
+    ASP_CHECK(knn_row_norms(s, distance));
+    if (kk == 0) return ASP_OK;
+    if (small) return item_knn_scan_all(s, gp, distance, kk, lists);
+    return item_knn_tc(s, gp, distance, kk, 0, n, lists);
 }
 
 // neighbour lists of rows [row_begin, row_end) only (multi-GPU item graph: every rank holds all items and resolves
 // its own rows); tensor-core pass only
-int asp_item_knn_rows_impl(asp_space *s, const asp_graph_params *gp, int64_t row_begin, int64_t row_end, asp_knn_lists *lists)
+int asp_item_knn_rows_impl(asp_space *s, const asp_graph_params *gp, int distance, int64_t row_begin, int64_t row_end,
+                           asp_knn_lists *lists)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
@@ -591,10 +680,7 @@ int asp_item_knn_rows_impl(asp_space *s, const asp_graph_params *gp, int64_t row
     ASP_CUDA(cudaMallocAsync(&lists->dist, sizeof(double) * (size_t)(rows > 0 ? rows : 1) * lists->kk, st));
     ASP_CUDA(cudaMallocAsync(&lists->cnt, sizeof(int32_t) * (size_t)(rows > 0 ? rows : 1), st));
     ASP_CUDA(cudaMemsetAsync(lists->cnt, 0, sizeof(int32_t) * (size_t)(rows > 0 ? rows : 1), st));
-    row_norms_kernel<<<(unsigned)(asp_ceil_div(n, 128) < 65535 ? asp_ceil_div(n, 128) : 65535), 128, 0, st>>>(
-        s->items, n, s->f, s->fp, s->norms, s->inv_norms);
-    ASP_CUDA(cudaGetLastError());
-    ASP_LAUNCHED(ctx);
+    ASP_CHECK(knn_row_norms(s, distance));
     if (rows == 0) return ASP_OK;
-    return item_knn_tc(s, gp, kk, row_begin, row_end, lists);
+    return item_knn_tc(s, gp, distance, kk, row_begin, row_end, lists);
 }

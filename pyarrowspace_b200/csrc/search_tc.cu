@@ -40,6 +40,7 @@
 #include "common.cuh"
 #include "ptx.cuh"
 #include "warp_sort.cuh"
+#include "l2_bound.cuh"
 
 #include <cuda_fp16.h>
 #include <math.h>
@@ -287,6 +288,17 @@ __global__ void row_delta_kernel(const double *__restrict__ rho_q, int64_t nq, d
         delta[i] = __double2float_ru(tau_abs * (rho_q[i] * c_main + c_fixed) + score_slack);
 }
 
+// per-row band of the approximate l2 score -d^2~ (f32, visiting order): 2 A B_max |cos~ - cos| plus the f32 roundings of
+// the score expression and of the two norms (< 1e-6 (A + B)^2, x2 margin), A = the row's norm
+__global__ void row_delta_l2_kernel(const double *__restrict__ rho_q, const double *__restrict__ qnorm, const int32_t *__restrict__ qperm,
+                                    int64_t nq, double c_main, double c_fixed, double b_max, float *__restrict__ delta)
+{
+    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < nq; i += (int64_t)gridDim.x * blockDim.x) {
+        const double a = qnorm[qperm ? qperm[i] : i];
+        delta[i] = __double2float_ru(2.0 * a * b_max * (rho_q[i] * c_main + c_fixed) + 2e-6 * (a + b_max) * (a + b_max) + 1e-36);
+    }
+}
+
 // f32 copies of the lambdas in visiting order + per-tile [min, max] rounded outwards
 __global__ void __launch_bounds__(TN) tile_lambda_kernel(const double *__restrict__ lam, const int32_t *__restrict__ perm,
                                                          int64_t n, float *__restrict__ lam32, float *__restrict__ tile_lo,
@@ -408,13 +420,17 @@ struct TcParams {
 // pipeline depth.  Barriers: TMA loads of both CTAs complete on the LEADER's full barrier; tcgen05.commit multicasts the
 // "stage free" / "accumulator ready" arrivals to both CTAs; the peer's epilogue warps arrive remotely on the leader's
 // "accumulator drained" barrier.
-template <bool DUMP, int VARIANT, bool ARES, bool PAIR, int LISTN>   // LISTN (>= topk): the four column-quarter threads of a query row keep LISTN / 4 scores each; VARIANT (profiling only): 0 normal, 2 epilogue does no work, 3 no MMA issued, 4 epilogue loads TMEM only
+// L2 (score kind of the Euclidean item graph): the score is -d^2~ (l2_bound.cuh) instead of tau cos~ + beta prox; lam_x /
+// lam_q / tile_lo / tile_hi then hold the f32 norms (items in norm order) and the per-(row, tile) raw-accumulator threshold
+// comes from asp_l2::threshold instead of the proximity bound.  The MMAs and the pipeline are the same.
+template <bool DUMP, int VARIANT, bool ARES, bool PAIR, int LISTN, bool L2 = false>   // LISTN (>= topk): the four column-quarter threads of a query row keep LISTN / 4 scores each; VARIANT (profiling only): 0 normal, 2 epilogue does no work, 3 no MMA issued, 4 epilogue loads TMEM only
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_constant__ CUtensorMap map_q_lo,
                const __grid_constant__ CUtensorMap map_x_hi, const __grid_constant__ CUtensorMap map_x_lo,
                const __grid_constant__ CUtensorMap map_q_nw, const __grid_constant__ CUtensorMap map_x_nw, const TcParams p)
 {
     static_assert(!PAIR || ARES, "the CTA-pair kernel keeps the query operand resident");
+    static_assert(!L2 || (!DUMP && VARIANT == 0), "the l2 score kind has no dump or profiling variants");
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     // SWIZZLE_128B tiles must start on 1024-byte boundaries
     constexpr int NST = PAIR ? 6 : ARES ? 3 : TC_STAGES;                         // ring depth
@@ -614,11 +630,17 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
                     const float sh = o2f(so);
                     if (sh > theta_k) { theta_k = sh; theta_emit = fmaxf(theta_k - delta2, floor_row); }
                 }
+                if constexpr (L2) {
+                    // lq = the row's norm, [tl, th] = the tile's norm interval: the smallest cos~ a column needs to reach
+                    // theta_emit (l2_bound.cuh).  It is not refreshed when theta_emit rises inside the tile (stale = lower = safe).
+                    theta_acc = asp_l2::threshold(lq, tl, th, theta_emit);
+                } else {
                 // s <= tau*cos + beta*prox_ub, prox_ub = 1/(1 + distance of lambda_q to the tile's lambda interval);
                 // the 2.5e-7 / 1.000001 keep the bound safe against the f32 roundings of lambda_q and the interval
                 const float gap = fmaxf(0.f, fmaxf(lq - th, tl - lq) - 2.5e-7f);
                 beta_ub = p.beta * __fdividef(1.0f, 1.0f + gap) * 1.000001f;
                 theta_acc = ((theta_emit - beta_ub) * inv_tau - 1e-6f) * ACC_SCALE;
+                }
             }
             asp::mbar_wait_suspend(&tmem_full[acc], (uint32_t)((t >> 1) & 1), 8000);
             asp::tc_fence_after();
@@ -658,7 +680,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
                             if (a < theta_acc) continue;                         // the threshold rose inside this loop
                             const int col = col0 + j;
                             const int64_t n = item0 + col;
-                            const float sc = fmaf(p.beta, __fdividef(1.0f, 1.0f + fabsf(lq - c_lam[col])), p.tau * (a * (1.0f / ACC_SCALE)));
+                            const float sc = L2 ? asp_l2::score(lq, c_lam[col], a)
+                                                : fmaf(p.beta, __fdividef(1.0f, 1.0f + fabsf(lq - c_lam[col])), p.tau * (a * (1.0f / ACC_SCALE)));
                             if (sc >= theta_emit && n < p.n_local) {
                                 const int pos = atomicAdd(&s_cnt[row], 1);
                                 if (pos < p.capb) { p.emit_sc[ebase + pos] = sc; p.emit_ix[ebase + pos] = p.perm[n]; }
@@ -676,7 +699,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
                                     if (kth > theta_k) {
                                         theta_k = kth;
                                         theta_emit = fmaxf(theta_k - delta2, floor_row);
-                                        theta_acc = ((theta_emit - beta_ub) * inv_tau - 1e-6f) * ACC_SCALE;
+                                        if constexpr (!L2) theta_acc = ((theta_emit - beta_ub) * inv_tau - 1e-6f) * ACC_SCALE;
                                         const uint32_t ko = f2o(kth);
                                         atomicMax(&s_theta[row], ko);
                                         atomicMax(&p.theta_glob[gq], ko);
@@ -977,9 +1000,11 @@ tc_rescore_kernel(const double *__restrict__ q, int qpitch, int64_t nq, const do
 // ------------------------------------------------------------------ host side
 struct asp_tc_cache {               // per-space fp16 operands in lambda order, built on the first tensor-core search
     __half *hi = nullptr, *lo = nullptr;      // lo (remainder of the residual columns) only once a 3-term search needs it
-    float *lam32 = nullptr, *tile_lo = nullptr, *tile_hi = nullptr;
+    float *lam32 = nullptr, *tile_lo = nullptr, *tile_hi = nullptr;   // the order key (lambda | norm) per item and tile
     int32_t *perm = nullptr;
-    bool lambda_ordered = false;    // items in lambda order (needs the lambdas); else identity order (item graph before the lambdas)
+    int order = ASP_TC_ORDER_IDENTITY;   // visiting order of the items: lambda (search), norm (l2 item graph) or identity
+                                         // (cosine item graph before the lambdas exist)
+    double norm_max = 0.0;          // ASP_TC_ORDER_NORM: the shard's largest norm
     double *mdir = nullptr;         // [f] unit mean direction of the shard's unit vectors
     double rho_max = 1.0;           // largest residual norm |x^ - (m.x^) m| of the shard
     int kp = 0;                     // operand row: f residual columns + 3 rank-1 columns, padded to a multiple of 64
@@ -988,7 +1013,7 @@ struct asp_tc_cache {               // per-space fp16 operands in lambda order, 
     int nw = 0;
 };
 
-static int device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out)
+int asp_device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out)
 {
     cudaStream_t st = ctx->stream;
     double *d_mm = nullptr;
@@ -1036,13 +1061,18 @@ __global__ void iota_kernel(int32_t *__restrict__ p, int64_t n)
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) p[i] = (int32_t)i;
 }
 
-static int ensure_tc_cache(const asp_space *s, asp_tc_cache **out)
+// by_norm: the l2 item graph's cache (items in norm order).  Otherwise the cosine one: lambda order once the space has
+// lambdas, identity order before.  A cache of the other kind is rebuilt, so a search sees the same operands whatever graph
+// was built before it.
+static int ensure_tc_cache(const asp_space *s, bool by_norm, asp_tc_cache **out)
 {
     asp_space *ms = const_cast<asp_space *>(s);
     if (ms->tc_cache) {
         asp_tc_cache *have = static_cast<asp_tc_cache *>(ms->tc_cache);
-        if (have->lambda_ordered || !s->have_lambdas) { *out = have; return ASP_OK; }
-        asp_free_tc_cache(ms);                                          // built before the lambdas existed: rebuild in lambda order
+        const bool ok = by_norm ? have->order == ASP_TC_ORDER_NORM
+                                : have->order == ASP_TC_ORDER_LAMBDA || (have->order == ASP_TC_ORDER_IDENTITY && !s->have_lambdas);
+        if (ok) { *out = have; return ASP_OK; }
+        asp_free_tc_cache(ms);                                          // other order (or built before the lambdas existed): rebuild
     }
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
@@ -1060,9 +1090,9 @@ static int ensure_tc_cache(const asp_space *s, asp_tc_cache **out)
     ASP_CUDA(cudaMallocAsync(&c->mdir, sizeof(double) * s->f, st));
     ASP_CUDA(cudaMallocAsync(&partials, sizeof(double) * (size_t)MD_BLOCKS * s->f, st));
     ASP_CUDA(cudaMallocAsync(&rho, sizeof(double) * n, st));
-    // visiting order: bucket sort of the shard by lambda (identity while the space has no lambdas: item graph)
-    c->lambda_ordered = s->have_lambdas;
-    if (s->have_lambdas) ASP_CHECK(bucket_order(ctx, s->lambdas, n, c->perm));
+    // visiting order: bucket sort of the shard by lambda (identity while the space has no lambdas: item graph), or by norm
+    c->order = by_norm ? ASP_TC_ORDER_NORM : s->have_lambdas ? ASP_TC_ORDER_LAMBDA : ASP_TC_ORDER_IDENTITY;
+    if (c->order != ASP_TC_ORDER_IDENTITY) ASP_CHECK(bucket_order(ctx, by_norm ? s->norms : s->lambdas, n, c->perm));
     else { iota_kernel<<<ctx->num_sms * 4, 256, 0, st>>>(c->perm, n); ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx); }
     // mean direction, projection, fp16 operands
     colsum_unit_kernel<<<MD_BLOCKS, 256, 0, st>>>(s->items, n, s->f, s->fp, s->inv_norms, partials);
@@ -1072,10 +1102,11 @@ static int ensure_tc_cache(const asp_space *s, asp_tc_cache **out)
     project_split_kernel<<<ctx->num_sms * 8, 256, 0, st>>>(s->items, n, s->f, s->fp, c->kp, s->inv_norms, c->perm, c->mdir, 0,
                                                           c->hi, nullptr, rho);
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
-    ASP_CHECK(device_max(ctx, rho, n, &c->rho_max));
-    if (s->have_lambdas) {
-        tile_lambda_kernel<<<(unsigned)ntile, TN, 0, st>>>(s->lambdas, c->perm, n, c->lam32, c->tile_lo, c->tile_hi);
+    ASP_CHECK(asp_device_max(ctx, rho, n, &c->rho_max));
+    if (c->order != ASP_TC_ORDER_IDENTITY) {
+        tile_lambda_kernel<<<(unsigned)ntile, TN, 0, st>>>(by_norm ? s->norms : s->lambdas, c->perm, n, c->lam32, c->tile_lo, c->tile_hi);
         ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
+        if (by_norm) ASP_CHECK(asp_device_max(ctx, s->norms, n, &c->norm_max));
     } else {
         ASP_CUDA(cudaMemsetAsync(c->lam32, 0, sizeof(float) * n, st));
         ASP_CUDA(cudaMemsetAsync(c->tile_lo, 0, sizeof(float) * ntile, st));
@@ -1136,17 +1167,20 @@ bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, doubl
 // ------------------------------------------------------------------ stage 1 for one batch of query vectors
 // Prepares the query operands (lambda_q order when lambdas are given, projection, per-row bands), runs tc_gemm_kernel and
 // leaves the emission lists in `b` for the caller's stage 2 (search: tc_rescore_kernel; item graph: knn.cu).
-// lambda_q_dev == nullptr: no lambda term (kNN): identity query order.  dump_dev != nullptr: approximate cosines
-// [nq][n_local] f32 (tests), no emission.
+// lambda_q_dev == nullptr: no lambda term (cosine kNN): identity query order.  dump_dev != nullptr: approximate cosines
+// [nq][n_local] f32 (tests), no emission.  l2 (Euclidean item graph): score -d^2~, items in norm order, queries visited in
+// the order of their norms (qnorm_dev is the key; lambda_q_dev and tau are unused).
 int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                   const double *qnorm_dev, double tau, int64_t topk, double score_floor, int force_terms, int capb_override,
-                  float *dump_dev, asp_tc_batch *b)
+                  float *dump_dev, asp_tc_batch *b, bool l2)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
     const double t_stage1 = asp_now_us();
     asp_tc_cache *c = nullptr;
-    ASP_CHECK(ensure_tc_cache(s, &c));
+    if (l2 && dump_dev) ASP_FAIL(ASP_ERR_ARG, "asp_tc_stage1: no dump of the l2 score");
+    ASP_CHECK(ensure_tc_cache(s, l2, &c));
+    if (l2) { lambda_q_dev = qnorm_dev; tau = 1.0; }
     const int kp = c->kp;
     *b = asp_tc_batch();
     b->nq = nq;
@@ -1161,7 +1195,7 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     ASP_CUDA(cudaMallocAsync(&b->rho_q, sizeof(double) * nq, st));
     ASP_CUDA(cudaMallocAsync(&b->delta_q, sizeof(float) * nq, st));
     ASP_CHECK(asp_launch_reciprocal(ctx, qnorm_dev, nq, b->inv_nq));
-    const bool by_lambda = !dump_dev && lambda_q_dev && c->lambda_ordered;
+    const bool by_lambda = !dump_dev && lambda_q_dev && c->order != ASP_TC_ORDER_IDENTITY;   // (l2: by the query norms)
     if (by_lambda) {
         // queries visited in lambda_q order: coherent blocks -> one visiting order per block
         ASP_CUDA(cudaMallocAsync(&b->qperm, sizeof(int32_t) * nq, st));
@@ -1177,7 +1211,7 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     // error band of one approximate cosine, |cos~ - cos| <= rho_q rho_x c_main + c_fixed (margin x2 on a worst-case
     // model: fp16 roundings of both residuals, round-toward-zero f32 accumulation, truncated rank-1 split)
     double rho_q_max = 1.0;
-    ASP_CHECK(device_max(ctx, b->rho_q, nq, &rho_q_max));
+    ASP_CHECK(asp_device_max(ctx, b->rho_q, nq, &rho_q_max));
     ctx->stats["search_host_prep_us"] = asp_now_us() - t_stage1;
     const double steps = (double)((s->f + 15) / 16);
     const double c_main1 = 2.0 * c->rho_max * (ldexp(1.0, -10) * (1.0 + ldexp(1.0, -11)) + steps * ldexp(1.0, -23));
@@ -1188,7 +1222,8 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     if (force_terms == 1 || force_terms == 3) nterms = force_terms;
     if (nterms == 3) ASP_CHECK(ensure_tc_lo(s, c));
     const double c_main = (nterms == 1) ? c_main1 : c_main3;
-    row_delta_kernel<<<64, 256, 0, st>>>(b->rho_q, nq, c_main, c_fixed, fabs(tau), (fabs(tau) + fabs(1.0 - tau)) * 2e-6, b->delta_q);
+    if (l2) row_delta_l2_kernel<<<64, 256, 0, st>>>(b->rho_q, qnorm_dev, b->qperm, nq, c_main, c_fixed, c->norm_max, b->delta_q);
+    else row_delta_kernel<<<64, 256, 0, st>>>(b->rho_q, nq, c_main, c_fixed, fabs(tau), (fabs(tau) + fabs(1.0 - tau)) * 2e-6, b->delta_q);
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
     b->nterms = nterms;
     b->delta_cos_max = rho_q_max * c_main + c_fixed;
@@ -1274,11 +1309,12 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     // (python -m pyarrowspace_b200.build --profiling); the shipped library has no knob that changes a result.
 #ifdef ASP_PROFILING
     const char *var = getenv("ASP_TC_VARIANT");
-    const int v = (var && !dump_dev && !wide) ? atoi(var) : 0;
+    int v = (var && !dump_dev && !wide) ? atoi(var) : 0;
 #else
-    const int v = 0;
+    int v = 0;
 #endif
     if (pair) p.nw_hi = 0;                                        // (the CTA-pair kernel keeps full boxes)
+    if (l2) v = 0;
     void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, TcParams) =
         dump_dev ? (ares ? tc_gemm_kernel<true, 0, true, false, 16> : tc_gemm_kernel<true, 0, false, false, 16>)
         : wide ? (pair ? tc_gemm_kernel<false, 0, true, true, 32> : ares ? tc_gemm_kernel<false, 0, true, false, 32> : tc_gemm_kernel<false, 0, false, false, 32>)
@@ -1292,6 +1328,11 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
         : pair ? tc_gemm_kernel<false, 0, true, true, 16>
 #endif
         : (ares ? tc_gemm_kernel<false, 0, true, false, 16> : tc_gemm_kernel<false, 0, false, false, 16>);
+    if (l2)
+        k = wide ? (pair ? tc_gemm_kernel<false, 0, true, true, 32, true> : ares ? tc_gemm_kernel<false, 0, true, false, 32, true>
+                         : tc_gemm_kernel<false, 0, false, false, 32, true>)
+                 : (pair ? tc_gemm_kernel<false, 0, true, true, 16, true> : ares ? tc_gemm_kernel<false, 0, true, false, 16, true>
+                         : tc_gemm_kernel<false, 0, false, false, 16, true>);
     ASP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ASP_CUDA(cudaEventRecord(ctx->ev0, st));
     if (pair) {

@@ -24,6 +24,7 @@ from pyarrowspace_b200.api import ArrowSpaceBuilder  # noqa: E402
 def main():
     m = int(sys.argv[1]) if len(sys.argv) > 1 else 100000
     eps_list = [float(e) for e in (sys.argv[2] if len(sys.argv) > 2 else "5,10,15").split(",")]
+    distance = sys.argv[3] if len(sys.argv) > 3 else "cosine"         # third argument: cosine | l2 | l2sq (recorded in the JSON)
     n, f = 8_800_000, 768
     dev = torch.device("cuda", 0)
     centres = torch.randn(c5_sweep.NCL, f, generator=torch.Generator(device=dev).manual_seed(c5_sweep.SEED), device=dev, dtype=torch.float64)
@@ -33,16 +34,16 @@ def main():
         oracle.set_num_threads(len(os.sched_getaffinity(0)))
     except AttributeError:
         pass
-    out = {"slice_rows": m, "f": f, "of_n": n, "runs": [], "oracle_threads": oracle.num_threads()}
+    out = {"slice_rows": m, "f": f, "distance": distance, "of_n": n, "runs": [], "oracle_threads": oracle.num_threads()}
     ok = True
     for eps in eps_list:
         gp = {"eps": eps, "k": 25, "topk": 10, "p": 2.0, "sigma": None}
         torch.cuda.synchronize(); t0 = time.time()
-        aspace, gl = ArrowSpaceBuilder.build_item_graph(gp, x)
+        aspace, gl = ArrowSpaceBuilder.build_item_graph(gp, x, distance=distance)
         torch.cuda.synchronize(); t_gpu = time.time() - t0
         st = {k: api.stat(k) for k in ("knn_stage1_ms", "knn_stage2_ms", "knn_slow_rows", "knn_rows_two_term", "knn_rescored_per_row")}
         t0 = time.time()
-        s, g = oracle.build(gp, xh, nodes="items")
+        s, g = oracle.build(gp, xh, nodes="items", distance=distance)
         t_cpu = time.time() - t0
         ip, ix, dt = gl.csr()
         oip, oix, odt = g.csr()
