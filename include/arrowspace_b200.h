@@ -220,9 +220,30 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
  *      min(topk, n) by (score desc, index asc).
  * pool >= n: no shortlist, i.e. asp_search_batch without the assertion; otherwise pool <= 1024 (what the exact scan keeps).
  * Output layout as asp_search_batch.  Needs every item on this GPU (world-1 space or a replicated item shard);
- * ASP_ERR_UNSUPPORTED on a row shard. */
+ * ASP_ERR_UNSUPPORTED on a row shard: a row-sharded space answers with asp_search_hybrid_shard + asp_hybrid_merge. */
 int asp_search_hybrid_batch(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                             int64_t pool, int64_t *out_idx, double *out_score, double *out_lambda_q);
+
+/* The shortlist length m of H2 for n_total items: pool (<= 0: min(2 * topk, 31)), raised to topk, cut to n_total.
+ * m == n_total (with n_total > 0) means no shortlist: the whole set. */
+int64_t asp_hybrid_pool(int64_t n_total, int64_t topk, int64_t pool);
+
+/* Hybrid search on a row-sharded space, bit for bit the one-GPU asp_search_hybrid_batch over all n_total items.  Every
+ * rank holding an item shard calls asp_search_hybrid_shard with the same queries; [exchange]: all-gather the outputs;
+ * then merge.  With m = asp_hybrid_pool(n_total, topk, pool):
+ *   m < n_total   out_idx / out_cos / out_score are [nq][m]: the shard's own top-m by (cosine desc, index asc) -- the
+ *                 search at tau = 1 with topk = m -- as GLOBAL indices, their cosines and their H3 scores at tau; lists
+ *                 padded with -1 / NaN.  m <= 1024, else ASP_ERR_UNSUPPORTED.  asp_hybrid_merge of the parts' lists
+ *                 ([parts][nq][m], shards in any order) takes the global top-m by cosine, which lies in the union of the
+ *                 shards' top-m lists, and returns its best topk by (score desc, index asc).
+ *   m == n_total  no shortlist: out_idx / out_score are [nq][topk], the shard's best topk by the lambda-aware score at tau
+ *                 (asp_search_batch without the assertion); out_cos is not used; merge with asp_topk_merge.
+ * H1 as asp_search_hybrid_batch (no lambda_q != 0 assertion; every rank gets the same lambda_q).  Host or device
+ * pointers.  asp_hybrid_merge output layout as asp_search_batch. */
+int asp_search_hybrid_shard(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
+                            int64_t pool, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q);
+int asp_hybrid_merge(asp_ctx *ctx, const int64_t *idx, const double *cos, const double *score, int parts, int64_t nq,
+                     int64_t m, int64_t topk, int64_t *out_idx, double *out_score);
 
 /* Test hook of the tcgen05 candidate pass: the approximate cosines (unit-scaled operands, bf16 two-term split,
  * f32 accumulation in TMEM) of nq queries against every item of the shard, out[nq][n_local] f32 (host or device). */

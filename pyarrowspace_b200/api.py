@@ -473,14 +473,15 @@ class ArrowSpace:
 
     def search_hybrid_batch(self, queries, gl, tau, *, pool=None, want_lambda=False):
         """Extension: search_hybrid for a host batch; (idx int64[Q, topk], score f64[Q, topk]) padded with -1 / NaN
-        (+ lambda_q with want_lambda).  Every item must be on this GPU: one GPU, or the replicated layout of
-        build_sharded (item_shards = 1), where each rank answers on its own."""
+        (+ lambda_q with want_lambda).  On one GPU, and on the replicated layout of build_sharded (item_shards = 1), each
+        rank answers on its own.  On an item-sharded space (item_shards > 1) it is called collectively, like `search`, and
+        every rank returns the whole batch: the one-GPU answer, bit for bit (distributed.sharded_search_hybrid)."""
         if not isinstance(gl, GraphLaplacian):
             raise TypeError("argument 'gl': 'GraphLaplacian' object expected")
         n_local, f, _, n_total = self._dims()
-        if n_local != n_total:
-            raise NotImplementedError("search_hybrid needs every item on this GPU (this rank holds %d of %d rows); build with "
-                                      "item_shards=1" % (n_local, n_total))
+        if n_local != n_total and self._grid is None:
+            raise NotImplementedError("search_hybrid on a row shard needs the search grid of build_sharded (this rank holds "
+                                      "%d of %d rows)" % (n_local, n_total))
         q = np.ascontiguousarray(queries, dtype=np.float64)
         if q.ndim != 2 or q.shape[1] != f:
             raise ValueError("query length %d must match nfeatures %d" % (q.shape[-1], f))
@@ -488,10 +489,16 @@ class ArrowSpace:
             raise ValueError("pool must be a positive integer (the shortlist length; default min(2 * topk, 31))")
         topk = gl.graph_params["topk"]
         nq = q.shape[0]
-        idx = np.empty((nq, topk), dtype=np.int64)
-        score = np.empty((nq, topk), dtype=np.float64)
-        lam = np.empty(nq, dtype=np.float64)
         try:
+            if n_local != n_total:
+                from .distributed import CudaEngine, sharded_search_hybrid
+                engine = CudaEngine(_lib.load().asp_ctx_device(self._ctx))
+                idx, score, lam = sharded_search_hybrid(engine, self._h, gl._h, q, float(tau), int(pool or 0), topk, n_total,
+                                                        self._grid)
+                return (idx, score, lam) if want_lambda else (idx, score)
+            idx = np.empty((nq, topk), dtype=np.int64)
+            score = np.empty((nq, topk), dtype=np.float64)
+            lam = np.empty(nq, dtype=np.float64)
             _lib.check(_lib.load().asp_search_hybrid_batch(self._h, gl._h, q.ctypes.data, nq, float(tau), int(pool or 0),
                                                            idx.ctypes.data, score.ctypes.data, lam.ctypes.data))
         except LibraryError as e:

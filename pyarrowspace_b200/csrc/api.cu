@@ -94,7 +94,7 @@ int upload_pitched(cudaStream_t st, const double *src, int64_t n, int32_t f, int
     return ASP_OK;
 }
 
-// stream-ordered scratch of asp_search_hybrid_batch, released on every exit path
+// stream-ordered scratch of the hybrid search entry points, released on every exit path
 struct HybridScratch {
     cudaStream_t st;
     std::vector<void *> ptrs;
@@ -897,6 +897,13 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
     return rc;
 }
 
+int64_t asp_hybrid_pool(int64_t n_total, int64_t topk, int64_t pool)
+{
+    int64_t m = pool > 0 ? pool : std::min<int64_t>(2 * topk, 31);   // H2: shortlist length (31: the longest tensor-core list)
+    if (m < topk) m = topk;
+    return std::min(m, n_total);
+}
+
 // Hybrid search (src/lib.rs:182-219 -> the crate's search_lambda_aware_hybrid; restatement H1-H3 of the header): the cosine
 // shortlist is the search above at tau = 1 with topk = pool (same candidate passes, same exact stage 2), the re-ranking is
 // hybrid.cuh.  No lambda_q != 0 assertion (search_hybrid has none).
@@ -919,9 +926,7 @@ int asp_search_hybrid_batch(const asp_space *s, const asp_graph *g, const double
     cudaStream_t st = ctx->stream;
     const int64_t topk = g->gp.topk;                              // src/lib.rs:214
     const int32_t f = s->f, fp = s->fp;
-    int64_t m = pool > 0 ? pool : std::min<int64_t>(2 * topk, 31);   // H2: shortlist length (31: the longest tensor-core list)
-    if (m < topk) m = topk;
-    if (m > s->n_local) m = s->n_local;
+    const int64_t m = asp_hybrid_pool(s->n_local, topk, pool);
     const bool whole_set = (m >= s->n_local);                     // the shortlist is every item: H3 is the plain search
     if (!whole_set && m > 1024)
         ASP_FAIL(ASP_ERR_UNSUPPORTED, "hybrid search: a shortlist of %lld items is beyond the 1024 the exact scan keeps per query "
@@ -969,6 +974,131 @@ int asp_search_hybrid_batch(const asp_space *s, const asp_graph *g, const double
     }
     ASP_CUDA(cudaStreamSynchronize(st));
     ctx->stats["hybrid_pool"] = (double)m;
+    return ASP_OK;
+}
+
+// One row shard's half of the hybrid search of a row-sharded space: H1, then the shard's own top-m by cosine (the search at
+// tau = 1 with topk = m, m from the WHOLE item count) and the H3 score of every slot beside its cosine.  asp_hybrid_merge
+// takes the global top-m by cosine from the shards' lists and re-ranks it, which is what the one-GPU shortlist holds.
+int asp_search_hybrid_shard(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                            int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q)
+{
+    if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score)))
+        ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_shard: NULL argument");
+    if (!s->have_lambdas) ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_shard: item lambdas have not been computed");
+    if (g->nnodes != s->f)
+        ASP_FAIL(ASP_ERR_ARG, "graph has %lld nodes but items have %d features", (long long)g->nnodes, s->f);
+    if (nq == 0) return ASP_OK;
+    if (s->f > 6144) ASP_FAIL(ASP_ERR_UNSUPPORTED, "search supports at most 6144 features (got %d)", s->f);
+    asp_ctx *ctx = s->ctx;
+    ASP_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t topk = g->gp.topk;
+    const int32_t f = s->f, fp = s->fp;
+    const int64_t m = asp_hybrid_pool(s->n_total, topk, pool);
+    const bool whole_set = (m >= s->n_total);
+    if (!whole_set && m > 1024)
+        ASP_FAIL(ASP_ERR_UNSUPPORTED, "hybrid search: a shortlist of %lld items is beyond the 1024 the exact scan keeps per query "
+                 "(use pool >= nitems = %lld for no shortlist at all)", (long long)m, (long long)s->n_total);
+    if (!whole_set && topk > 0 && !out_cos) ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_shard: NULL out_cos");
+    const int64_t width = whole_set ? topk : m;                   // entries per query of the outputs
+    const int64_t kl = std::min(m, s->n_local);                   // a shard smaller than m answers all its rows
+
+    HybridScratch scratch{st, {}};
+    double *dq = nullptr, *dlam = nullptr, *dnorm = nullptr, *dcos = nullptr, *dscore = nullptr;
+    int64_t *didx = nullptr;
+    int *flags = nullptr;
+    ASP_CHECK(scratch.get(&dq, (size_t)nq * fp));
+    ASP_CHECK(scratch.get(&dlam, (size_t)nq));
+    ASP_CHECK(scratch.get(&dnorm, (size_t)nq));
+    ASP_CHECK(scratch.get(&flags, 2));
+    if (topk > 0) {
+        ASP_CHECK(scratch.get(&didx, (size_t)nq * width));
+        ASP_CHECK(scratch.get(&dscore, (size_t)nq * width));
+        if (!whole_set) ASP_CHECK(scratch.get(&dcos, (size_t)nq * width));
+    }
+    ASP_CHECK(upload_pitched(st, queries, nq, f, fp, dq));
+    if (whole_set) {
+        // no shortlist: the shard's best topk by the lambda-aware score, merged like asp_search_batch's lists
+        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false));
+    } else {
+        int64_t *sidx = didx;
+        double *scos = dcos;
+        if (topk > 0 && kl < m) {
+            ASP_CHECK(scratch.get(&sidx, (size_t)nq * kl));
+            ASP_CHECK(scratch.get(&scos, (size_t)nq * kl));
+        }
+        // the score at tau = 1 is the cosine
+        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? kl : 0, dlam, dnorm, flags, sidx, scos, false));
+        if (topk > 0) {
+            if (kl < m) {                                         // lists padded to m with -1 / NaN
+                ASP_CUDA(cudaMemsetAsync(didx, 0xff, sizeof(int64_t) * (size_t)nq * m, st));
+                ASP_CUDA(cudaMemsetAsync(dcos, 0xff, sizeof(double) * (size_t)nq * m, st));
+                if (kl > 0) {
+                    ASP_CUDA(cudaMemcpy2DAsync(didx, sizeof(int64_t) * m, sidx, sizeof(int64_t) * kl, sizeof(int64_t) * kl,
+                                               (size_t)nq, cudaMemcpyDeviceToDevice, st));
+                    ASP_CUDA(cudaMemcpy2DAsync(dcos, sizeof(double) * m, scos, sizeof(double) * kl, sizeof(double) * kl,
+                                               (size_t)nq, cudaMemcpyDeviceToDevice, st));
+                }
+            }
+            const int64_t total = nq * m;
+            const unsigned blocks = (unsigned)std::min<int64_t>(asp_ceil_div(total, 256), (int64_t)ctx->num_sms * 8);
+            asp_hybrid::hybrid_rescore_kernel<<<blocks, 256, 0, st>>>(total, m, dq, fp, s->items, fp, f, s->row0, s->norms,
+                                                                       s->lambdas, dnorm, dlam, tau, didx, dscore);
+            ASP_CUDA(cudaGetLastError());
+            ASP_LAUNCHED(ctx);
+        }
+    }
+    if (out_lambda_q) ASP_CHECK(asp_copy_out(ctx, out_lambda_q, dlam, sizeof(double) * nq));
+    if (topk > 0) {
+        ASP_CHECK(asp_copy_out(ctx, out_idx, didx, sizeof(int64_t) * (size_t)nq * width));
+        ASP_CHECK(asp_copy_out(ctx, out_score, dscore, sizeof(double) * (size_t)nq * width));
+        if (!whole_set) ASP_CHECK(asp_copy_out(ctx, out_cos, dcos, sizeof(double) * (size_t)nq * width));
+    }
+    ASP_CUDA(cudaStreamSynchronize(st));
+    ctx->stats["hybrid_pool"] = (double)m;
+    return ASP_OK;
+}
+
+int asp_hybrid_merge(asp_ctx *ctx, const int64_t *idx, const double *cosv, const double *score, int parts, int64_t nq, int64_t m,
+                     int64_t topk, int64_t *out_idx, double *out_score)
+{
+    if (!ctx || parts <= 0 || nq < 0 || m < 0 || topk < 0 ||
+        (nq > 0 && topk > 0 && (!idx || !cosv || !score || !out_idx || !out_score)))
+        ASP_FAIL(ASP_ERR_ARG, "asp_hybrid_merge: bad argument");
+    if (nq == 0 || topk == 0) return ASP_OK;
+    ASP_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const size_t n_in = (size_t)parts * nq * m, n_pool = (size_t)nq * m, n_out = (size_t)nq * topk;
+    HybridScratch scratch{st, {}};
+    int64_t *d_idx = nullptr, *d_pidx = nullptr, *d_oidx = nullptr;
+    double *d_cos = nullptr, *d_sc = nullptr, *d_psc = nullptr, *d_osc = nullptr;
+    ASP_CHECK(scratch.get(&d_idx, n_in));
+    ASP_CHECK(scratch.get(&d_cos, n_in));
+    ASP_CHECK(scratch.get(&d_sc, n_in));
+    ASP_CHECK(scratch.get(&d_pidx, n_pool));
+    ASP_CHECK(scratch.get(&d_psc, n_pool));
+    ASP_CHECK(scratch.get(&d_oidx, n_out));
+    ASP_CHECK(scratch.get(&d_osc, n_out));
+    if (n_in) {
+        ASP_CUDA(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * n_in, cudaMemcpyDefault, st));
+        ASP_CUDA(cudaMemcpyAsync(d_cos, cosv, sizeof(double) * n_in, cudaMemcpyDefault, st));
+        ASP_CUDA(cudaMemcpyAsync(d_sc, score, sizeof(double) * n_in, cudaMemcpyDefault, st));
+    }
+    ASP_CUDA(cudaMemsetAsync(d_pidx, 0xff, sizeof(int64_t) * n_pool, st));   // -1: a position no slot reaches stays padding
+    if (n_in) {
+        const unsigned blocks = (unsigned)std::min<int64_t>(asp_ceil_div((int64_t)n_in, 256), (int64_t)ctx->num_sms * 8);
+        asp_hybrid::hybrid_merge_kernel<<<blocks, 256, 0, st>>>((int64_t)n_in, parts, nq, m, d_idx, d_cos, d_sc, d_pidx, d_psc);
+        ASP_CUDA(cudaGetLastError());
+        ASP_LAUNCHED(ctx);
+    }
+    const unsigned blocks_s = (unsigned)std::min<int64_t>(asp_ceil_div(nq, 128), (int64_t)ctx->num_sms * 8);
+    asp_hybrid::hybrid_select_kernel<<<blocks_s, 128, 0, st>>>(nq, m, topk, d_pidx, d_psc, d_oidx, d_osc);
+    ASP_CUDA(cudaGetLastError());
+    ASP_LAUNCHED(ctx);
+    ASP_CHECK(asp_copy_out(ctx, out_idx, d_oidx, sizeof(int64_t) * n_out));
+    ASP_CHECK(asp_copy_out(ctx, out_score, d_osc, sizeof(double) * n_out));
+    ASP_CUDA(cudaStreamSynchronize(st));
     return ASP_OK;
 }
 

@@ -9,8 +9,15 @@
 //   hybrid_select_kernel   one thread per query: the best topk slots by (score desc, index asc).
 // Both are a few hundred steps per query next to a scan of every item for the shortlist; no shared memory, no barriers.
 //
-// The per-thread bodies are plain functions so that tests/test_hybrid_host.py can compile this header with g++
-// (-ffp-contract=off) and walk the thread grid on the CPU against the oracle.
+// Row-sharded spaces (asp_search_hybrid_shard + asp_hybrid_merge) add one step between the two:
+//   hybrid_merge_kernel    one thread per (shard, query, slot) of the per-shard shortlists: the slot's rank among the union
+//                          of the query's shortlists by (cosine desc, index asc), by binary search in each other list.  The
+//                          global top-m by cosine is contained in that union (each shard holds its own top-m), so a slot of
+//                          rank < m is one of the m entries the one-GPU shortlist holds, and it is written to position
+//                          `rank` of that shortlist.  hybrid_select_kernel then picks from it exactly as on one GPU.
+//
+// The per-thread bodies are plain functions so that tests/test_hybrid_host.py and tests/test_hybrid_sharded_cpu.py can
+// compile this header with g++ (-ffp-contract=off) and walk the thread grid on the CPU against the oracle.
 #pragma once
 
 #include <math.h>
@@ -101,7 +108,48 @@ ASP_HYB_FN void select_query(int64_t qi, int64_t pool, int64_t topk, int64_t *po
     }
 }
 
+// Slot t = (r * nq + qi) * m + p of `parts` per-shard shortlists ([parts][nq][m]: GLOBAL indices, their cosines and H3
+// scores, each list sorted by (cosine desc, index asc) and padded with -1).  A slot whose rank in the union of the query's
+// lists is below m goes to position `rank` of the query's merged shortlist pool_idx / pool_score ([nq][m], filled with -1
+// beforehand).  Ranks are distinct because the shards hold disjoint rows, so every position is written at most once.
+ASP_HYB_FN void merge_slot(int64_t t, int parts, int64_t nq, int64_t m, const int64_t *idx, const double *cosv,
+                           const double *score, int64_t *pool_idx, double *pool_score)
+{
+    const int64_t id = idx[t];
+    if (id < 0) return;
+    const int64_t per = nq * m;
+    const int r = (int)(t / per);
+    const int64_t qi = (t - r * per) / m;
+    const double c = cosv[t];
+    int64_t rank = t - r * per - qi * m;                       // the entries before it in its own list
+    for (int o = 0; o < parts && rank < m; ++o) {
+        if (o == r) continue;
+        const int64_t *oi = idx + o * per + qi * m;
+        const double *oc = cosv + o * per + qi * m;
+        int64_t lo = 0, hi = m;                                // entries of list o before (c, id): a prefix of the list
+        while (lo < hi) {
+            const int64_t mid = (lo + hi) >> 1;
+            if (oi[mid] >= 0 && (oc[mid] > c || (oc[mid] == c && oi[mid] < id))) lo = mid + 1;
+            else hi = mid;
+        }
+        rank += lo;
+    }
+    if (rank < m) {
+        pool_idx[qi * m + rank] = id;
+        pool_score[qi * m + rank] = score[t];
+    }
+}
+
 #if defined(__CUDACC__)
+__global__ void __launch_bounds__(256)
+hybrid_merge_kernel(int64_t total, int parts, int64_t nq, int64_t m, const int64_t *__restrict__ idx,
+                    const double *__restrict__ cosv, const double *__restrict__ score, int64_t *__restrict__ pool_idx,
+                    double *__restrict__ pool_score)
+{
+    for (int64_t t = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; t < total; t += (int64_t)gridDim.x * blockDim.x)
+        merge_slot(t, parts, nq, m, idx, cosv, score, pool_idx, pool_score);
+}
+
 __global__ void __launch_bounds__(256)
 hybrid_rescore_kernel(int64_t total, int64_t pool, const double *__restrict__ q, int qpitch, const double *__restrict__ items,
                       int pitch, int f, int64_t row0, const double *__restrict__ norm_x, const double *__restrict__ lam_x,

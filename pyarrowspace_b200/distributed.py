@@ -16,6 +16,9 @@ The path shards by rows (SURVEY.md section 8(e)): rank r owns the rows of Gram s
              rank then answers 1/C of each query batch against item shard r.  Per-query work (lambda_q, operand
              projection, stage 2, merge) is divided by C instead of being replicated G times; R = 1 needs no cross-GPU
              merge at all.  R = G is the fully item-sharded layout (every rank scores every query).
+  hybrid search (R > 1; `sharded_search_hybrid`)
+          7. all-gather of the per-shard cosine shortlists (idx, cosine, score: 24 * Q * m bytes per rank) among the R ranks
+             of a query slot + merge kernel; the C slots all-gather their finished slices
 
 The summation tree of the Gram is fixed (segments -> slices), so every world size produces
 bit-identical graphs, lambdas and result lists.
@@ -216,6 +219,42 @@ class CudaEngine:
                                                C.byref(cgp), C.byref(sw), C.byref(hg)))
         return hg
 
+    # ---- hybrid search on row-sharded spaces
+    def hybrid_pool(self, n_total, topk, pool):
+        return self.lib.asp_hybrid_pool(int(n_total), int(topk), int(pool))
+
+    def hybrid_shard(self, space, graph, q, tau, pool, idx, cos, score, lam):
+        """asp_search_hybrid_shard of the host rows q into the device tensors idx / cos / score [rows, width] and lam [rows]
+        (cos is None when the shortlist is the whole set)."""
+        self.torch.cuda.current_stream(self.device).synchronize()      # the outputs were filled on torch's stream
+        _lib.check(self.lib.asp_search_hybrid_shard(space, graph, q.ctypes.data, q.shape[0], float(tau), int(pool),
+                                                    idx.data_ptr(), None if cos is None else cos.data_ptr(),
+                                                    score.data_ptr(), lam.data_ptr()))
+
+    def hybrid_merge(self, idx, cos, score, m, topk):
+        """[parts, nq, m] shortlists of the shards -> (idx, score) [nq, topk] device tensors (asp_hybrid_merge)."""
+        t = self.torch
+        parts, nq = idx.shape[0], idx.shape[1]
+        out_idx = t.empty((nq, topk), dtype=t.int64, device=self.device)
+        out_sc = t.empty((nq, topk), dtype=t.float64, device=self.device)
+        idx, cos, score = idx.contiguous(), cos.contiguous(), score.contiguous()
+        t.cuda.current_stream(self.device).synchronize()
+        _lib.check(self.lib.asp_hybrid_merge(self.ctx, idx.data_ptr(), cos.data_ptr(), score.data_ptr(), parts, nq, m, topk,
+                                             out_idx.data_ptr(), out_sc.data_ptr()))
+        return out_idx, out_sc
+
+    def topk_merge(self, idx, score):
+        """[parts, nq, topk] lists -> (idx, score) [nq, topk] device tensors (asp_topk_merge)."""
+        t = self.torch
+        parts, nq, topk = idx.shape
+        out_idx = t.empty((nq, topk), dtype=t.int64, device=self.device)
+        out_sc = t.empty((nq, topk), dtype=t.float64, device=self.device)
+        idx, score = idx.contiguous(), score.contiguous()
+        t.cuda.current_stream(self.device).synchronize()
+        _lib.check(self.lib.asp_topk_merge(self.ctx, idx.data_ptr(), score.data_ptr(), parts, nq, topk, out_idx.data_ptr(),
+                                           out_sc.data_ptr()))
+        return out_idx, out_sc
+
     def to_comm(self, arr):
         return self.torch.from_numpy(arr).to(self.device)
 
@@ -393,6 +432,64 @@ def regroup(engine, space, rows_dev, n_total, item_shards, group=None):
     new_space = engine.space_from_gathered(x, lam, nrm, n_total, r_, r)
     engine.free_space(space)
     return new_space, grid
+
+
+def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_total, grid):
+    """Hybrid search (step 7) on an item-sharded grid (grid["R"] > 1), bit for bit the one-GPU search_hybrid_batch over all
+    n_total items.  Called collectively with the same host batch `queries` [Q, F] on every rank.  Query slot c answers rows
+    [a, b) of the batch: each of its R ranks computes its item shard's shortlist (engine.hybrid_shard), the R lists are
+    all-gathered over the slot's merge group (R * m * 24 bytes per query) and merged on every one of them; the C slots then
+    all-gather their finished slices, as the grid search does.  Returns (idx, score, lambda_q) host arrays of the whole
+    batch on every rank.  A failure on any rank raises the same LibraryError (same code) on every rank."""
+    import torch
+    from ._lib import LibraryError
+    r_, c_ = grid["R"], grid["C"]
+    nq = queries.shape[0]
+    a, b, per = query_slice(nq, c_, grid["c"])
+    m = engine.hybrid_pool(n_total, topk, pool)
+    whole = m >= n_total                                     # no shortlist: the plain search's lists, merged as such
+    width = topk if whole else m
+    dev = engine.device
+    nan = float("nan")
+    idx = torch.full((per, width), -1, dtype=torch.int64, device=dev)
+    cos = None if whole else torch.full((per, width), nan, dtype=torch.float64, device=dev)
+    score = torch.full((per, width), nan, dtype=torch.float64, device=dev)
+    lam = torch.full((per + 1,), nan, dtype=torch.float64, device=dev)
+    lam[per] = 0.0                                           # the last element carries the status of this slot
+    err = None
+    if b > a:
+        try:
+            engine.hybrid_shard(space, graph, queries[a:b], tau, pool, idx[:b - a], None if whole else cos[:b - a],
+                                score[:b - a], lam[:b - a])
+        except LibraryError as e:
+            err = e
+    status = torch.tensor([float(err.code) if err is not None else 0.0], dtype=torch.float64, device=dev)
+    status = _all_gather_blocks(status, r_, grid["merge_group"]).reshape(-1)
+    g_idx = _all_gather_blocks(idx, r_, grid["merge_group"])
+    g_sc = _all_gather_blocks(score, r_, grid["merge_group"])
+    g_cos = None if whole else _all_gather_blocks(cos, r_, grid["merge_group"])
+    if hasattr(engine, "after_collective"):
+        engine.after_collective()
+    bad = [float(s) for s in status.tolist() if s != 0.0]
+    lam[per] = bad[0] if bad else 0.0
+    out_idx = torch.full((per, topk), -1, dtype=torch.int64, device=dev)
+    out_sc = torch.full((per, topk), nan, dtype=torch.float64, device=dev)
+    if not bad and per > 0 and topk > 0:
+        out_idx, out_sc = engine.topk_merge(g_idx, g_sc) if whole else engine.hybrid_merge(g_idx, g_cos, g_sc, m, topk)
+    if c_ > 1:
+        out_idx = _all_gather_blocks(out_idx, c_, grid["item_group"]).reshape(c_ * per, topk)
+        out_sc = _all_gather_blocks(out_sc, c_, grid["item_group"]).reshape(c_ * per, topk)
+        lam = _all_gather_blocks(lam, c_, grid["item_group"])
+        if hasattr(engine, "after_collective"):
+            engine.after_collective()
+    lam = lam.reshape(c_, per + 1).cpu()
+    codes = [int(cd) for cd in lam[:, per].tolist() if cd != 0]
+    if codes:
+        msg = err.message if err is not None and err.code == codes[0] else \
+            "a rank of the query grid failed with error %d" % codes[0]
+        raise LibraryError(codes[0], msg)
+    return (out_idx[:nq].cpu().numpy(), out_sc[:nq].cpu().numpy(),
+            np.ascontiguousarray(lam[:, :per].reshape(-1)[:nq].numpy()))
 
 
 def _all_gather_ragged(t_local, counts, group):

@@ -1,6 +1,7 @@
 """torchrun --nproc-per-node N tools/mgpu_check.py : multi-GPU build + search over NCCL against the CPU oracle and against
 the single-GPU result (bit identical), for EVERY layout of the search grid (R item shards x N / R query slots: R = N fully
-item-sharded ... R = 1 items replicated), with host and with device-resident query batches.
+item-sharded ... R = 1 items replicated), with host and with device-resident query batches, and search_hybrid (host
+batches, default shortlist and pool 40) against the single-GPU result (bit identical) and the oracle.
 
     BIG=1      adds the 1M x 384 case (BASELINE.json C4 shape; oracle check on a 96-query sample)
     CHECK_PEER=1 also runs the peer-memory merge (csrc/peer.cu) on the fully item-sharded layout
@@ -9,6 +10,7 @@ Prints one line per check and MGPU_CHECK OK / FAILED; exit code 0 / 1."""
 import os
 import sys
 import time
+import zlib
 
 import numpy as np
 
@@ -19,6 +21,8 @@ import torch.distributed as dist  # noqa: E402
 
 from pyarrowspace_b200 import shard_rows, synth  # noqa: E402
 from pyarrowspace_b200.api import ArrowSpaceBuilder  # noqa: E402
+
+HYBRID_POOLS = (None, 40)     # search_hybrid shortlists: the default (tensor-core candidates) and the batched exact scan
 
 
 def all_ranks(flag):
@@ -56,6 +60,9 @@ def main():
             s, g = oracle.build(gp, full)
             oidx, osc, _ = s.search_batch(q[pick], g, 0.62)
             ref = dict(idx1=idx1, sc1=sc1, lam1=a1.lambdas(), csr1=g1.csr(), pick=pick, oidx=oidx, osc=osc, olam=s.lambdas(), oedges=g.edges())
+            for pool in HYBRID_POOLS:                         # search_hybrid: one GPU and the oracle's restatement
+                ref["hyb1", pool] = a1.search_hybrid_batch(q, g1, 0.62, pool=pool)
+                ref["hybo", pool] = s.search_hybrid_batch(q[pick], g, 0.62, pool or 0)[:2]
             ar, gr = ArrowSpaceBuilder.build(gp, full, device=local, reduction=True)      # pre-graph reduction, one GPU
             ref.update(red_csr=gr.csr(), red_lam=ar.lambdas(), red_cent=gr.centroids(), red_info=gr.reduction)
             del a1, g1, s, g, full, ar, gr
@@ -92,6 +99,22 @@ def main():
                       % (world, n, f, R, world // R, len(ref["pick"]), e_or, e_1, same_dev, time.time() - t0), flush=True)
                 ok = ok and all(e_or) and all(e_1)
             ok = ok and same_dev
+            for pool in HYBRID_POOLS:                         # collective on item shards; every rank returns the whole batch
+                hi, hs = aspace.search_hybrid_batch(q, gl, 0.62, pool=pool)
+                crc = torch.tensor([zlib.crc32(hi.tobytes() + hs.tobytes())], dtype=torch.int64, device="cuda")
+                lo, hi_crc = crc.clone(), crc.clone()
+                dist.all_reduce(lo, op=dist.ReduceOp.MIN)
+                dist.all_reduce(hi_crc, op=dist.ReduceOp.MAX)
+                if rank == 0:
+                    i1, s1 = ref["hyb1", pool]
+                    oi, os_ = ref["hybo", pool]
+                    e = [np.array_equal(hi, i1) and np.array_equal(hs, s1, equal_nan=True),
+                         np.array_equal(hi[ref["pick"]], oi) and bool(np.allclose(hs[ref["pick"]], os_, rtol=1e-9, atol=0)),
+                         bool(lo.item() == hi_crc.item())]
+                    print("world %d n %d f %d grid %d item shard(s) x %d query slot(s): search_hybrid pool %s == single GPU "
+                          "(bitwise) %s, == oracle (%d queries) %s, same bits on every rank %s"
+                          % (world, n, f, R, world // R, pool, e[0], len(ref["pick"]), e[1], e[2]), flush=True)
+                    ok = ok and all(e)
             if os.environ.get("CHECK_PEER") and R == world and world > 1:    # csrc/peer.cu: P2P exchange + flag-driven merge
                 os.environ["ASP_PEER_MERGE"] = "1"
                 same = True
