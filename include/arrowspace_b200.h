@@ -206,6 +206,16 @@ int asp_query_lambda(asp_ctx *ctx, const asp_graph *g, const asp_switches *sw, c
 int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq,
                      double tau, int64_t *out_idx, double *out_score, double *out_lambda_q);
 
+/* Filtered search: asp_search_batch over the items whose bit is set in allowed_bits only -- per query the best topk ALLOWED
+ * items by (score desc, index asc), the oracle's scores bit for bit, rows padded with -1 / NaN when fewer items are allowed.
+ * allowed_bits: a packed mask over this space's LOCAL rows, ceil(n_local / 8) bytes, LSB-first (bit i % 8 of byte i / 8 =
+ * local row i; numpy.packbits(mask, bitorder="little")), host or device memory; NULL = every row, which is asp_search_batch
+ * itself.  The mask is the same for every query of the call and changes neither lambda_q nor the lambda_q != 0 assertion.
+ * A row shard passes the slice of the global mask for its own rows [row0, row0 + n_local); the per-shard lists merge with
+ * asp_topk_merge as they are. */
+int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
+                              int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits);
+
 /* Hybrid search, batched (SURVEY.md 8(f)-2).  Replaces prepare_query_item + search_lambda_aware_hybrid(&query,
  * gl.graph_params.topk, tau) of ArrowSpace.search_hybrid (src/lib.rs:182-219).  The crate function's body is not in the
  * reference and nothing there documents or tests it, so this is a restatement (PARITY UNPINNED against the crate; GPU ==
@@ -223,6 +233,12 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
  * ASP_ERR_UNSUPPORTED on a row shard: a row-sharded space answers with asp_search_hybrid_shard + asp_hybrid_merge. */
 int asp_search_hybrid_batch(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                             int64_t pool, int64_t *out_idx, double *out_score, double *out_lambda_q);
+
+/* Filtered hybrid search: H2's shortlist is the m ALLOWED items of largest cosine (ties -> smaller index), with m still
+ * asp_hybrid_pool(n, topk, pool) of the whole item count; H3 re-ranks it.  allowed_bits as in asp_search_batch_filtered. */
+int asp_search_hybrid_batch_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
+                                     int64_t pool, int64_t *out_idx, double *out_score, double *out_lambda_q,
+                                     const uint8_t *allowed_bits);
 
 /* The shortlist length m of H2 for n_total items: pool (<= 0: min(2 * topk, 31)), raised to topk, cut to n_total.
  * m == n_total (with n_total > 0) means no shortlist: the whole set. */
@@ -242,6 +258,11 @@ int64_t asp_hybrid_pool(int64_t n_total, int64_t topk, int64_t pool);
  * pointers.  asp_hybrid_merge output layout as asp_search_batch. */
 int asp_search_hybrid_shard(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                             int64_t pool, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q);
+/* The same over this shard's allowed rows (allowed_bits: the shard's slice of the global mask, as in
+ * asp_search_batch_filtered).  asp_hybrid_merge / asp_topk_merge of the filtered lists give the filtered one-GPU answer. */
+int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
+                                     int64_t pool, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q,
+                                     const uint8_t *allowed_bits);
 int asp_hybrid_merge(asp_ctx *ctx, const int64_t *idx, const double *cos, const double *score, int parts, int64_t nq,
                      int64_t m, int64_t topk, int64_t *out_idx, double *out_score);
 

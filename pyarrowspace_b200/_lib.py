@@ -116,6 +116,9 @@ SYMBOLS = {
     "asp_hybrid_pool": (_i64, [_i64, _i64, _i64]),
     "asp_search_hybrid_shard": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _vp, _vp, _vp, _vp]),
     "asp_hybrid_merge": (_int, [_vp, _vp, _vp, _vp, _int, _i64, _i64, _i64, _vp, _vp]),
+    "asp_search_batch_filtered": (_int, [_vp, _vp, _vp, _i64, _dbl, _vp, _vp, _vp, _vp]),
+    "asp_search_hybrid_batch_filtered": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _vp, _vp, _vp, _vp]),
+    "asp_search_hybrid_shard_filtered": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _vp, _vp, _vp, _vp, _vp]),
     "asp_debug_tc_dots": (_int, [_vp, _vp, _i64, _vp]),
     "asp_topk_merge": (_int, [_vp, _vp, _vp, _int, _i64, _i64, _vp, _vp]),
     "asp_peer_exchange_bytes": (C.c_size_t, [_int, _i64, _i64]),

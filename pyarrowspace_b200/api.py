@@ -62,6 +62,18 @@ def _unwrap(exc):
         % (type(exc).__name__, type(exc).__name__, str(exc)))
 
 
+def _check_allowed(allowed, nitems):
+    """The `allowed=` argument of the searches: None, or a 1-D host numpy bool array of one entry per item."""
+    if allowed is None:
+        return None
+    if not isinstance(allowed, np.ndarray) or allowed.dtype != np.bool_:
+        raise TypeError("allowed must be a numpy.ndarray of bool (got %s)" % (
+            "ndarray of %s" % allowed.dtype if isinstance(allowed, np.ndarray) else type(allowed).__name__))
+    if allowed.ndim != 1 or allowed.shape[0] != nitems:
+        raise ValueError("allowed must be 1-D with one entry per item (%d), got shape %s" % (nitems, allowed.shape))
+    return allowed
+
+
 def parse_graph_params(graph_params):
     """src/helpers.rs:48-77: eps, k, topk, p required; sigma missing/None -> eps * 0.5."""
     if graph_params is None:
@@ -271,7 +283,8 @@ class ArrowSpace:
 
     # ------------------------------------------------------------------ search
     def search(self, item, gl, tau):
-        """list[(index, score)], best first, length min(topk, nitems) -- src/lib.rs:132-174."""
+        """list[(index, score)], best first, length min(topk, nitems) -- src/lib.rs:132-174.  (The reference's signature;
+        a filtered single query is search_batch(item.reshape(1, -1), gl, tau, allowed=mask).)"""
         if not isinstance(gl, GraphLaplacian):
             raise TypeError("argument 'gl': 'GraphLaplacian' object expected")
         if not isinstance(item, np.ndarray) or item.dtype != np.float64 or item.ndim != 1:
@@ -285,11 +298,14 @@ class ArrowSpace:
         dbg_println("search: qlen=%d, lambda_q=%.6f" % (item.shape[0], lam_q[0]))
         return [(int(i), float(s)) for i, s in zip(idx[0], score[0]) if i >= 0]
 
-    def search_batch(self, queries, gl, tau, out=None):
+    def search_batch(self, queries, gl, tau, out=None, *, allowed=None):
         """Extension: (idx int64[Q, topk], score f64[Q, topk]); rows padded with -1 / NaN.
         out = (idx, score) host arrays to fill (C-contiguous, right shapes / dtypes; e.g. pinned memory that the caller
         reuses from call to call: the device -> host read then runs at the PCIe rate instead of the page-fault rate of
-        freshly allocated memory).  Host query batches only."""
+        freshly allocated memory).  Host query batches only.
+        allowed = numpy bool[nitems] (keyword only): per query the best topk among the allowed items, padded with -1 / NaN
+        when fewer are allowed; the same mask for every query.  Collective calls: every rank passes the same mask."""
+        allowed = _check_allowed(allowed, self.nitems)
         if out is not None:
             topk = gl.graph_params["topk"]
             nq = queries.shape[0]
@@ -299,13 +315,21 @@ class ArrowSpace:
                 raise ValueError("out must be (int64[%d, %d], float64[%d, %d]) C-contiguous host arrays" % (nq, topk, nq, topk))
             if _is_device_tensor(queries):
                 raise ValueError("out= is for host query batches (device batches return device tensors)")
-        idx, score, _ = self._search_batch(queries, gl, float(tau), want_lambda=False, out=out)
+        idx, score, _ = self._search_batch(queries, gl, float(tau), want_lambda=False, out=out, allowed=allowed)
         return idx, score
 
-    def _search_batch(self, queries, gl, tau, want_lambda, out=None):
+    def _allowed_bits(self, allowed):
+        """This rank's slice of the mask, packed for the library (None: no filter)."""
+        if allowed is None:
+            return None
+        from .distributed import pack_allowed
+        n_local, _, row0, _ = self._dims()
+        return pack_allowed(allowed, row0, n_local)
+
+    def _search_batch(self, queries, gl, tau, want_lambda, out=None, allowed=None):
         import time
         if self._grid is not None and self._grid["C"] > 1:
-            return self._search_batch_grid(queries, gl, tau, out)
+            return self._search_batch_grid(queries, gl, tau, out, allowed)
         t_a = time.perf_counter()
         lib = _lib.load()
         f = self.nfeatures
@@ -352,9 +376,13 @@ class ArrowSpace:
             score = out[1] if out is not None else np.empty((nq, topk), dtype=np.float64)
             lam = np.empty(nq, dtype=np.float64)
             qp, ip, sp, lp = q.ctypes.data, idx.ctypes.data, score.ctypes.data, lam.ctypes.data
+        bits = self._allowed_bits(allowed)
         t_b = time.perf_counter()
         try:
-            _lib.check(lib.asp_search_batch(self._h, gl._h, qp, nq, tau, ip, sp, lp))
+            if bits is None:
+                _lib.check(lib.asp_search_batch(self._h, gl._h, qp, nq, tau, ip, sp, lp))
+            else:
+                _lib.check(lib.asp_search_batch_filtered(self._h, gl._h, qp, nq, tau, ip, sp, lp, bits.ctypes.data))
             LAST_CALL_TRACE["prepare_ms"] = (t_b - t_a) * 1e3
             LAST_CALL_TRACE["library_ms"] = (time.perf_counter() - t_b) * 1e3
         except LibraryError as e:
@@ -372,7 +400,7 @@ class ArrowSpace:
                 _to_host(lam, host_out and host_out[2])
         return idx, score, lam
 
-    def _search_batch_grid(self, queries, gl, tau, out=None):
+    def _search_batch_grid(self, queries, gl, tau, out=None, allowed=None):
         """R item shards x C query slots (distributed.regroup): this rank answers rows [a, b) of the batch against its item
         shard; R > 1: the R ranks of the slot merge their lists (K5); the C slots all-gather the finished slices, so every
         rank returns the whole batch.  Host batches: this rank uploads only ITS slice (over its own PCIe link)."""
@@ -415,7 +443,12 @@ class ArrowSpace:
         if b > a:
             qp = q[a:b].ctypes.data if host_in else q[a:b].data_ptr()
             torch.cuda.current_stream(dev).synchronize()                 # the library runs on its own stream
-            rc = lib.asp_search_batch(self._h, gl._h, qp, b - a, tau, idx_p.data_ptr(), sc_p.data_ptr(), lam_p.data_ptr())
+            bits = self._allowed_bits(allowed)
+            if bits is None:
+                rc = lib.asp_search_batch(self._h, gl._h, qp, b - a, tau, idx_p.data_ptr(), sc_p.data_ptr(), lam_p.data_ptr())
+            else:
+                rc = lib.asp_search_batch_filtered(self._h, gl._h, qp, b - a, tau, idx_p.data_ptr(), sc_p.data_ptr(),
+                                                   lam_p.data_ptr(), bits.ctypes.data)
             if rc != _lib.ASP_OK:
                 msg = lib.asp_last_error()
                 err = LibraryError(rc, msg.decode("utf-8", "replace") if msg else "unknown error")
@@ -454,11 +487,12 @@ class ArrowSpace:
         return persist.save(path, self, gl, items)
 
     # ------------------------------------------------------------------ hybrid search (SURVEY.md 8(f)-2)
-    def search_hybrid(self, item, gl, tau, *, pool=None):
+    def search_hybrid(self, item, gl, tau, *, pool=None, allowed=None):
         """list[(index, score)], best first -- src/lib.rs:182-219: same argument checks and lambda_q as `search`, no
         lambda_q != 0 assertion, k = gl.graph_params.topk, then the crate's search_lambda_aware_hybrid.  That function is not
         in the reference (PARITY UNPINNED): restated as a cosine shortlist of `pool` items (keyword-only extra, default
-        min(2 * topk, 31)) re-ranked by the lambda-aware score (include/arrowspace_b200.h, asp_search_hybrid_batch)."""
+        min(2 * topk, 31)) re-ranked by the lambda-aware score (include/arrowspace_b200.h, asp_search_hybrid_batch).
+        allowed (keyword only, numpy bool[nitems]): the shortlist is the `pool` ALLOWED items of largest cosine."""
         if not isinstance(gl, GraphLaplacian):
             raise TypeError("argument 'gl': 'GraphLaplacian' object expected")
         if not isinstance(item, np.ndarray) or item.dtype != np.float64 or item.ndim != 1:
@@ -467,15 +501,18 @@ class ArrowSpace:
             raise ValueError("The given array is not contiguous")           # as_slice()? src/lib.rs:189
         if item.shape[0] != self.nfeatures:
             raise ValueError("query length %d must match nfeatures %d" % (item.shape[0], self.nfeatures))   # src/lib.rs:190-196
-        idx, score, lam_q = self.search_hybrid_batch(item.reshape(1, -1), gl, float(tau), pool=pool, want_lambda=True)
+        idx, score, lam_q = self.search_hybrid_batch(item.reshape(1, -1), gl, float(tau), pool=pool, want_lambda=True,
+                                                     allowed=allowed)
         dbg_println("search: qlen=%d, lambda_q=%.6f" % (item.shape[0], lam_q[0]))     # src/lib.rs:207-211 (same text as search)
         return [(int(i), float(s)) for i, s in zip(idx[0], score[0]) if i >= 0]
 
-    def search_hybrid_batch(self, queries, gl, tau, *, pool=None, want_lambda=False):
+    def search_hybrid_batch(self, queries, gl, tau, *, pool=None, want_lambda=False, allowed=None):
         """Extension: search_hybrid for a host batch; (idx int64[Q, topk], score f64[Q, topk]) padded with -1 / NaN
         (+ lambda_q with want_lambda).  On one GPU, and on the replicated layout of build_sharded (item_shards = 1), each
         rank answers on its own.  On an item-sharded space (item_shards > 1) it is called collectively, like `search`, and
-        every rank returns the whole batch: the one-GPU answer, bit for bit (distributed.sharded_search_hybrid)."""
+        every rank returns the whole batch: the one-GPU answer, bit for bit (distributed.sharded_search_hybrid).
+        allowed = numpy bool[nitems]: H2's shortlist is taken from the allowed items only (the pool length is unchanged);
+        collective calls pass the same mask on every rank."""
         if not isinstance(gl, GraphLaplacian):
             raise TypeError("argument 'gl': 'GraphLaplacian' object expected")
         n_local, f, _, n_total = self._dims()
@@ -487,6 +524,7 @@ class ArrowSpace:
             raise ValueError("query length %d must match nfeatures %d" % (q.shape[-1], f))
         if pool is not None and (isinstance(pool, bool) or not isinstance(pool, (int, np.integer)) or pool < 1):
             raise ValueError("pool must be a positive integer (the shortlist length; default min(2 * topk, 31))")
+        allowed = _check_allowed(allowed, n_total)
         topk = gl.graph_params["topk"]
         nq = q.shape[0]
         try:
@@ -494,13 +532,19 @@ class ArrowSpace:
                 from .distributed import CudaEngine, sharded_search_hybrid
                 engine = CudaEngine(_lib.load().asp_ctx_device(self._ctx))
                 idx, score, lam = sharded_search_hybrid(engine, self._h, gl._h, q, float(tau), int(pool or 0), topk, n_total,
-                                                        self._grid)
+                                                        self._grid, allowed=allowed)
                 return (idx, score, lam) if want_lambda else (idx, score)
             idx = np.empty((nq, topk), dtype=np.int64)
             score = np.empty((nq, topk), dtype=np.float64)
             lam = np.empty(nq, dtype=np.float64)
-            _lib.check(_lib.load().asp_search_hybrid_batch(self._h, gl._h, q.ctypes.data, nq, float(tau), int(pool or 0),
-                                                           idx.ctypes.data, score.ctypes.data, lam.ctypes.data))
+            bits = self._allowed_bits(allowed)
+            if bits is None:
+                _lib.check(_lib.load().asp_search_hybrid_batch(self._h, gl._h, q.ctypes.data, nq, float(tau), int(pool or 0),
+                                                               idx.ctypes.data, score.ctypes.data, lam.ctypes.data))
+            else:
+                _lib.check(_lib.load().asp_search_hybrid_batch_filtered(self._h, gl._h, q.ctypes.data, nq, float(tau),
+                                                                        int(pool or 0), idx.ctypes.data, score.ctypes.data,
+                                                                        lam.ctypes.data, bits.ctypes.data))
         except LibraryError as e:
             if e.code == _lib.ASP_ERR_ZERO_VECTOR:
                 raise PanicException(e.message)

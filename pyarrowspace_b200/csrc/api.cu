@@ -113,6 +113,19 @@ struct HybridScratch {
     ~HybridScratch() { for (void *p : ptrs) cudaFreeAsync(p, st); }
 };
 
+// The packed item mask of a filtered call (ceil(n / 8) bytes, host or device) on the device as 32-bit words, the rest of the
+// last word zero.  NULL bits: *out = NULL (every row).
+int upload_allowed(cudaStream_t st, const uint8_t *bits, int64_t n, uint32_t **out)
+{
+    *out = nullptr;
+    if (!bits) return ASP_OK;
+    const size_t nbytes = (size_t)((n + 7) / 8), nwords = (size_t)((n + 31) / 32);
+    ASP_CUDA(cudaMallocAsync(out, sizeof(uint32_t) * (nwords ? nwords : 1), st));
+    ASP_CUDA(cudaMemsetAsync(*out, 0, sizeof(uint32_t) * (nwords ? nwords : 1), st));
+    if (nbytes) ASP_CUDA(cudaMemcpyAsync(*out, bits, nbytes, cudaMemcpyDefault, st));
+    return ASP_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -731,10 +744,11 @@ int asp_query_lambda(asp_ctx *ctx, const asp_graph *g, const asp_switches *sw_in
 }
 
 // One device-resident batch: lambda_q (src/lib.rs:154), the lambda_q != 0 guard (src/lib.rs:156-159), candidate pass +
-// exact stage 2.  `flags` is a 2-int device scratch.  Synchronises ctx->stream before returning.
+// exact stage 2.  `flags` is a 2-int device scratch.  allowed: the item mask as upload_allowed left it, or nullptr.
+// Synchronises ctx->stream before returning.
 static int search_device_batch(const asp_space *s, const asp_graph *g, const double *dq, int64_t nq, double tau, int64_t topk,
                                double *dlam, double *dnorm, int *flags, int64_t *didx, double *dscore,
-                               bool assert_lambda_nonzero = true)
+                               bool assert_lambda_nonzero = true, const uint32_t *allowed = nullptr)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
@@ -759,9 +773,9 @@ static int search_device_batch(const asp_space *s, const asp_graph *g, const dou
     int rc;
     // small batches against a large shard stream the fp16 operands (2 * kp bytes per item) instead of the f64 rows
     if (!want_fp64 && asp_search_tc_supported(s, nq, topk, tau) && (want_tc || nq >= 256 || s->n_local >= 131072))
-        rc = asp_search_tc_impl(s, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore, nullptr);
+        rc = asp_search_tc_impl(s, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore, nullptr, allowed);
     else
-        rc = asp_search_impl(s, g, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore);
+        rc = asp_search_impl(s, g, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore, allowed);
     if (rc == ASP_OK) ASP_CUDA(cudaStreamSynchronize(st));
     ctx->stats["search_host_device_batch_us"] = asp_now_us() - t_in;
     return rc;
@@ -779,6 +793,12 @@ constexpr int64_t ASP_PIPE_MIN_BATCH = 32768;
 
 int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                      int64_t *out_idx, double *out_score, double *out_lambda_q)
+{
+    return asp_search_batch_filtered(s, g, queries, nq, tau, out_idx, out_score, out_lambda_q, nullptr);
+}
+
+int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
+                              int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits)
 {
     if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score))) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch: NULL argument");
     if (!s->have_lambdas) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch: item lambdas have not been computed");
@@ -805,12 +825,13 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
         ASP_CUDA(cudaMallocAsync(&didx, sizeof(int64_t) * (size_t)nq * topk, st));
         ASP_CUDA(cudaMallocAsync(&dscore, sizeof(double) * (size_t)nq * topk, st));
     }
+    uint32_t *dallowed = nullptr;                                 // once per call, before the batch is split
+    int rc = upload_allowed(st, allowed_bits, s->n_local, &dallowed);
     const char *nopipe = getenv("ASP_NO_PIPELINE");
     const bool host_io = !asp_is_device_ptr(queries) && !asp_is_device_ptr(out_idx) && !asp_is_device_ptr(out_score) &&
                          (!out_lambda_q || !asp_is_device_ptr(out_lambda_q));
     int64_t head = std::max<int64_t>(1024, (nq * 3 / 64 + 127) / 128 * 128);   // 3072 of 65536: its kernels (~2.5 ms) cover most of the rest's upload
     if (const char *e = getenv("ASP_PIPE_HEAD")) { const long v = atol(e); if (v >= 128 && v < nq) head = v; }   // tuning knob
-    int rc = ASP_OK;
     auto prefault = [=](int64_t q0, int64_t qn) {                 // first touch of the caller's result pages
         if (out_lambda_q) memset(out_lambda_q + q0, 0, sizeof(double) * qn);
         if (topk > 0) {
@@ -819,7 +840,7 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
         }
     };
     const bool touch = host_io && (size_t)nq * (topk + 1) * 16 >= (1u << 18);
-    if (host_io && nq >= ASP_PIPE_MIN_BATCH && !(nopipe && nopipe[0] == '1')) {
+    if (rc == ASP_OK && host_io && nq >= ASP_PIPE_MIN_BATCH && !(nopipe && nopipe[0] == '1')) {
         if (!ctx->up_stream) {                                     // streams and events live as long as the context
             ASP_CUDA(cudaStreamCreateWithFlags(&ctx->up_stream, cudaStreamNonBlocking));
             ASP_CUDA(cudaStreamCreateWithFlags(&ctx->down_stream, cudaStreamNonBlocking));
@@ -847,7 +868,7 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
             cudaEventRecord(start_c[c], st);
             if (c == 1) ctx->on_wait = [=]() { prefault(head, nq - head); };   // under the kernels of the rest (the head's are too short)
             rc = search_device_batch(s, g, dq + q0 * fp, qn, tau, topk, dlam + q0, dnorm + q0, flags,
-                                     didx ? didx + q0 * topk : nullptr, dscore ? dscore + q0 * topk : nullptr);
+                                     didx ? didx + q0 * topk : nullptr, dscore ? dscore + q0 * topk : nullptr, true, dallowed);
             if (ctx->on_wait) { auto fn = std::move(ctx->on_wait); ctx->on_wait = nullptr; if (rc == ASP_OK) fn(); }
             if (rc != ASP_OK) break;
             // results of this piece: D2H on the second copy stream (for pageable destinations the runtime stages the copy
@@ -875,10 +896,10 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
                 if (cudaEventElapsedTime(&ms, alloc_ready, evs[i]) == cudaSuccess) ctx->stats[names[i]] = ms; else cudaGetLastError();
         }
         ctx->stats["search_pipeline_chunks"] = nch;
-    } else {
+    } else if (rc == ASP_OK) {
         rc = upload_pitched(st, queries, nq, f, fp, dq);
         if (touch) ctx->on_wait = [=]() { prefault(0, nq); };
-        if (rc == ASP_OK) rc = search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore);
+        if (rc == ASP_OK) rc = search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, true, dallowed);
         if (ctx->on_wait) { auto fn = std::move(ctx->on_wait); ctx->on_wait = nullptr; if (rc == ASP_OK) fn(); }
         if (rc == ASP_OK && out_lambda_q) rc = asp_copy_out(ctx, out_lambda_q, dlam, sizeof(double) * nq);
         if (rc == ASP_OK && topk > 0) {
@@ -894,6 +915,7 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
     cudaFreeAsync(flags, st);
     if (didx) cudaFreeAsync(didx, st);
     if (dscore) cudaFreeAsync(dscore, st);
+    if (dallowed) cudaFreeAsync(dallowed, st);
     return rc;
 }
 
@@ -909,6 +931,14 @@ int64_t asp_hybrid_pool(int64_t n_total, int64_t topk, int64_t pool)
 // hybrid.cuh.  No lambda_q != 0 assertion (search_hybrid has none).
 int asp_search_hybrid_batch(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
                             int64_t *out_idx, double *out_score, double *out_lambda_q)
+{
+    return asp_search_hybrid_batch_filtered(s, g, queries, nq, tau, pool, out_idx, out_score, out_lambda_q, nullptr);
+}
+
+// Filtered: the shortlist is the m ALLOWED items of largest cosine (the filtered search at tau = 1), m still from n.
+int asp_search_hybrid_batch_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
+                                     int64_t pool, int64_t *out_idx, double *out_score, double *out_lambda_q,
+                                     const uint8_t *allowed_bits)
 {
     if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score)))
         ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_batch: NULL argument");
@@ -949,11 +979,14 @@ int asp_search_hybrid_batch(const asp_space *s, const asp_graph *g, const double
         ASP_CHECK(scratch.get(&dscore, (size_t)nq * topk));
     }
     ASP_CHECK(upload_pitched(st, queries, nq, f, fp, dq));
+    uint32_t *dallowed = nullptr;
+    ASP_CHECK(upload_allowed(st, allowed_bits, s->n_local, &dallowed));
+    if (dallowed) scratch.ptrs.push_back(dallowed);
     // H1 + H2: lambda_q, then the m largest cosines per query (the score at tau = 1 is the cosine), ties by the smaller index
     if (whole_set)
-        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false));
+        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false, dallowed));
     else
-        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? m : 0, dlam, dnorm, flags, pidx, pscore, false));
+        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? m : 0, dlam, dnorm, flags, pidx, pscore, false, dallowed));
     if (topk > 0 && !whole_set) {
         // H3: reference-order scores of the shortlist, best topk by (score desc, index asc)
         const int64_t total = nq * m;
@@ -982,6 +1015,13 @@ int asp_search_hybrid_batch(const asp_space *s, const asp_graph *g, const double
 // takes the global top-m by cosine from the shards' lists and re-ranks it, which is what the one-GPU shortlist holds.
 int asp_search_hybrid_shard(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
                             int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q)
+{
+    return asp_search_hybrid_shard_filtered(s, g, queries, nq, tau, pool, out_idx, out_cos, out_score, out_lambda_q, nullptr);
+}
+
+int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
+                                     int64_t pool, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q,
+                                     const uint8_t *allowed_bits)
 {
     if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score)))
         ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_shard: NULL argument");
@@ -1018,9 +1058,12 @@ int asp_search_hybrid_shard(const asp_space *s, const asp_graph *g, const double
         if (!whole_set) ASP_CHECK(scratch.get(&dcos, (size_t)nq * width));
     }
     ASP_CHECK(upload_pitched(st, queries, nq, f, fp, dq));
+    uint32_t *dallowed = nullptr;
+    ASP_CHECK(upload_allowed(st, allowed_bits, s->n_local, &dallowed));
+    if (dallowed) scratch.ptrs.push_back(dallowed);
     if (whole_set) {
         // no shortlist: the shard's best topk by the lambda-aware score, merged like asp_search_batch's lists
-        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false));
+        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false, dallowed));
     } else {
         int64_t *sidx = didx;
         double *scos = dcos;
@@ -1029,7 +1072,7 @@ int asp_search_hybrid_shard(const asp_space *s, const asp_graph *g, const double
             ASP_CHECK(scratch.get(&scos, (size_t)nq * kl));
         }
         // the score at tau = 1 is the cosine
-        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? kl : 0, dlam, dnorm, flags, sidx, scos, false));
+        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? kl : 0, dlam, dnorm, flags, sidx, scos, false, dallowed));
         if (topk > 0) {
             if (kl < m) {                                         // lists padded to m with -1 / NaN
                 ASP_CUDA(cudaMemsetAsync(didx, 0xff, sizeof(int64_t) * (size_t)nq * m, st));

@@ -109,6 +109,10 @@ static inline int64_t asp_neighbour_cap(const asp_graph_params *gp, const asp_sw
     return kk < 0 ? 0 : kk;
 }
 
+// Item filter of a search: bit i of the packed mask (LSB-first bytes, read as little-endian 32-bit words) says whether local
+// row i may be returned.  nullptr = every row.
+__device__ __forceinline__ bool asp_allowed(const uint32_t *bits, int64_t i) { return (bits[i >> 5] >> (i & 31)) & 1u; }
+
 // host helpers implemented in api.cu
 int  asp_copy_in(asp_ctx *ctx, void *dst_dev, const void *src, size_t bytes);
 int  asp_copy_out(asp_ctx *ctx, void *dst, const void *src_dev, size_t bytes);
@@ -148,7 +152,7 @@ int asp_launch_taumode(asp_ctx *ctx, const asp_graph *g, const asp_switches *sw,
 // search.cu
 int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev, int64_t nq, int32_t qpitch,
                     const double *lambda_q_dev, const double *qnorm_dev, double tau, int64_t topk,
-                    int64_t *out_idx_dev, double *out_score_dev);
+                    int64_t *out_idx_dev, double *out_score_dev, const uint32_t *allowed_dev = nullptr);
 int asp_topk_merge_impl(asp_ctx *ctx, const int64_t *idx_dev, const double *score_dev, int parts,
                         int64_t nq, int64_t topk, int64_t *out_idx_dev, double *out_score_dev);
 
@@ -164,22 +168,23 @@ struct asp_tc_batch {                     // device buffers of one batch of quer
     float *emit_sc = nullptr;                        // [nq][nsub][capb] approximate scores
     int32_t *emit_ix = nullptr, *emit_cnt = nullptr; // local item indices; [nq][nsub] counts (> capb: overflow)
     uint32_t *theta_glob = nullptr;
+    uint32_t *vbits = nullptr;                       // filtered search: the item mask in visiting order
 };
 enum { ASP_TC_ORDER_IDENTITY = 0, ASP_TC_ORDER_LAMBDA = 1, ASP_TC_ORDER_NORM = 2 };   // item order of the operand cache
 int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                   const double *qnorm_dev, double tau, int64_t topk, double score_floor, int force_terms, int capb_override,
-                  float *dump_dev, asp_tc_batch *b, bool l2 = false);
+                  float *dump_dev, asp_tc_batch *b, bool l2 = false, const uint32_t *allowed_dev = nullptr);
 int asp_device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out);   // max(0, max v), synchronises
 void asp_tc_batch_free(asp_ctx *ctx, asp_tc_batch *b);
 bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, double tau);
 int asp_search_tc_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                        const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
-                       float *dump_dev);
+                       float *dump_dev, const uint32_t *allowed_dev = nullptr);
 void asp_free_tc_cache(asp_space *s);
 int asp_launch_reciprocal(asp_ctx *ctx, const double *x, int64_t n, double *out);
 int asp_search_slow_path(const asp_space *s, const double *q_dev, int32_t qpitch, const double *lambda_q_dev,
                          const double *qnorm_dev, double tau, int64_t topk, const int32_t *slow_list_dev, int nslow,
-                         int64_t *out_idx_dev, double *out_score_dev);
+                         int64_t *out_idx_dev, double *out_score_dev, const uint32_t *allowed_dev = nullptr);
 int asp_make_f16_tmap(CUtensorMap *out, const void *base, int64_t rows, int32_t kp, int box_rows);
 int asp_make_f16_tmap_narrow(CUtensorMap *out, const void *base, int64_t rows, int32_t kp, int box_rows, int nw);
 

@@ -3,6 +3,8 @@
 //
 // MODE 0 (search):     score = tau*cos(q,x) + (1-tau)/(1+|lambda_q - lambda_x|)
 // MODE 1 (item graph): score = max(0, cos(x_i, x_j)), j != i, score >= smin (= 1 - eps - band)
+// FILTER (MODE 0 only): a column whose bit in `allowed` is clear is treated like one beyond n_local -- it never enters a
+// row's list, so it never raises the row's threshold.
 #pragma once
 #include "common.cuh"
 #include "ptx.cuh"
@@ -61,14 +63,16 @@ __device__ __noinline__ void compact_row(ListSmem<LIST> *ls, int row, int lane)
     __syncwarp();
 }
 
-template <int LIST, int STAGES, bool USE_TMA, int MODE>
+template <int LIST, int STAGES, bool USE_TMA, int MODE, bool FILTER = false>
 __global__ void __launch_bounds__(MMA_WARPS * 32, 1)
 search_gemm_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_x,
                    const double *__restrict__ q, const double *__restrict__ items, int64_t nq, int64_t n_local, int fp,
                    const double *__restrict__ inv_nx, const double *__restrict__ lam_x,
                    const double *__restrict__ inv_nq, const double *__restrict__ lam_q, double tau, double smin,
-                   int nchunks, double *__restrict__ cand_score, int32_t *__restrict__ cand_idx)
+                   int nchunks, double *__restrict__ cand_score, int32_t *__restrict__ cand_idx,
+                   const uint32_t *__restrict__ allowed)
 {
+    static_assert(!FILTER || MODE == 0, "only the search is filtered");
     constexpr int CAP = 2 * LIST;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     double *stages = reinterpret_cast<double *>(smem_raw);
@@ -211,6 +215,7 @@ search_gemm_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_cons
 #pragma unroll
             for (int e = 0; e < 2; ++e) {
                 cvalid[e] = (c0 + e) < n_local;
+                if (FILTER) cvalid[e] = cvalid[e] && asp_allowed(allowed, c0 + e);
                 inx[e] = cvalid[e] ? inv_nx[c0 + e] : 0.0;
                 lmx[e] = (MODE == 0 && cvalid[e]) ? lam_x[c0 + e] : 0.0;
             }

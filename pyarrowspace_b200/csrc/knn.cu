@@ -404,12 +404,12 @@ static int item_knn_fp64(asp_space *s, const asp_graph_params *gp, asp_knn_lists
             auto k = search_gemm_kernel<LIST, STAGES, true, 1>;
             ASP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             k<<<grid, MMA_WARPS * 32, smem, st>>>(s->tmap_rows, s->tmap_rows, s->items, s->items, n, n, s->fp, s->inv_norms,
-                                                   nullptr, s->inv_norms, nullptr, 1.0, smin, nparts, cand_score, cand_idx);
+                                                   nullptr, s->inv_norms, nullptr, 1.0, smin, nparts, cand_score, cand_idx, nullptr);
         } else {
             auto k = search_gemm_kernel<LIST, STAGES, false, 1>;
             ASP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             k<<<grid, MMA_WARPS * 32, smem, st>>>(s->tmap_rows, s->tmap_rows, s->items, s->items, n, n, s->fp, s->inv_norms,
-                                                   nullptr, s->inv_norms, nullptr, 1.0, smin, nparts, cand_score, cand_idx);
+                                                   nullptr, s->inv_norms, nullptr, 1.0, smin, nparts, cand_score, cand_idx, nullptr);
         }
         ASP_CUDA(cudaGetLastError());
         ASP_LAUNCHED(ctx);

@@ -16,10 +16,14 @@
 //            complete iff  s~(LIST) < s~(k) - 2 DELTA  (or the shard has <= LIST items); otherwise the
 //            query takes the exact full scan (exact_scan.cuh, SearchScanPolicy).
 //   K5       topk_merge_kernel: merge of per-shard results (cross-GPU), (score desc, index asc).
+// Filtered search (FILTER instantiations, `allowed` = packed item mask): stage 1 skips a row that is not allowed before it can
+// enter a list, so every threshold is the k-th score of k allowed rows and the completeness test above holds over the allowed
+// set; the exact scan marks such rows invalid.  Stage 2 needs no change.
 #include "gemm_topk.cuh"
 #include "exact_scan.cuh"
 
 #include <math.h>
+#include <type_traits>
 
 namespace {
 
@@ -30,12 +34,12 @@ using namespace asp_gemm;
 constexpr int GV_MAXQ = 8;
 constexpr int GV_WARPS = 8;
 
-template <int LIST, int FPL>
+template <int LIST, int FPL, bool FILTER>
 __global__ void __launch_bounds__(GV_WARPS * 32)
 search_gemv_kernel(const double *__restrict__ q, int qpitch, int nq, const double *__restrict__ items, int64_t n_local,
                    int f, int pitch, const double *__restrict__ inv_nx, const double *__restrict__ lam_x,
                    const double *__restrict__ inv_nq, const double *__restrict__ lam_q, double tau,
-                   double *__restrict__ cand_score, int32_t *__restrict__ cand_idx)
+                   double *__restrict__ cand_score, int32_t *__restrict__ cand_idx, const uint32_t *__restrict__ allowed)
 {
     constexpr int CAP = 2 * LIST;
     constexpr int NPL = CAP / 32;
@@ -81,6 +85,7 @@ search_gemv_kernel(const double *__restrict__ q, int qpitch, int nq, const doubl
 
     const int64_t gw = (int64_t)blockIdx.x * GV_WARPS + warp, nw = (int64_t)gridDim.x * GV_WARPS;
     for (int64_t item = gw; item < n_local; item += nw) {
+        if (FILTER && !asp_allowed(allowed, item)) continue;                         // warp-uniform: one item per warp
         const double *row = items + item * pitch;
         double xv[FPL];
 #pragma unroll
@@ -238,19 +243,20 @@ rescore_kernel(const double *__restrict__ q, int qpitch, int64_t nq, const doubl
 }
 
 // ============================================================================ slow path: exact full scan (exact_scan.cuh)
-// value = the reference-order score; every item is admissible
+// value = the reference-order score; every item is admissible (FILTER: the allowed ones)
+template <bool FILTER>
 struct SearchScanPolicy {
     const double *q; int qpitch; const int32_t *slow_list;
     const double *norm_x, *lam_x, *norm_q, *lam_q; double tau;
-    int64_t row0; int topk; int64_t *out_idx; double *out_score;
+    int64_t row0; int topk; int64_t *out_idx; double *out_score; const uint32_t *allowed;
     struct Row { double nq, lq; };
     struct Item { double nx, lx; };
     __device__ const double *query(int slot) const { return q + (int64_t)slow_list[slot] * qpitch; }
     __device__ Row row(int slot) const { const int64_t qi = slow_list[slot]; return Row{norm_q[qi], lam_q[qi]}; }
     __device__ Item item(int64_t it) const { return Item{norm_x[it], lam_x[it]}; }
-    __device__ double value(const Row &r, const Item &i, double dot, int64_t, bool &valid) const
+    __device__ double value(const Row &r, const Item &i, double dot, int64_t it, bool &valid) const
     {
-        valid = true;
+        valid = !FILTER || asp_allowed(allowed, it);
         return exact_score(dot, r.nq, i.nx, tau, r.lq, i.lx);
     }
     __device__ void emit(int slot, int r, bool ok, double v, int64_t it) const
@@ -305,35 +311,35 @@ __global__ void topk_merge_kernel(const int64_t *__restrict__ idx, const double 
     }
 }
 
-template <int LIST>
+template <int LIST, bool FILTER>
 int launch_gemm(const asp_space *s, const CUtensorMap &tmap_q, const double *q_dev, int64_t nq, const double *inv_nq,
-                const double *lam_q, double tau, int nchunks, double *cand_score, int32_t *cand_idx)
+                const double *lam_q, double tau, int nchunks, double *cand_score, int32_t *cand_idx, const uint32_t *allowed)
 {
     asp_ctx *ctx = s->ctx;
     constexpr int STAGES = (LIST == 16) ? 4 : 3;
     const size_t smem = (size_t)STAGES * STAGE_DOUBLES_S * 8 + sizeof(ListSmem<LIST>) + 128;
     dim3 grid((unsigned)asp_ceil_div(nq, QT), nchunks);
     if (ctx->use_tma) {
-        auto k = search_gemm_kernel<LIST, STAGES, true, 0>;
+        auto k = search_gemm_kernel<LIST, STAGES, true, 0, FILTER>;
         ASP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         k<<<grid, MMA_WARPS * 32, smem, ctx->stream>>>(tmap_q, s->tmap_rows, q_dev, s->items, nq, s->n_local, s->fp,
                                                            s->inv_norms, s->lambdas, inv_nq, lam_q, tau, 0.0, nchunks, cand_score,
-                                                           cand_idx);
+                                                           cand_idx, allowed);
     } else {
-        auto k = search_gemm_kernel<LIST, STAGES, false, 0>;
+        auto k = search_gemm_kernel<LIST, STAGES, false, 0, FILTER>;
         ASP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         k<<<grid, MMA_WARPS * 32, smem, ctx->stream>>>(tmap_q, s->tmap_rows, q_dev, s->items, nq, s->n_local, s->fp,
                                                      s->inv_norms, s->lambdas, inv_nq, lam_q, tau, 0.0, nchunks, cand_score,
-                                                     cand_idx);
+                                                     cand_idx, allowed);
     }
     ASP_CUDA(cudaGetLastError());
     ASP_LAUNCHED(ctx);
     return ASP_OK;
 }
 
-template <int LIST>
+template <int LIST, bool FILTER>
 int launch_gemv(const asp_space *s, const double *q_dev, int qpitch, int nq, const double *inv_nq, const double *lam_q,
-                double tau, int nblocks, double *cand_score, int32_t *cand_idx)
+                double tau, int nblocks, double *cand_score, int32_t *cand_idx, const uint32_t *allowed)
 {
     asp_ctx *ctx = s->ctx;
     constexpr int CAP = 2 * LIST;
@@ -342,12 +348,12 @@ int launch_gemv(const asp_space *s, const double *q_dev, int qpitch, int nq, con
     auto smem_for = [&](int FPL) { return (size_t)GV_MAXQ * FPL * 32 * 8 + (size_t)GV_WARPS * GV_MAXQ * CAP * 12; };
 #define ASP_GEMV_CASE(FPLV)                                                                                         \
     {                                                                                                               \
-        auto k = search_gemv_kernel<LIST, FPLV>;                                                                    \
+        auto k = search_gemv_kernel<LIST, FPLV, FILTER>;                                                            \
         const size_t smem = smem_for(FPLV);                                                                         \
         ASP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                  \
         k<<<nblocks, GV_WARPS * 32, smem, ctx->stream>>>(q_dev, qpitch, nq, s->items, s->n_local, f, s->fp,         \
                                                         s->inv_norms, s->lambdas, inv_nq, lam_q, tau, cand_score,   \
-                                                        cand_idx);                                                  \
+                                                        cand_idx, allowed);                                         \
     }
     if (fpl <= 4) ASP_GEMV_CASE(4)
     else if (fpl <= 12) ASP_GEMV_CASE(12)
@@ -373,13 +379,17 @@ int asp_launch_reciprocal(asp_ctx *ctx, const double *x, int64_t n, double *out)
 // exact full scan of the listed queries (completeness test failed / emission buffer full)
 int asp_search_slow_path(const asp_space *s, const double *q_dev, int32_t qpitch, const double *lambda_q_dev,
                          const double *qnorm_dev, double tau, int64_t topk, const int32_t *slow_list, int nslow,
-                         int64_t *out_idx_dev, double *out_score_dev)
+                         int64_t *out_idx_dev, double *out_score_dev, const uint32_t *allowed)
 {
     asp_ctx *ctx = s->ctx;
-    const SearchScanPolicy pol{q_dev, qpitch, slow_list, s->norms, s->lambdas, qnorm_dev, lambda_q_dev, tau,
-                               s->row0, (int)topk, out_idx_dev, out_score_dev};
-    const int rc = asp_xs::run(ctx->stream, ctx->num_sms, pol, nslow, s->items, s->n_local, s->f, s->fp, topk,
-                               [&](int k) { ctx->launches += k; });
+    auto scan = [&](auto pol) {
+        return asp_xs::run(ctx->stream, ctx->num_sms, pol, nslow, s->items, s->n_local, s->f, s->fp, topk,
+                           [&](int k) { ctx->launches += k; });
+    };
+    const int rc = allowed ? scan(SearchScanPolicy<true>{q_dev, qpitch, slow_list, s->norms, s->lambdas, qnorm_dev, lambda_q_dev,
+                                                         tau, s->row0, (int)topk, out_idx_dev, out_score_dev, allowed})
+                           : scan(SearchScanPolicy<false>{q_dev, qpitch, slow_list, s->norms, s->lambdas, qnorm_dev, lambda_q_dev,
+                                                          tau, s->row0, (int)topk, out_idx_dev, out_score_dev, nullptr});
     if (rc == 1) ASP_FAIL(ASP_ERR_UNSUPPORTED, "exact scan supports topk <= %d (got %lld)", asp_xs::TOPK_MAX, (long long)topk);
     if (rc == 2) ASP_FAIL(ASP_ERR_UNSUPPORTED, "exact scan: %d features x topk %lld do not fit in shared memory", s->f, (long long)topk);
     if (rc == 3) ASP_FAIL(ASP_ERR_NOMEM, "out of device memory in the exact scan");
@@ -389,7 +399,7 @@ int asp_search_slow_path(const asp_space *s, const double *q_dev, int32_t qpitch
 
 int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev, int64_t nq, int32_t qpitch,
                     const double *lambda_q_dev, const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev,
-                    double *out_score_dev)
+                    double *out_score_dev, const uint32_t *allowed)
 {
     (void)g;
     asp_ctx *ctx = s->ctx;
@@ -421,8 +431,13 @@ int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev,
         nparts = (int)(want < ctx->num_sms * 2 ? (want > 0 ? want : 1) : ctx->num_sms * 2);
         ASP_CUDA(cudaMallocAsync(&cand_score, sizeof(double) * (size_t)nq * nparts * LISTSEL, st));
         ASP_CUDA(cudaMallocAsync(&cand_idx, sizeof(int32_t) * (size_t)nq * nparts * LISTSEL, st));
-        if (LISTSEL == 16) ASP_CHECK(launch_gemv<16>(s, q_dev, qpitch, (int)nq, inv_nq, lambda_q_dev, tau, nparts, cand_score, cand_idx));
-        else ASP_CHECK(launch_gemv<32>(s, q_dev, qpitch, (int)nq, inv_nq, lambda_q_dev, tau, nparts, cand_score, cand_idx));
+        auto gemv = [&](auto list, auto filter) {
+            return launch_gemv<decltype(list)::value, decltype(filter)::value>(s, q_dev, qpitch, (int)nq, inv_nq, lambda_q_dev, tau,
+                                                                               nparts, cand_score, cand_idx, allowed);
+        };
+        using L16 = std::integral_constant<int, 16>; using L32 = std::integral_constant<int, 32>;
+        using F0 = std::false_type; using F1 = std::true_type;
+        ASP_CHECK(LISTSEL == 16 ? (allowed ? gemv(L16(), F1()) : gemv(L16(), F0())) : (allowed ? gemv(L32(), F1()) : gemv(L32(), F0())));
     } else {
         const int64_t tiles_total = asp_ceil_div(s->n_local, IT);
         const int64_t qblocks = asp_ceil_div(nq, QT);
@@ -444,8 +459,13 @@ int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev,
         ASP_CHECK(asp_make_items_tmap(&tmap_q, q_dev, nq, qpitch, QT, KSTEP / 4));
         ASP_CUDA(cudaMallocAsync(&cand_score, sizeof(double) * (size_t)nq * nparts * LISTSEL, st));
         ASP_CUDA(cudaMallocAsync(&cand_idx, sizeof(int32_t) * (size_t)nq * nparts * LISTSEL, st));
-        if (LISTSEL == 16) ASP_CHECK(launch_gemm<16>(s, tmap_q, q_dev, nq, inv_nq, lambda_q_dev, tau, nparts, cand_score, cand_idx));
-        else ASP_CHECK(launch_gemm<32>(s, tmap_q, q_dev, nq, inv_nq, lambda_q_dev, tau, nparts, cand_score, cand_idx));
+        auto gemm = [&](auto list, auto filter) {
+            return launch_gemm<decltype(list)::value, decltype(filter)::value>(s, tmap_q, q_dev, nq, inv_nq, lambda_q_dev, tau,
+                                                                               nparts, cand_score, cand_idx, allowed);
+        };
+        using L16 = std::integral_constant<int, 16>; using L32 = std::integral_constant<int, 32>;
+        using F0 = std::false_type; using F1 = std::true_type;
+        ASP_CHECK(LISTSEL == 16 ? (allowed ? gemm(L16(), F1()) : gemm(L16(), F0())) : (allowed ? gemm(L32(), F1()) : gemm(L32(), F0())));
     }
     ASP_CUDA(cudaEventRecord(ctx->ev1, st));
 
@@ -479,7 +499,7 @@ int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev,
     ctx->stats["search_stage1_is_tc"] = 0.0;
     if (nslow > 0)
         ASP_CHECK(asp_search_slow_path(s, q_dev, qpitch, lambda_q_dev, qnorm_dev, tau, topk, slow_list, nslow, out_idx_dev,
-                                       out_score_dev));
+                                       out_score_dev, allowed));
     ASP_CUDA(cudaFreeAsync(cand_score, st));
     ASP_CUDA(cudaFreeAsync(cand_idx, st));
     ASP_CUDA(cudaFreeAsync(slow_list, st));

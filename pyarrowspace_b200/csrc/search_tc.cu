@@ -31,6 +31,13 @@
 // has s >= t_k, hence s~ >= s - DELTA >= theta - 2 DELTA: it passes every emission test and the final cut.  The same
 // argument with EPS in place of DELTA covers (A) -> (B).
 //
+// Filtered search (FILTER instantiations): a per-call bitmask in VISITING order, vbits[pos] = allowed[perm[pos]], gives the
+// 32 columns of one TMEM load in one word.  The rare path drops the columns that are not allowed before anything else, so no
+// such item is emitted, enters a quarter list or raises theta_k / s_theta / theta_glob: every threshold stays the k-th best
+// approximate score of k distinct allowed items and the argument above holds over the allowed set.  The common path is
+// unchanged.  A query with fewer allowed items than topk never gets a finite threshold; stage 2 sees fewer than k
+// candidates in the band and sends it to the exact scan (search_slow_queries), which skips the rows that are not allowed.
+//
 // Kernel (one CTA per SM, 64 + 512 threads):
 //   warp 0     TMA producer: 4-stage ring of {128 queries x 64 k, 256 items x 64 k} fp16 tiles, SWIZZLE_128B
 //   warp 1     allocates TMEM (512 columns = 2 accumulators of 128 x 256 f32), issues tcgen05.mma (one lane),
@@ -43,6 +50,7 @@
 #include "l2_bound.cuh"
 
 #include <cuda_fp16.h>
+#include <algorithm>
 #include <math.h>
 #include <stdlib.h>
 
@@ -198,6 +206,19 @@ __global__ void gather_f32_kernel(const double *__restrict__ a, const int32_t *_
 {
     for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x)
         fa[i] = (float)a[perm ? perm[i] : i];
+}
+
+// filtered search: vbits[pos] = allowed[perm[pos]] for the nwords * 32 visiting positions (0 from n on)
+__global__ void visit_bits_kernel(const uint32_t *__restrict__ allowed, const int32_t *__restrict__ perm, int64_t n, int64_t nwords,
+                                  uint32_t *__restrict__ vbits)
+{
+    const int lane = threadIdx.x & 31;
+    const int64_t warp = (blockIdx.x * (int64_t)blockDim.x + threadIdx.x) >> 5, nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    for (int64_t w = warp; w < nwords; w += nwarps) {
+        const int64_t pos = w * 32 + lane;
+        const unsigned word = __ballot_sync(0xffffffffu, pos < n && asp_allowed(allowed, perm[pos]));
+        if (lane == 0) vbits[w] = word;
+    }
 }
 
 // ---- mean direction of the unit vectors (any unit vector keeps the identity below exact; the mean makes the residuals small)
@@ -408,6 +429,7 @@ struct TcParams {
     int32_t *emit_ix;
     int32_t *emit_cnt;
     float *dump;                  // DUMP mode: approximate cosines [nq][n_local], local item order
+    const uint32_t *vbits;        // FILTER: item mask in visiting order, zero beyond n_local (whole tiles)
 };
 
 // ARES (1-term mode, <= 7 k blocks): the query operand (128 x kp fp16, <= 112 KB) is loaded ONCE and stays resident in
@@ -423,7 +445,7 @@ struct TcParams {
 // L2 (score kind of the Euclidean item graph): the score is -d^2~ (l2_bound.cuh) instead of tau cos~ + beta prox; lam_x /
 // lam_q / tile_lo / tile_hi then hold the f32 norms (items in norm order) and the per-(row, tile) raw-accumulator threshold
 // comes from asp_l2::threshold instead of the proximity bound.  The MMAs and the pipeline are the same.
-template <bool DUMP, int VARIANT, bool ARES, bool PAIR, int LISTN, bool L2 = false>   // LISTN (>= topk): the four column-quarter threads of a query row keep LISTN / 4 scores each; VARIANT (profiling only): 0 normal, 2 epilogue does no work, 3 no MMA issued, 4 epilogue loads TMEM only
+template <bool DUMP, int VARIANT, bool ARES, bool PAIR, int LISTN, bool L2 = false, bool FILTER = false>   // LISTN (>= topk): the four column-quarter threads of a query row keep LISTN / 4 scores each; VARIANT (profiling only): 0 normal, 2 epilogue does no work, 3 no MMA issued, 4 epilogue loads TMEM only
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_constant__ CUtensorMap map_q_lo,
                const __grid_constant__ CUtensorMap map_x_hi, const __grid_constant__ CUtensorMap map_x_lo,
@@ -431,6 +453,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
 {
     static_assert(!PAIR || ARES, "the CTA-pair kernel keeps the query operand resident");
     static_assert(!L2 || (!DUMP && VARIANT == 0), "the l2 score kind has no dump or profiling variants");
+    static_assert(!FILTER || (!L2 && !DUMP && VARIANT == 0), "only the search is filtered");
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     // SWIZZLE_128B tiles must start on 1024-byte boundaries
     constexpr int NST = PAIR ? 6 : ARES ? 3 : TC_STAGES;                         // ring depth
@@ -673,6 +696,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
                         uint32_t mask = 0;
 #pragma unroll
                         for (int j = 0; j < 32; ++j) mask |= (__uint_as_float(r[j]) >= theta_acc) ? (1u << j) : 0u;
+                        if constexpr (FILTER) mask &= p.vbits[(item0 + col0) >> 5];       // col0 % 32 == 0: one word
                         while (mask) {
                             const int j = __ffs(mask) - 1;
                             mask &= mask - 1;
@@ -1172,13 +1196,14 @@ bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, doubl
 // the order of their norms (qnorm_dev is the key; lambda_q_dev and tau are unused).
 int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                   const double *qnorm_dev, double tau, int64_t topk, double score_floor, int force_terms, int capb_override,
-                  float *dump_dev, asp_tc_batch *b, bool l2)
+                  float *dump_dev, asp_tc_batch *b, bool l2, const uint32_t *allowed_dev)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
     const double t_stage1 = asp_now_us();
     asp_tc_cache *c = nullptr;
     if (l2 && dump_dev) ASP_FAIL(ASP_ERR_ARG, "asp_tc_stage1: no dump of the l2 score");
+    if (allowed_dev && (l2 || dump_dev)) ASP_FAIL(ASP_ERR_ARG, "asp_tc_stage1: only the search is filtered");
     ASP_CHECK(ensure_tc_cache(s, l2, &c));
     if (l2) { lambda_q_dev = qnorm_dev; tau = 1.0; }
     const int kp = c->kp;
@@ -1283,7 +1308,15 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     p.sub_hi_last = (s->f + 3 - (p.kb_hi - 1) * TKB + 15) / 16;
     p.nw_hi = c->nw;
     p.lam_x = c->lam32; p.lam_q = b->lam_q32; p.tile_lo = c->tile_lo; p.tile_hi = c->tile_hi; p.perm = c->perm; p.center = b->center;
-    p.theta_glob = nullptr; p.emit_sc = nullptr; p.emit_ix = nullptr; p.emit_cnt = nullptr; p.dump = dump_dev;
+    p.theta_glob = nullptr; p.emit_sc = nullptr; p.emit_ix = nullptr; p.emit_cnt = nullptr; p.dump = dump_dev; p.vbits = nullptr;
+    if (allowed_dev) {                                            // from the cache's current order (it may have been rebuilt)
+        const int64_t nwords = tiles_total * (TN / 32);
+        ASP_CUDA(cudaMallocAsync(&b->vbits, sizeof(uint32_t) * (size_t)nwords, st));
+        visit_bits_kernel<<<(unsigned)std::min<int64_t>(asp_ceil_div(nwords, 8), (int64_t)ctx->num_sms * 8), 256, 0, st>>>(
+            allowed_dev, c->perm, s->n_local, nwords, b->vbits);
+        ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
+        p.vbits = b->vbits;
+    }
     if (!dump_dev) {
         ASP_CUDA(cudaMallocAsync(&b->emit_sc, sizeof(float) * (size_t)nq * nchunks * capb, st));
         ASP_CUDA(cudaMallocAsync(&b->emit_ix, sizeof(int32_t) * (size_t)nq * nchunks * capb, st));
@@ -1314,7 +1347,7 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     int v = 0;
 #endif
     if (pair) p.nw_hi = 0;                                        // (the CTA-pair kernel keeps full boxes)
-    if (l2) v = 0;
+    if (l2 || allowed_dev) v = 0;
     void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, TcParams) =
         dump_dev ? (ares ? tc_gemm_kernel<true, 0, true, false, 16> : tc_gemm_kernel<true, 0, false, false, 16>)
         : wide ? (pair ? tc_gemm_kernel<false, 0, true, true, 32> : ares ? tc_gemm_kernel<false, 0, true, false, 32> : tc_gemm_kernel<false, 0, false, false, 32>)
@@ -1328,6 +1361,11 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
         : pair ? tc_gemm_kernel<false, 0, true, true, 16>
 #endif
         : (ares ? tc_gemm_kernel<false, 0, true, false, 16> : tc_gemm_kernel<false, 0, false, false, 16>);
+    if (allowed_dev)
+        k = wide ? (pair ? tc_gemm_kernel<false, 0, true, true, 32, false, true> : ares ? tc_gemm_kernel<false, 0, true, false, 32, false, true>
+                         : tc_gemm_kernel<false, 0, false, false, 32, false, true>)
+                 : (pair ? tc_gemm_kernel<false, 0, true, true, 16, false, true> : ares ? tc_gemm_kernel<false, 0, true, false, 16, false, true>
+                         : tc_gemm_kernel<false, 0, false, false, 16, false, true>);
     if (l2)
         k = wide ? (pair ? tc_gemm_kernel<false, 0, true, true, 32, true> : ares ? tc_gemm_kernel<false, 0, true, false, 32, true>
                          : tc_gemm_kernel<false, 0, false, false, 32, true>)
@@ -1359,7 +1397,7 @@ void asp_tc_batch_free(asp_ctx *ctx, asp_tc_batch *b)
 {
     cudaStream_t st = ctx->stream;
     void *ptrs[] = {b->q_hi, b->q_lo, b->lam_q32, b->inv_nq, b->rho_q, b->delta_q, b->qperm, b->center,
-                    b->emit_sc, b->emit_ix, b->emit_cnt, b->theta_glob};
+                    b->emit_sc, b->emit_ix, b->emit_cnt, b->theta_glob, b->vbits};
     for (void *ptr : ptrs)
         if (ptr) cudaFreeAsync(ptr, st);
     *b = asp_tc_batch();
@@ -1393,29 +1431,31 @@ __global__ void scatter_results_kernel(const int64_t *__restrict__ idx2, const d
 // three-term split (retry), and what is still undecided (exact ties around the k-th score) takes the exact scan.
 static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                              const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
-                             float *dump_dev, int force_terms, bool may_retry);
+                             float *dump_dev, int force_terms, bool may_retry, const uint32_t *allowed_dev);
 
-// dump == nullptr: full search.  dump != nullptr: approximate cosines [nq][n_local] f32 (tests).
+// dump == nullptr: full search.  dump != nullptr: approximate cosines [nq][n_local] f32 (tests).  allowed_dev: item mask
+// (local item order, packed) or nullptr.
 int asp_search_tc_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                        const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
-                       float *dump_dev)
+                       float *dump_dev, const uint32_t *allowed_dev)
 {
     const char *e = getenv("ASP_TC_FIRST_TERMS");                  // A/B knob: "auto" = the band rule decides (the earlier behaviour)
     int first = dump_dev ? 0 : (e && e[0] == 'a') ? 0 : 1;
     if (const char *t = getenv("ASP_TC_TERMS")) { const int v = atoi(t); if (v == 1 || v == 3) first = v; }   // test knob: that mode, no retry
     const bool pinned = getenv("ASP_TC_TERMS") != nullptr;
     return search_tc_attempt(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, out_idx_dev, out_score_dev, dump_dev, first,
-                             first == 1 && !pinned);
+                             first == 1 && !pinned, allowed_dev);
 }
 
 static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                              const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
-                             float *dump_dev, int force_terms, bool may_retry)
+                             float *dump_dev, int force_terms, bool may_retry, const uint32_t *allowed_dev)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
     asp_tc_batch b;
-    int rc = asp_tc_stage1(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, -INFINITY, force_terms, 0, dump_dev, &b);
+    int rc = asp_tc_stage1(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, -INFINITY, force_terms, 0, dump_dev, &b, false,
+                           allowed_dev);
     if (rc != ASP_OK || dump_dev) { asp_tc_batch_free(ctx, &b); return rc; }
 
     if (b.variant != 0) {                                         // profiling variants: stage 1 only, results are garbage
@@ -1483,7 +1523,7 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
         gather_queries_kernel<<<(unsigned)nslow, 128, 0, st>>>(q_dev, qpitch, lambda_q_dev, qnorm_dev, slow_list, nslow, q2, lam2, nrm2);
         ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
         asp_tc_batch_free(ctx, &b);                                   // the retry allocates its own emission buffers
-        rc = search_tc_attempt(s, q2, nslow, qpitch, lam2, nrm2, tau, topk, idx2, sc2, nullptr, 3, false);
+        rc = search_tc_attempt(s, q2, nslow, qpitch, lam2, nrm2, tau, topk, idx2, sc2, nullptr, 3, false, allowed_dev);
         if (rc == ASP_OK) {
             scatter_results_kernel<<<(unsigned)nslow, 32, 0, st>>>(idx2, sc2, slow_list, nslow, (int)topk, out_idx_dev, out_score_dev);
             ASP_LAUNCHED(ctx);
@@ -1496,7 +1536,8 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
         ctx->stats["search_slow_queries"] = retry_slow;              // what finally took the exact scan
         cudaFreeAsync(q2, st); cudaFreeAsync(lam2, st); cudaFreeAsync(nrm2, st); cudaFreeAsync(idx2, st); cudaFreeAsync(sc2, st);
     } else if (nslow > 0) {
-        rc = asp_search_slow_path(s, q_dev, qpitch, lambda_q_dev, qnorm_dev, tau, topk, slow_list, nslow, out_idx_dev, out_score_dev);
+        rc = asp_search_slow_path(s, q_dev, qpitch, lambda_q_dev, qnorm_dev, tau, topk, slow_list, nslow, out_idx_dev, out_score_dev,
+                                  allowed_dev);
     }
     cudaFreeAsync(slow_list, st); cudaFreeAsync(slow_count, st); cudaFreeAsync(counters, st);
     asp_tc_batch_free(ctx, &b);

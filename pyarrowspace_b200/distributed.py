@@ -44,6 +44,12 @@ def shard_rows(n_total, world, rank):
     return r0.value, r1.value
 
 
+def pack_allowed(allowed, row0, n_local):
+    """A rank's slice [row0, row0 + n_local) of the global bool mask `allowed`, packed LSB-first as the library takes it
+    (ceil(n_local / 8) bytes: bit i % 8 of byte i / 8 is local row i)."""
+    return np.packbits(np.ascontiguousarray(allowed[row0:row0 + n_local], dtype=np.bool_), bitorder="little")
+
+
 class CudaEngine:
     """The product engine: every method is one call into libarrowspace_b200.so."""
 
@@ -223,13 +229,19 @@ class CudaEngine:
     def hybrid_pool(self, n_total, topk, pool):
         return self.lib.asp_hybrid_pool(int(n_total), int(topk), int(pool))
 
-    def hybrid_shard(self, space, graph, q, tau, pool, idx, cos, score, lam):
+    def hybrid_shard(self, space, graph, q, tau, pool, idx, cos, score, lam, allowed=None):
         """asp_search_hybrid_shard of the host rows q into the device tensors idx / cos / score [rows, width] and lam [rows]
-        (cos is None when the shortlist is the whole set)."""
+        (cos is None when the shortlist is the whole set).  allowed: the global item mask (this shard's rows are used)."""
         self.torch.cuda.current_stream(self.device).synchronize()      # the outputs were filled on torch's stream
-        _lib.check(self.lib.asp_search_hybrid_shard(space, graph, q.ctypes.data, q.shape[0], float(tau), int(pool),
-                                                    idx.data_ptr(), None if cos is None else cos.data_ptr(),
-                                                    score.data_ptr(), lam.data_ptr()))
+        args = (space, graph, q.ctypes.data, q.shape[0], float(tau), int(pool), idx.data_ptr(),
+                None if cos is None else cos.data_ptr(), score.data_ptr(), lam.data_ptr())
+        if allowed is None:
+            _lib.check(self.lib.asp_search_hybrid_shard(*args))
+        else:
+            n_local, row0 = C.c_int64(), C.c_int64()
+            _lib.check(self.lib.asp_space_dims(space, C.byref(n_local), C.byref(C.c_int32()), C.byref(row0), C.byref(C.c_int64())))
+            bits = pack_allowed(allowed, row0.value, n_local.value)
+            _lib.check(self.lib.asp_search_hybrid_shard_filtered(*args, bits.ctypes.data))
 
     def hybrid_merge(self, idx, cos, score, m, topk):
         """[parts, nq, m] shortlists of the shards -> (idx, score) [nq, topk] device tensors (asp_hybrid_merge)."""
@@ -434,13 +446,15 @@ def regroup(engine, space, rows_dev, n_total, item_shards, group=None):
     return new_space, grid
 
 
-def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_total, grid):
+def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_total, grid, allowed=None):
     """Hybrid search (step 7) on an item-sharded grid (grid["R"] > 1), bit for bit the one-GPU search_hybrid_batch over all
     n_total items.  Called collectively with the same host batch `queries` [Q, F] on every rank.  Query slot c answers rows
     [a, b) of the batch: each of its R ranks computes its item shard's shortlist (engine.hybrid_shard), the R lists are
     all-gathered over the slot's merge group (R * m * 24 bytes per query) and merged on every one of them; the C slots then
     all-gather their finished slices, as the grid search does.  Returns (idx, score, lambda_q) host arrays of the whole
-    batch on every rank.  A failure on any rank raises the same LibraryError (same code) on every rank."""
+    batch on every rank.  A failure on any rank raises the same LibraryError (same code) on every rank.
+    allowed: the global bool item mask, the same on every rank (each shard filters its own rows; the merges take the
+    -1-padded lists as they are), or None."""
     import torch
     from ._lib import LibraryError
     r_, c_ = grid["R"], grid["C"]
@@ -459,8 +473,9 @@ def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_tota
     err = None
     if b > a:
         try:
+            extra = {} if allowed is None else {"allowed": allowed}
             engine.hybrid_shard(space, graph, queries[a:b], tau, pool, idx[:b - a], None if whole else cos[:b - a],
-                                score[:b - a], lam[:b - a])
+                                score[:b - a], lam[:b - a], **extra)
         except LibraryError as e:
             err = e
     status = torch.tensor([float(err.code) if err is not None else 0.0], dtype=torch.float64, device=dev)

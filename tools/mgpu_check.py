@@ -22,7 +22,17 @@ import torch.distributed as dist  # noqa: E402
 from pyarrowspace_b200 import shard_rows, synth  # noqa: E402
 from pyarrowspace_b200.api import ArrowSpaceBuilder  # noqa: E402
 
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+from test_filtered_search_cpu import want_hybrid, want_search  # noqa: E402  (the filtered searches by definition)
+
 HYBRID_POOLS = (None, 40)     # search_hybrid shortlists: the default (tensor-core candidates) and the batched exact scan
+
+
+def filter_mask(n):
+    """The allowed= mask of the filtered checks: half the items, and none of the last rank's rows, the same on every rank."""
+    mask = np.random.default_rng(n).random(n) < 0.5
+    mask[shard_rows(n, dist.get_world_size(), dist.get_world_size() - 1)[0]:] = False
+    return mask
 
 
 def all_ranks(flag):
@@ -63,6 +73,11 @@ def main():
             for pool in HYBRID_POOLS:                         # search_hybrid: one GPU and the oracle's restatement
                 ref["hyb1", pool] = a1.search_hybrid_batch(q, g1, 0.62, pool=pool)
                 ref["hybo", pool] = s.search_hybrid_batch(q[pick], g, 0.62, pool or 0)[:2]
+            fmask = filter_mask(n)                            # filtered search and hybrid: one GPU and the oracle
+            ref["filt1"] = a1.search_batch(q, g1, 0.62, allowed=fmask)
+            ref["filto"] = want_search(s, q[pick], s.search_batch(q[pick], g, 0.62)[2], 0.62, fmask, gp["topk"])
+            ref["fhyb1"] = a1.search_hybrid_batch(q, g1, 0.62, allowed=fmask)
+            ref["fhybo"] = want_hybrid(s, q[pick], s.search_hybrid_batch(q[pick], g, 0.62, 0)[2], 0.62, 0, fmask, gp["topk"])
             ar, gr = ArrowSpaceBuilder.build(gp, full, device=local, reduction=True)      # pre-graph reduction, one GPU
             ref.update(red_csr=gr.csr(), red_lam=ar.lambdas(), red_cent=gr.centroids(), red_info=gr.reduction)
             del a1, g1, s, g, full, ar, gr
@@ -114,6 +129,22 @@ def main():
                     print("world %d n %d f %d grid %d item shard(s) x %d query slot(s): search_hybrid pool %s == single GPU "
                           "(bitwise) %s, == oracle (%d queries) %s, same bits on every rank %s"
                           % (world, n, f, R, world // R, pool, e[0], len(ref["pick"]), e[1], e[2]), flush=True)
+                    ok = ok and all(e)
+            fmask = filter_mask(n)                            # collective, the same mask on every rank
+            checks = [("search", aspace.search_batch(q, gl, 0.62, allowed=fmask), "filt"),
+                      ("search_hybrid", aspace.search_hybrid_batch(q, gl, 0.62, allowed=fmask), "fhyb")]
+            for name, (fi, fs), key in checks:
+                fi, fs = (t.cpu().numpy() if torch.is_tensor(t) else t for t in (fi, fs))
+                if rank == 0:
+                    i1, s1 = ref[key + "1"]
+                    oi, os_ = ref[key + "o"]
+                    ok_o = oi >= 0
+                    e = [np.array_equal(fi, i1) and np.array_equal(fs, s1, equal_nan=True),
+                         np.array_equal(fi[ref["pick"]], oi) and bool(np.allclose(fs[ref["pick"]][ok_o], os_[ok_o], rtol=1e-9, atol=0)),
+                         bool(fmask[fi[fi >= 0]].all())]
+                    print("world %d n %d f %d grid %d item shard(s) x %d query slot(s): filtered %s == single GPU (bitwise) %s, "
+                          "== oracle (%d queries) %s, only allowed items %s" % (world, n, f, R, world // R, name, e[0],
+                                                                                len(ref["pick"]), e[1], e[2]), flush=True)
                     ok = ok and all(e)
             if os.environ.get("CHECK_PEER") and R == world and world > 1:    # csrc/peer.cu: P2P exchange + flag-driven merge
                 os.environ["ASP_PEER_MERGE"] = "1"
