@@ -46,7 +46,8 @@ enum {
     ASP_ERR_NOMEM = 5,
     ASP_ERR_CUDA = 6,         /* no device / CUDA failure: there is no CPU fallback */
     ASP_ERR_UNSUPPORTED = 7,
-    ASP_NEED_EXACT = 8        /* asp_graph_from_gram: decisions inside the rounding band, see below */
+    ASP_NEED_EXACT = 8,       /* asp_graph_from_gram: decisions inside the rounding band, see below */
+    ASP_ERR_LIMIT = 9         /* asp_search_range_batch: more hits than max_hits */
 };
 
 /* (eps, k, topk, p, sigma) as parsed by parse_graph_params, src/helpers.rs:48-77.
@@ -85,6 +86,7 @@ typedef struct {
 typedef struct asp_ctx   asp_ctx;    /* device, streams, scratch */
 typedef struct asp_space asp_space;  /* replaces arrowspace::core::ArrowSpace   (src/lib.rs:64-67)  */
 typedef struct asp_graph asp_graph;  /* replaces arrowspace::graph::GraphLaplacian (src/lib.rs:26-29) */
+typedef struct asp_range_result asp_range_result;   /* hits of asp_search_range_batch, in device memory */
 
 const char *asp_last_error(void);
 int  asp_abi_version(void);
@@ -265,6 +267,31 @@ int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, con
                                      const uint8_t *allowed_bits);
 int asp_hybrid_merge(asp_ctx *ctx, const int64_t *idx, const double *cos, const double *score, int parts, int64_t nq,
                      int64_t m, int64_t topk, int64_t *out_idx, double *out_score);
+
+/* Range search (no reference counterpart): per query EVERY item with score >= min_score, ordered by (score desc, index asc),
+ * GLOBAL indices, the oracle-order scores bit for bit (score and lambda_q as in asp_search_batch, including the
+ * lambda_q != 0 assertion and the zero-vector check).  min_score is inclusive and compared in f64 against the reference-order
+ * value; -inf returns every item, > 1 returns empty rows, NaN is ASP_ERR_ARG.  allowed_bits as in asp_search_batch_filtered
+ * (NULL = all).  out_counts[nq] (host or device) receives the per-query hit counts; the hits stay in device memory owned by
+ * *out until asp_range_result_fetch copies them out (sum(counts) entries, query-major; host or device) and
+ * asp_range_result_free releases them.  max_hits > 0: when the running total of the call exceeds it the call fails with
+ * ASP_ERR_LIMIT, naming the total and the query at which it was crossed; batches are processed in sub-batches of
+ * asp_range_sub_batch() queries and the cap is checked on each sub-batch's counts before its hits get device memory.
+ * Candidates: the tcgen05 pass of the search with topk = 0 and min_score (clamped to [-2, 2]) as its emission floor, for
+ * 0.001 < tau <= 1 and <= 6144 features; queries whose emission buffers overflow, and every query outside those bounds, take
+ * the exact range scan (env ASP_RANGE_STAGE1=scan forces it: a test knob, the same bits).  [exchange]: a row shard passes
+ * its slice of the mask; the per-shard results merge with asp_range_merge. */
+int  asp_search_range_batch(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
+                            double min_score, const uint8_t *allowed_bits, int64_t max_hits, int64_t *out_counts,
+                            double *out_lambda_q, asp_range_result **out);
+int  asp_range_result_fetch(const asp_range_result *r, int64_t *out_idx, double *out_score);
+void asp_range_result_free(asp_range_result *r);
+int64_t asp_range_sub_batch(void);
+/* Merge of per-shard range results over the same nq queries into the one-GPU order: counts [parts][nq] and the concatenated
+ * parts' hits (each part query-major, each query's hits sorted) -> sum(counts) hits query-major.  Shards must be contiguous
+ * global row ranges (then ties resolve as on one GPU, whatever the number or order of the shards).  Host or device pointers. */
+int  asp_range_merge(asp_ctx *ctx, int parts, int64_t nq, const int64_t *counts, const int64_t *idx, const double *score,
+                     int64_t *out_idx, double *out_score);
 
 /* Test hook of the tcgen05 candidate pass: the approximate cosines (unit-scaled operands, bf16 two-term split,
  * f32 accumulation in TMEM) of nq queries against every item of the shard, out[nq][n_local] f32 (host or device). */

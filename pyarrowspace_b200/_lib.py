@@ -19,6 +19,7 @@ ASP_ERR_NOMEM = 5
 ASP_ERR_CUDA = 6
 ASP_ERR_UNSUPPORTED = 7
 ASP_NEED_EXACT = 8
+ASP_ERR_LIMIT = 9
 
 GRAM_SEGMENTS = 8
 GRAM_SLICES = 24
@@ -119,6 +120,11 @@ SYMBOLS = {
     "asp_search_batch_filtered": (_int, [_vp, _vp, _vp, _i64, _dbl, _vp, _vp, _vp, _vp]),
     "asp_search_hybrid_batch_filtered": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _vp, _vp, _vp, _vp]),
     "asp_search_hybrid_shard_filtered": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "asp_search_range_batch": (_int, [_vp, _vp, _vp, _i64, _dbl, _dbl, _vp, _i64, _vp, _vp, C.POINTER(_vp)]),
+    "asp_range_result_fetch": (_int, [_vp, _vp, _vp]),
+    "asp_range_result_free": (None, [_vp]),
+    "asp_range_sub_batch": (_i64, []),
+    "asp_range_merge": (_int, [_vp, _int, _i64, _vp, _vp, _vp, _vp, _vp]),
     "asp_debug_tc_dots": (_int, [_vp, _vp, _i64, _vp]),
     "asp_topk_merge": (_int, [_vp, _vp, _vp, _int, _i64, _i64, _vp, _vp]),
     "asp_peer_exchange_bytes": (C.c_size_t, [_int, _i64, _i64]),

@@ -9,7 +9,8 @@ names, argument order / keyword names, return shapes and error behaviour.
     GraphLaplacian.nnodes / shape() / graph_params                                 src/lib.rs:40-61
     set_debug(enabled)                                                             src/helpers.rs:12-21
 
-Extensions (not in the reference): ``ArrowSpace.search_batch``, ``ArrowSpaceBuilder.build_sharded``
+Extensions (not in the reference): ``ArrowSpace.search_batch``, ``ArrowSpace.search_range`` /
+``search_range_batch`` (every item at or above a score threshold), ``ArrowSpaceBuilder.build_sharded``
 and device-tensor inputs (anything exposing ``data_ptr()``), used by bench.py.
 
 Every numeric step runs in libarrowspace_b200.so (hand-written sm_100a CUDA).  There is no CPU
@@ -72,6 +73,43 @@ def _check_allowed(allowed, nitems):
     if allowed.ndim != 1 or allowed.shape[0] != nitems:
         raise ValueError("allowed must be 1-D with one entry per item (%d), got shape %s" % (nitems, allowed.shape))
     return allowed
+
+
+# Default cap of a range search: 2**26 hits, 1 GiB of results (int64 index + f64 score) -- a threshold far below the
+# scores of a data set would otherwise ask for every item of every query.  max_results= raises or lowers it.
+DEFAULT_MAX_RESULTS = 1 << 26
+
+
+def _check_min_score(min_score):
+    """min_score of a range search: a real number (inclusive, compared in f64; -inf = every item); NaN is refused."""
+    if isinstance(min_score, bool) or not isinstance(min_score, (int, float, np.integer, np.floating)):
+        raise TypeError("min_score must be a real number (got %s)" % type(min_score).__name__)
+    v = float(min_score)
+    if v != v:
+        raise ValueError("min_score must not be NaN")
+    return v
+
+
+def _check_max_results(max_results):
+    if max_results is None:
+        return DEFAULT_MAX_RESULTS
+    if isinstance(max_results, bool) or not isinstance(max_results, (int, np.integer)):
+        raise TypeError("max_results must be an integer (got %s)" % type(max_results).__name__)
+    if max_results < 1:
+        raise ValueError("max_results must be at least 1 (got %d)" % max_results)
+    return int(max_results)
+
+
+def _range_error(e):
+    """What a failed range search raises: the search's panics, ValueError for the result cap, else the LibraryError."""
+    if e.code == _lib.ASP_ERR_LAMBDA_ZERO:
+        return PanicException("assertion `left != right` failed: The lambdas are zero, check the magnitude of items and eps.\n"
+                              "  left: 0.0\n right: 0.0")
+    if e.code == _lib.ASP_ERR_ZERO_VECTOR:
+        return PanicException(e.message)
+    if e.code == _lib.ASP_ERR_LIMIT:
+        return ValueError(e.message)
+    return e
 
 
 def parse_graph_params(graph_params):
@@ -479,6 +517,101 @@ class ArrowSpace:
             return (_to_host(idx, host_out and host_out[0]), _to_host(score, host_out and host_out[1]),
                     _to_host(lam.contiguous(), host_out and host_out[2]))
         return idx, score, lam.contiguous()
+
+    # ------------------------------------------------------------------ range search (extension)
+    def search_range(self, item, gl, tau, min_score):
+        """list[(index, score)] of EVERY item with score >= min_score, best first (score desc, index asc).  Same argument
+        checks, lambda_q and panics as `search`; a filtered single query is search_range_batch(item.reshape(1, -1), ...)."""
+        if not isinstance(gl, GraphLaplacian):
+            raise TypeError("argument 'gl': 'GraphLaplacian' object expected")
+        if not isinstance(item, np.ndarray) or item.dtype != np.float64 or item.ndim != 1:
+            raise TypeError("argument 'item': expected 1-D numpy.ndarray of float64")
+        if not item.flags.c_contiguous:
+            raise ValueError("The given array is not contiguous")
+        if item.shape[0] != self.nfeatures:
+            raise ValueError("query length %d must match nfeatures %d" % (item.shape[0], self.nfeatures))
+        indptr, idx, score = self.search_range_batch(item.reshape(1, -1), gl, tau, min_score)
+        return [(int(i), float(s)) for i, s in zip(idx, score)]
+
+    def search_range_batch(self, queries, gl, tau, min_score, *, allowed=None, max_results=None):
+        """Range search: per query every item whose score (the search's, evaluated in the reference order) is >= min_score,
+        ordered by (score desc, index asc).  Returns CSR (indptr int64[Q + 1], idx int64[nnz], score f64[nnz]): the hits of
+        query q are idx[indptr[q]:indptr[q + 1]].  Host batches return numpy arrays, device batches device tensors.
+        min_score: inclusive, compared in f64; -inf returns every item, > 1 empty rows, NaN raises ValueError.
+        allowed = numpy bool[nitems]: only allowed items are hits (collective calls: the same mask on every rank).
+        max_results: the cap on the total number of hits of the call (default DEFAULT_MAX_RESULTS = 2**26, 1 GiB of
+        results); more raises ValueError stating the count.  lambda_q == 0 and zero vectors panic as in `search`.
+        Row-sharded spaces (build_sharded) are called collectively and every rank returns the whole batch."""
+        if not isinstance(gl, GraphLaplacian):
+            raise TypeError("argument 'gl': 'GraphLaplacian' object expected")
+        min_score = _check_min_score(min_score)
+        max_hits = _check_max_results(max_results)
+        tau = float(tau)
+        n_local, f, _, n_total = self._dims()
+        allowed = _check_allowed(allowed, n_total)
+        device_in = _is_device_tensor(queries)
+        if device_in:
+            import torch
+            if queries.dim() != 2 or queries.shape[1] != f:
+                raise ValueError("query length %d must match nfeatures %d" % (queries.shape[-1], f))
+            if queries.dtype != torch.float64:
+                raise TypeError("queries must be float64")
+        else:
+            queries = np.ascontiguousarray(queries, dtype=np.float64)
+            if queries.ndim != 2 or queries.shape[1] != f:
+                raise ValueError("query length %d must match nfeatures %d" % (queries.shape[-1], f))
+        if self._grid is not None:
+            from .distributed import CudaEngine, sharded_search_range
+            engine = CudaEngine(_lib.load().asp_ctx_device(self._ctx))
+            q_host = queries.cpu().numpy() if device_in else queries
+            try:
+                indptr, idx, score, _ = sharded_search_range(engine, self._h, gl._h, q_host, tau, min_score, n_total, self._grid,
+                                                             allowed=allowed, max_hits=max_hits)
+            except LibraryError as e:
+                raise _range_error(e)
+            if device_in:
+                import torch
+                return tuple(torch.from_numpy(a).to(queries.device) for a in (indptr, idx, score))
+            return indptr, idx, score
+        if n_local != n_total:
+            raise NotImplementedError("search_range on a row shard needs the search grid of build_sharded")
+        return self._search_range_local(queries, gl, tau, min_score, allowed, max_hits, device_in)
+
+    def _search_range_local(self, queries, gl, tau, min_score, allowed, max_hits, device_in):
+        lib = _lib.load()
+        nq = queries.shape[0]
+        counts = np.empty(nq, dtype=np.int64)
+        lam = np.empty(nq, dtype=np.float64)
+        if device_in:
+            import torch
+            q = queries.contiguous()
+            qp = q.data_ptr()
+            torch.cuda.current_stream(q.device).synchronize()      # the library runs on its own stream
+        else:
+            qp = queries.ctypes.data
+        bits = self._allowed_bits(allowed)
+        h = C.c_void_p()
+        try:
+            _lib.check(lib.asp_search_range_batch(self._h, gl._h, qp, nq, tau, min_score, None if bits is None else bits.ctypes.data,
+                                                  max_hits, counts.ctypes.data, lam.ctypes.data, C.byref(h)))
+        except LibraryError as e:
+            raise _range_error(e)
+        try:
+            indptr = np.zeros(nq + 1, dtype=np.int64)
+            np.cumsum(counts, out=indptr[1:])
+            nnz = int(indptr[-1])
+            if device_in:
+                import torch
+                idx = torch.empty(nnz, dtype=torch.int64, device=q.device)
+                score = torch.empty(nnz, dtype=torch.float64, device=q.device)
+                _lib.check(lib.asp_range_result_fetch(h, idx.data_ptr(), score.data_ptr()))
+                return torch.from_numpy(indptr).to(q.device), idx, score
+            idx = np.empty(nnz, dtype=np.int64)
+            score = np.empty(nnz, dtype=np.float64)
+            _lib.check(lib.asp_range_result_fetch(h, idx.ctypes.data, score.ctypes.data))
+            return indptr, idx, score
+        finally:
+            lib.asp_range_result_free(h)
 
     # ------------------------------------------------------------------ persistence (extension, SURVEY.md 8(f)-4)
     def save(self, path, gl, items=None):

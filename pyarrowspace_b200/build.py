@@ -14,7 +14,7 @@ OBJ = os.path.join(HERE, "_obj")
 LIB = os.path.join(HERE, "libarrowspace_b200.so")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 
-SOURCES = ["api.cu", "tensormap.cu", "gram.cu", "graph_select.cu", "csr.cu", "taumode.cu", "search.cu", "search_tc.cu", "knn.cu", "peer.cu", "reduce.cu"]
+SOURCES = ["api.cu", "tensormap.cu", "gram.cu", "graph_select.cu", "csr.cu", "taumode.cu", "search.cu", "search_tc.cu", "knn.cu", "peer.cu", "reduce.cu", "range.cu"]
 FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O2", "-ccbin", "/usr/bin/g++",

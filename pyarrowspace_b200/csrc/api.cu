@@ -1,10 +1,11 @@
 // api.cu -- the C ABI declared in include/arrowspace_b200.h (extern "C", plain pointers).
 // Host-side orchestration only; every numeric step is a kernel in gram.cu / graph_select.cu /
-// csr.cu / taumode.cu / search.cu / knn.cu.  There is no CPU fallback anywhere in this file.
+// csr.cu / taumode.cu / search.cu / knn.cu / range.cu.  There is no CPU fallback anywhere in this file.
 #include "common.cuh"
 #include "hybrid.cuh"
 
 #include <algorithm>
+#include <cmath>
 #include <math.h>
 #include <stdarg.h>
 #include <stdlib.h>
@@ -1201,6 +1202,113 @@ int asp_topk_merge(asp_ctx *ctx, const int64_t *idx, const double *score, int pa
     cudaFreeAsync(d_oidx, st);
     cudaFreeAsync(d_osc, st);
     return rc;
+}
+
+// ------------------------------------------------------------------ range search (csrc/range.cu)
+int asp_search_range_batch(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, double min_score,
+                           const uint8_t *allowed_bits, int64_t max_hits, int64_t *out_counts, double *out_lambda_q,
+                           asp_range_result **out)
+{
+    if (!s || !g || !out || nq < 0 || (nq > 0 && (!queries || !out_counts))) ASP_FAIL(ASP_ERR_ARG, "asp_search_range_batch: NULL argument");
+    *out = nullptr;
+    if (!s->have_lambdas) ASP_FAIL(ASP_ERR_ARG, "asp_search_range_batch: item lambdas have not been computed");
+    if (g->nnodes != s->f) ASP_FAIL(ASP_ERR_ARG, "graph has %lld nodes but items have %d features", (long long)g->nnodes, s->f);
+    if (std::isnan(min_score)) ASP_FAIL(ASP_ERR_ARG, "asp_search_range_batch: min_score is NaN");
+    if (std::isnan(tau)) ASP_FAIL(ASP_ERR_ARG, "asp_search_range_batch: tau is NaN");
+    asp_ctx *ctx = s->ctx;
+    ASP_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    asp_range_result *res = new asp_range_result();
+    res->ctx = ctx;
+    ctx->stats["search_slow_queries"] = 0.0;
+    ctx->stats["range_stage1_ms"] = 0.0;
+    ctx->stats["range_stage2_ms"] = 0.0;
+    const int32_t f = s->f, fp = s->fp;
+    const int64_t sub = std::min<int64_t>(std::max<int64_t>(nq, 1), asp_range_sub_batch());
+    std::vector<int64_t> h_counts((size_t)nq);
+    HybridScratch scratch{st, {}};
+    double *dq = nullptr, *dlam = nullptr, *dnorm = nullptr;
+    int *flags = nullptr;
+    uint32_t *dallowed = nullptr;
+    int rc = scratch.get(&dq, (size_t)sub * fp);
+    if (rc == ASP_OK) rc = scratch.get(&dlam, (size_t)sub);
+    if (rc == ASP_OK) rc = scratch.get(&dnorm, (size_t)sub);
+    if (rc == ASP_OK) rc = scratch.get(&flags, 2);
+    if (rc == ASP_OK) rc = upload_allowed(st, allowed_bits, s->n_local, &dallowed);   // once per call
+    for (int64_t q0 = 0; q0 < nq && rc == ASP_OK; q0 += sub) {
+        const int64_t qn = std::min(sub, nq - q0);
+        rc = upload_pitched(st, queries + q0 * f, qn, f, fp, dq);
+        // lambda_q, the zero-vector check and the lambda_q != 0 assertion of the search (topk = 0: no search)
+        if (rc == ASP_OK) rc = search_device_batch(s, g, dq, qn, tau, 0, dlam, dnorm, flags, nullptr, nullptr, true, nullptr);
+        asp_range_result::Piece p;
+        if (rc == ASP_OK)
+            rc = asp_range_impl(s, dq, qn, fp, dlam, dnorm, tau, min_score, dallowed, max_hits, res->total, q0, h_counts.data() + q0,
+                                &p.idx, &p.score, &p.n);
+        if (p.n > 0) { res->pieces.push_back(p); res->total += p.n; }
+        if (rc == ASP_OK && out_lambda_q) rc = asp_copy_out(ctx, out_lambda_q + q0, dlam, sizeof(double) * qn);
+    }
+    if (dallowed) cudaFreeAsync(dallowed, st);
+    if (rc == ASP_OK && nq > 0) rc = asp_copy_out(ctx, out_counts, h_counts.data(), sizeof(int64_t) * nq);
+    if (rc == ASP_OK && cudaStreamSynchronize(st) != cudaSuccess) { asp_set_error("range search: stream failed"); rc = ASP_ERR_CUDA; }
+    if (rc != ASP_OK) { asp_range_result_free(res); return rc; }
+    *out = res;
+    return ASP_OK;
+}
+
+int asp_range_result_fetch(const asp_range_result *r, int64_t *out_idx, double *out_score)
+{
+    if (!r || (r->total > 0 && (!out_idx || !out_score))) ASP_FAIL(ASP_ERR_ARG, "asp_range_result_fetch: NULL argument");
+    asp_ctx *ctx = r->ctx;
+    ASP_CUDA(cudaSetDevice(ctx->device));
+    int64_t o = 0;
+    for (const auto &p : r->pieces) {
+        ASP_CHECK(asp_copy_out(ctx, out_idx + o, p.idx, sizeof(int64_t) * p.n));
+        ASP_CHECK(asp_copy_out(ctx, out_score + o, p.score, sizeof(double) * p.n));
+        o += p.n;
+    }
+    ASP_CUDA(cudaStreamSynchronize(ctx->stream));
+    return ASP_OK;
+}
+
+void asp_range_result_free(asp_range_result *r)
+{
+    if (!r) return;
+    cudaSetDevice(r->ctx->device);
+    for (auto &p : r->pieces) { cudaFreeAsync(p.idx, r->ctx->stream); cudaFreeAsync(p.score, r->ctx->stream); }
+    delete r;
+}
+
+int asp_range_merge(asp_ctx *ctx, int parts, int64_t nq, const int64_t *counts, const int64_t *idx, const double *score,
+                    int64_t *out_idx, double *out_score)
+{
+    if (!ctx || parts <= 0 || nq < 0 || (nq > 0 && !counts)) ASP_FAIL(ASP_ERR_ARG, "asp_range_merge: bad argument");
+    if (nq == 0) return ASP_OK;
+    ASP_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    std::vector<int64_t> h_counts((size_t)parts * nq);
+    ASP_CUDA(cudaMemcpyAsync(h_counts.data(), counts, sizeof(int64_t) * h_counts.size(), cudaMemcpyDefault, st));
+    ASP_CUDA(cudaStreamSynchronize(st));
+    int64_t total = 0;
+    for (int64_t c : h_counts) {
+        if (c < 0) ASP_FAIL(ASP_ERR_ARG, "asp_range_merge: negative count");
+        total += c;
+    }
+    if (total == 0) return ASP_OK;
+    if (!idx || !score || !out_idx || !out_score) ASP_FAIL(ASP_ERR_ARG, "asp_range_merge: NULL argument");
+    HybridScratch scratch{st, {}};
+    int64_t *d_idx = nullptr, *d_oidx = nullptr;
+    double *d_sc = nullptr, *d_osc = nullptr;
+    ASP_CHECK(scratch.get(&d_idx, (size_t)total));
+    ASP_CHECK(scratch.get(&d_sc, (size_t)total));
+    ASP_CHECK(scratch.get(&d_oidx, (size_t)total));
+    ASP_CHECK(scratch.get(&d_osc, (size_t)total));
+    ASP_CUDA(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * total, cudaMemcpyDefault, st));
+    ASP_CUDA(cudaMemcpyAsync(d_sc, score, sizeof(double) * total, cudaMemcpyDefault, st));
+    ASP_CHECK(asp_range_merge_impl(ctx, parts, nq, h_counts.data(), d_idx, d_sc, d_oidx, d_osc));
+    ASP_CHECK(asp_copy_out(ctx, out_idx, d_oidx, sizeof(int64_t) * total));
+    ASP_CHECK(asp_copy_out(ctx, out_score, d_osc, sizeof(double) * total));
+    ASP_CUDA(cudaStreamSynchronize(st));
+    return ASP_OK;
 }
 
 // Persistence: a graph handle from a stored Laplacian (what asp_graph_csr exported).  feature_graph != 0 also prepares the

@@ -86,6 +86,14 @@ struct asp_graph {
     void *tm_blob = nullptr;
 };
 
+// hits of asp_search_range_batch: one device piece per sub-batch (query-major, concatenated in query order)
+struct asp_range_result {
+    asp_ctx *ctx = nullptr;
+    int64_t total = 0;
+    struct Piece { int64_t *idx = nullptr; double *score = nullptr; int64_t n = 0; };
+    std::vector<Piece> pieces;
+};
+
 // host wall clock in microseconds (diagnostic stats "search_host_*_us": where a call's time goes between the kernels)
 #include <chrono>
 static inline double asp_now_us()
@@ -187,6 +195,13 @@ int asp_search_slow_path(const asp_space *s, const double *q_dev, int32_t qpitch
                          int64_t *out_idx_dev, double *out_score_dev, const uint32_t *allowed_dev = nullptr);
 int asp_make_f16_tmap(CUtensorMap *out, const void *base, int64_t rows, int32_t kp, int box_rows);
 int asp_make_f16_tmap_narrow(CUtensorMap *out, const void *base, int64_t rows, int32_t kp, int box_rows, int nw);
+
+// range.cu (range search after the tcgen05 candidate pass)
+int asp_range_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lam_dev, const double *norm_dev,
+                   double tau, double min_score, const uint32_t *allowed_dev, int64_t max_hits, int64_t hits_before, int64_t q_base,
+                   int64_t *h_counts, int64_t **out_idx, double **out_score, int64_t *out_nnz);
+int asp_range_merge_impl(asp_ctx *ctx, int parts, int64_t nq, const int64_t *h_counts, const int64_t *idx_dev,
+                         const double *score_dev, int64_t *out_idx_dev, double *out_score_dev);
 
 // knn.cu
 // distance: ASP_DISTANCE_COSINE | L2 | L2SQ

@@ -19,6 +19,9 @@ The path shards by rows (SURVEY.md section 8(e)): rank r owns the rows of Gram s
   hybrid search (R > 1; `sharded_search_hybrid`)
           7. all-gather of the per-shard cosine shortlists (idx, cosine, score: 24 * Q * m bytes per rank) among the R ranks
              of a query slot + merge kernel; the C slots all-gather their finished slices
+  range search (`sharded_search_range`)
+          8. all-gather of the per-shard hit counts (8 bytes per query), then of the ragged hits (16 bytes each) among the R
+             ranks of a query slot + merge kernel; the C slots all-gather their counts and finished slices
 
 The summation tree of the Gram is fixed (segments -> slices), so every world size produces
 bit-identical graphs, lambdas and result lists.
@@ -267,6 +270,46 @@ class CudaEngine:
                                            out_sc.data_ptr()))
         return out_idx, out_sc
 
+    # ---- range search
+    def range_shard(self, space, graph, q, tau, min_score, allowed=None, max_hits=0):
+        """asp_search_range_batch of the host rows q on this rank's item shard -> (idx, score) device tensors of the hits
+        (GLOBAL indices, query-major, each query sorted), counts [rows] and lambda_q [rows] as host arrays."""
+        t = self.torch
+        nq = q.shape[0]
+        counts = np.empty(nq, dtype=np.int64)
+        lam = np.empty(nq, dtype=np.float64)
+        bits = None
+        if allowed is not None:
+            n_local, row0 = C.c_int64(), C.c_int64()
+            _lib.check(self.lib.asp_space_dims(space, C.byref(n_local), C.byref(C.c_int32()), C.byref(row0), C.byref(C.c_int64())))
+            bits = pack_allowed(allowed, row0.value, n_local.value)
+        h = C.c_void_p()
+        _lib.check(self.lib.asp_search_range_batch(space, graph, q.ctypes.data, nq, float(tau), float(min_score),
+                                                   None if bits is None else bits.ctypes.data, int(max_hits), counts.ctypes.data,
+                                                   lam.ctypes.data, C.byref(h)))
+        try:
+            nnz = int(counts.sum())
+            idx = t.empty(nnz, dtype=t.int64, device=self.device)
+            score = t.empty(nnz, dtype=t.float64, device=self.device)
+            _lib.check(self.lib.asp_range_result_fetch(h, idx.data_ptr(), score.data_ptr()))
+        finally:
+            self.lib.asp_range_result_free(h)
+        return idx, score, counts, lam
+
+    def range_merge(self, counts, idx, score):
+        """counts [parts, nq] (host), the parts' hits concatenated (device tensors) -> the merged hits (asp_range_merge)."""
+        t = self.torch
+        counts = np.ascontiguousarray(counts, dtype=np.int64)
+        parts, nq = counts.shape
+        total = int(counts.sum())
+        out_idx = t.empty(total, dtype=t.int64, device=self.device)
+        out_sc = t.empty(total, dtype=t.float64, device=self.device)
+        idx, score = idx.contiguous(), score.contiguous()
+        t.cuda.current_stream(self.device).synchronize()
+        _lib.check(self.lib.asp_range_merge(self.ctx, parts, nq, counts.ctypes.data, idx.data_ptr(), score.data_ptr(),
+                                            out_idx.data_ptr(), out_sc.data_ptr()))
+        return out_idx, out_sc
+
     def to_comm(self, arr):
         return self.torch.from_numpy(arr).to(self.device)
 
@@ -505,6 +548,94 @@ def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_tota
         raise LibraryError(codes[0], msg)
     return (out_idx[:nq].cpu().numpy(), out_sc[:nq].cpu().numpy(),
             np.ascontiguousarray(lam[:, :per].reshape(-1)[:nq].numpy()))
+
+
+def _limit_message(total, query, max_hits):
+    """The text of ASP_ERR_LIMIT, as asp_search_range_batch words it."""
+    return "range search: %d hits reached at query %d, more than max_hits = %d" % (total, query, max_hits)
+
+
+def sharded_search_range(engine, space, graph, queries, tau, min_score, n_total, grid, allowed=None, max_hits=1 << 26):
+    """Range search (step 8) on the search grid of build_sharded, bit for bit the one-GPU search_range_batch over all n_total
+    items.  Called collectively with the same host batch `queries` [Q, F] on every rank.  Query slot c answers rows [a, b):
+    each of its R ranks runs its item shard (engine.range_shard); the slot's merge group all-gathers the per-query counts,
+    then the ragged hits, and engine.range_merge orders them; the C slots all-gather their counts and finished slices.
+    Every rank returns (indptr, idx, score, lambda_q) host arrays of the whole batch.  A failure on any rank -- the result
+    cap (max_hits > 0: ASP_ERR_LIMIT, checked on every rank against the merged counts) and the panics included -- raises
+    the same LibraryError code on every rank.  allowed: the global bool item mask, the same on every rank, or None."""
+    import torch
+    from ._lib import ASP_ERR_LIMIT, LibraryError
+    r_, c_ = grid["R"], grid["C"]
+    nq = queries.shape[0]
+    a, b, per = query_slice(nq, c_, grid["c"])
+    dev = engine.device
+    counts = torch.zeros(per + 1, dtype=torch.int64)       # the last element carries this rank's status
+    lam = torch.full((per,), float("nan"), dtype=torch.float64)
+    idx = torch.empty(0, dtype=torch.int64, device=dev)
+    score = torch.empty(0, dtype=torch.float64, device=dev)
+    err = None
+    if b > a:
+        try:
+            idx, score, cnt, lq = engine.range_shard(space, graph, queries[a:b], tau, min_score, allowed, max_hits)
+            counts[:b - a] = torch.from_numpy(np.asarray(cnt, dtype=np.int64))
+            lam[:b - a] = torch.from_numpy(np.asarray(lq, dtype=np.float64))
+        except LibraryError as e:
+            err = e
+            counts[per] = e.code
+    # counts and statuses first: every rank learns every failure and every count before any hit moves
+    shard_counts = counts.to(dev)
+    if r_ > 1:
+        shard_counts = _all_gather_blocks(shard_counts, r_, grid["merge_group"])
+    else:
+        shard_counts = shard_counts.reshape(1, per + 1)
+    if hasattr(engine, "after_collective"):
+        engine.after_collective()
+    shard_counts = shard_counts.cpu()
+    slot = torch.zeros(per + 1, dtype=torch.float64)
+    slot[:per] = shard_counts[:, :per].sum(dim=0).to(torch.float64)
+    bad = [int(v) for v in shard_counts[:, per].tolist() if v != 0]
+    slot[per] = bad[0] if bad else 0
+    slot_lam = torch.cat([slot, lam])                       # [per + 1 counts / status | per lambda_q]
+    if c_ > 1:
+        all_slots = _all_gather_blocks(slot_lam.to(dev), c_, grid["item_group"])
+        if hasattr(engine, "after_collective"):
+            engine.after_collective()
+        all_slots = all_slots.cpu()
+    else:
+        all_slots = slot_lam.reshape(1, -1)
+    codes = [int(v) for v in all_slots[:, per].tolist() if v != 0]
+    if codes:
+        code = codes[0]
+        if err is not None and err.code == code:
+            raise LibraryError(code, err.message)
+        msg = ("range search: more than max_hits = %d hits" % max_hits) if code == ASP_ERR_LIMIT else \
+            "a rank of the query grid failed with error %d" % code
+        raise LibraryError(code, msg)
+    q_counts = all_slots[:, :per].reshape(-1)[:nq].to(torch.int64).numpy()
+    lam_all = np.ascontiguousarray(all_slots[:, per + 1:].reshape(-1)[:nq].numpy())
+    indptr = np.zeros(nq + 1, dtype=np.int64)
+    np.cumsum(q_counts, out=indptr[1:])
+    if max_hits > 0 and indptr[-1] > max_hits:                # the merged total: the same decision on every rank
+        qi = int(np.searchsorted(indptr[1:], max_hits, side="right"))
+        raise LibraryError(ASP_ERR_LIMIT, _limit_message(int(indptr[qi + 1]), qi, max_hits))
+    # the slot's hits: ragged all-gather over its R ranks, merged into the one-GPU order
+    if r_ > 1:
+        per_rank = [int(v) for v in shard_counts[:, :per].sum(dim=1).tolist()]
+        if sum(per_rank) > 0:
+            g_idx = _all_gather_ragged(idx, per_rank, grid["merge_group"])
+            g_sc = _all_gather_ragged(score, per_rank, grid["merge_group"])
+            if hasattr(engine, "after_collective"):
+                engine.after_collective()
+            idx, score = engine.range_merge(shard_counts[:, :per].numpy(), g_idx, g_sc)
+    # the C slots' finished slices
+    if c_ > 1:
+        per_slot = [int(v) for v in all_slots[:, :per].sum(dim=1).tolist()]
+        if sum(per_slot) > 0:
+            idx = _all_gather_ragged(idx, per_slot, grid["item_group"])
+            score = _all_gather_ragged(score, per_slot, grid["item_group"])
+            if hasattr(engine, "after_collective"):
+                engine.after_collective()
+    return indptr, idx.cpu().numpy(), score.cpu().numpy(), lam_all
 
 
 def _all_gather_ragged(t_local, counts, group):

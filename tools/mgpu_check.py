@@ -1,7 +1,8 @@
 """torchrun --nproc-per-node N tools/mgpu_check.py : multi-GPU build + search over NCCL against the CPU oracle and against
 the single-GPU result (bit identical), for EVERY layout of the search grid (R item shards x N / R query slots: R = N fully
 item-sharded ... R = 1 items replicated), with host and with device-resident query batches, and search_hybrid (host
-batches, default shortlist and pool 40) against the single-GPU result (bit identical) and the oracle.
+batches, default shortlist and pool 40) against the single-GPU result (bit identical) and the oracle, and search_range_batch
+(with and without a mask) against the single-GPU result (bit identical) and the definition over the oracle.
 
     BIG=1      adds the 1M x 384 case (BASELINE.json C4 shape; oracle check on a 96-query sample)
     CHECK_PEER=1 also runs the peer-memory merge (csrc/peer.cu) on the fully item-sharded layout
@@ -24,6 +25,7 @@ from pyarrowspace_b200.api import ArrowSpaceBuilder  # noqa: E402
 
 sys.path.insert(0, os.path.join(ROOT, "tests"))
 from test_filtered_search_cpu import want_hybrid, want_search  # noqa: E402  (the filtered searches by definition)
+from test_range_search_cpu import want_range  # noqa: E402  (the range search by definition)
 
 HYBRID_POOLS = (None, 40)     # search_hybrid shortlists: the default (tensor-core candidates) and the batched exact scan
 
@@ -78,6 +80,12 @@ def main():
             ref["filto"] = want_search(s, q[pick], s.search_batch(q[pick], g, 0.62)[2], 0.62, fmask, gp["topk"])
             ref["fhyb1"] = a1.search_hybrid_batch(q, g1, 0.62, allowed=fmask)
             ref["fhybo"] = want_hybrid(s, q[pick], s.search_hybrid_batch(q[pick], g, 0.62, 0)[2], 0.62, 0, fmask, gp["topk"])
+            thr = float(np.median(sc1[:, -1]))                # range search: about topk hits per query
+            olq = s.search_batch(q[pick], g, 0.62)[2]
+            for m_ in (None, fmask):
+                ref["rng1", m_ is None] = a1.search_range_batch(q, g1, 0.62, thr, allowed=m_)
+                ref["rngo", m_ is None] = [want_range(s, q[i], olq[j], 0.62, thr, m_) for j, i in enumerate(pick)]
+            ref["thr"] = thr
             ar, gr = ArrowSpaceBuilder.build(gp, full, device=local, reduction=True)      # pre-graph reduction, one GPU
             ref.update(red_csr=gr.csr(), red_lam=ar.lambdas(), red_cent=gr.centroids(), red_info=gr.reduction)
             del a1, g1, s, g, full, ar, gr
@@ -145,6 +153,26 @@ def main():
                     print("world %d n %d f %d grid %d item shard(s) x %d query slot(s): filtered %s == single GPU (bitwise) %s, "
                           "== oracle (%d queries) %s, only allowed items %s" % (world, n, f, R, world // R, name, e[0],
                                                                                 len(ref["pick"]), e[1], e[2]), flush=True)
+                    ok = ok and all(e)
+            thr = torch.tensor([ref["thr"] if rank == 0 else 0.0], dtype=torch.float64, device="cuda")
+            dist.broadcast(thr, 0)
+            for m_ in (None, fmask):                          # range search, collective: every rank returns the whole batch
+                rp, ri, rs = aspace.search_range_batch(q, gl, 0.62, float(thr.item()), allowed=m_)
+                crc = torch.tensor([zlib.crc32(rp.tobytes() + ri.tobytes() + rs.tobytes())], dtype=torch.int64, device="cuda")
+                lo, hi_crc = crc.clone(), crc.clone()
+                dist.all_reduce(lo, op=dist.ReduceOp.MIN)
+                dist.all_reduce(hi_crc, op=dist.ReduceOp.MAX)
+                if rank == 0:
+                    p1, i1, s1 = ref["rng1", m_ is None]
+                    e_o = True
+                    for j, i in enumerate(ref["pick"]):
+                        wi, ws = ref["rngo", m_ is None][j]
+                        e_o = e_o and np.array_equal(ri[rp[i]:rp[i + 1]], wi) and bool(np.allclose(rs[rp[i]:rp[i + 1]], ws, rtol=1e-9, atol=0))
+                    e = [np.array_equal(rp, p1) and np.array_equal(ri, i1) and np.array_equal(rs, s1), e_o, bool(lo.item() == hi_crc.item())]
+                    print("world %d n %d f %d grid %d item shard(s) x %d query slot(s): search_range%s (%.1f hits/query) == single "
+                          "GPU (bitwise) %s, == definition (%d queries) %s, same bits on every rank %s"
+                          % (world, n, f, R, world // R, "" if m_ is None else " masked", rp[-1] / nq, e[0], len(ref["pick"]),
+                             e[1], e[2]), flush=True)
                     ok = ok and all(e)
             if os.environ.get("CHECK_PEER") and R == world and world > 1:    # csrc/peer.cu: P2P exchange + flag-driven merge
                 os.environ["ASP_PEER_MERGE"] = "1"
