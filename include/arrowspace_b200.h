@@ -43,7 +43,7 @@ enum {
     ASP_ERR_ZERO_VECTOR = 2,  /* all-zero vector in the Rayleigh quotient      TAUMODE.md:13 */
     ASP_ERR_LAMBDA_ZERO = 3,  /* "The lambdas are zero, check the magnitude of items and eps."  src/lib.rs:156-159 */
     ASP_ERR_ARG = 4,
-    ASP_ERR_NOMEM = 5,
+    ASP_ERR_NOMEM = 5,        /* a device allocation failed (every path; the message gives the bytes asked for) */
     ASP_ERR_CUDA = 6,         /* no device / CUDA failure: there is no CPU fallback */
     ASP_ERR_UNSUPPORTED = 7,
     ASP_NEED_EXACT = 8,       /* asp_graph_from_gram: decisions inside the rounding band, see below */

@@ -95,33 +95,15 @@ int upload_pitched(cudaStream_t st, const double *src, int64_t n, int32_t f, int
     return ASP_OK;
 }
 
-// stream-ordered scratch of the hybrid search entry points, released on every exit path
-struct HybridScratch {
-    cudaStream_t st;
-    std::vector<void *> ptrs;
-    template <typename T> int get(T **out, size_t count)
-    {
-        void *p = nullptr;
-        if (cudaMallocAsync(&p, sizeof(T) * (count ? count : 1), st) != cudaSuccess) {
-            cudaGetLastError();
-            asp_set_error("out of device memory in the hybrid search (%zu bytes)", sizeof(T) * count);
-            return ASP_ERR_NOMEM;
-        }
-        ptrs.push_back(p);
-        *out = static_cast<T *>(p);
-        return ASP_OK;
-    }
-    ~HybridScratch() { for (void *p : ptrs) cudaFreeAsync(p, st); }
-};
-
 // The packed item mask of a filtered call (ceil(n / 8) bytes, host or device) on the device as 32-bit words, the rest of the
-// last word zero.  NULL bits: *out = NULL (every row).
-int upload_allowed(cudaStream_t st, const uint8_t *bits, int64_t n, uint32_t **out)
+// last word zero, held by the caller's scratch.  NULL bits: *out = NULL (every row).
+int upload_allowed(asp_scratch &sc, const uint8_t *bits, int64_t n, uint32_t **out)
 {
     *out = nullptr;
     if (!bits) return ASP_OK;
+    cudaStream_t st = sc.st;
     const size_t nbytes = (size_t)((n + 7) / 8), nwords = (size_t)((n + 31) / 32);
-    ASP_CUDA(cudaMallocAsync(out, sizeof(uint32_t) * (nwords ? nwords : 1), st));
+    ASP_CHECK(sc.get(out, nwords));
     ASP_CUDA(cudaMemsetAsync(*out, 0, sizeof(uint32_t) * (nwords ? nwords : 1), st));
     if (nbytes) ASP_CUDA(cudaMemcpyAsync(*out, bits, nbytes, cudaMemcpyDefault, st));
     return ASP_OK;
@@ -284,11 +266,16 @@ int asp_space_create(asp_ctx *ctx, const double *items_shard, int64_t n_local, i
     s->fp = (f + 3) & ~3;
     s->world = world;
     s->rank = rank;
-    ASP_CUDA(cudaMallocAsync(&s->items, sizeof(double) * (size_t)n_local * s->fp, ctx->stream));
-    ASP_CUDA(cudaMallocAsync(&s->norms, sizeof(double) * n_local, ctx->stream));
-    ASP_CUDA(cudaMallocAsync(&s->inv_norms, sizeof(double) * n_local, ctx->stream));
-    ASP_CUDA(cudaMallocAsync(&s->lambdas, sizeof(double) * n_local, ctx->stream));
-    int rc = upload_pitched(ctx->stream, items_shard, n_local, f, s->fp, s->items);
+    int rc = ASP_OK;
+    if (cudaMallocAsync(&s->items, sizeof(double) * (size_t)n_local * s->fp, ctx->stream) != cudaSuccess ||
+        cudaMallocAsync(&s->norms, sizeof(double) * n_local, ctx->stream) != cudaSuccess ||
+        cudaMallocAsync(&s->inv_norms, sizeof(double) * n_local, ctx->stream) != cudaSuccess ||
+        cudaMallocAsync(&s->lambdas, sizeof(double) * n_local, ctx->stream) != cudaSuccess) {
+        cudaGetLastError();
+        asp_set_error("out of device memory for the item shard");
+        rc = ASP_ERR_NOMEM;
+    }
+    if (rc == ASP_OK) rc = upload_pitched(ctx->stream, items_shard, n_local, f, s->fp, s->items);
     if (rc == ASP_OK) rc = asp_make_items_tmap(&s->tmap_gram, s->items, n_local, s->fp, ASP_ROW_UNIT, 32);
     if (rc == ASP_OK) rc = asp_make_items_tmap(&s->tmap_rows, s->items, n_local, s->fp, 128, 4);
     if (rc == ASP_OK && cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
@@ -322,10 +309,15 @@ int asp_space_adopt_shard(asp_ctx *ctx, double *items_dev, int64_t n_local, int3
     s->world = world; s->rank = rank;
     s->items = items_dev;
     s->owns_items = false;
-    ASP_CUDA(cudaMallocAsync(&s->norms, sizeof(double) * n_local, ctx->stream));
-    ASP_CUDA(cudaMallocAsync(&s->inv_norms, sizeof(double) * n_local, ctx->stream));
-    ASP_CUDA(cudaMallocAsync(&s->lambdas, sizeof(double) * n_local, ctx->stream));
-    int rc = asp_make_items_tmap(&s->tmap_gram, s->items, n_local, s->fp, ASP_ROW_UNIT, 32);
+    int rc = ASP_OK;
+    if (cudaMallocAsync(&s->norms, sizeof(double) * n_local, ctx->stream) != cudaSuccess ||
+        cudaMallocAsync(&s->inv_norms, sizeof(double) * n_local, ctx->stream) != cudaSuccess ||
+        cudaMallocAsync(&s->lambdas, sizeof(double) * n_local, ctx->stream) != cudaSuccess) {
+        cudaGetLastError();
+        asp_set_error("out of device memory for the item norms and lambdas");
+        rc = ASP_ERR_NOMEM;
+    }
+    if (rc == ASP_OK) rc = asp_make_items_tmap(&s->tmap_gram, s->items, n_local, s->fp, ASP_ROW_UNIT, 32);
     if (rc == ASP_OK) rc = asp_make_items_tmap(&s->tmap_rows, s->items, n_local, s->fp, 128, 4);
     if (rc != ASP_OK) { asp_free_space(s); return rc; }
     *out = s;
@@ -405,9 +397,10 @@ int asp_graph_from_gram(asp_ctx *ctx, const double *gram_segments_dev, int32_t f
     cudaStream_t st = ctx->stream;
     if (n_need) *n_need = 0;
     StageTimer timer(ctx, "graph_ms");
+    asp_scratch sc(st);
 
     double *gram = nullptr;
-    ASP_CUDA(cudaMallocAsync(&gram, sizeof(double) * (size_t)f * f, st));
+    ASP_CHECK(sc.get(&gram, (size_t)f * f));
     ASP_CHECK(asp_launch_gram_reduce(ctx, gram_segments_dev, f, gram));
 
     // exact pairs, sorted by (a, b) for the device binary search
@@ -427,8 +420,8 @@ int asp_graph_from_gram(asp_ctx *ctx, const double *gram_segments_dev, int32_t f
             hp[2 * i + 1] = exact_pairs[2 * order[i] + 1];
             for (int c = 0; c < 3; ++c) hs[3 * i + c] = exact_sums[3 * order[i] + c];
         }
-        ASP_CUDA(cudaMallocAsync(&d_pairs, sizeof(int32_t) * 2 * n_exact, st));
-        ASP_CUDA(cudaMallocAsync(&d_sums, sizeof(double) * 3 * n_exact, st));
+        ASP_CHECK(sc.get(&d_pairs, 2 * (size_t)n_exact));
+        ASP_CHECK(sc.get(&d_sums, 3 * (size_t)n_exact));
         ASP_CUDA(cudaMemcpyAsync(d_pairs, hp.data(), sizeof(int32_t) * 2 * n_exact, cudaMemcpyHostToDevice, st));
         ASP_CUDA(cudaMemcpyAsync(d_sums, hs.data(), sizeof(double) * 3 * n_exact, cudaMemcpyHostToDevice, st));
         ASP_CUDA(cudaStreamSynchronize(st));
@@ -438,8 +431,8 @@ int asp_graph_from_gram(asp_ctx *ctx, const double *gram_segments_dev, int32_t f
     const int64_t all_pairs = (int64_t)f * (f - 1) / 2;
     const int64_t dev_cap = std::max<int64_t>(1, std::min<int64_t>(all_pairs * 2, (int64_t)1 << 24));
     int32_t *d_need = nullptr, *d_need_count = nullptr;
-    ASP_CUDA(cudaMallocAsync(&d_need, sizeof(int32_t) * 2 * dev_cap, st));
-    ASP_CUDA(cudaMallocAsync(&d_need_count, sizeof(int32_t), st));
+    ASP_CHECK(sc.get(&d_need, 2 * (size_t)dev_cap));
+    ASP_CHECK(sc.get(&d_need_count, 1));
     ASP_CUDA(cudaMemsetAsync(d_need_count, 0, sizeof(int32_t), st));
 
     asp_knn_lists lists;
@@ -480,14 +473,6 @@ int asp_graph_from_gram(asp_ctx *ctx, const double *gram_segments_dev, int32_t f
         if (rc == ASP_OK) rc = asp_graph_upload_upper(g);
         if (rc != ASP_OK) { asp_free_graph(g); g = nullptr; }
     }
-    cudaFreeAsync(lists.idx, st);
-    cudaFreeAsync(lists.dist, st);
-    cudaFreeAsync(lists.cnt, st);
-    cudaFreeAsync(d_need, st);
-    cudaFreeAsync(d_need_count, st);
-    if (d_pairs) cudaFreeAsync(d_pairs, st);
-    if (d_sums) cudaFreeAsync(d_sums, st);
-    cudaFreeAsync(gram, st);
     timer.stop();
     if (rc == ASP_OK) *out_graph = g;
     return rc;
@@ -500,10 +485,11 @@ int asp_space_exact_pairs(asp_space *s, const int32_t *pairs, int64_t n_pairs, d
     asp_ctx *ctx = s->ctx;
     ASP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
+    asp_scratch sc(st);
     int32_t *d_pairs = nullptr;
     double *d_sums = nullptr;
-    ASP_CUDA(cudaMallocAsync(&d_pairs, sizeof(int32_t) * 2 * n_pairs, st));
-    ASP_CUDA(cudaMallocAsync(&d_sums, sizeof(double) * 3 * n_pairs, st));
+    ASP_CHECK(sc.get(&d_pairs, 2 * (size_t)n_pairs));
+    ASP_CHECK(sc.get(&d_sums, 3 * (size_t)n_pairs));
     ASP_CUDA(cudaMemcpyAsync(d_pairs, pairs, sizeof(int32_t) * 2 * n_pairs, cudaMemcpyDefault, st));
     ASP_CUDA(cudaMemcpyAsync(d_sums, sums, sizeof(double) * 3 * n_pairs, cudaMemcpyDefault, st));
     int rc = asp_launch_exact_pairs(s, d_pairs, n_pairs, d_sums);
@@ -511,8 +497,6 @@ int asp_space_exact_pairs(asp_space *s, const int32_t *pairs, int64_t n_pairs, d
         ASP_CUDA(cudaMemcpyAsync(sums, d_sums, sizeof(double) * 3 * n_pairs, cudaMemcpyDefault, st));
         ASP_CUDA(cudaStreamSynchronize(st));
     }
-    cudaFreeAsync(d_pairs, st);
-    cudaFreeAsync(d_sums, st);
     return rc;
 }
 
@@ -521,8 +505,9 @@ int asp_space_compute_lambdas(asp_space *s, const asp_graph *g)
     if (!s || !g) ASP_FAIL(ASP_ERR_ARG, "asp_space_compute_lambdas: NULL argument");
     asp_ctx *ctx = s->ctx;
     ASP_CUDA(cudaSetDevice(ctx->device));
+    asp_scratch sc(ctx->stream);
     int *flag = nullptr;
-    ASP_CUDA(cudaMallocAsync(&flag, sizeof(int), ctx->stream));
+    ASP_CHECK(sc.get(&flag, 1));
     ASP_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), ctx->stream));
     StageTimer timer(ctx, "lambda_ms");
     int rc = asp_launch_taumode(ctx, g, &g->sw, s->items, s->n_local, s->f, s->fp, nullptr, nullptr, s->lambdas, s->norms,
@@ -533,7 +518,6 @@ int asp_space_compute_lambdas(asp_space *s, const asp_graph *g)
         ASP_CUDA(cudaMemcpyAsync(&h, flag, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
         ASP_CUDA(cudaStreamSynchronize(ctx->stream));
     }
-    cudaFreeAsync(flag, ctx->stream);
     if (rc != ASP_OK) return rc;
     if (h) ASP_FAIL(ASP_ERR_ZERO_VECTOR, "an item vector is all zeros: its Rayleigh quotient is undefined");
     s->have_lambdas = true;
@@ -549,12 +533,10 @@ int asp_space_feature_graph(asp_space *s, const asp_graph_params *gp, const asp_
     const int32_t f = s->f;
     const int64_t n = s->n_local;
     ASP_CUDA(cudaSetDevice(ctx->device));
+    asp_scratch sc(ctx->stream);
     double *segs = nullptr;
     asp_graph *g = nullptr;
-    if (cudaMallocAsync(&segs, sizeof(double) * (size_t)ASP_GRAM_SEGMENTS * f * f, ctx->stream) != cudaSuccess) {
-        cudaGetLastError();
-        ASP_FAIL(ASP_ERR_NOMEM, "out of device memory for the Gram segments");
-    }
+    ASP_CHECK(sc.get(&segs, (size_t)ASP_GRAM_SEGMENTS * f * f));
     int rc = asp_space_gram_partials(s, segs);
     if (rc == ASP_OK) {
         double graph_ms = 0.0;
@@ -584,7 +566,6 @@ int asp_space_feature_graph(asp_space *s, const asp_graph_params *gp, const asp_
         if (rc == ASP_NEED_EXACT) { asp_set_error("exact-pair resolution did not converge"); rc = ASP_ERR_CUDA; }
         ctx->stats["graph_ms"] = graph_ms;
     }
-    cudaFreeAsync(segs, ctx->stream);
     if (rc != ASP_OK) { asp_free_graph(g); return rc; }
     *out_graph = g;
     return ASP_OK;
@@ -720,11 +701,12 @@ int asp_query_lambda(asp_ctx *ctx, const asp_graph *g, const asp_switches *sw_in
     const asp_switches sw = sw_in ? *sw_in : g->sw;
     const int32_t f = (int32_t)g->nnodes;
     cudaStream_t st = ctx->stream;
+    asp_scratch sc(st);
     double *dq = nullptr, *de = nullptr;
     int *flag = nullptr;
-    ASP_CUDA(cudaMallocAsync(&dq, sizeof(double) * (size_t)nq * f, st));
-    ASP_CUDA(cudaMallocAsync(&de, sizeof(double) * 3 * nq, st));
-    ASP_CUDA(cudaMallocAsync(&flag, sizeof(int), st));
+    ASP_CHECK(sc.get(&dq, (size_t)nq * f));
+    ASP_CHECK(sc.get(&de, 3 * (size_t)nq));
+    ASP_CHECK(sc.get(&flag, 1));
     ASP_CUDA(cudaMemsetAsync(flag, 0, sizeof(int), st));
     ASP_CUDA(cudaMemcpyAsync(dq, queries, sizeof(double) * (size_t)nq * f, cudaMemcpyDefault, st));
     int rc = asp_launch_taumode(ctx, g, &sw, dq, nq, f, f, de, de + nq, de + 2 * nq, nullptr, nullptr, flag);
@@ -736,9 +718,6 @@ int asp_query_lambda(asp_ctx *ctx, const asp_graph *g, const asp_switches *sw_in
         if (rc == ASP_OK && out_lambda) rc = asp_copy_out(ctx, out_lambda, de + 2 * nq, sizeof(double) * nq);
         ASP_CUDA(cudaStreamSynchronize(st));
     }
-    cudaFreeAsync(dq, st);
-    cudaFreeAsync(de, st);
-    cudaFreeAsync(flag, st);
     if (rc != ASP_OK) return rc;
     if (h) ASP_FAIL(ASP_ERR_ZERO_VECTOR, "a query vector is all zeros: its Rayleigh quotient is undefined");
     return ASP_OK;
@@ -815,19 +794,20 @@ int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const doub
     const int64_t topk = g->gp.topk;                              // src/lib.rs:169
     const int32_t f = s->f, fp = s->fp;
 
+    asp_scratch sc(st);
     double *dq = nullptr, *dlam = nullptr, *dnorm = nullptr, *dscore = nullptr;
     int64_t *didx = nullptr;
     int *flags = nullptr;
-    ASP_CUDA(cudaMallocAsync(&dq, sizeof(double) * (size_t)nq * fp, st));
-    ASP_CUDA(cudaMallocAsync(&dlam, sizeof(double) * nq, st));
-    ASP_CUDA(cudaMallocAsync(&dnorm, sizeof(double) * nq, st));
-    ASP_CUDA(cudaMallocAsync(&flags, sizeof(int) * 2, st));
+    ASP_CHECK(sc.get(&dq, (size_t)nq * fp));
+    ASP_CHECK(sc.get(&dlam, (size_t)nq));
+    ASP_CHECK(sc.get(&dnorm, (size_t)nq));
+    ASP_CHECK(sc.get(&flags, 2));
     if (topk > 0) {
-        ASP_CUDA(cudaMallocAsync(&didx, sizeof(int64_t) * (size_t)nq * topk, st));
-        ASP_CUDA(cudaMallocAsync(&dscore, sizeof(double) * (size_t)nq * topk, st));
+        ASP_CHECK(sc.get(&didx, (size_t)nq * topk));
+        ASP_CHECK(sc.get(&dscore, (size_t)nq * topk));
     }
     uint32_t *dallowed = nullptr;                                 // once per call, before the batch is split
-    int rc = upload_allowed(st, allowed_bits, s->n_local, &dallowed);
+    int rc = upload_allowed(sc, allowed_bits, s->n_local, &dallowed);
     const char *nopipe = getenv("ASP_NO_PIPELINE");
     const bool host_io = !asp_is_device_ptr(queries) && !asp_is_device_ptr(out_idx) && !asp_is_device_ptr(out_score) &&
                          (!out_lambda_q || !asp_is_device_ptr(out_lambda_q));
@@ -910,13 +890,6 @@ int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const doub
         }
         ctx->stats["search_pipeline_chunks"] = 1;
     }
-    cudaFreeAsync(dq, st);
-    cudaFreeAsync(dlam, st);
-    cudaFreeAsync(dnorm, st);
-    cudaFreeAsync(flags, st);
-    if (didx) cudaFreeAsync(didx, st);
-    if (dscore) cudaFreeAsync(dscore, st);
-    if (dallowed) cudaFreeAsync(dallowed, st);
     return rc;
 }
 
@@ -963,7 +936,7 @@ int asp_search_hybrid_batch_filtered(const asp_space *s, const asp_graph *g, con
         ASP_FAIL(ASP_ERR_UNSUPPORTED, "hybrid search: a shortlist of %lld items is beyond the 1024 the exact scan keeps per query "
                  "(use pool >= nitems = %lld for no shortlist at all)", (long long)m, (long long)s->n_local);
 
-    HybridScratch scratch{st, {}};
+    asp_scratch scratch(st);
     double *dq = nullptr, *dlam = nullptr, *dnorm = nullptr, *pscore = nullptr, *dscore = nullptr;
     int64_t *pidx = nullptr, *didx = nullptr;
     int *flags = nullptr;
@@ -981,8 +954,7 @@ int asp_search_hybrid_batch_filtered(const asp_space *s, const asp_graph *g, con
     }
     ASP_CHECK(upload_pitched(st, queries, nq, f, fp, dq));
     uint32_t *dallowed = nullptr;
-    ASP_CHECK(upload_allowed(st, allowed_bits, s->n_local, &dallowed));
-    if (dallowed) scratch.ptrs.push_back(dallowed);
+    ASP_CHECK(upload_allowed(scratch, allowed_bits, s->n_local, &dallowed));
     // H1 + H2: lambda_q, then the m largest cosines per query (the score at tau = 1 is the cosine), ties by the smaller index
     if (whole_set)
         ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false, dallowed));
@@ -1045,7 +1017,7 @@ int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, con
     const int64_t width = whole_set ? topk : m;                   // entries per query of the outputs
     const int64_t kl = std::min(m, s->n_local);                   // a shard smaller than m answers all its rows
 
-    HybridScratch scratch{st, {}};
+    asp_scratch scratch(st);
     double *dq = nullptr, *dlam = nullptr, *dnorm = nullptr, *dcos = nullptr, *dscore = nullptr;
     int64_t *didx = nullptr;
     int *flags = nullptr;
@@ -1060,8 +1032,7 @@ int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, con
     }
     ASP_CHECK(upload_pitched(st, queries, nq, f, fp, dq));
     uint32_t *dallowed = nullptr;
-    ASP_CHECK(upload_allowed(st, allowed_bits, s->n_local, &dallowed));
-    if (dallowed) scratch.ptrs.push_back(dallowed);
+    ASP_CHECK(upload_allowed(scratch, allowed_bits, s->n_local, &dallowed));
     if (whole_set) {
         // no shortlist: the shard's best topk by the lambda-aware score, merged like asp_search_batch's lists
         ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false, dallowed));
@@ -1114,7 +1085,7 @@ int asp_hybrid_merge(asp_ctx *ctx, const int64_t *idx, const double *cosv, const
     ASP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const size_t n_in = (size_t)parts * nq * m, n_pool = (size_t)nq * m, n_out = (size_t)nq * topk;
-    HybridScratch scratch{st, {}};
+    asp_scratch scratch(st);
     int64_t *d_idx = nullptr, *d_pidx = nullptr, *d_oidx = nullptr;
     double *d_cos = nullptr, *d_sc = nullptr, *d_psc = nullptr, *d_osc = nullptr;
     ASP_CHECK(scratch.get(&d_idx, n_in));
@@ -1162,18 +1133,18 @@ int asp_debug_tc_dots(const asp_space *s, const double *queries, int64_t nq, flo
         for (int j = 0; j < s->f; ++j) n2 += hq[i * s->f + j] * hq[i * s->f + j];
         hz[nq + i] = sqrt(n2);
     }
+    asp_scratch sc(st);
     double *dq = nullptr, *dz = nullptr;
     float *dd = nullptr;
-    ASP_CUDA(cudaMallocAsync(&dq, sizeof(double) * (size_t)nq * s->fp, st));
-    ASP_CUDA(cudaMallocAsync(&dz, sizeof(double) * 2 * nq, st));
-    ASP_CUDA(cudaMallocAsync(&dd, sizeof(float) * (size_t)nq * s->n_local, st));
+    ASP_CHECK(sc.get(&dq, (size_t)nq * s->fp));
+    ASP_CHECK(sc.get(&dz, 2 * (size_t)nq));
+    ASP_CHECK(sc.get(&dd, (size_t)nq * s->n_local));
     ASP_CUDA(cudaMemcpyAsync(dz, hz.data(), sizeof(double) * 2 * nq, cudaMemcpyHostToDevice, st));
     ASP_CUDA(cudaMemsetAsync(dd, 0, sizeof(float) * (size_t)nq * s->n_local, st));
     int rc = upload_pitched(ctx->stream, hq.data(), nq, s->f, s->fp, dq);
     if (rc == ASP_OK) rc = asp_search_tc_impl(s, dq, nq, s->fp, dz, dz + nq, 1.0, 1, nullptr, nullptr, dd);
     if (rc == ASP_OK) rc = asp_copy_out(ctx, out, dd, sizeof(float) * (size_t)nq * s->n_local);
     ASP_CUDA(cudaStreamSynchronize(st));
-    cudaFreeAsync(dq, st); cudaFreeAsync(dz, st); cudaFreeAsync(dd, st);
     return rc;
 }
 
@@ -1185,22 +1156,19 @@ int asp_topk_merge(asp_ctx *ctx, const int64_t *idx, const double *score, int pa
     ASP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const size_t n_in = (size_t)parts * nq * topk, n_out = (size_t)nq * topk;
+    asp_scratch sc(st);
     int64_t *d_idx = nullptr, *d_oidx = nullptr;
     double *d_sc = nullptr, *d_osc = nullptr;
-    ASP_CUDA(cudaMallocAsync(&d_idx, sizeof(int64_t) * n_in, st));
-    ASP_CUDA(cudaMallocAsync(&d_sc, sizeof(double) * n_in, st));
-    ASP_CUDA(cudaMallocAsync(&d_oidx, sizeof(int64_t) * n_out, st));
-    ASP_CUDA(cudaMallocAsync(&d_osc, sizeof(double) * n_out, st));
+    ASP_CHECK(sc.get(&d_idx, n_in));
+    ASP_CHECK(sc.get(&d_sc, n_in));
+    ASP_CHECK(sc.get(&d_oidx, n_out));
+    ASP_CHECK(sc.get(&d_osc, n_out));
     ASP_CUDA(cudaMemcpyAsync(d_idx, idx, sizeof(int64_t) * n_in, cudaMemcpyDefault, st));
     ASP_CUDA(cudaMemcpyAsync(d_sc, score, sizeof(double) * n_in, cudaMemcpyDefault, st));
     int rc = asp_topk_merge_impl(ctx, d_idx, d_sc, parts, nq, topk, d_oidx, d_osc);
     if (rc == ASP_OK) rc = asp_copy_out(ctx, out_idx, d_oidx, sizeof(int64_t) * n_out);
     if (rc == ASP_OK) rc = asp_copy_out(ctx, out_score, d_osc, sizeof(double) * n_out);
     ASP_CUDA(cudaStreamSynchronize(st));
-    cudaFreeAsync(d_idx, st);
-    cudaFreeAsync(d_sc, st);
-    cudaFreeAsync(d_oidx, st);
-    cudaFreeAsync(d_osc, st);
     return rc;
 }
 
@@ -1226,7 +1194,7 @@ int asp_search_range_batch(const asp_space *s, const asp_graph *g, const double 
     const int32_t f = s->f, fp = s->fp;
     const int64_t sub = std::min<int64_t>(std::max<int64_t>(nq, 1), asp_range_sub_batch());
     std::vector<int64_t> h_counts((size_t)nq);
-    HybridScratch scratch{st, {}};
+    asp_scratch scratch(st);
     double *dq = nullptr, *dlam = nullptr, *dnorm = nullptr;
     int *flags = nullptr;
     uint32_t *dallowed = nullptr;
@@ -1234,7 +1202,7 @@ int asp_search_range_batch(const asp_space *s, const asp_graph *g, const double 
     if (rc == ASP_OK) rc = scratch.get(&dlam, (size_t)sub);
     if (rc == ASP_OK) rc = scratch.get(&dnorm, (size_t)sub);
     if (rc == ASP_OK) rc = scratch.get(&flags, 2);
-    if (rc == ASP_OK) rc = upload_allowed(st, allowed_bits, s->n_local, &dallowed);   // once per call
+    if (rc == ASP_OK) rc = upload_allowed(scratch, allowed_bits, s->n_local, &dallowed);   // once per call
     for (int64_t q0 = 0; q0 < nq && rc == ASP_OK; q0 += sub) {
         const int64_t qn = std::min(sub, nq - q0);
         rc = upload_pitched(st, queries + q0 * f, qn, f, fp, dq);
@@ -1242,12 +1210,10 @@ int asp_search_range_batch(const asp_space *s, const asp_graph *g, const double 
         if (rc == ASP_OK) rc = search_device_batch(s, g, dq, qn, tau, 0, dlam, dnorm, flags, nullptr, nullptr, true, nullptr);
         asp_range_result::Piece p;
         if (rc == ASP_OK)
-            rc = asp_range_impl(s, dq, qn, fp, dlam, dnorm, tau, min_score, dallowed, max_hits, res->total, q0, h_counts.data() + q0,
-                                &p.idx, &p.score, &p.n);
-        if (p.n > 0) { res->pieces.push_back(p); res->total += p.n; }
+            rc = asp_range_impl(s, dq, qn, fp, dlam, dnorm, tau, min_score, dallowed, max_hits, res->total, q0, h_counts.data() + q0, &p);
+        if (p.n > 0) { res->total += p.n; res->pieces.push_back(std::move(p)); }
         if (rc == ASP_OK && out_lambda_q) rc = asp_copy_out(ctx, out_lambda_q + q0, dlam, sizeof(double) * qn);
     }
-    if (dallowed) cudaFreeAsync(dallowed, st);
     if (rc == ASP_OK && nq > 0) rc = asp_copy_out(ctx, out_counts, h_counts.data(), sizeof(int64_t) * nq);
     if (rc == ASP_OK && cudaStreamSynchronize(st) != cudaSuccess) { asp_set_error("range search: stream failed"); rc = ASP_ERR_CUDA; }
     if (rc != ASP_OK) { asp_range_result_free(res); return rc; }
@@ -1274,7 +1240,6 @@ void asp_range_result_free(asp_range_result *r)
 {
     if (!r) return;
     cudaSetDevice(r->ctx->device);
-    for (auto &p : r->pieces) { cudaFreeAsync(p.idx, r->ctx->stream); cudaFreeAsync(p.score, r->ctx->stream); }
     delete r;
 }
 
@@ -1295,7 +1260,7 @@ int asp_range_merge(asp_ctx *ctx, int parts, int64_t nq, const int64_t *counts, 
     }
     if (total == 0) return ASP_OK;
     if (!idx || !score || !out_idx || !out_score) ASP_FAIL(ASP_ERR_ARG, "asp_range_merge: NULL argument");
-    HybridScratch scratch{st, {}};
+    asp_scratch scratch(st);
     int64_t *d_idx = nullptr, *d_oidx = nullptr;
     double *d_sc = nullptr, *d_osc = nullptr;
     ASP_CHECK(scratch.get(&d_idx, (size_t)total));
@@ -1373,11 +1338,11 @@ int asp_item_graph(asp_space *s, const asp_graph_params *gp, const asp_switches 
     if (!g->gp.has_sigma) { g->gp.sigma = gp->eps * 0.5; g->gp.has_sigma = 1; }
     g->sw = sw;
     int rc = asp_assemble_laplacian(ctx, &lists, gp, &sw, g);
-    cudaFreeAsync(lists.idx, ctx->stream);
-    cudaFreeAsync(lists.dist, ctx->stream);
-    cudaFreeAsync(lists.cnt, ctx->stream);
+    if (rc == ASP_OK && cudaStreamSynchronize(ctx->stream) != cudaSuccess) {
+        asp_set_error("item graph: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = ASP_ERR_CUDA;
+    }
     if (rc != ASP_OK) { asp_free_graph(g); return rc; }
-    ASP_CUDA(cudaStreamSynchronize(ctx->stream));
     *out_graph = g;
     return ASP_OK;
 }
@@ -1403,9 +1368,6 @@ int asp_item_knn_rows(asp_space *s, const asp_graph_params *gp, const asp_switch
         if (rc == ASP_OK && rows > 0) rc = asp_copy_out(ctx, out_cnt, lists.cnt, sizeof(int32_t) * rows);
         cudaStreamSynchronize(ctx->stream);
     }
-    if (lists.idx) cudaFreeAsync(lists.idx, ctx->stream);
-    if (lists.dist) cudaFreeAsync(lists.dist, ctx->stream);
-    if (lists.cnt) cudaFreeAsync(lists.cnt, ctx->stream);
     return rc;
 }
 
@@ -1419,10 +1381,7 @@ int asp_graph_from_knn(asp_ctx *ctx, int64_t m, int32_t kk, const int32_t *idx, 
     if (sw_in) sw = *sw_in; else asp_default_switches(&sw);
     ASP_CHECK(check_switches(&sw));
     asp_knn_lists lists;
-    lists.m = m; lists.kk = kk;
-    ASP_CUDA(cudaMallocAsync(&lists.idx, sizeof(int32_t) * (size_t)m * kk, st));
-    ASP_CUDA(cudaMallocAsync(&lists.dist, sizeof(double) * (size_t)m * kk, st));
-    ASP_CUDA(cudaMallocAsync(&lists.cnt, sizeof(int32_t) * (size_t)m, st));
+    ASP_CHECK(lists.alloc(st, m, kk));
     int rc = asp_copy_in(ctx, lists.idx, idx, sizeof(int32_t) * (size_t)m * kk);
     if (rc == ASP_OK) rc = asp_copy_in(ctx, lists.dist, dist, sizeof(double) * (size_t)m * kk);
     if (rc == ASP_OK) rc = asp_copy_in(ctx, lists.cnt, cnt, sizeof(int32_t) * (size_t)m);
@@ -1435,9 +1394,11 @@ int asp_graph_from_knn(asp_ctx *ctx, int64_t m, int32_t kk, const int32_t *idx, 
         g->sw = sw;
         rc = asp_assemble_laplacian(ctx, &lists, gp, &sw, g);
     }
-    cudaFreeAsync(lists.idx, st); cudaFreeAsync(lists.dist, st); cudaFreeAsync(lists.cnt, st);
-    if (rc != ASP_OK) { if (g) asp_free_graph(g); return rc; }
-    ASP_CUDA(cudaStreamSynchronize(st));
+    if (rc == ASP_OK && cudaStreamSynchronize(st) != cudaSuccess) {
+        asp_set_error("graph from kNN lists: %s", cudaGetErrorString(cudaGetLastError()));
+        rc = ASP_ERR_CUDA;
+    }
+    if (rc != ASP_OK) { asp_free_graph(g); return rc; }
     *out_graph = g;
     return ASP_OK;
 }

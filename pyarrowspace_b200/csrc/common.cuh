@@ -37,6 +37,46 @@ void asp_set_error(const char *fmt, ...);
         return (code);                                                                       \
     } while (0)
 
+// ------------------------------------------------------------------ device scratch
+// Owner of stream-ordered device buffers: every buffer taken with get() is given back (cudaFreeAsync on the owner's
+// stream) by release() or by the destructor, so no return path leaks one.  Move-only: a moved-from owner holds nothing.
+struct asp_scratch {
+    cudaStream_t st = nullptr;
+    std::vector<void *> ptrs;
+
+    asp_scratch() = default;
+    explicit asp_scratch(cudaStream_t s) : st(s) {}
+    asp_scratch(const asp_scratch &) = delete;
+    asp_scratch &operator=(const asp_scratch &) = delete;
+    asp_scratch(asp_scratch &&o) noexcept : st(o.st), ptrs(std::move(o.ptrs)) { o.ptrs.clear(); }
+    asp_scratch &operator=(asp_scratch &&o) noexcept
+    {
+        if (this != &o) { release(); st = o.st; ptrs = std::move(o.ptrs); o.ptrs.clear(); }
+        return *this;
+    }
+    ~asp_scratch() { release(); }
+
+    // count elements of T (count == 0: one element); ASP_ERR_NOMEM with the byte count when the pool has no room
+    template <class T> int get(T **out, size_t count)
+    {
+        const size_t bytes = sizeof(T) * (count ? count : 1);
+        void *p = nullptr;
+        if (cudaMallocAsync(&p, bytes, st) != cudaSuccess) {
+            cudaGetLastError();
+            asp_set_error("out of device memory (%zu bytes)", bytes);
+            return ASP_ERR_NOMEM;
+        }
+        ptrs.push_back(p);
+        *out = static_cast<T *>(p);
+        return ASP_OK;
+    }
+    void release()
+    {
+        for (void *p : ptrs) cudaFreeAsync(p, st);
+        ptrs.clear();
+    }
+};
+
 // ------------------------------------------------------------------ handles
 struct asp_ctx {
     int device = 0;
@@ -90,7 +130,7 @@ struct asp_graph {
 struct asp_range_result {
     asp_ctx *ctx = nullptr;
     int64_t total = 0;
-    struct Piece { int64_t *idx = nullptr; double *score = nullptr; int64_t n = 0; };
+    struct Piece { int64_t *idx = nullptr; double *score = nullptr; int64_t n = 0; asp_scratch mem; };   // mem owns idx, score
     std::vector<Piece> pieces;
 };
 
@@ -138,6 +178,16 @@ int asp_launch_gram_reduce(asp_ctx *ctx, const double *segments_dev, int32_t f, 
 struct asp_knn_lists {                    // device buffers, m rows x kk slots
     int64_t m = 0; int32_t kk = 0;
     int32_t *idx = nullptr; double *dist = nullptr; int32_t *cnt = nullptr;
+    asp_scratch mem;                      // owns idx, dist, cnt
+    int alloc(cudaStream_t st, int64_t rows, int32_t k)   // room for max(rows, 1) rows
+    {
+        m = rows; kk = k; mem = asp_scratch(st);
+        const size_t r = (size_t)(rows > 0 ? rows : 1);
+        int rc = mem.get(&idx, r * k);
+        if (rc == ASP_OK) rc = mem.get(&dist, r * k);
+        if (rc == ASP_OK) rc = mem.get(&cnt, r);
+        return rc;
+    }
 };
 int asp_feature_select(asp_ctx *ctx, const double *gram_dev, int32_t f, int64_t n_total,
                        const asp_graph_params *gp, const asp_switches *sw, const int32_t *exact_pairs_dev,
@@ -177,13 +227,13 @@ struct asp_tc_batch {                     // device buffers of one batch of quer
     int32_t *emit_ix = nullptr, *emit_cnt = nullptr; // local item indices; [nq][nsub] counts (> capb: overflow)
     uint32_t *theta_glob = nullptr;
     uint32_t *vbits = nullptr;                       // filtered search: the item mask in visiting order
+    asp_scratch mem;                                 // owns every buffer above; *b = asp_tc_batch() frees them
 };
 enum { ASP_TC_ORDER_IDENTITY = 0, ASP_TC_ORDER_LAMBDA = 1, ASP_TC_ORDER_NORM = 2 };   // item order of the operand cache
 int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                   const double *qnorm_dev, double tau, int64_t topk, double score_floor, int force_terms, int capb_override,
                   float *dump_dev, asp_tc_batch *b, bool l2 = false, const uint32_t *allowed_dev = nullptr);
 int asp_device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out);   // max(0, max v), synchronises
-void asp_tc_batch_free(asp_ctx *ctx, asp_tc_batch *b);
 bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, double tau);
 int asp_search_tc_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                        const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
@@ -199,7 +249,7 @@ int asp_make_f16_tmap_narrow(CUtensorMap *out, const void *base, int64_t rows, i
 // range.cu (range search after the tcgen05 candidate pass)
 int asp_range_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lam_dev, const double *norm_dev,
                    double tau, double min_score, const uint32_t *allowed_dev, int64_t max_hits, int64_t hits_before, int64_t q_base,
-                   int64_t *h_counts, int64_t **out_idx, double **out_score, int64_t *out_nnz);
+                   int64_t *h_counts, asp_range_result::Piece *out);
 int asp_range_merge_impl(asp_ctx *ctx, int parts, int64_t nq, const int64_t *h_counts, const int64_t *idx_dev,
                          const double *score_dev, int64_t *out_idx_dev, double *out_score_dev);
 

@@ -348,15 +348,16 @@ int asp_assemble_laplacian(asp_ctx *ctx, const asp_knn_lists *lists, const asp_g
     }
     const int mirror = (sw->symmetrise == ASP_SYM_NONE || sw->symmetrise == ASP_SYM_MIN) ? 0 : 1;
 
+    asp_scratch sc(st);                                                   // temporaries; the g-> arrays belong to the graph
     int32_t *extra = nullptr, *cursor = nullptr, *long_count = nullptr;
     int64_t *block_sums = nullptr, *total = nullptr, *long_rows = nullptr;
     const int64_t nblocks = asp_ceil_div(m, SCAN_BLOCK);
-    ASP_CUDA(cudaMallocAsync(&extra, sizeof(int32_t) * m, st));
-    ASP_CUDA(cudaMallocAsync(&cursor, sizeof(int32_t) * m, st));
-    ASP_CUDA(cudaMallocAsync(&long_count, sizeof(int32_t), st));
-    ASP_CUDA(cudaMallocAsync(&block_sums, sizeof(int64_t) * nblocks, st));
-    ASP_CUDA(cudaMallocAsync(&total, sizeof(int64_t), st));
-    ASP_CUDA(cudaMallocAsync(&long_rows, sizeof(int64_t) * m, st));
+    ASP_CHECK(sc.get(&extra, (size_t)m));
+    ASP_CHECK(sc.get(&cursor, (size_t)m));
+    ASP_CHECK(sc.get(&long_count, 1));
+    ASP_CHECK(sc.get(&block_sums, (size_t)nblocks));
+    ASP_CHECK(sc.get(&total, 1));
+    ASP_CHECK(sc.get(&long_rows, (size_t)m));
     ASP_CUDA(cudaMemsetAsync(extra, 0, sizeof(int32_t) * m, st));
     ASP_CUDA(cudaMemsetAsync(cursor, 0, sizeof(int32_t) * m, st));
     ASP_CUDA(cudaMemsetAsync(long_count, 0, sizeof(int32_t), st));
@@ -390,29 +391,19 @@ int asp_assemble_laplacian(asp_ctx *ctx, const asp_knn_lists *lists, const asp_g
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
     int32_t *scratch_col = nullptr;
     double *scratch_w = nullptr;
-    ASP_CUDA(cudaMallocAsync(&scratch_col, sizeof(int32_t) * 2 * (size_t)nnz, st));
-    ASP_CUDA(cudaMallocAsync(&scratch_w, sizeof(double) * 2 * (size_t)nnz, st));
+    ASP_CHECK(sc.get(&scratch_col, 2 * (size_t)nnz));
+    ASP_CHECK(sc.get(&scratch_w, 2 * (size_t)nnz));
     sort_rows_block_kernel<<<ctx->num_sms * 2, 256, 0, st>>>(long_rows, long_count, g->d_indptr, g->d_indices, g->d_data,
                                                              scratch_col, scratch_w);
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
 
     if (sw->laplacian != ASP_LAPLACIAN_COMBINATORIAL) {
         double *deg = nullptr;
-        ASP_CUDA(cudaMallocAsync(&deg, sizeof(double) * m, st));
+        ASP_CHECK(sc.get(&deg, (size_t)m));
         extract_degree_kernel<<<grid, 256, 0, st>>>(m, g->d_indptr, g->d_indices, g->d_data, deg);
         ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
         normalise_kernel<<<grid, 256, 0, st>>>(m, g->d_indptr, g->d_indices, g->d_data, deg, sw->laplacian);
         ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
-        ASP_CUDA(cudaFreeAsync(deg, st));
     }
-
-    ASP_CUDA(cudaFreeAsync(scratch_col, st));
-    ASP_CUDA(cudaFreeAsync(scratch_w, st));
-    ASP_CUDA(cudaFreeAsync(extra, st));
-    ASP_CUDA(cudaFreeAsync(cursor, st));
-    ASP_CUDA(cudaFreeAsync(long_count, st));
-    ASP_CUDA(cudaFreeAsync(block_sums, st));
-    ASP_CUDA(cudaFreeAsync(total, st));
-    ASP_CUDA(cudaFreeAsync(long_rows, st));
     return ASP_OK;
 }

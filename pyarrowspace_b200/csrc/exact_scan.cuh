@@ -196,10 +196,11 @@ int run(cudaStream_t st, int num_sms, const Policy &pol, int nslow, const double
     if (max_groups > 65535) max_groups = 65535;
     if (max_groups < 1) max_groups = 1;
     const int64_t alloc_groups = ngroups < max_groups ? ngroups : max_groups;
+    asp_scratch sc(st);
     double *part_value = nullptr;
     int64_t *part_idx = nullptr;
-    if (cudaMallocAsync(&part_value, sizeof(double) * (size_t)alloc_groups * qpb * nparts * topk, st) != cudaSuccess) return 3;
-    if (cudaMallocAsync(&part_idx, sizeof(int64_t) * (size_t)alloc_groups * qpb * nparts * topk, st) != cudaSuccess) { cudaFreeAsync(part_value, st); return 3; }
+    if (sc.get(&part_value, (size_t)alloc_groups * qpb * nparts * topk) != ASP_OK) return 3;
+    if (sc.get(&part_idx, (size_t)alloc_groups * qpb * nparts * topk) != ASP_OK) return 3;
     int rc = 0;
     if (qpb == 4) { if (cudaFuncSetAttribute(scan_topk_kernel<4, Policy>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) rc = 4; }
     else { if (cudaFuncSetAttribute(scan_topk_kernel<1, Policy>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) rc = 4; }
@@ -215,8 +216,6 @@ int run(cudaStream_t st, int num_sms, const Policy &pol, int nslow, const double
         launched(1);
         if (cudaGetLastError() != cudaSuccess) rc = 4;
     }
-    cudaFreeAsync(part_value, st);
-    cudaFreeAsync(part_idx, st);
     return rc;
 }
 

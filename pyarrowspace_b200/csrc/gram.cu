@@ -232,10 +232,11 @@ int asp_launch_gram_partials(asp_space *s, double *out_dev)
     // under 2 GB (one group -- one launch -- for the usual feature counts).
     const size_t seg_bytes = sizeof(double) * (size_t)ASP_GRAM_SLICES * ntu * TILE * TILE;
     int group = (int)std::max<size_t>(1, std::min<size_t>((size_t)nseg, ((size_t)2 << 30) / seg_bytes));
+    asp_scratch sc(ctx->stream);
     SliceRange *d_slices = nullptr;
     double *d_partial = nullptr;
-    ASP_CUDA(cudaMallocAsync(&d_slices, sizeof(SliceRange) * nslices, ctx->stream));
-    ASP_CUDA(cudaMallocAsync(&d_partial, seg_bytes * group, ctx->stream));
+    ASP_CHECK(sc.get(&d_slices, (size_t)nslices));
+    ASP_CHECK(sc.get(&d_partial, seg_bytes / sizeof(double) * group));
     ASP_CUDA(cudaMemcpyAsync(d_slices, h_slices.data(), sizeof(SliceRange) * nslices, cudaMemcpyHostToDevice,
                              ctx->stream));
 
@@ -258,8 +259,6 @@ int asp_launch_gram_partials(asp_space *s, double *out_dev)
         ASP_CUDA(cudaGetLastError());
         ASP_LAUNCHED(ctx);
     }
-    ASP_CUDA(cudaFreeAsync(d_partial, ctx->stream));
-    ASP_CUDA(cudaFreeAsync(d_slices, ctx->stream));
     return ASP_OK;
 }
 

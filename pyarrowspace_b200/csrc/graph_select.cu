@@ -243,11 +243,7 @@ int asp_feature_select(asp_ctx *ctx, const double *gram_dev, int32_t f, int64_t 
 {
     if (f > 8192) ASP_FAIL(ASP_ERR_UNSUPPORTED, "feature graph supports at most 8192 features (got %d)", f);
     const int64_t kk = asp_neighbour_cap(gp, sw, f);
-    lists->m = f;
-    lists->kk = (int32_t)(kk > 0 ? kk : 1);
-    ASP_CUDA(cudaMallocAsync(&lists->idx, sizeof(int32_t) * (size_t)f * lists->kk, ctx->stream));
-    ASP_CUDA(cudaMallocAsync(&lists->dist, sizeof(double) * (size_t)f * lists->kk, ctx->stream));
-    ASP_CUDA(cudaMallocAsync(&lists->cnt, sizeof(int32_t) * (size_t)f, ctx->stream));
+    ASP_CHECK(lists->alloc(ctx->stream, f, (int32_t)(kk > 0 ? kk : 1)));
     if (kk == 0) {
         ASP_CUDA(cudaMemsetAsync(lists->cnt, 0, sizeof(int32_t) * (size_t)f, ctx->stream));
         return ASP_OK;

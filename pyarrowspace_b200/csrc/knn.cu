@@ -328,12 +328,12 @@ knn_tc_rescore_kernel(const double *__restrict__ items, int64_t n, int f, int pi
 
 }  // namespace
 
-// exact scan of the rows listed in slow_list (device)
+// exact scan of the rows listed in slow_list (device) into lists indexed by item row
 static int knn_slow_rows(asp_space *s, const asp_graph_params *gp, int distance, int64_t kk, const int32_t *slow_list, int nslow,
-                         asp_knn_lists *lists)
+                         int32_t *idx, double *dist, int32_t *cnt)
 {
     asp_ctx *ctx = s->ctx;
-    const KnnScanPolicy pol{s->items, s->fp, s->norms, gp->eps, slow_list, (int)kk, lists->idx, lists->dist, lists->cnt, s->nsq, distance};
+    const KnnScanPolicy pol{s->items, s->fp, s->norms, gp->eps, slow_list, (int)kk, idx, dist, cnt, s->nsq, distance};
     const int rc = asp_xs::run(ctx->stream, ctx->num_sms, pol, nslow, s->items, s->n_local, s->f, s->fp, kk,
                                [&](int k) { ctx->launches += k; });
     if (rc == 3) ASP_FAIL(ASP_ERR_NOMEM, "out of device memory in the exact scan of the item graph");
@@ -355,11 +355,7 @@ static int item_knn_fp64(asp_space *s, const asp_graph_params *gp, asp_knn_lists
     if (kk > n - 1) kk = n - 1;
     if (kk < 0) kk = 0;
     if (kk > LIST - 4) ASP_FAIL(ASP_ERR_UNSUPPORTED, "item graph supports k <= %d (got %lld)", LIST - 4, (long long)gp->k);
-    lists->m = n;
-    lists->kk = (int32_t)(kk > 0 ? kk : 1);
-    ASP_CUDA(cudaMallocAsync(&lists->idx, sizeof(int32_t) * (size_t)n * lists->kk, st));
-    ASP_CUDA(cudaMallocAsync(&lists->dist, sizeof(double) * (size_t)n * lists->kk, st));
-    ASP_CUDA(cudaMallocAsync(&lists->cnt, sizeof(int32_t) * (size_t)n, st));
+    ASP_CHECK(lists->alloc(st, n, (int32_t)(kk > 0 ? kk : 1)));
     ASP_CUDA(cudaMemsetAsync(lists->cnt, 0, sizeof(int32_t) * (size_t)n, st));
     if (kk == 0) return ASP_OK;
 
@@ -388,12 +384,13 @@ static int item_knn_fp64(asp_space *s, const asp_graph_params *gp, asp_knn_lists
     }
     const int nparts = (int)best_chunks;
 
+    asp_scratch sc(st);
     double *cand_score = nullptr;
     int32_t *cand_idx = nullptr, *slow_list = nullptr, *slow_count = nullptr;
-    ASP_CUDA(cudaMallocAsync(&cand_score, sizeof(double) * (size_t)n * nparts * LIST, st));
-    ASP_CUDA(cudaMallocAsync(&cand_idx, sizeof(int32_t) * (size_t)n * nparts * LIST, st));
-    ASP_CUDA(cudaMallocAsync(&slow_list, sizeof(int32_t) * (n + 1), st));
-    ASP_CUDA(cudaMallocAsync(&slow_count, sizeof(int32_t), st));
+    ASP_CHECK(sc.get(&cand_score, (size_t)n * nparts * LIST));
+    ASP_CHECK(sc.get(&cand_idx, (size_t)n * nparts * LIST));
+    ASP_CHECK(sc.get(&slow_list, (size_t)n + 1));
+    ASP_CHECK(sc.get(&slow_count, 1));
     ASP_CUDA(cudaMemsetAsync(slow_count, 0, sizeof(int32_t), st));
 
     ASP_CUDA(cudaEventRecord(ctx->ev0, st));
@@ -432,11 +429,7 @@ static int item_knn_fp64(asp_space *s, const asp_graph_params *gp, asp_knn_lists
     ctx->stats["knn_stage1_ms"] = ms;
     ctx->stats["knn_slow_rows"] = nslow;
     ctx->stats["knn_stage1_is_tc"] = 0.0;
-    if (nslow > 0) ASP_CHECK(knn_slow_rows(s, gp, ASP_DISTANCE_COSINE, kk, slow_list, nslow, lists));
-    ASP_CUDA(cudaFreeAsync(cand_score, st));
-    ASP_CUDA(cudaFreeAsync(cand_idx, st));
-    ASP_CUDA(cudaFreeAsync(slow_list, st));
-    ASP_CUDA(cudaFreeAsync(slow_count, st));
+    if (nslow > 0) ASP_CHECK(knn_slow_rows(s, gp, ASP_DISTANCE_COSINE, kk, slow_list, nslow, lists->idx, lists->dist, lists->cnt));
     return ASP_OK;
 }
 
@@ -482,12 +475,13 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int distance, i
         floor = (gp->eps >= 0.0 && e2 < 1e300) ? -(e2 * (1.0 + 1e-12)) : -INFINITY;
     }
     const int64_t rows = row_end - row_begin;
+    asp_scratch sc(st);
     int32_t *slow1 = nullptr, *slow2 = nullptr, *counts = nullptr;                  // counts[0], counts[1]
     unsigned long long *counter = nullptr;
-    ASP_CUDA(cudaMallocAsync(&slow1, sizeof(int32_t) * (rows + 1), st));
-    ASP_CUDA(cudaMallocAsync(&slow2, sizeof(int32_t) * (rows + 1), st));
-    ASP_CUDA(cudaMallocAsync(&counts, sizeof(int32_t) * 2, st));
-    ASP_CUDA(cudaMallocAsync(&counter, sizeof(unsigned long long), st));
+    ASP_CHECK(sc.get(&slow1, (size_t)rows + 1));
+    ASP_CHECK(sc.get(&slow2, (size_t)rows + 1));
+    ASP_CHECK(sc.get(&counts, 2));
+    ASP_CHECK(sc.get(&counter, 1));
     ASP_CUDA(cudaMemsetAsync(counts, 0, sizeof(int32_t) * 2, st));
     ASP_CUDA(cudaMemsetAsync(counter, 0, sizeof(unsigned long long), st));
     const size_t rsmem = (size_t)KR_WARPS * s->fp * 8 + KR_WARPS * KT_QUEUE * 4;
@@ -518,7 +512,6 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int distance, i
             stage1_ms += m1; stage2_ms += m2;
             *terms_used = b.nterms;
         }
-        asp_tc_batch_free(ctx, &b);
         return r;
     };
 
@@ -554,10 +547,11 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int distance, i
     const int32_t *final_list = direct3 ? slow2 : slow1;
     int32_t n_final = direct3 ? h_counts[1] : h_counts[0];
     if (rc == ASP_OK && n_pass2 > 0) {
+        asp_scratch qsc(st);
         double *qbuf = nullptr, *qnorm = nullptr;
         const int64_t chunk = n_pass2 < batch ? n_pass2 : batch;
-        ASP_CUDA(cudaMallocAsync(&qbuf, sizeof(double) * (size_t)chunk * s->fp, st));
-        ASP_CUDA(cudaMallocAsync(&qnorm, sizeof(double) * (size_t)chunk, st));
+        ASP_CHECK(qsc.get(&qbuf, (size_t)chunk * s->fp));
+        ASP_CHECK(qsc.get(&qnorm, (size_t)chunk));
         for (int64_t c0 = 0; c0 < n_pass2 && rc == ASP_OK; c0 += chunk) {
             const int64_t nq = (n_pass2 - c0 < chunk) ? n_pass2 - c0 : chunk;
             gather_rows_kernel<<<ctx->num_sms * 4, 256, 0, st>>>(s->items, s->fp, s->norms, slow1 + c0, nq, qbuf, qnorm);
@@ -565,7 +559,6 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int distance, i
             int used = 0;
             rc = run_batch(qbuf, qnorm, nq, 0, slow1 + c0, 3, slow2, counts + 1, &used);
         }
-        cudaFreeAsync(qbuf, st); cudaFreeAsync(qnorm, st);
         if (rc == ASP_OK) {
             ASP_CUDA(cudaMemcpyAsync(h_counts, counts, sizeof(h_counts), cudaMemcpyDeviceToHost, st));
             ASP_CUDA(cudaStreamSynchronize(st));
@@ -589,12 +582,10 @@ static int item_knn_tc(asp_space *s, const asp_graph_params *gp, int distance, i
                           "k-th neighbour?); use ASP_KNN_STAGE1=fp64", n_final);
             rc = ASP_ERR_UNSUPPORTED;
         } else if (n_final > 0) {                                     // the exact kernels index the lists by GLOBAL row
-            asp_knn_lists shifted = *lists;
-            shifted.idx = lists->idx - row_begin * kk; shifted.dist = lists->dist - row_begin * kk; shifted.cnt = lists->cnt - row_begin;
-            rc = knn_slow_rows(s, gp, distance, kk, final_list, n_final, &shifted);
+            rc = knn_slow_rows(s, gp, distance, kk, final_list, n_final, lists->idx - row_begin * kk, lists->dist - row_begin * kk,
+                               lists->cnt - row_begin);
         }
     }
-    cudaFreeAsync(slow1, st); cudaFreeAsync(slow2, st); cudaFreeAsync(counts, st); cudaFreeAsync(counter, st);
     return rc;
 }
 
@@ -618,13 +609,13 @@ static int item_knn_scan_all(asp_space *s, const asp_graph_params *gp, int dista
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
     const int64_t n = s->n_local;
+    asp_scratch sc(st);
     int32_t *rows = nullptr;
-    ASP_CUDA(cudaMallocAsync(&rows, sizeof(int32_t) * (size_t)(n > 0 ? n : 1), st));
+    ASP_CHECK(sc.get(&rows, (size_t)n));
     iota_rows_kernel<<<ctx->num_sms * 4, 256, 0, st>>>(rows, n);
     ASP_CUDA(cudaGetLastError());
     ASP_LAUNCHED(ctx);
-    const int rc = knn_slow_rows(s, gp, distance, kk, rows, (int)n, lists);
-    cudaFreeAsync(rows, st);
+    const int rc = knn_slow_rows(s, gp, distance, kk, rows, (int)n, lists->idx, lists->dist, lists->cnt);
     ctx->stats["knn_stage1_ms"] = 0.0;
     ctx->stats["knn_slow_rows"] = (double)n;
     ctx->stats["knn_stage1_is_tc"] = 0.0;
@@ -649,11 +640,7 @@ int asp_item_knn(asp_space *s, const asp_graph_params *gp, int distance, asp_knn
     if (l2 && !small && !tc_ok)
         ASP_FAIL(ASP_ERR_UNSUPPORTED, "the Euclidean item graph on the tensor cores supports at most 6144 features (got %d)", s->f);
 
-    lists->m = n;
-    lists->kk = (int32_t)(kk > 0 ? kk : 1);
-    ASP_CUDA(cudaMallocAsync(&lists->idx, sizeof(int32_t) * (size_t)n * lists->kk, st));
-    ASP_CUDA(cudaMallocAsync(&lists->dist, sizeof(double) * (size_t)n * lists->kk, st));
-    ASP_CUDA(cudaMallocAsync(&lists->cnt, sizeof(int32_t) * (size_t)n, st));
+    ASP_CHECK(lists->alloc(st, n, (int32_t)(kk > 0 ? kk : 1)));
     ASP_CUDA(cudaMemsetAsync(lists->cnt, 0, sizeof(int32_t) * (size_t)n, st));
     ASP_CHECK(knn_row_norms(s, distance));
     if (kk == 0) return ASP_OK;
@@ -674,11 +661,7 @@ int asp_item_knn_rows_impl(asp_space *s, const asp_graph_params *gp, int distanc
     if (row_begin < 0 || row_end > n || rows < 0) ASP_FAIL(ASP_ERR_ARG, "row range [%lld, %lld) outside [0, %lld)", (long long)row_begin, (long long)row_end, (long long)n);
     if (kk < 1 || kk + 1 > 31 || n >= 2147483647LL || s->fp > 6144)
         ASP_FAIL(ASP_ERR_UNSUPPORTED, "the row-range item graph needs 1 <= k <= 30 (got %lld) and <= 6144 features", (long long)gp->k);
-    lists->m = rows;
-    lists->kk = (int32_t)kk;
-    ASP_CUDA(cudaMallocAsync(&lists->idx, sizeof(int32_t) * (size_t)(rows > 0 ? rows : 1) * lists->kk, st));
-    ASP_CUDA(cudaMallocAsync(&lists->dist, sizeof(double) * (size_t)(rows > 0 ? rows : 1) * lists->kk, st));
-    ASP_CUDA(cudaMallocAsync(&lists->cnt, sizeof(int32_t) * (size_t)(rows > 0 ? rows : 1), st));
+    ASP_CHECK(lists->alloc(st, rows, (int32_t)kk));
     ASP_CUDA(cudaMemsetAsync(lists->cnt, 0, sizeof(int32_t) * (size_t)(rows > 0 ? rows : 1), st));
     ASP_CHECK(knn_row_norms(s, distance));
     if (rows == 0) return ASP_OK;

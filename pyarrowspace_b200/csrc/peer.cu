@@ -179,8 +179,9 @@ int asp_peer_merge(asp_ctx *ctx, int world, int rank, const uint64_t *peer_bases
     while (p2 < world * topk) p2 <<= 1;
     const size_t smem = (size_t)p2 * sizeof(PKey);
     if (smem > 200 * 1024) ASP_FAIL(ASP_ERR_UNSUPPORTED, "peer merge of %d x %lld entries does not fit in shared memory", world, (long long)topk);
+    asp_scratch sc(st);
     unsigned int *scratch = nullptr;                                    // [0] block counter of the scatter, [1] status
-    ASP_CUDA(cudaMallocAsync(&scratch, 2 * sizeof(unsigned int), st));
+    ASP_CHECK(sc.get(&scratch, 2));
     ASP_CUDA(cudaMemsetAsync(scratch, 0, 2 * sizeof(unsigned int), st));
     const int parity = (int)(epoch & 1);
     const uint32_t e32 = (uint32_t)epoch;
@@ -202,7 +203,6 @@ int asp_peer_merge(asp_ctx *ctx, int world, int rank, const uint64_t *peer_bases
     int status = 0;
     ASP_CUDA(cudaMemcpyAsync(&status, scratch + 1, sizeof(int), cudaMemcpyDeviceToHost, st));
     ASP_CUDA(cudaStreamSynchronize(st));
-    cudaFreeAsync(scratch, st);
     if (status != 0) ASP_FAIL(ASP_ERR_CUDA, "asp_peer_merge: timed out waiting for the lists of the other ranks (epoch %lld)", (long long)epoch);
     return ASP_OK;
 }

@@ -301,25 +301,6 @@ __global__ void merge_pass_kernel(int nseg, const int64_t *__restrict__ segs, in
     }
 }
 
-// stream-ordered scratch, released on every exit path
-struct Scratch {
-    cudaStream_t st;
-    std::vector<void *> ptrs;
-    template <typename T> int get(T **out, size_t count)
-    {
-        void *p = nullptr;
-        if (cudaMallocAsync(&p, sizeof(T) * (count ? count : 1), st) != cudaSuccess) {
-            cudaGetLastError();
-            asp_set_error("out of device memory in the range search (%zu bytes)", sizeof(T) * count);
-            return ASP_ERR_NOMEM;
-        }
-        ptrs.push_back(p);
-        *out = static_cast<T *>(p);
-        return ASP_OK;
-    }
-    ~Scratch() { for (void *p : ptrs) cudaFreeAsync(p, st); }
-};
-
 template <int QPB, bool FILL, bool FILTER>
 int launch_scan(const asp_space *s, const double *q_dev, int32_t qpitch, const int32_t *list, int nslow, int nparts,
                 const double *lam_dev, const double *norm_dev, double tau, double min_score, const uint32_t *allowed,
@@ -382,7 +363,7 @@ int sort_segments(asp_ctx *ctx, int64_t nq, const int64_t *h_off, const int64_t 
         ASP_LAUNCHED(ctx);
     }
     if (segs.empty()) return ASP_OK;
-    Scratch sc{st, {}};
+    asp_scratch sc(st);
     int64_t *d_segs = nullptr, *d_blocks = nullptr, *t_idx = nullptr;
     double *t_score = nullptr;
     ASP_CHECK(sc.get(&d_segs, segs.size()));
@@ -430,7 +411,7 @@ int asp_range_merge_impl(asp_ctx *ctx, int parts, int64_t nq, const int64_t *h_c
     std::vector<int64_t> part_off((size_t)parts * (nq + 1)), out_off((size_t)nq + 1);
     const int64_t total = asp_range::merge_tables(parts, nq, h_counts, part_off.data(), out_off.data());
     if (total == 0) return ASP_OK;
-    Scratch sc{st, {}};
+    asp_scratch sc(st);
     int64_t *d_po = nullptr, *d_oo = nullptr;
     ASP_CHECK(sc.get(&d_po, part_off.size()));
     ASP_CHECK(sc.get(&d_oo, out_off.size()));
@@ -446,17 +427,16 @@ int asp_range_merge_impl(asp_ctx *ctx, int parts, int64_t nq, const int64_t *h_c
 
 int asp_range_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lam_dev, const double *norm_dev,
                    double tau, double min_score, const uint32_t *allowed_dev, int64_t max_hits, int64_t hits_before, int64_t q_base,
-                   int64_t *h_counts, int64_t **out_idx, double **out_score, int64_t *out_nnz)
+                   int64_t *h_counts, asp_range_result::Piece *out)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
-    *out_idx = nullptr; *out_score = nullptr; *out_nnz = 0;
     if (nq == 0) return ASP_OK;
     // the f32 emission floor: from a value inside [-2, 2] (every score lies in [-1, 1] for tau in [0, 1]; > 1 gives empty rows)
     const double emit_floor = std::min(2.0, std::max(-2.0, min_score));
     bool use_tc = tau > 1e-3 && tau <= 1.0 && s->fp <= 6144 && s->n_local >= 1 && s->n_local < 2147483647LL;
     if (const char *e = getenv("ASP_RANGE_STAGE1")) { if (e[0] == 's') use_tc = false; }   // test knob: both routes, same bits
-    Scratch sc{st, {}};
+    asp_scratch sc(st);
     int64_t *d_counts = nullptr, *d_off = nullptr;
     int32_t *slow_list = nullptr, *slow_count = nullptr;
     ASP_CHECK(sc.get(&d_counts, nq));
@@ -466,7 +446,6 @@ int asp_range_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t 
     ASP_CUDA(cudaMemsetAsync(d_counts, 0, sizeof(int64_t) * nq, st));
     ASP_CUDA(cudaMemsetAsync(slow_count, 0, sizeof(int32_t), st));
     asp_tc_batch b;
-    struct BatchGuard { asp_ctx *c; asp_tc_batch *b; ~BatchGuard() { asp_tc_batch_free(c, b); } } guard{ctx, &b};
     double *exact = nullptr;
     int nslow = 0;
     float ms1 = 0.f;
@@ -517,15 +496,12 @@ int asp_range_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t 
     ctx->stats["search_slow_queries"] += nslow;
     if (run > 0) {
         ASP_CUDA(cudaMemcpyAsync(d_off, h_off.data(), sizeof(int64_t) * (nq + 1), cudaMemcpyHostToDevice, st));
+        out->mem = asp_scratch(st);                               // the hits belong to the caller's piece
         int64_t *didx = nullptr;
         double *dsc = nullptr;
-        if (cudaMallocAsync(&didx, sizeof(int64_t) * (size_t)run, st) != cudaSuccess ||
-            cudaMallocAsync(&dsc, sizeof(double) * (size_t)run, st) != cudaSuccess) {
-            cudaGetLastError();
-            if (didx) cudaFreeAsync(didx, st);
-            ASP_FAIL(ASP_ERR_NOMEM, "out of device memory for %lld range-search hits", (long long)run);
-        }
-        *out_idx = didx; *out_score = dsc; *out_nnz = run;        // owned by the caller from here on
+        ASP_CHECK(out->mem.get(&didx, (size_t)run));
+        ASP_CHECK(out->mem.get(&dsc, (size_t)run));
+        out->idx = didx; out->score = dsc; out->n = run;
         if (use_tc) {
             tc_range_fill_kernel<<<(unsigned)asp_ceil_div(nq, RW), RW * 32, 0, st>>>(nq, b.nsub, b.capb, b.emit_ix, b.emit_cnt, b.qperm,
                                                                                    exact, d_off, s->row0, didx, dsc);

@@ -319,11 +319,12 @@ int min2_all(asp_ctx *ctx, const double *XA, int pitchA, const int32_t *a_rows, 
     if (a_tiles > 2147483647LL || nsplit > 65535) ASP_FAIL(ASP_ERR_UNSUPPORTED, "reduction: too many rows for one launch");
     const int64_t per = asp_ceil_div(asp_ceil_div(nb, nsplit), tb) * tb;
     nsplit = asp_ceil_div(nb, per);
+    asp_scratch sc(ctx->stream);
     double *pd = fin_d;
     int32_t *pi = fin_i;
     if (nsplit > 1) {
-        ASP_CUDA(cudaMallocAsync(&pd, sizeof(double) * 2 * na * nsplit, ctx->stream));
-        ASP_CUDA(cudaMallocAsync(&pi, sizeof(int32_t) * 2 * na * nsplit, ctx->stream));
+        ASP_CHECK(sc.get(&pd, 2 * (size_t)na * nsplit));
+        ASP_CHECK(sc.get(&pi, 2 * (size_t)na * nsplit));
     }
     const dim3 grid((unsigned)a_tiles, (unsigned)nsplit);
     if (jb == 4) launch_min2<4>(ctx->stream, grid, XA, pitchA, a_rows, na, XB, pitchB, b_rows, nb, per, excl, fp, pd, pi);
@@ -335,30 +336,9 @@ int min2_all(asp_ctx *ctx, const double *XA, int pitchA, const int32_t *a_rows, 
         min2_merge_splits_kernel<<<(unsigned)asp_ceil_div(na, 256), 256, 0, ctx->stream>>>(pd, pi, (int)nsplit, na, fin_d, fin_i);
         ASP_LAUNCHED(ctx);
         ASP_CUDA(cudaGetLastError());
-        ASP_CUDA(cudaFreeAsync(pd, ctx->stream));
-        ASP_CUDA(cudaFreeAsync(pi, ctx->stream));
     }
     return ASP_OK;
 }
-
-struct DevBuf {                                           // stream-ordered scratch released on scope exit
-    cudaStream_t st;
-    std::vector<void *> ptrs;
-    explicit DevBuf(cudaStream_t s) : st(s) {}
-    template <typename T> int get(T **out, size_t count)
-    {
-        void *p = nullptr;
-        if (cudaMallocAsync(&p, sizeof(T) * (count ? count : 1), st) != cudaSuccess) {
-            cudaGetLastError();
-            asp_set_error("out of device memory in the reduction (%zu bytes)", sizeof(T) * count);
-            return ASP_ERR_NOMEM;
-        }
-        ptrs.push_back(p);
-        *out = static_cast<T *>(p);
-        return ASP_OK;
-    }
-    ~DevBuf() { for (void *p : ptrs) cudaFreeAsync(p, st); }
-};
 
 }  // namespace
 
@@ -406,7 +386,7 @@ int asp_space_reduce(asp_space *s, const asp_reduction *red_in, int64_t n_total_
     asp_ctx *ctx = s->ctx;
     ASP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    DevBuf scratch(st);
+    asp_scratch scratch(st);
     const int fp = s->fp;
     const int64_t n = s->n_local;
 

@@ -413,13 +413,14 @@ int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev,
     const double delta = (4.0 * f + 64.0) * u * (fabs(tau) + fabs(1.0 - tau) + 1.0);
 
     // 1/norm of the queries
+    asp_scratch sc(st);
     double *inv_nq = nullptr;
-    ASP_CUDA(cudaMallocAsync(&inv_nq, sizeof(double) * nq, st));
+    ASP_CHECK(sc.get(&inv_nq, (size_t)nq));
     ASP_CHECK(asp_launch_reciprocal(ctx, qnorm_dev, nq, inv_nq));
 
     int32_t *slow_list = nullptr, *slow_count = nullptr;
-    ASP_CUDA(cudaMallocAsync(&slow_list, sizeof(int32_t) * (nq + 1), st));
-    ASP_CUDA(cudaMallocAsync(&slow_count, sizeof(int32_t), st));
+    ASP_CHECK(sc.get(&slow_list, (size_t)nq + 1));
+    ASP_CHECK(sc.get(&slow_count, 1));
     ASP_CUDA(cudaMemsetAsync(slow_count, 0, sizeof(int32_t), st));
 
     int nparts = 0;
@@ -429,8 +430,8 @@ int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev,
     if (nq <= GV_MAXQ && f <= 1536) {            // the GEMV kernel keeps a query in registers: wider vectors take the DMMA tile kernel
         int64_t want = asp_ceil_div(s->n_local, GV_WARPS * 16);
         nparts = (int)(want < ctx->num_sms * 2 ? (want > 0 ? want : 1) : ctx->num_sms * 2);
-        ASP_CUDA(cudaMallocAsync(&cand_score, sizeof(double) * (size_t)nq * nparts * LISTSEL, st));
-        ASP_CUDA(cudaMallocAsync(&cand_idx, sizeof(int32_t) * (size_t)nq * nparts * LISTSEL, st));
+        ASP_CHECK(sc.get(&cand_score, (size_t)nq * nparts * LISTSEL));
+        ASP_CHECK(sc.get(&cand_idx, (size_t)nq * nparts * LISTSEL));
         auto gemv = [&](auto list, auto filter) {
             return launch_gemv<decltype(list)::value, decltype(filter)::value>(s, q_dev, qpitch, (int)nq, inv_nq, lambda_q_dev, tau,
                                                                                nparts, cand_score, cand_idx, allowed);
@@ -457,8 +458,8 @@ int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev,
         nparts = (int)best_chunks;
         CUtensorMap tmap_q;
         ASP_CHECK(asp_make_items_tmap(&tmap_q, q_dev, nq, qpitch, QT, KSTEP / 4));
-        ASP_CUDA(cudaMallocAsync(&cand_score, sizeof(double) * (size_t)nq * nparts * LISTSEL, st));
-        ASP_CUDA(cudaMallocAsync(&cand_idx, sizeof(int32_t) * (size_t)nq * nparts * LISTSEL, st));
+        ASP_CHECK(sc.get(&cand_score, (size_t)nq * nparts * LISTSEL));
+        ASP_CHECK(sc.get(&cand_idx, (size_t)nq * nparts * LISTSEL));
         auto gemm = [&](auto list, auto filter) {
             return launch_gemm<decltype(list)::value, decltype(filter)::value>(s, tmap_q, q_dev, nq, inv_nq, lambda_q_dev, tau,
                                                                                nparts, cand_score, cand_idx, allowed);
@@ -500,11 +501,6 @@ int asp_search_impl(const asp_space *s, const asp_graph *g, const double *q_dev,
     if (nslow > 0)
         ASP_CHECK(asp_search_slow_path(s, q_dev, qpitch, lambda_q_dev, qnorm_dev, tau, topk, slow_list, nslow, out_idx_dev,
                                        out_score_dev, allowed));
-    ASP_CUDA(cudaFreeAsync(cand_score, st));
-    ASP_CUDA(cudaFreeAsync(cand_idx, st));
-    ASP_CUDA(cudaFreeAsync(slow_list, st));
-    ASP_CUDA(cudaFreeAsync(slow_count, st));
-    ASP_CUDA(cudaFreeAsync(inv_nq, st));
     return ASP_OK;
 }
 

@@ -52,6 +52,7 @@
 #include <cuda_fp16.h>
 #include <algorithm>
 #include <math.h>
+#include <memory>
 #include <stdlib.h>
 
 namespace {
@@ -1035,19 +1036,20 @@ struct asp_tc_cache {               // per-space fp16 operands in lambda order, 
     CUtensorMap map_hi, map_lo, map_hi_half;      // boxes of 256 item rows; 128 for the CTA-pair kernel
     CUtensorMap map_hi_nw;                        // narrow box (16 | 32 halves) over the last k block, see TcParams::nw_hi
     int nw = 0;
+    asp_scratch mem;                // owns hi, lo, lam32, tile_lo, tile_hi, perm, mdir
 };
 
 int asp_device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out)
 {
     cudaStream_t st = ctx->stream;
+    asp_scratch sc(st);
     double *d_mm = nullptr;
     std::vector<double> h_mm(512);
-    ASP_CUDA(cudaMallocAsync(&d_mm, sizeof(double) * 512, st));
+    ASP_CHECK(sc.get(&d_mm, 512));
     minmax_kernel<<<256, 256, 0, st>>>(v_dev, n, d_mm);
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
     ASP_CUDA(cudaMemcpyAsync(h_mm.data(), d_mm, sizeof(double) * 512, cudaMemcpyDeviceToHost, st));
     ASP_CUDA(cudaStreamSynchronize(st));
-    ASP_CUDA(cudaFreeAsync(d_mm, st));
     double hi = 0.0;
     for (int i = 0; i < 256; ++i) hi = fmax(hi, h_mm[2 * i + 1]);
     *out = hi;
@@ -1059,10 +1061,11 @@ int asp_device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out)
 static int bucket_order(asp_ctx *ctx, const double *keys_dev, int64_t n, int32_t *perm_dev)
 {
     cudaStream_t st = ctx->stream;
+    asp_scratch sc(st);
     double *scratch = nullptr;                                              // [256][2] partials + [2] range
     uint32_t *cursor = nullptr;
-    ASP_CUDA(cudaMallocAsync(&scratch, sizeof(double) * 514, st));
-    ASP_CUDA(cudaMallocAsync(&cursor, sizeof(uint32_t) * LAM_BUCKETS, st));
+    ASP_CHECK(sc.get(&scratch, 514));
+    ASP_CHECK(sc.get(&cursor, LAM_BUCKETS));
     ASP_CUDA(cudaMemsetAsync(cursor, 0, sizeof(uint32_t) * LAM_BUCKETS, st));
     const int grid = (int)(asp_ceil_div(n, 256) < ctx->num_sms * 4 ? asp_ceil_div(n, 256) : ctx->num_sms * 4);
     minmax_kernel<<<256, 256, 0, st>>>(keys_dev, n, scratch);
@@ -1075,8 +1078,6 @@ static int bucket_order(asp_ctx *ctx, const double *keys_dev, int64_t n, int32_t
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
     bucket_scatter_kernel<<<grid, 256, 0, st>>>(keys_dev, n, scratch + 512, cursor, perm_dev);
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
-    ASP_CUDA(cudaFreeAsync(scratch, st));
-    ASP_CUDA(cudaFreeAsync(cursor, st));
     return ASP_OK;
 }
 
@@ -1100,20 +1101,22 @@ static int ensure_tc_cache(const asp_space *s, bool by_norm, asp_tc_cache **out)
     }
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
-    asp_tc_cache *c = new asp_tc_cache();
+    std::unique_ptr<asp_tc_cache> c(new asp_tc_cache());           // the space holds it once it is complete
+    c->mem = asp_scratch(st);
     c->kp = (s->f + 3 + TKB - 1) / TKB * TKB;
     const int64_t n = s->n_local;
     const size_t ne = (size_t)n * c->kp;
     const int64_t ntile = asp_ceil_div(n, TN);
+    asp_scratch tmp(st);
     double *partials = nullptr, *rho = nullptr;
-    ASP_CUDA(cudaMallocAsync(&c->hi, ne * 2, st));
-    ASP_CUDA(cudaMallocAsync(&c->lam32, sizeof(float) * n, st));
-    ASP_CUDA(cudaMallocAsync(&c->perm, sizeof(int32_t) * n, st));
-    ASP_CUDA(cudaMallocAsync(&c->tile_lo, sizeof(float) * ntile, st));
-    ASP_CUDA(cudaMallocAsync(&c->tile_hi, sizeof(float) * ntile, st));
-    ASP_CUDA(cudaMallocAsync(&c->mdir, sizeof(double) * s->f, st));
-    ASP_CUDA(cudaMallocAsync(&partials, sizeof(double) * (size_t)MD_BLOCKS * s->f, st));
-    ASP_CUDA(cudaMallocAsync(&rho, sizeof(double) * n, st));
+    ASP_CHECK(c->mem.get(&c->hi, ne));
+    ASP_CHECK(c->mem.get(&c->lam32, (size_t)n));
+    ASP_CHECK(c->mem.get(&c->perm, (size_t)n));
+    ASP_CHECK(c->mem.get(&c->tile_lo, (size_t)ntile));
+    ASP_CHECK(c->mem.get(&c->tile_hi, (size_t)ntile));
+    ASP_CHECK(c->mem.get(&c->mdir, (size_t)s->f));
+    ASP_CHECK(tmp.get(&partials, (size_t)MD_BLOCKS * s->f));
+    ASP_CHECK(tmp.get(&rho, (size_t)n));
     // visiting order: bucket sort of the shard by lambda (identity while the space has no lambdas: item graph), or by norm
     c->order = by_norm ? ASP_TC_ORDER_NORM : s->have_lambdas ? ASP_TC_ORDER_LAMBDA : ASP_TC_ORDER_IDENTITY;
     if (c->order != ASP_TC_ORDER_IDENTITY) ASP_CHECK(bucket_order(ctx, by_norm ? s->norms : s->lambdas, n, c->perm));
@@ -1136,8 +1139,6 @@ static int ensure_tc_cache(const asp_space *s, bool by_norm, asp_tc_cache **out)
         ASP_CUDA(cudaMemsetAsync(c->tile_lo, 0, sizeof(float) * ntile, st));
         ASP_CUDA(cudaMemsetAsync(c->tile_hi, 0, sizeof(float) * ntile, st));
     }
-    ASP_CUDA(cudaFreeAsync(partials, st));
-    ASP_CUDA(cudaFreeAsync(rho, st));
     ASP_CHECK(asp_make_f16_tmap(&c->map_hi, c->hi, n, c->kp, TN));
     ASP_CHECK(asp_make_f16_tmap(&c->map_hi_half, c->hi, n, c->kp, TN / 2));
     c->map_lo = c->map_hi;
@@ -1148,8 +1149,8 @@ static int ensure_tc_cache(const asp_space *s, bool by_norm, asp_tc_cache **out)
         c->map_hi_nw = c->map_hi;
         if (c->nw) ASP_CHECK(asp_make_f16_tmap_narrow(&c->map_hi_nw, c->hi, n, c->kp, TN, c->nw));
     }
-    ms->tc_cache = c;
-    *out = c;
+    *out = c.release();
+    ms->tc_cache = *out;
     return ASP_OK;
 }
 
@@ -1159,26 +1160,20 @@ static int ensure_tc_lo(const asp_space *s, asp_tc_cache *c)
     if (c->lo) return ASP_OK;
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
+    asp_scratch tmp(st);
     double *rho = nullptr;
-    ASP_CUDA(cudaMallocAsync(&c->lo, (size_t)s->n_local * c->kp * 2, st));
-    ASP_CUDA(cudaMallocAsync(&rho, sizeof(double) * s->n_local, st));
+    ASP_CHECK(c->mem.get(&c->lo, (size_t)s->n_local * c->kp));
+    ASP_CHECK(tmp.get(&rho, (size_t)s->n_local));
     project_split_kernel<<<ctx->num_sms * 8, 256, 0, st>>>(s->items, s->n_local, s->f, s->fp, c->kp, s->inv_norms, c->perm, c->mdir, 0,
                                                           c->hi, c->lo, rho);
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
-    ASP_CUDA(cudaFreeAsync(rho, st));
     ASP_CHECK(asp_make_f16_tmap(&c->map_lo, c->lo, s->n_local, c->kp, TN));
     return ASP_OK;
 }
 
 void asp_free_tc_cache(asp_space *s)
 {
-    if (!s->tc_cache) return;
-    asp_tc_cache *c = static_cast<asp_tc_cache *>(s->tc_cache);
-    cudaStream_t st = s->ctx->stream;
-    cudaFreeAsync(c->hi, st); if (c->lo) cudaFreeAsync(c->lo, st); cudaFreeAsync(c->lam32, st); cudaFreeAsync(c->perm, st);
-    cudaFreeAsync(c->mdir, st);
-    cudaFreeAsync(c->tile_lo, st); cudaFreeAsync(c->tile_hi, st);
-    delete c;
+    delete static_cast<asp_tc_cache *>(s->tc_cache);
     s->tc_cache = nullptr;
 }
 
@@ -1208,23 +1203,24 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     if (l2) { lambda_q_dev = qnorm_dev; tau = 1.0; }
     const int kp = c->kp;
     *b = asp_tc_batch();
+    b->mem = asp_scratch(st);
     b->nq = nq;
 
     __half *q_hi = nullptr, *q_lo = nullptr;
     const int64_t qblocks = asp_ceil_div(nq, TQ);
-    ASP_CUDA(cudaMallocAsync(&q_hi, (size_t)nq * kp * 2, st));
-    ASP_CUDA(cudaMallocAsync(&q_lo, (size_t)nq * kp * 2, st));
+    ASP_CHECK(b->mem.get(&q_hi, (size_t)nq * kp));
+    ASP_CHECK(b->mem.get(&q_lo, (size_t)nq * kp));
     b->q_hi = q_hi; b->q_lo = q_lo;
-    ASP_CUDA(cudaMallocAsync(&b->lam_q32, sizeof(float) * nq, st));
-    ASP_CUDA(cudaMallocAsync(&b->inv_nq, sizeof(double) * nq, st));
-    ASP_CUDA(cudaMallocAsync(&b->rho_q, sizeof(double) * nq, st));
-    ASP_CUDA(cudaMallocAsync(&b->delta_q, sizeof(float) * nq, st));
+    ASP_CHECK(b->mem.get(&b->lam_q32, (size_t)nq));
+    ASP_CHECK(b->mem.get(&b->inv_nq, (size_t)nq));
+    ASP_CHECK(b->mem.get(&b->rho_q, (size_t)nq));
+    ASP_CHECK(b->mem.get(&b->delta_q, (size_t)nq));
     ASP_CHECK(asp_launch_reciprocal(ctx, qnorm_dev, nq, b->inv_nq));
     const bool by_lambda = !dump_dev && lambda_q_dev && c->order != ASP_TC_ORDER_IDENTITY;   // (l2: by the query norms)
     if (by_lambda) {
         // queries visited in lambda_q order: coherent blocks -> one visiting order per block
-        ASP_CUDA(cudaMallocAsync(&b->qperm, sizeof(int32_t) * nq, st));
-        ASP_CUDA(cudaMallocAsync(&b->center, sizeof(int32_t) * qblocks, st));
+        ASP_CHECK(b->mem.get(&b->qperm, (size_t)nq));
+        ASP_CHECK(b->mem.get(&b->center, (size_t)qblocks));
         if (nq > TQ) ASP_CHECK(bucket_order(ctx, lambda_q_dev, nq, b->qperm));
         else {              // one query block: its visiting order starts at one of its own lambdas whatever the query order
             iota_kernel<<<1, 128, 0, st>>>(b->qperm, nq);
@@ -1311,17 +1307,17 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     p.theta_glob = nullptr; p.emit_sc = nullptr; p.emit_ix = nullptr; p.emit_cnt = nullptr; p.dump = dump_dev; p.vbits = nullptr;
     if (allowed_dev) {                                            // from the cache's current order (it may have been rebuilt)
         const int64_t nwords = tiles_total * (TN / 32);
-        ASP_CUDA(cudaMallocAsync(&b->vbits, sizeof(uint32_t) * (size_t)nwords, st));
+        ASP_CHECK(b->mem.get(&b->vbits, (size_t)nwords));
         visit_bits_kernel<<<(unsigned)std::min<int64_t>(asp_ceil_div(nwords, 8), (int64_t)ctx->num_sms * 8), 256, 0, st>>>(
             allowed_dev, c->perm, s->n_local, nwords, b->vbits);
         ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
         p.vbits = b->vbits;
     }
     if (!dump_dev) {
-        ASP_CUDA(cudaMallocAsync(&b->emit_sc, sizeof(float) * (size_t)nq * nchunks * capb, st));
-        ASP_CUDA(cudaMallocAsync(&b->emit_ix, sizeof(int32_t) * (size_t)nq * nchunks * capb, st));
-        ASP_CUDA(cudaMallocAsync(&b->emit_cnt, sizeof(int32_t) * (size_t)nq * nchunks, st));
-        ASP_CUDA(cudaMallocAsync(&b->theta_glob, sizeof(uint32_t) * (size_t)nq, st));
+        ASP_CHECK(b->mem.get(&b->emit_sc, (size_t)nq * nchunks * capb));
+        ASP_CHECK(b->mem.get(&b->emit_ix, (size_t)nq * nchunks * capb));
+        ASP_CHECK(b->mem.get(&b->emit_cnt, (size_t)nq * nchunks));
+        ASP_CHECK(b->mem.get(&b->theta_glob, (size_t)nq));
         ASP_CUDA(cudaMemsetAsync(b->theta_glob, 0, sizeof(uint32_t) * (size_t)nq, st));
         p.emit_sc = b->emit_sc; p.emit_ix = b->emit_ix; p.emit_cnt = b->emit_cnt; p.theta_glob = b->theta_glob;
     }
@@ -1393,16 +1389,6 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     return ASP_OK;
 }
 
-void asp_tc_batch_free(asp_ctx *ctx, asp_tc_batch *b)
-{
-    cudaStream_t st = ctx->stream;
-    void *ptrs[] = {b->q_hi, b->q_lo, b->lam_q32, b->inv_nq, b->rho_q, b->delta_q, b->qperm, b->center,
-                    b->emit_sc, b->emit_ix, b->emit_cnt, b->theta_glob, b->vbits};
-    for (void *ptr : ptrs)
-        if (ptr) cudaFreeAsync(ptr, st);
-    *b = asp_tc_batch();
-}
-
 namespace {
 __global__ void gather_queries_kernel(const double *__restrict__ q, int qpitch, const double *__restrict__ lam, const double *__restrict__ nrm,
                                       const int32_t *__restrict__ list, int count, double *__restrict__ q2, double *__restrict__ lam2,
@@ -1456,7 +1442,7 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
     asp_tc_batch b;
     int rc = asp_tc_stage1(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, -INFINITY, force_terms, 0, dump_dev, &b, false,
                            allowed_dev);
-    if (rc != ASP_OK || dump_dev) { asp_tc_batch_free(ctx, &b); return rc; }
+    if (rc != ASP_OK || dump_dev) return rc;
 
     if (b.variant != 0) {                                         // profiling variants: stage 1 only, results are garbage
         ASP_CUDA(cudaStreamSynchronize(st));
@@ -1465,14 +1451,14 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
         ctx->stats["search_stage1_ms"] = ms;
         ASP_CUDA(cudaMemsetAsync(out_idx_dev, 0xff, sizeof(int64_t) * (size_t)nq * topk, st));
         ASP_CUDA(cudaMemsetAsync(out_score_dev, 0, sizeof(double) * (size_t)nq * topk, st));
-        asp_tc_batch_free(ctx, &b);
         return ASP_OK;
     }
+    asp_scratch sc(st);
     int32_t *slow_list = nullptr, *slow_count = nullptr;
     unsigned long long *counters = nullptr;
-    ASP_CUDA(cudaMallocAsync(&slow_list, sizeof(int32_t) * (nq + 1), st));
-    ASP_CUDA(cudaMallocAsync(&slow_count, sizeof(int32_t), st));
-    ASP_CUDA(cudaMallocAsync(&counters, 2 * sizeof(unsigned long long), st));
+    ASP_CHECK(sc.get(&slow_list, (size_t)nq + 1));
+    ASP_CHECK(sc.get(&slow_count, 1));
+    ASP_CHECK(sc.get(&counters, 2));
     ASP_CUDA(cudaMemsetAsync(slow_count, 0, sizeof(int32_t), st));
     ASP_CUDA(cudaMemsetAsync(counters, 0, 2 * sizeof(unsigned long long), st));
     const double u = 1.1102230246251565e-16;
@@ -1513,16 +1499,17 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
     const bool wide_band = b.nterms == 1 && b.delta_cos_max > 2.5e-4;   // the three-term split has a much tighter band to offer
     if (nslow > 0 && may_retry && wide_band) {
         const std::map<std::string, double> first_stats = ctx->stats;
+        asp_scratch retry(st);
         double *q2 = nullptr, *lam2 = nullptr, *nrm2 = nullptr, *sc2 = nullptr;
         int64_t *idx2 = nullptr;
-        ASP_CUDA(cudaMallocAsync(&q2, sizeof(double) * (size_t)nslow * qpitch, st));
-        ASP_CUDA(cudaMallocAsync(&lam2, sizeof(double) * nslow, st));
-        ASP_CUDA(cudaMallocAsync(&nrm2, sizeof(double) * nslow, st));
-        ASP_CUDA(cudaMallocAsync(&idx2, sizeof(int64_t) * (size_t)nslow * topk, st));
-        ASP_CUDA(cudaMallocAsync(&sc2, sizeof(double) * (size_t)nslow * topk, st));
+        ASP_CHECK(retry.get(&q2, (size_t)nslow * qpitch));
+        ASP_CHECK(retry.get(&lam2, (size_t)nslow));
+        ASP_CHECK(retry.get(&nrm2, (size_t)nslow));
+        ASP_CHECK(retry.get(&idx2, (size_t)nslow * topk));
+        ASP_CHECK(retry.get(&sc2, (size_t)nslow * topk));
         gather_queries_kernel<<<(unsigned)nslow, 128, 0, st>>>(q_dev, qpitch, lambda_q_dev, qnorm_dev, slow_list, nslow, q2, lam2, nrm2);
         ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
-        asp_tc_batch_free(ctx, &b);                                   // the retry allocates its own emission buffers
+        b.mem.release();                                              // the retry allocates its own emission buffers
         rc = search_tc_attempt(s, q2, nslow, qpitch, lam2, nrm2, tau, topk, idx2, sc2, nullptr, 3, false, allowed_dev);
         if (rc == ASP_OK) {
             scatter_results_kernel<<<(unsigned)nslow, 32, 0, st>>>(idx2, sc2, slow_list, nslow, (int)topk, out_idx_dev, out_score_dev);
@@ -1534,12 +1521,9 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
         ctx->stats["search_retry_queries"] = nslow;
         ctx->stats["search_retry_ms"] = retry_ms;
         ctx->stats["search_slow_queries"] = retry_slow;              // what finally took the exact scan
-        cudaFreeAsync(q2, st); cudaFreeAsync(lam2, st); cudaFreeAsync(nrm2, st); cudaFreeAsync(idx2, st); cudaFreeAsync(sc2, st);
     } else if (nslow > 0) {
         rc = asp_search_slow_path(s, q_dev, qpitch, lambda_q_dev, qnorm_dev, tau, topk, slow_list, nslow, out_idx_dev, out_score_dev,
                                   allowed_dev);
     }
-    cudaFreeAsync(slow_list, st); cudaFreeAsync(slow_count, st); cudaFreeAsync(counters, st);
-    asp_tc_batch_free(ctx, &b);
     return rc;
 }

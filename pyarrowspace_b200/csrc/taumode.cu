@@ -785,10 +785,10 @@ int asp_graph_upload_upper(asp_graph *g)
 {
     ASP_CHECK(asp_graph_host_mirror(g));
     TmBlob *b = new TmBlob();
+    g->tm_blob = b;                                                    // a partly built blob is freed like a complete one
     const int rc = build_tm_blob(g->ctx, g, b);
-    if (rc != ASP_OK) { delete b; return rc; }
-    g->tm_blob = b;
-    return ASP_OK;
+    if (rc != ASP_OK) asp_graph_free_upper(g);
+    return rc;
 }
 
 void asp_graph_free_upper(asp_graph *g)
