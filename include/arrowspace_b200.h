@@ -200,6 +200,7 @@ int asp_query_lambda(asp_ctx *ctx, const asp_graph *g, const asp_switches *sw, c
  * kernel (nq <= 8) otherwise; env ASP_SEARCH_STAGE1=fp64|tc forces one.  The answers are bit-identical whichever
  * stage 1 produced the candidates.  topk >= 32 is answered by the batched exact scan of every query (reference-order score of
  * every item; ~3300 queries/s at 1M x 384: the completeness test needs one kept candidate beyond the k-th and the kernels keep 32).
+ * asp_search_batch_k with k = 32 .. 64 keeps such lists on the tensor cores.
  * queries / outputs may be host or device memory.  Host batches of >= 32768 queries are processed in two pieces so that
  * the PCIe copies run under the kernels (env ASP_NO_PIPELINE=1: single shot); the result is the same either way.
  * One caller per ctx at a time (the reference holds the GIL for the whole call, src/lib.rs:132).
@@ -217,6 +218,19 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
  * asp_topk_merge as they are. */
 int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                               int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits);
+
+/* Search with a per-call k: asp_search_batch_filtered returning k hits per query instead of gl.graph_params.topk, so a
+ * different k needs no rebuild (under topk_prunes a rebuild would also change the graph and every lambda).  out_idx /
+ * out_score are [nq][k], padded with -1 / NaN when fewer than k items exist or are allowed; allowed_bits NULL = every row.
+ * 1 <= k <= 1024 (k < 1: ASP_ERR_ARG; k > 1024, the exact scan's list length: ASP_ERR_UNSUPPORTED).  Same answers, bit for
+ * bit, as asp_search_batch on a graph of topk = k.  Route: k <= 31 as asp_search_batch; 32 <= k <= 64 stays on the tcgen05
+ * candidate pass (64-entry running lists) with a wide stage 2 of one CTA per query that keeps every survivor of the
+ * cut (csrc/large_k.cuh), on the tensor-core pass's conditions (0.001 < tau <= 1, <= 6144 features, nq >= 256 or >= 131072
+ * items); k > 64 (a 128-entry list spills registers in stage 1) and everything else take the batched exact scan.  The graph-topk entry points keep their routes: a graph
+ * topk >= 32 there still takes the exact scan; moving them onto the wide route is a separate change that needs its own
+ * B200 measurements. */
+int asp_search_batch_k(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t k,
+                       int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits);
 
 /* Hybrid search, batched (SURVEY.md 8(f)-2).  Replaces prepare_query_item + search_lambda_aware_hybrid(&query,
  * gl.graph_params.topk, tau) of ArrowSpace.search_hybrid (src/lib.rs:182-219).  The crate function's body is not in the
@@ -242,6 +256,12 @@ int asp_search_hybrid_batch_filtered(const asp_space *s, const asp_graph *g, con
                                      int64_t pool, int64_t *out_idx, double *out_score, double *out_lambda_q,
                                      const uint8_t *allowed_bits);
 
+/* Hybrid search with a per-call k: k replaces gl.graph_params.topk in H2 and H3 (pool <= 0: asp_hybrid_pool(n, k, 0) =
+ * min(2k, 31) raised to k), outputs [nq][k].  k as in asp_search_batch_k; shortlists of up to 64 stay on the tensor-core
+ * route.  allowed_bits NULL = every row. */
+int asp_search_hybrid_batch_k(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                              int64_t k, int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits);
+
 /* The shortlist length m of H2 for n_total items: pool (<= 0: min(2 * topk, 31)), raised to topk, cut to n_total.
  * m == n_total (with n_total > 0) means no shortlist: the whole set. */
 int64_t asp_hybrid_pool(int64_t n_total, int64_t topk, int64_t pool);
@@ -265,6 +285,11 @@ int asp_search_hybrid_shard(const asp_space *s, const asp_graph *g, const double
 int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                                      int64_t pool, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q,
                                      const uint8_t *allowed_bits);
+/* The same with a per-call k in place of gl.graph_params.topk (m = asp_hybrid_pool(n_total, k, pool); [nq][k] lists when
+ * m == n_total), k as in asp_search_batch_k; merge with asp_hybrid_merge / asp_topk_merge at list width k. */
+int asp_search_hybrid_shard_k(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                              int64_t k, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q,
+                              const uint8_t *allowed_bits);
 int asp_hybrid_merge(asp_ctx *ctx, const int64_t *idx, const double *cos, const double *score, int parts, int64_t nq,
                      int64_t m, int64_t topk, int64_t *out_idx, double *out_score);
 

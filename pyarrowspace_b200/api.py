@@ -75,6 +75,21 @@ def _check_allowed(allowed, nitems):
     return allowed
 
 
+# Longest per-call k: the list length the batched exact scan keeps per query (asp_xs::TOPK_MAX, asp_search_batch_k).
+K_MAX = 1024
+
+
+def _check_k(k):
+    """The `k=` argument of the searches: None (the graph's topk, today's call), or an integer 1 <= k <= K_MAX."""
+    if k is None:
+        return None
+    if isinstance(k, bool) or not isinstance(k, (int, np.integer)) or k < 1:
+        raise ValueError("k must be a positive integer (the number of results per query)")
+    if k > K_MAX:
+        raise LibraryError(_lib.ASP_ERR_UNSUPPORTED, "k = %d is beyond the %d results the exact scan keeps per query" % (k, K_MAX))
+    return int(k)
+
+
 # Default cap of a range search: 2**26 hits, 1 GiB of results (int64 index + f64 score) -- a threshold far below the
 # scores of a data set would otherwise ask for every item of every query.  max_results= raises or lowers it.
 DEFAULT_MAX_RESULTS = 1 << 26
@@ -336,16 +351,19 @@ class ArrowSpace:
         dbg_println("search: qlen=%d, lambda_q=%.6f" % (item.shape[0], lam_q[0]))
         return [(int(i), float(s)) for i, s in zip(idx[0], score[0]) if i >= 0]
 
-    def search_batch(self, queries, gl, tau, out=None, *, allowed=None):
+    def search_batch(self, queries, gl, tau, out=None, *, allowed=None, k=None):
         """Extension: (idx int64[Q, topk], score f64[Q, topk]); rows padded with -1 / NaN.
         out = (idx, score) host arrays to fill (C-contiguous, right shapes / dtypes; e.g. pinned memory that the caller
         reuses from call to call: the device -> host read then runs at the PCIe rate instead of the page-fault rate of
         freshly allocated memory).  Host query batches only.
         allowed = numpy bool[nitems] (keyword only): per query the best topk among the allowed items, padded with -1 / NaN
-        when fewer are allowed; the same mask for every query.  Collective calls: every rank passes the same mask."""
+        when fewer are allowed; the same mask for every query.  Collective calls: every rank passes the same mask.
+        k = int (keyword only, 1 .. 1024): k results per query instead of gl.graph_params["topk"] (no rebuild; the answer is
+        the one a graph of topk = k gives, bit for bit); out shapes are then (Q, k).  k = None is the graph's topk."""
         allowed = _check_allowed(allowed, self.nitems)
+        k = _check_k(k)
         if out is not None:
-            topk = gl.graph_params["topk"]
+            topk = gl.graph_params["topk"] if k is None else k
             nq = queries.shape[0]
             oi, os_ = out
             if not (isinstance(oi, np.ndarray) and isinstance(os_, np.ndarray) and oi.dtype == np.int64 and os_.dtype == np.float64
@@ -353,7 +371,7 @@ class ArrowSpace:
                 raise ValueError("out must be (int64[%d, %d], float64[%d, %d]) C-contiguous host arrays" % (nq, topk, nq, topk))
             if _is_device_tensor(queries):
                 raise ValueError("out= is for host query batches (device batches return device tensors)")
-        idx, score, _ = self._search_batch(queries, gl, float(tau), want_lambda=False, out=out, allowed=allowed)
+        idx, score, _ = self._search_batch(queries, gl, float(tau), want_lambda=False, out=out, allowed=allowed, k=k)
         return idx, score
 
     def _allowed_bits(self, allowed):
@@ -364,14 +382,14 @@ class ArrowSpace:
         n_local, _, row0, _ = self._dims()
         return pack_allowed(allowed, row0, n_local)
 
-    def _search_batch(self, queries, gl, tau, want_lambda, out=None, allowed=None):
+    def _search_batch(self, queries, gl, tau, want_lambda, out=None, allowed=None, k=None):
         import time
         if self._grid is not None and self._grid["C"] > 1:
-            return self._search_batch_grid(queries, gl, tau, out, allowed)
+            return self._search_batch_grid(queries, gl, tau, out, allowed, k)
         t_a = time.perf_counter()
         lib = _lib.load()
         f = self.nfeatures
-        topk = gl.graph_params["topk"]
+        topk = gl.graph_params["topk"] if k is None else k
         host_in = not _is_device_tensor(queries)
         host_out, toucher = None, None
         if host_in and self._group is not None:
@@ -417,7 +435,9 @@ class ArrowSpace:
         bits = self._allowed_bits(allowed)
         t_b = time.perf_counter()
         try:
-            if bits is None:
+            if k is not None:
+                _lib.check(lib.asp_search_batch_k(self._h, gl._h, qp, nq, tau, k, ip, sp, lp, None if bits is None else bits.ctypes.data))
+            elif bits is None:
                 _lib.check(lib.asp_search_batch(self._h, gl._h, qp, nq, tau, ip, sp, lp))
             else:
                 _lib.check(lib.asp_search_batch_filtered(self._h, gl._h, qp, nq, tau, ip, sp, lp, bits.ctypes.data))
@@ -438,7 +458,7 @@ class ArrowSpace:
                 _to_host(lam, host_out and host_out[2])
         return idx, score, lam
 
-    def _search_batch_grid(self, queries, gl, tau, out=None, allowed=None):
+    def _search_batch_grid(self, queries, gl, tau, out=None, allowed=None, k=None):
         """R item shards x C query slots (distributed.regroup): this rank answers rows [a, b) of the batch against its item
         shard; R > 1: the R ranks of the slot merge their lists (K5); the C slots all-gather the finished slices, so every
         rank returns the whole batch.  Host batches: this rank uploads only ITS slice (over its own PCIe link)."""
@@ -449,7 +469,7 @@ class ArrowSpace:
         lib = _lib.load()
         g = self._grid
         f = self.nfeatures
-        topk = gl.graph_params["topk"]
+        topk = gl.graph_params["topk"] if k is None else k
         dev = torch.device("cuda", lib.asp_ctx_device(self._ctx))
         host_in = not _is_device_tensor(queries)
         if host_in:
@@ -482,7 +502,10 @@ class ArrowSpace:
             qp = q[a:b].ctypes.data if host_in else q[a:b].data_ptr()
             torch.cuda.current_stream(dev).synchronize()                 # the library runs on its own stream
             bits = self._allowed_bits(allowed)
-            if bits is None:
+            if k is not None:
+                rc = lib.asp_search_batch_k(self._h, gl._h, qp, b - a, tau, k, idx_p.data_ptr(), sc_p.data_ptr(), lam_p.data_ptr(),
+                                            None if bits is None else bits.ctypes.data)
+            elif bits is None:
                 rc = lib.asp_search_batch(self._h, gl._h, qp, b - a, tau, idx_p.data_ptr(), sc_p.data_ptr(), lam_p.data_ptr())
             else:
                 rc = lib.asp_search_batch_filtered(self._h, gl._h, qp, b - a, tau, idx_p.data_ptr(), sc_p.data_ptr(),
@@ -620,12 +643,13 @@ class ArrowSpace:
         return persist.save(path, self, gl, items)
 
     # ------------------------------------------------------------------ hybrid search (SURVEY.md 8(f)-2)
-    def search_hybrid(self, item, gl, tau, *, pool=None, allowed=None):
+    def search_hybrid(self, item, gl, tau, *, pool=None, allowed=None, k=None):
         """list[(index, score)], best first -- src/lib.rs:182-219: same argument checks and lambda_q as `search`, no
         lambda_q != 0 assertion, k = gl.graph_params.topk, then the crate's search_lambda_aware_hybrid.  That function is not
         in the reference (PARITY UNPINNED): restated as a cosine shortlist of `pool` items (keyword-only extra, default
         min(2 * topk, 31)) re-ranked by the lambda-aware score (include/arrowspace_b200.h, asp_search_hybrid_batch).
-        allowed (keyword only, numpy bool[nitems]): the shortlist is the `pool` ALLOWED items of largest cosine."""
+        allowed (keyword only, numpy bool[nitems]): the shortlist is the `pool` ALLOWED items of largest cosine.
+        k (keyword only): k results instead of gl.graph_params["topk"], as in search_hybrid_batch."""
         if not isinstance(gl, GraphLaplacian):
             raise TypeError("argument 'gl': 'GraphLaplacian' object expected")
         if not isinstance(item, np.ndarray) or item.dtype != np.float64 or item.ndim != 1:
@@ -635,17 +659,19 @@ class ArrowSpace:
         if item.shape[0] != self.nfeatures:
             raise ValueError("query length %d must match nfeatures %d" % (item.shape[0], self.nfeatures))   # src/lib.rs:190-196
         idx, score, lam_q = self.search_hybrid_batch(item.reshape(1, -1), gl, float(tau), pool=pool, want_lambda=True,
-                                                     allowed=allowed)
+                                                     allowed=allowed, k=k)
         dbg_println("search: qlen=%d, lambda_q=%.6f" % (item.shape[0], lam_q[0]))     # src/lib.rs:207-211 (same text as search)
         return [(int(i), float(s)) for i, s in zip(idx[0], score[0]) if i >= 0]
 
-    def search_hybrid_batch(self, queries, gl, tau, *, pool=None, want_lambda=False, allowed=None):
+    def search_hybrid_batch(self, queries, gl, tau, *, pool=None, want_lambda=False, allowed=None, k=None):
         """Extension: search_hybrid for a host batch; (idx int64[Q, topk], score f64[Q, topk]) padded with -1 / NaN
         (+ lambda_q with want_lambda).  On one GPU, and on the replicated layout of build_sharded (item_shards = 1), each
         rank answers on its own.  On an item-sharded space (item_shards > 1) it is called collectively, like `search`, and
         every rank returns the whole batch: the one-GPU answer, bit for bit (distributed.sharded_search_hybrid).
         allowed = numpy bool[nitems]: H2's shortlist is taken from the allowed items only (the pool length is unchanged);
-        collective calls pass the same mask on every rank."""
+        collective calls pass the same mask on every rank.
+        k = int (1 .. 1024): k replaces gl.graph_params["topk"] in H2 and H3 (default pool min(2k, 31) raised to k), outputs
+        (Q, k); the answer of a graph built with topk = k where topk does not prune."""
         if not isinstance(gl, GraphLaplacian):
             raise TypeError("argument 'gl': 'GraphLaplacian' object expected")
         n_local, f, _, n_total = self._dims()
@@ -658,20 +684,25 @@ class ArrowSpace:
         if pool is not None and (isinstance(pool, bool) or not isinstance(pool, (int, np.integer)) or pool < 1):
             raise ValueError("pool must be a positive integer (the shortlist length; default min(2 * topk, 31))")
         allowed = _check_allowed(allowed, n_total)
-        topk = gl.graph_params["topk"]
+        k = _check_k(k)
+        topk = gl.graph_params["topk"] if k is None else k
         nq = q.shape[0]
         try:
             if n_local != n_total:
                 from .distributed import CudaEngine, sharded_search_hybrid
                 engine = CudaEngine(_lib.load().asp_ctx_device(self._ctx))
                 idx, score, lam = sharded_search_hybrid(engine, self._h, gl._h, q, float(tau), int(pool or 0), topk, n_total,
-                                                        self._grid, allowed=allowed)
+                                                        self._grid, allowed=allowed, call_k=k is not None)
                 return (idx, score, lam) if want_lambda else (idx, score)
             idx = np.empty((nq, topk), dtype=np.int64)
             score = np.empty((nq, topk), dtype=np.float64)
             lam = np.empty(nq, dtype=np.float64)
             bits = self._allowed_bits(allowed)
-            if bits is None:
+            if k is not None:
+                _lib.check(_lib.load().asp_search_hybrid_batch_k(self._h, gl._h, q.ctypes.data, nq, float(tau), int(pool or 0), k,
+                                                                 idx.ctypes.data, score.ctypes.data, lam.ctypes.data,
+                                                                 None if bits is None else bits.ctypes.data))
+            elif bits is None:
                 _lib.check(_lib.load().asp_search_hybrid_batch(self._h, gl._h, q.ctypes.data, nq, float(tau), int(pool or 0),
                                                                idx.ctypes.data, score.ctypes.data, lam.ctypes.data))
             else:

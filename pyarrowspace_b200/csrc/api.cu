@@ -725,10 +725,11 @@ int asp_query_lambda(asp_ctx *ctx, const asp_graph *g, const asp_switches *sw_in
 
 // One device-resident batch: lambda_q (src/lib.rs:154), the lambda_q != 0 guard (src/lib.rs:156-159), candidate pass +
 // exact stage 2.  `flags` is a 2-int device scratch.  allowed: the item mask as upload_allowed left it, or nullptr.
-// Synchronises ctx->stream before returning.
+// Synchronises ctx->stream before returning.  wide (the _k entry points only): topk 32 .. 64 stays on the tensor-core route
+// with the wide stage 2; without it such a topk takes the batched exact scan, as the graph-topk entry points always have.
 static int search_device_batch(const asp_space *s, const asp_graph *g, const double *dq, int64_t nq, double tau, int64_t topk,
                                double *dlam, double *dnorm, int *flags, int64_t *didx, double *dscore,
-                               bool assert_lambda_nonzero = true, const uint32_t *allowed = nullptr)
+                               bool assert_lambda_nonzero = true, const uint32_t *allowed = nullptr, bool wide = false)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
@@ -752,8 +753,8 @@ static int search_device_batch(const asp_space *s, const asp_graph *g, const dou
     const bool want_tc = force && force[0] == 't';
     int rc;
     // small batches against a large shard stream the fp16 operands (2 * kp bytes per item) instead of the f64 rows
-    if (!want_fp64 && asp_search_tc_supported(s, nq, topk, tau) && (want_tc || nq >= 256 || s->n_local >= 131072))
-        rc = asp_search_tc_impl(s, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore, nullptr, allowed);
+    if (!want_fp64 && asp_search_tc_supported(s, nq, topk, tau, wide) && (want_tc || nq >= 256 || s->n_local >= 131072))
+        rc = asp_search_tc_impl(s, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore, nullptr, allowed, wide);
     else
         rc = asp_search_impl(s, g, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore, allowed);
     if (rc == ASP_OK) ASP_CUDA(cudaStreamSynchronize(st));
@@ -770,6 +771,7 @@ static int search_device_batch(const asp_space *s, const asp_graph *g, const dou
 // ~3 GB/s inside the D2H copy (10.5 MB per 64k queries: 3 ms after the last kernel); they are touched on this thread
 // while the kernels run instead (ctx->on_wait).
 constexpr int64_t ASP_PIPE_MIN_BATCH = 32768;
+constexpr int ASP_CALL_K_MAX = 1024;          // asp_xs::TOPK_MAX: the longest list the batched exact scan keeps
 
 int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                      int64_t *out_idx, double *out_score, double *out_lambda_q)
@@ -777,8 +779,34 @@ int asp_search_batch(const asp_space *s, const asp_graph *g, const double *queri
     return asp_search_batch_filtered(s, g, queries, nq, tau, out_idx, out_score, out_lambda_q, nullptr);
 }
 
+// k of a per-call search: 1 .. the exact scan's list length
+static int check_call_k(int64_t k)
+{
+    if (k < 1) ASP_FAIL(ASP_ERR_ARG, "k must be >= 1 (got %lld)", (long long)k);
+    if (k > ASP_CALL_K_MAX) ASP_FAIL(ASP_ERR_UNSUPPORTED, "k = %lld is beyond the %d results the exact scan keeps per query", (long long)k, ASP_CALL_K_MAX);
+    return ASP_OK;
+}
+
+static int search_batch_topk(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t topk,
+                             bool wide, int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits);
+
 int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                               int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits)
+{
+    return search_batch_topk(s, g, queries, nq, tau, g ? g->gp.topk : 0, false, out_idx, out_score, out_lambda_q, allowed_bits);
+}
+
+int asp_search_batch_k(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t k,
+                       int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits)
+{
+    if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score))) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch_k: NULL argument");
+    ASP_CHECK(check_call_k(k));
+    return search_batch_topk(s, g, queries, nq, tau, k, true, out_idx, out_score, out_lambda_q, allowed_bits);
+}
+
+// topk: the graph's (src/lib.rs:169) or the call's k (wide: the _k route, see search_device_batch)
+static int search_batch_topk(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t topk,
+                             bool wide, int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits)
 {
     if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score))) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch: NULL argument");
     if (!s->have_lambdas) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch: item lambdas have not been computed");
@@ -791,7 +819,6 @@ int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const doub
     struct CallTimer { asp_ctx *c; double t0; ~CallTimer() { c->stats["search_host_call_us"] = asp_now_us() - t0; } } call_timer{ctx, t_call};
     ASP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const int64_t topk = g->gp.topk;                              // src/lib.rs:169
     const int32_t f = s->f, fp = s->fp;
 
     asp_scratch sc(st);
@@ -849,7 +876,8 @@ int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const doub
             cudaEventRecord(start_c[c], st);
             if (c == 1) ctx->on_wait = [=]() { prefault(head, nq - head); };   // under the kernels of the rest (the head's are too short)
             rc = search_device_batch(s, g, dq + q0 * fp, qn, tau, topk, dlam + q0, dnorm + q0, flags,
-                                     didx ? didx + q0 * topk : nullptr, dscore ? dscore + q0 * topk : nullptr, true, dallowed);
+                                     didx ? didx + q0 * topk : nullptr, dscore ? dscore + q0 * topk : nullptr, true, dallowed,
+                                     wide);
             if (ctx->on_wait) { auto fn = std::move(ctx->on_wait); ctx->on_wait = nullptr; if (rc == ASP_OK) fn(); }
             if (rc != ASP_OK) break;
             // results of this piece: D2H on the second copy stream (for pageable destinations the runtime stages the copy
@@ -880,7 +908,7 @@ int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const doub
     } else if (rc == ASP_OK) {
         rc = upload_pitched(st, queries, nq, f, fp, dq);
         if (touch) ctx->on_wait = [=]() { prefault(0, nq); };
-        if (rc == ASP_OK) rc = search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, true, dallowed);
+        if (rc == ASP_OK) rc = search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, true, dallowed, wide);
         if (ctx->on_wait) { auto fn = std::move(ctx->on_wait); ctx->on_wait = nullptr; if (rc == ASP_OK) fn(); }
         if (rc == ASP_OK && out_lambda_q) rc = asp_copy_out(ctx, out_lambda_q, dlam, sizeof(double) * nq);
         if (rc == ASP_OK && topk > 0) {
@@ -910,9 +938,30 @@ int asp_search_hybrid_batch(const asp_space *s, const asp_graph *g, const double
 }
 
 // Filtered: the shortlist is the m ALLOWED items of largest cosine (the filtered search at tau = 1), m still from n.
+static int hybrid_batch_topk(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                             int64_t topk, bool wide, int64_t *out_idx, double *out_score, double *out_lambda_q,
+                             const uint8_t *allowed_bits);
+
 int asp_search_hybrid_batch_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                                      int64_t pool, int64_t *out_idx, double *out_score, double *out_lambda_q,
                                      const uint8_t *allowed_bits)
+{
+    return hybrid_batch_topk(s, g, queries, nq, tau, pool, g ? g->gp.topk : 0, false, out_idx, out_score, out_lambda_q, allowed_bits);
+}
+
+int asp_search_hybrid_batch_k(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                              int64_t k, int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits)
+{
+    if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score)))
+        ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_batch_k: NULL argument");
+    ASP_CHECK(check_call_k(k));
+    return hybrid_batch_topk(s, g, queries, nq, tau, pool, k, true, out_idx, out_score, out_lambda_q, allowed_bits);
+}
+
+// topk: the graph's (src/lib.rs:214) or the call's k, which also sets the default shortlist (asp_hybrid_pool)
+static int hybrid_batch_topk(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                             int64_t topk, bool wide, int64_t *out_idx, double *out_score, double *out_lambda_q,
+                             const uint8_t *allowed_bits)
 {
     if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score)))
         ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_batch: NULL argument");
@@ -928,7 +977,6 @@ int asp_search_hybrid_batch_filtered(const asp_space *s, const asp_graph *g, con
     asp_ctx *ctx = s->ctx;
     ASP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const int64_t topk = g->gp.topk;                              // src/lib.rs:214
     const int32_t f = s->f, fp = s->fp;
     const int64_t m = asp_hybrid_pool(s->n_local, topk, pool);
     const bool whole_set = (m >= s->n_local);                     // the shortlist is every item: H3 is the plain search
@@ -957,9 +1005,9 @@ int asp_search_hybrid_batch_filtered(const asp_space *s, const asp_graph *g, con
     ASP_CHECK(upload_allowed(scratch, allowed_bits, s->n_local, &dallowed));
     // H1 + H2: lambda_q, then the m largest cosines per query (the score at tau = 1 is the cosine), ties by the smaller index
     if (whole_set)
-        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false, dallowed));
+        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false, dallowed, wide));
     else
-        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? m : 0, dlam, dnorm, flags, pidx, pscore, false, dallowed));
+        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? m : 0, dlam, dnorm, flags, pidx, pscore, false, dallowed, wide));
     if (topk > 0 && !whole_set) {
         // H3: reference-order scores of the shortlist, best topk by (score desc, index asc)
         const int64_t total = nq * m;
@@ -992,9 +1040,31 @@ int asp_search_hybrid_shard(const asp_space *s, const asp_graph *g, const double
     return asp_search_hybrid_shard_filtered(s, g, queries, nq, tau, pool, out_idx, out_cos, out_score, out_lambda_q, nullptr);
 }
 
+static int hybrid_shard_topk(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                             int64_t topk, bool wide, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q,
+                             const uint8_t *allowed_bits);
+
 int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau,
                                      int64_t pool, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q,
                                      const uint8_t *allowed_bits)
+{
+    return hybrid_shard_topk(s, g, queries, nq, tau, pool, g ? g->gp.topk : 0, false, out_idx, out_cos, out_score, out_lambda_q,
+                             allowed_bits);
+}
+
+int asp_search_hybrid_shard_k(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                              int64_t k, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q,
+                              const uint8_t *allowed_bits)
+{
+    if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score)))
+        ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_shard_k: NULL argument");
+    ASP_CHECK(check_call_k(k));
+    return hybrid_shard_topk(s, g, queries, nq, tau, pool, k, true, out_idx, out_cos, out_score, out_lambda_q, allowed_bits);
+}
+
+static int hybrid_shard_topk(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t pool,
+                             int64_t topk, bool wide, int64_t *out_idx, double *out_cos, double *out_score, double *out_lambda_q,
+                             const uint8_t *allowed_bits)
 {
     if (!s || !g || (nq > 0 && (!queries || !out_idx || !out_score)))
         ASP_FAIL(ASP_ERR_ARG, "asp_search_hybrid_shard: NULL argument");
@@ -1006,7 +1076,6 @@ int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, con
     asp_ctx *ctx = s->ctx;
     ASP_CUDA(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    const int64_t topk = g->gp.topk;
     const int32_t f = s->f, fp = s->fp;
     const int64_t m = asp_hybrid_pool(s->n_total, topk, pool);
     const bool whole_set = (m >= s->n_total);
@@ -1035,7 +1104,7 @@ int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, con
     ASP_CHECK(upload_allowed(scratch, allowed_bits, s->n_local, &dallowed));
     if (whole_set) {
         // no shortlist: the shard's best topk by the lambda-aware score, merged like asp_search_batch's lists
-        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false, dallowed));
+        ASP_CHECK(search_device_batch(s, g, dq, nq, tau, topk, dlam, dnorm, flags, didx, dscore, false, dallowed, wide));
     } else {
         int64_t *sidx = didx;
         double *scos = dcos;
@@ -1044,7 +1113,7 @@ int asp_search_hybrid_shard_filtered(const asp_space *s, const asp_graph *g, con
             ASP_CHECK(scratch.get(&scos, (size_t)nq * kl));
         }
         // the score at tau = 1 is the cosine
-        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? kl : 0, dlam, dnorm, flags, sidx, scos, false, dallowed));
+        ASP_CHECK(search_device_batch(s, g, dq, nq, 1.0, topk > 0 ? kl : 0, dlam, dnorm, flags, sidx, scos, false, dallowed, wide));
         if (topk > 0) {
             if (kl < m) {                                         // lists padded to m with -1 / NaN
                 ASP_CUDA(cudaMemsetAsync(didx, 0xff, sizeof(int64_t) * (size_t)nq * m, st));

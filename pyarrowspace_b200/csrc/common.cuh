@@ -234,10 +234,11 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
                   const double *qnorm_dev, double tau, int64_t topk, double score_floor, int force_terms, int capb_override,
                   float *dump_dev, asp_tc_batch *b, bool l2 = false, const uint32_t *allowed_dev = nullptr);
 int asp_device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out);   // max(0, max v), synchronises
-bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, double tau);
+// wide: topk up to 128 on the tensor-core route (wide stage 2 from 32 on); otherwise topk <= 32 as the graph-topk entry points use
+bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, double tau, bool wide = false);
 int asp_search_tc_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                        const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
-                       float *dump_dev, const uint32_t *allowed_dev = nullptr);
+                       float *dump_dev, const uint32_t *allowed_dev = nullptr, bool wide = false);
 void asp_free_tc_cache(asp_space *s);
 int asp_launch_reciprocal(asp_ctx *ctx, const double *x, int64_t n, double *out);
 int asp_search_slow_path(const asp_space *s, const double *q_dev, int32_t qpitch, const double *lambda_q_dev,

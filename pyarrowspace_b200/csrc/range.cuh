@@ -105,7 +105,7 @@ ASP_RNG_FN void merge_elem(int64_t t, int parts, int64_t nq, const int64_t *part
     out_score[pos] = s;
 }
 
-#if defined(__CUDACC__)
+#if defined(__CUDACC__) && !defined(ASP_RANGE_KEYS_ONLY)          // (large_k.cuh takes the keys only: one kernel definition)
 __global__ void __launch_bounds__(256)
 range_merge_kernel(int64_t total, int parts, int64_t nq, const int64_t *__restrict__ part_off, const int64_t *__restrict__ out_off,
                    const int64_t *__restrict__ idx, const double *__restrict__ score, int64_t *__restrict__ out_idx,

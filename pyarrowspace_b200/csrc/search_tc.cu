@@ -26,6 +26,13 @@
 // expression) and sorted by (score desc, index asc).  More than 32 candidates inside that band, or a full emission
 // buffer, send the query to the exact scan.  The result is bit-identical to the FP64 path's (tests assert it).
 //
+// Per-call k of 32 .. 64 (asp_search_batch_k and the hybrid _k entry points only; their `wide` flag): stage 1 runs with
+// 64-entry running lists (ceil(k / 4) <= 16 scores per column-quarter thread, so every threshold is still a lower bound of
+// the k-th best score) and a larger emission capacity; stage 2 is tc_rescore_wide_kernel, one CTA per query, which keeps
+// every survivor of the cut (up to asp_lk::SURV_CAP) instead of 32 per warp: large_k.cuh.  The graph-topk entry points never
+// set the flag, so a graph topk >= 32 still takes the exact scan there; moving them onto this route needs its own B200
+// measurements and a deliberate change of the test that pins their route.
+//
 // Completeness.  Let t_k be the exact k-th best score.  Any running threshold theta is the k-th best APPROXIMATE score
 // of some k distinct items, whose exact scores are >= theta - DELTA, so t_k >= theta - DELTA.  An item of the true top-k
 // has s >= t_k, hence s~ >= s - DELTA >= theta - 2 DELTA: it passes every emission test and the final cut.  The same
@@ -48,6 +55,7 @@
 #include "ptx.cuh"
 #include "warp_sort.cuh"
 #include "l2_bound.cuh"
+#include "large_k.cuh"
 
 #include <cuda_fp16.h>
 #include <algorithm>
@@ -1020,6 +1028,152 @@ tc_rescore_kernel(const double *__restrict__ q, int qpitch, int64_t nq, const do
     }
 }
 
+constexpr int TW_THREADS = 256;
+static_assert(TW_THREADS == 256, "one thread per radix digit");
+
+// block-wide bitonic sort of n (a power of two) (key, index) pairs in shared memory
+__device__ __forceinline__ void block_bitonic(uint64_t *key, int32_t *ix, int n)
+{
+    for (int size = 2; size <= n; size <<= 1)
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            for (int t = threadIdx.x; t < n / 2; t += TW_THREADS) asp_lk::bitonic_cx(key, ix, t, size, stride);
+            __syncthreads();
+        }
+}
+
+// Wide stage 2 (k = 32 .. 128, the _k entry points): one CTA per query, every survivor of the cut kept in shared memory.
+// The phases and their reasons are in large_k.cuh.  Dynamic shared memory: the query row (pitch doubles), then SURV_CAP
+// sort keys and SURV_CAP item indices.
+__global__ void __launch_bounds__(TW_THREADS)
+tc_rescore_wide_kernel(const double *__restrict__ q, int qpitch, const double *__restrict__ items, int64_t n_local, int f,
+                       int pitch, int64_t row0, const double *__restrict__ norm_x, const double *__restrict__ lam_x,
+                       const double *__restrict__ norm_q, const double *__restrict__ lam_q, double tau, int topk, int nstreams,
+                       int capb, const float *__restrict__ delta_q, double eps_fast, const float *__restrict__ emit_sc,
+                       const int32_t *__restrict__ emit_ix, const int32_t *__restrict__ emit_cnt, const int32_t *__restrict__ qperm,
+                       int64_t *__restrict__ out_idx, double *__restrict__ out_score, int32_t *slow_list, int32_t *slow_count,
+                       unsigned long long *survivor_total, unsigned long long *exact_total)
+{
+    extern __shared__ __align__(1024) unsigned char smem_raw[];
+    double *qs = reinterpret_cast<double *>(smem_raw);
+    uint64_t *key = reinterpret_cast<uint64_t *>(qs + pitch);
+    int32_t *ix = reinterpret_cast<int32_t *>(key + asp_lk::SURV_CAP);
+    __shared__ int s_hist[256];
+    __shared__ int s_krem, s_nsurv;
+    __shared__ uint32_t s_prefix;
+    __shared__ unsigned long long s_emitted;
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int64_t qi = blockIdx.x;                                               // position in lambda_q order
+    const int64_t oq = qperm ? (int64_t)qperm[qi] : qi;
+    const int kk = topk < n_local ? topk : (int)n_local;
+    for (int j = tid; j < pitch; j += TW_THREADS) qs[j] = (j < f) ? q[oq * qpitch + j] : 0.0;
+    if (tid == 0) { s_emitted = 0ull; s_nsurv = 0; s_prefix = 0u; s_krem = kk; }
+    bool overflow = false;
+    unsigned long long mine = 0;
+    for (int c = tid; c < nstreams; c += TW_THREADS) {
+        const int cnt = emit_cnt[qi * nstreams + c];
+        overflow |= cnt > capb;
+        mine += (unsigned long long)cnt;
+    }
+    overflow = __syncthreads_or(overflow ? 1 : 0) != 0;
+    if (overflow) {
+        if (tid == 0) slow_list[atomicAdd(slow_count, 1)] = (int32_t)oq;
+        return;
+    }
+    if (mine) atomicAdd(&s_emitted, mine);
+    __syncthreads();
+    const int64_t emitted = (int64_t)s_emitted;
+
+    // (1) cut: radix select of the kk-th largest approximate score over every emitted candidate
+    float cutoff = -INFINITY;
+    if (emitted >= kk) {
+        for (int pass = 0; pass < 4; ++pass) {
+            s_hist[tid] = 0;                                                     // TW_THREADS == 256 digits
+            __syncthreads();
+            const uint32_t prefix = s_prefix;
+            for (int c = 0; c < nstreams; ++c) {
+                const int cnt = emit_cnt[qi * nstreams + c];
+                const float *sc = emit_sc + ((size_t)qi * nstreams + c) * (size_t)capb;
+                for (int e = tid; e < cnt; e += TW_THREADS) {
+                    const uint32_t k = asp_lk::f32_key(sc[e]);
+                    if (asp_lk::prefix_match(k, prefix, pass)) atomicAdd(&s_hist[asp_lk::digit(k, pass)], 1);
+                }
+            }
+            __syncthreads();
+            if (tid == 0) {
+                int kr = s_krem;
+                const int d = asp_lk::select_digit(s_hist, &kr);
+                s_krem = kr;
+                s_prefix = prefix | ((uint32_t)d << (24 - 8 * pass));
+            }
+            __syncthreads();
+        }
+        cutoff = asp_lk::survivor_cutoff(s_prefix, delta_q[qi]);
+    }
+
+    // (2) survivors of the cut (their order here depends on the schedule; the sorts below make it irrelevant)
+    for (int c = 0; c < nstreams; ++c) {
+        const int cnt = emit_cnt[qi * nstreams + c];
+        const size_t base = ((size_t)qi * nstreams + c) * (size_t)capb;
+        for (int e = tid; e < cnt; e += TW_THREADS)
+            if (emit_sc[base + e] >= cutoff) {
+                const int pos = atomicAdd(&s_nsurv, 1);
+                if (pos < asp_lk::SURV_CAP) ix[pos] = emit_ix[base + e];
+            }
+    }
+    __syncthreads();
+    const int nsurv = s_nsurv;
+    if (asp_lk::route(false, emitted, nsurv, kk) != asp_lk::ROUTE_OK) {
+        if (tid == 0) slow_list[atomicAdd(slow_count, 1)] = (int32_t)oq;
+        return;
+    }
+
+    // (3) f64 re-score of every survivor (one warp per survivor, coalesced 16 B loads), sort by (fast desc, index asc)
+    const double nqv = norm_q[oq], lqv = lam_q[oq];
+    for (int s = warp; s < nsurv; s += TW_THREADS / 32) {
+        const int it = ix[s];
+        const double *row = items + (int64_t)it * pitch;
+        double d = 0.0;
+        for (int j = 2 * lane; j < pitch; j += 64) {
+            const double2 qq = *reinterpret_cast<const double2 *>(qs + j);
+            const double2 a = *reinterpret_cast<const double2 *>(row + j);
+            d = fma(qq.x, a.x, d);
+            d = fma(qq.y, a.y, d);
+        }
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) d += __shfl_xor_sync(0xffffffffu, d, off);
+        if (lane == 0) key[s] = asp_range::desc_key(exact_score_tc(d, nqv, norm_x[it], tau, lqv, lam_x[it]));
+    }
+    const int n2 = asp_lk::next_pow2(nsurv);
+    for (int s = nsurv + tid; s < n2; s += TW_THREADS) { key[s] = ~0ull; ix[s] = 0x7fffffff; }
+    __syncthreads();
+    block_bitonic(key, ix, n2);
+
+    // (4) the band of the kk-th best fast score (a prefix of the sorted survivors), in the reference order
+    int nb = 0;
+    for (int i0 = 0; i0 < nsurv; i0 += TW_THREADS) {
+        const int i = i0 + tid;
+        const int cnt = __syncthreads_count(i < nsurv && asp_lk::in_band(key, i, kk, eps_fast));
+        nb += cnt;
+        if (cnt < TW_THREADS) break;
+    }
+    __syncthreads();                                                             // every thread has read the fast keys
+    const int n3 = asp_lk::next_pow2(nb);
+    for (int i = tid; i < n3; i += TW_THREADS) {
+        if (i < nb) {
+            const int it = ix[i];
+            const double d = seq_dot_row_tc(qs, items + (int64_t)it * pitch, f);
+            key[i] = asp_range::desc_key(exact_score_tc(d, nqv, norm_x[it], tau, lqv, lam_x[it]));
+        } else {
+            key[i] = ~0ull;
+            ix[i] = 0x7fffffff;
+        }
+    }
+    __syncthreads();
+    block_bitonic(key, ix, n3);
+    for (int j = tid; j < topk; j += TW_THREADS) asp_lk::emit_slot(j, kk, key, ix, row0, out_idx + oq * topk, out_score + oq * topk);
+    if (tid == 0) { atomicAdd(survivor_total, (unsigned long long)nsurv); atomicAdd(exact_total, (unsigned long long)nb); }
+}
+
 }  // namespace
 
 // ------------------------------------------------------------------ host side
@@ -1177,9 +1331,9 @@ void asp_free_tc_cache(asp_space *s)
     s->tc_cache = nullptr;
 }
 
-bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, double tau)
+bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, double tau, bool wide)
 {
-    return topk >= 1 && topk <= TK_LIST_MAX && nq >= 1 && s->n_local >= 1 && s->n_local < 2147483647LL && tau > 1e-3 &&
+    return topk >= 1 && topk <= (wide ? asp_lk::KMAX : TK_LIST_MAX) && nq >= 1 && s->n_local >= 1 && s->n_local < 2147483647LL && tau > 1e-3 &&
            tau <= 1.0 && s->fp <= 6144;   // beta = 1 - tau >= 0: the proximity term is bounded from above by prox_ub
 }
 
@@ -1326,6 +1480,7 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     bool ares = (nterms == 1) && (p.kb_hi <= 7);
     if (const char *e = getenv("ASP_TC_ARES")) ares = ares && atoi(e) != 0;
     const bool wide = topk > 16;                                  // 32-entry running lists
+    const int listn = topk > 32 ? 64 : 0;                         // k = 33 .. 64 (the _k entry points): 64-entry lists
     // CTA pairs (cta_group::2: two query blocks share one M = 256 MMA, each SM loads half of every item tile) whenever there
     // are two query blocks to pair: -18 % stage-1 time at C4 / 64k queries (ASP_TC_PAIR=0: the 1-SM kernel, same bits)
     bool pair = ares && !dump_dev && qblocks >= 2;
@@ -1343,7 +1498,7 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     int v = 0;
 #endif
     if (pair) p.nw_hi = 0;                                        // (the CTA-pair kernel keeps full boxes)
-    if (l2 || allowed_dev) v = 0;
+    if (l2 || allowed_dev || listn) v = 0;
     void (*k)(CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap, TcParams) =
         dump_dev ? (ares ? tc_gemm_kernel<true, 0, true, false, 16> : tc_gemm_kernel<true, 0, false, false, 16>)
         : wide ? (pair ? tc_gemm_kernel<false, 0, true, true, 32> : ares ? tc_gemm_kernel<false, 0, true, false, 32> : tc_gemm_kernel<false, 0, false, false, 32>)
@@ -1362,6 +1517,11 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
                          : tc_gemm_kernel<false, 0, false, false, 32, false, true>)
                  : (pair ? tc_gemm_kernel<false, 0, true, true, 16, false, true> : ares ? tc_gemm_kernel<false, 0, true, false, 16, false, true>
                          : tc_gemm_kernel<false, 0, false, false, 16, false, true>);
+    if (listn == 64)
+        k = allowed_dev ? (pair ? tc_gemm_kernel<false, 0, true, true, 64, false, true> : ares ? tc_gemm_kernel<false, 0, true, false, 64, false, true>
+                                : tc_gemm_kernel<false, 0, false, false, 64, false, true>)
+                        : (pair ? tc_gemm_kernel<false, 0, true, true, 64> : ares ? tc_gemm_kernel<false, 0, true, false, 64>
+                                : tc_gemm_kernel<false, 0, false, false, 64>);
     if (l2)
         k = wide ? (pair ? tc_gemm_kernel<false, 0, true, true, 32, true> : ares ? tc_gemm_kernel<false, 0, true, false, 32, true>
                          : tc_gemm_kernel<false, 0, false, false, 32, true>)
@@ -1417,31 +1577,35 @@ __global__ void scatter_results_kernel(const int64_t *__restrict__ idx2, const d
 // three-term split (retry), and what is still undecided (exact ties around the k-th score) takes the exact scan.
 static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                              const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
-                             float *dump_dev, int force_terms, bool may_retry, const uint32_t *allowed_dev);
+                             float *dump_dev, int force_terms, bool may_retry, const uint32_t *allowed_dev, bool wide);
 
 // dump == nullptr: full search.  dump != nullptr: approximate cosines [nq][n_local] f32 (tests).  allowed_dev: item mask
-// (local item order, packed) or nullptr.
+// (local item order, packed) or nullptr.  wide: topk = 32 .. 128 takes the wide stage 2 (tc_rescore_wide_kernel) instead of
+// the 32-per-warp one, whose lists cannot hold a candidate beyond the 32nd (the _k entry points only).
 int asp_search_tc_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                        const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
-                       float *dump_dev, const uint32_t *allowed_dev)
+                       float *dump_dev, const uint32_t *allowed_dev, bool wide)
 {
     const char *e = getenv("ASP_TC_FIRST_TERMS");                  // A/B knob: "auto" = the band rule decides (the earlier behaviour)
     int first = dump_dev ? 0 : (e && e[0] == 'a') ? 0 : 1;
     if (const char *t = getenv("ASP_TC_TERMS")) { const int v = atoi(t); if (v == 1 || v == 3) first = v; }   // test knob: that mode, no retry
     const bool pinned = getenv("ASP_TC_TERMS") != nullptr;
     return search_tc_attempt(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, out_idx_dev, out_score_dev, dump_dev, first,
-                             first == 1 && !pinned, allowed_dev);
+                             first == 1 && !pinned, allowed_dev, wide);
 }
 
 static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                              const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
-                             float *dump_dev, int force_terms, bool may_retry, const uint32_t *allowed_dev)
+                             float *dump_dev, int force_terms, bool may_retry, const uint32_t *allowed_dev, bool wide)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
     asp_tc_batch b;
-    int rc = asp_tc_stage1(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, -INFINITY, force_terms, 0, dump_dev, &b, false,
-                           allowed_dev);
+    // the wide stage 2 keeps every survivor, so its emission lists get room for k-sized lists plus the band: a chunk of a
+    // million items emits about k (1 + ln(items / k)) records plus every item within the band of the k-th score
+    const bool wide2 = wide && topk >= asp_lk::KMIN;
+    int rc = asp_tc_stage1(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, -INFINITY, force_terms,
+                           wide2 ? (int)(64 * topk) : 0, dump_dev, &b, false, allowed_dev);
     if (rc != ASP_OK || dump_dev) return rc;
 
     if (b.variant != 0) {                                         // profiling variants: stage 1 only, results are garbage
@@ -1474,7 +1638,14 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
             out_score_dev, slow_list, slow_count, counters, counters + 1);
         return ASP_OK;
     };
-    if (wpq == 32) ASP_CHECK(launch_rescore(tc_rescore_kernel<32>, 32, 1, (unsigned)nq));
+    if (wide2) {
+        const size_t wsmem = (size_t)s->fp * 8 + (size_t)asp_lk::SURV_CAP * (sizeof(uint64_t) + sizeof(int32_t));
+        ASP_CUDA(cudaFuncSetAttribute(tc_rescore_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
+        tc_rescore_wide_kernel<<<(unsigned)nq, TW_THREADS, wsmem, st>>>(
+            q_dev, qpitch, s->items, s->n_local, s->f, s->fp, s->row0, s->norms, s->lambdas, qnorm_dev, lambda_q_dev, tau, (int)topk,
+            b.nsub, b.capb, b.delta_q, eps_fast, b.emit_sc, b.emit_ix, b.emit_cnt, b.qperm, out_idx_dev, out_score_dev, slow_list,
+            slow_count, counters, counters + 1);
+    } else if (wpq == 32) ASP_CHECK(launch_rescore(tc_rescore_kernel<32>, 32, 1, (unsigned)nq));
     else if (wpq == 8) ASP_CHECK(launch_rescore(tc_rescore_kernel<8>, 8, 1, (unsigned)nq));
     else if (getenv("ASP_TC_RESCORE_OCC6")) ASP_CHECK(launch_rescore(tc_rescore_kernel<1>, TR_WARPS, TR_WARPS, (unsigned)asp_ceil_div(nq, TR_WARPS)));
     else ASP_CHECK(launch_rescore(tc_rescore_kernel<1, TR_MIN_CTAS>, TR_WARPS, TR_WARPS, (unsigned)asp_ceil_div(nq, TR_WARPS)));
@@ -1510,7 +1681,7 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
         gather_queries_kernel<<<(unsigned)nslow, 128, 0, st>>>(q_dev, qpitch, lambda_q_dev, qnorm_dev, slow_list, nslow, q2, lam2, nrm2);
         ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
         b.mem.release();                                              // the retry allocates its own emission buffers
-        rc = search_tc_attempt(s, q2, nslow, qpitch, lam2, nrm2, tau, topk, idx2, sc2, nullptr, 3, false, allowed_dev);
+        rc = search_tc_attempt(s, q2, nslow, qpitch, lam2, nrm2, tau, topk, idx2, sc2, nullptr, 3, false, allowed_dev, wide);
         if (rc == ASP_OK) {
             scatter_results_kernel<<<(unsigned)nslow, 32, 0, st>>>(idx2, sc2, slow_list, nslow, (int)topk, out_idx_dev, out_score_dev);
             ASP_LAUNCHED(ctx);

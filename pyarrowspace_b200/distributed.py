@@ -232,13 +232,21 @@ class CudaEngine:
     def hybrid_pool(self, n_total, topk, pool):
         return self.lib.asp_hybrid_pool(int(n_total), int(topk), int(pool))
 
-    def hybrid_shard(self, space, graph, q, tau, pool, idx, cos, score, lam, allowed=None):
+    def hybrid_shard(self, space, graph, q, tau, pool, idx, cos, score, lam, allowed=None, k=None):
         """asp_search_hybrid_shard of the host rows q into the device tensors idx / cos / score [rows, width] and lam [rows]
-        (cos is None when the shortlist is the whole set).  allowed: the global item mask (this shard's rows are used)."""
+        (cos is None when the shortlist is the whole set).  allowed: the global item mask (this shard's rows are used).
+        k: a per-call k in place of the graph's topk (asp_search_hybrid_shard_k)."""
         self.torch.cuda.current_stream(self.device).synchronize()      # the outputs were filled on torch's stream
         args = (space, graph, q.ctypes.data, q.shape[0], float(tau), int(pool), idx.data_ptr(),
                 None if cos is None else cos.data_ptr(), score.data_ptr(), lam.data_ptr())
-        if allowed is None:
+        if k is not None:
+            bits = None
+            if allowed is not None:
+                n_local, row0 = C.c_int64(), C.c_int64()
+                _lib.check(self.lib.asp_space_dims(space, C.byref(n_local), C.byref(C.c_int32()), C.byref(row0), C.byref(C.c_int64())))
+                bits = pack_allowed(allowed, row0.value, n_local.value)
+            _lib.check(self.lib.asp_search_hybrid_shard_k(*args[:6], int(k), *args[6:], None if bits is None else bits.ctypes.data))
+        elif allowed is None:
             _lib.check(self.lib.asp_search_hybrid_shard(*args))
         else:
             n_local, row0 = C.c_int64(), C.c_int64()
@@ -489,7 +497,7 @@ def regroup(engine, space, rows_dev, n_total, item_shards, group=None):
     return new_space, grid
 
 
-def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_total, grid, allowed=None):
+def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_total, grid, allowed=None, call_k=False):
     """Hybrid search (step 7) on an item-sharded grid (grid["R"] > 1), bit for bit the one-GPU search_hybrid_batch over all
     n_total items.  Called collectively with the same host batch `queries` [Q, F] on every rank.  Query slot c answers rows
     [a, b) of the batch: each of its R ranks computes its item shard's shortlist (engine.hybrid_shard), the R lists are
@@ -497,7 +505,8 @@ def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_tota
     all-gather their finished slices, as the grid search does.  Returns (idx, score, lambda_q) host arrays of the whole
     batch on every rank.  A failure on any rank raises the same LibraryError (same code) on every rank.
     allowed: the global bool item mask, the same on every rank (each shard filters its own rows; the merges take the
-    -1-padded lists as they are), or None."""
+    -1-padded lists as they are), or None.  call_k: topk is the caller's per-call k, not the graph's (engine.hybrid_shard
+    gets k=topk, the merges take lists of that width)."""
     import torch
     from ._lib import LibraryError
     r_, c_ = grid["R"], grid["C"]
@@ -517,6 +526,8 @@ def sharded_search_hybrid(engine, space, graph, queries, tau, pool, topk, n_tota
     if b > a:
         try:
             extra = {} if allowed is None else {"allowed": allowed}
+            if call_k:
+                extra["k"] = topk
             engine.hybrid_shard(space, graph, queries[a:b], tau, pool, idx[:b - a], None if whole else cos[:b - a],
                                 score[:b - a], lam[:b - a], **extra)
         except LibraryError as e:
