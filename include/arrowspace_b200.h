@@ -232,6 +232,20 @@ int asp_search_batch_filtered(const asp_space *s, const asp_graph *g, const doub
 int asp_search_batch_k(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, double tau, int64_t k,
                        int64_t *out_idx, double *out_score, double *out_lambda_q, const uint8_t *allowed_bits);
 
+/* Tau sweep: the same queries at ntau >= 1 taus (host array taus, finite, duplicates allowed) in one call.  out_idx /
+ * out_score are [ntau][nq][k]; rows t are, bit for bit, asp_search_batch_k(s, g, queries, nq, taus[t], k, ...) with the same
+ * allowed_bits.  k as in asp_search_batch_k (the Python layer passes the graph topk for k=None).  lambda_q is computed once
+ * (out_lambda_q [nq], may be NULL); the lambda_q == 0 and zero-vector failures are those of asp_search_batch.  Route: the
+ * taus that take the tcgen05 candidate pass in asp_search_batch_k with k <= 16 share ONE candidate pass per group of at most
+ * 3 taus (two or more per group; tc_gemm_kernel holds every tau's running list in registers, and a fourth spills), then each
+ * runs its own stage 2 and slow-query remedies; every other tau, and a lone qualifying one, takes asp_search_batch_k's route.
+ * queries / outputs may be host or device memory.  Single-GPU spaces: a sharded layout loops over asp_search_batch_k in the
+ * Python layer.  asp_ctx_stat keys: sweep_fused_taus, sweep_stage1_passes (shared candidate passes), search_slow_queries
+ * (summed over the taus), sweep_slow_queries_<t>, sweep_stage1_ms / sweep_stage2_ms / sweep_emitted_per_query (shared passes). */
+int asp_search_batch_taus(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, const double *taus,
+                          int64_t ntau, int64_t k, int64_t *out_idx, double *out_score, double *out_lambda_q,
+                          const uint8_t *allowed_bits);
+
 /* Hybrid search, batched (SURVEY.md 8(f)-2).  Replaces prepare_query_item + search_lambda_aware_hybrid(&query,
  * gl.graph_params.topk, tau) of ArrowSpace.search_hybrid (src/lib.rs:182-219).  The crate function's body is not in the
  * reference and nothing there documents or tests it, so this is a restatement (PARITY UNPINNED against the crate; GPU ==

@@ -121,6 +121,7 @@ SYMBOLS = {
     "asp_search_hybrid_batch_filtered": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _vp, _vp, _vp, _vp]),
     "asp_search_hybrid_shard_filtered": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _vp, _vp, _vp, _vp, _vp]),
     "asp_search_batch_k": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _vp, _vp, _vp, _vp]),
+    "asp_search_batch_taus": (_int, [_vp, _vp, _vp, _i64, _vp, _i64, _i64, _vp, _vp, _vp, _vp]),
     "asp_search_hybrid_batch_k": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _i64, _vp, _vp, _vp, _vp]),
     "asp_search_hybrid_shard_k": (_int, [_vp, _vp, _vp, _i64, _dbl, _i64, _i64, _vp, _vp, _vp, _vp, _vp]),
     "asp_search_range_batch": (_int, [_vp, _vp, _vp, _i64, _dbl, _dbl, _vp, _i64, _vp, _vp, C.POINTER(_vp)]),

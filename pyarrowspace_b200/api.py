@@ -90,6 +90,29 @@ def _check_k(k):
     return int(k)
 
 
+def _check_taus(taus):
+    """The `taus` argument of search_batch_taus: a non-empty list, tuple or 1-D numpy array of finite real numbers, in the
+    caller's order (duplicates kept).  Returns a C-contiguous float64 array."""
+    if isinstance(taus, np.ndarray):
+        if taus.ndim != 1:
+            raise ValueError("taus must be 1-D (got shape %s)" % (taus.shape,))
+        if taus.dtype == np.bool_ or not (np.issubdtype(taus.dtype, np.integer) or np.issubdtype(taus.dtype, np.floating)):
+            raise TypeError("taus must hold real numbers (got ndarray of %s)" % taus.dtype)
+        vals = taus.astype(np.float64)
+    elif isinstance(taus, (list, tuple)):
+        for t in taus:
+            if isinstance(t, (bool, np.bool_)) or not isinstance(t, (int, float, np.integer, np.floating)):
+                raise TypeError("taus must hold real numbers (got %s)" % type(t).__name__)
+        vals = np.array([float(t) for t in taus], dtype=np.float64)
+    else:
+        raise TypeError("taus must be a list, tuple or 1-D numpy.ndarray of real numbers (got %s)" % type(taus).__name__)
+    if vals.size == 0:
+        raise ValueError("taus must not be empty")
+    if not np.isfinite(vals).all():
+        raise ValueError("taus must be finite (got %s)" % vals.tolist())
+    return np.ascontiguousarray(vals)
+
+
 # Default cap of a range search: 2**26 hits, 1 GiB of results (int64 index + f64 score) -- a threshold far below the
 # scores of a data set would otherwise ask for every item of every query.  max_results= raises or lowers it.
 DEFAULT_MAX_RESULTS = 1 << 26
@@ -372,6 +395,58 @@ class ArrowSpace:
             if _is_device_tensor(queries):
                 raise ValueError("out= is for host query batches (device batches return device tensors)")
         idx, score, _ = self._search_batch(queries, gl, float(tau), want_lambda=False, out=out, allowed=allowed, k=k)
+        return idx, score
+
+    def search_batch_taus(self, queries, gl, taus, *, allowed=None, k=None):
+        """Extension: the same queries at several taus.  Returns (idx int64[T, Q, k], score f64[T, Q, k]) where T = len(taus)
+        and k is the call's k or gl.graph_params["topk"]; idx[t], score[t] are, bit for bit, search_batch(queries, gl,
+        taus[t], allowed=allowed, k=k), -1 / NaN padding included.  taus: a list, tuple or 1-D ndarray of finite real
+        numbers (duplicates allowed).  lambda_q is computed once, with search_batch's panics.  On one GPU the taus that take
+        the tensor-core candidate pass with k <= 16 share one pass per group of up to 3; on multi-GPU layouts the call loops
+        over the collective search_batch.  Host batches return numpy arrays, device float64 batches device tensors."""
+        taus = _check_taus(taus)
+        allowed = _check_allowed(allowed, self.nitems)
+        k = _check_k(k)
+        if self._group is not None or (self._grid is not None and self._grid["C"] > 1):
+            outs = [self.search_batch(queries, gl, float(t), allowed=allowed, k=k) for t in taus]
+            if _is_device_tensor(outs[0][0]):
+                import torch
+                return torch.stack([o[0] for o in outs]), torch.stack([o[1] for o in outs])
+            return np.stack([o[0] for o in outs]), np.stack([o[1] for o in outs])
+        lib = _lib.load()
+        f = self.nfeatures
+        topk = gl.graph_params["topk"] if k is None else k
+        ntau = taus.shape[0]
+        if _is_device_tensor(queries):
+            if queries.dim() != 2 or queries.shape[1] != f:
+                raise ValueError("query length %d must match nfeatures %d" % (queries.shape[-1], f))
+            import torch
+            q = queries.contiguous()
+            if q.dtype != torch.float64:
+                raise TypeError("queries must be float64")
+            nq = q.shape[0]
+            idx = torch.empty((ntau, nq, topk), dtype=torch.int64, device=q.device)
+            score = torch.empty((ntau, nq, topk), dtype=torch.float64, device=q.device)
+            qp, ip, sp = q.data_ptr(), idx.data_ptr(), score.data_ptr()
+            torch.cuda.current_stream(q.device).synchronize()      # the library runs on its own stream
+        else:
+            q = np.ascontiguousarray(queries, dtype=np.float64)
+            if q.ndim != 2 or q.shape[1] != f:
+                raise ValueError("query length %d must match nfeatures %d" % (q.shape[-1], f))
+            nq = q.shape[0]
+            idx = np.empty((ntau, nq, topk), dtype=np.int64)
+            score = np.empty((ntau, nq, topk), dtype=np.float64)
+            qp, ip, sp = q.ctypes.data, idx.ctypes.data, score.ctypes.data
+        bits = self._allowed_bits(allowed)
+        try:
+            _lib.check(lib.asp_search_batch_taus(self._h, gl._h, qp, nq, taus.ctypes.data, ntau, topk, ip, sp, None,
+                                                 None if bits is None else bits.ctypes.data))
+        except LibraryError as e:
+            if e.code == _lib.ASP_ERR_LAMBDA_ZERO:                          # src/lib.rs:156-159
+                raise PanicException("assertion `left != right` failed: %s\n  left: 0.0\n right: 0.0" % e.message)
+            if e.code == _lib.ASP_ERR_ZERO_VECTOR:
+                raise PanicException(e.message)
+            raise
         return idx, score
 
     def _allowed_bits(self, allowed):

@@ -2,6 +2,7 @@
 // Host-side orchestration only; every numeric step is a kernel in gram.cu / graph_select.cu /
 // csr.cu / taumode.cu / search.cu / knn.cu / range.cu.  There is no CPU fallback anywhere in this file.
 #include "common.cuh"
+#include "sweep_bound.cuh"
 #include "hybrid.cuh"
 
 #include <algorithm>
@@ -727,6 +728,30 @@ int asp_query_lambda(asp_ctx *ctx, const asp_graph *g, const asp_switches *sw_in
 // exact stage 2.  `flags` is a 2-int device scratch.  allowed: the item mask as upload_allowed left it, or nullptr.
 // Synchronises ctx->stream before returning.  wide (the _k entry points only): topk 32 .. 64 stays on the tensor-core route
 // with the wide stage 2; without it such a topk takes the batched exact scan, as the graph-topk entry points always have.
+// Whether a batch of nq queries at tau with topk results takes stage 1 on tcgen05 (fp16 split); otherwise FP64 DMMA / GEMV.
+// Same exact stage 2, same answers.  Small batches against a large shard stream the fp16 operands (2 * kp bytes per item)
+// instead of the f64 rows.
+static bool search_takes_tc(const asp_space *s, int64_t nq, int64_t topk, double tau, bool wide)
+{
+    const char *force = getenv("ASP_SEARCH_STAGE1");
+    const bool want_fp64 = force && force[0] == 'f';
+    const bool want_tc = force && force[0] == 't';
+    return !want_fp64 && asp_search_tc_supported(s, nq, topk, tau, wide) && (want_tc || nq >= 256 || s->n_local >= 131072);
+}
+
+// The search of a device batch whose lambda_q (dlam) and norms (dnorm) are known.  Synchronises ctx->stream.
+static int search_device_stage(const asp_space *s, const asp_graph *g, const double *dq, int64_t nq, double tau, int64_t topk,
+                               const double *dlam, const double *dnorm, int64_t *didx, double *dscore, const uint32_t *allowed, bool wide)
+{
+    int rc;
+    if (search_takes_tc(s, nq, topk, tau, wide))
+        rc = asp_search_tc_impl(s, dq, nq, s->fp, dlam, dnorm, tau, topk, didx, dscore, nullptr, allowed, wide);
+    else
+        rc = asp_search_impl(s, g, dq, nq, s->fp, dlam, dnorm, tau, topk, didx, dscore, allowed);
+    if (rc == ASP_OK) ASP_CUDA(cudaStreamSynchronize(s->ctx->stream));
+    return rc;
+}
+
 static int search_device_batch(const asp_space *s, const asp_graph *g, const double *dq, int64_t nq, double tau, int64_t topk,
                                double *dlam, double *dnorm, int *flags, int64_t *didx, double *dscore,
                                bool assert_lambda_nonzero = true, const uint32_t *allowed = nullptr, bool wide = false)
@@ -747,17 +772,7 @@ static int search_device_batch(const asp_space *s, const asp_graph *g, const dou
         ASP_FAIL(ASP_ERR_LAMBDA_ZERO, "The lambdas are zero, check the magnitude of items and eps.");   // src/lib.rs:156-159
     ctx->stats["search_host_lambda_us"] = asp_now_us() - t_in;
     if (topk <= 0) return ASP_OK;
-    // stage 1 on tcgen05 (fp16 split) for batches, FP64 DMMA / GEMV otherwise; same exact stage 2, same answers
-    const char *force = getenv("ASP_SEARCH_STAGE1");
-    const bool want_fp64 = force && force[0] == 'f';
-    const bool want_tc = force && force[0] == 't';
-    int rc;
-    // small batches against a large shard stream the fp16 operands (2 * kp bytes per item) instead of the f64 rows
-    if (!want_fp64 && asp_search_tc_supported(s, nq, topk, tau, wide) && (want_tc || nq >= 256 || s->n_local >= 131072))
-        rc = asp_search_tc_impl(s, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore, nullptr, allowed, wide);
-    else
-        rc = asp_search_impl(s, g, dq, nq, fp, dlam, dnorm, tau, topk, didx, dscore, allowed);
-    if (rc == ASP_OK) ASP_CUDA(cudaStreamSynchronize(st));
+    const int rc = search_device_stage(s, g, dq, nq, tau, topk, dlam, dnorm, didx, dscore, allowed, wide);
     ctx->stats["search_host_device_batch_us"] = asp_now_us() - t_in;
     return rc;
 }
@@ -919,6 +934,95 @@ static int search_batch_topk(const asp_space *s, const asp_graph *g, const doubl
         ctx->stats["search_pipeline_chunks"] = 1;
     }
     return rc;
+}
+
+// Tau sweep (DESIGN §2 item 8): lambda_q once, then the taus that qualify for the tensor-core pass with k <= 16 in groups of at
+// most asp_sweep::NT_MAX, one candidate pass per group, and every other tau through the per-call-k search, in the caller's
+// order.  A lone qualifying tau takes the per-tau route too.  Each tau's rows are those of asp_search_batch_k at that tau.
+int asp_search_batch_taus(const asp_space *s, const asp_graph *g, const double *queries, int64_t nq, const double *taus,
+                          int64_t ntau, int64_t k, int64_t *out_idx, double *out_score, double *out_lambda_q,
+                          const uint8_t *allowed_bits)
+{
+    if (!s || !g || !taus || (nq > 0 && (!queries || !out_idx || !out_score))) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch_taus: NULL argument");
+    ASP_CHECK(check_call_k(k));
+    if (ntau < 1) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch_taus: at least one tau is needed (got %lld)", (long long)ntau);
+    for (int64_t t = 0; t < ntau; ++t)
+        if (!std::isfinite(taus[t])) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch_taus: tau %lld is not finite", (long long)t);
+    if (!s->have_lambdas) ASP_FAIL(ASP_ERR_ARG, "asp_search_batch: item lambdas have not been computed");
+    if (g->nnodes != s->f)
+        ASP_FAIL(ASP_ERR_ARG, "graph has %lld nodes but items have %d features", (long long)g->nnodes, s->f);
+    if (nq == 0) return ASP_OK;
+    if (s->f > 6144) ASP_FAIL(ASP_ERR_UNSUPPORTED, "search supports at most 6144 features (got %d)", s->f);
+    asp_ctx *ctx = s->ctx;
+    ASP_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const size_t rows = (size_t)nq * k;
+
+    asp_scratch sc(st);
+    double *dq = nullptr, *dlam = nullptr, *dnorm = nullptr, *dscore = nullptr;
+    int64_t *didx = nullptr;
+    int *flags = nullptr;
+    ASP_CHECK(sc.get(&dq, (size_t)nq * s->fp));
+    ASP_CHECK(sc.get(&dlam, (size_t)nq));
+    ASP_CHECK(sc.get(&dnorm, (size_t)nq));
+    ASP_CHECK(sc.get(&flags, 2));
+    ASP_CHECK(sc.get(&didx, rows * ntau));
+    ASP_CHECK(sc.get(&dscore, rows * ntau));
+    uint32_t *dallowed = nullptr;
+    ASP_CHECK(upload_allowed(sc, allowed_bits, s->n_local, &dallowed));
+    ASP_CHECK(upload_pitched(st, queries, nq, s->f, s->fp, dq));
+    ASP_CHECK(search_device_batch(s, g, dq, nq, taus[0], 0, dlam, dnorm, flags, nullptr, nullptr, true, dallowed));   // lambda_q, panics
+
+    // fused groups: the qualifying taus split into ceil(n / NT_MAX) groups of near-equal size (two or more each)
+    std::vector<int> fused;
+    for (int64_t t = 0; t < ntau; ++t)
+        if (k <= 16 && search_takes_tc(s, nq, k, taus[t], false)) fused.push_back((int)t);
+    if (fused.size() < 2) fused.clear();
+    const int ngroups = (int)asp_ceil_div((int64_t)fused.size(), asp_sweep::NT_MAX);
+    std::vector<int> group_of(ntau, -1);
+    for (size_t i = 0; i < fused.size(); ++i) group_of[fused[i]] = (int)(i * ngroups / fused.size());
+
+    for (const char *key : {"sweep_stage1_ms", "sweep_stage2_ms", "sweep_emitted"}) ctx->stats[key] = 0.0;
+    std::vector<int64_t> slow(ntau, 0);
+    std::vector<bool> done(ntau, false);
+    for (int64_t t = 0; t < ntau; ++t) {
+        if (done[t]) continue;
+        if (group_of[t] < 0) {
+            ctx->stats["search_slow_queries"] = 0.0;
+            ASP_CHECK(search_device_stage(s, g, dq, nq, taus[t], k, dlam, dnorm, didx + t * rows, dscore + t * rows, dallowed, true));
+            slow[t] = (int64_t)ctx->stats["search_slow_queries"];
+            done[t] = true;
+            continue;
+        }
+        std::vector<int> members;
+        std::vector<double> gt;
+        std::vector<int64_t *> gi;
+        std::vector<double *> gs;
+        for (int64_t u = t; u < ntau; ++u)
+            if (group_of[u] == group_of[t]) {
+                members.push_back((int)u); gt.push_back(taus[u]); gi.push_back(didx + u * rows); gs.push_back(dscore + u * rows);
+            }
+        std::vector<int64_t> gslow(members.size(), 0);
+        ASP_CHECK(asp_search_tc_sweep(s, dq, nq, s->fp, dlam, dnorm, gt.data(), (int)members.size(), k, gi.data(), gs.data(), dallowed,
+                                      gslow.data()));
+        ASP_CUDA(cudaStreamSynchronize(st));
+        for (size_t i = 0; i < members.size(); ++i) { slow[members[i]] = gslow[i]; done[members[i]] = true; }
+    }
+
+    if (out_lambda_q) ASP_CHECK(asp_copy_out(ctx, out_lambda_q, dlam, sizeof(double) * nq));
+    ASP_CHECK(asp_copy_out(ctx, out_idx, didx, sizeof(int64_t) * rows * ntau));
+    ASP_CHECK(asp_copy_out(ctx, out_score, dscore, sizeof(double) * rows * ntau));
+    ASP_CUDA(cudaStreamSynchronize(st));
+    double total = 0.0;
+    for (int64_t t = 0; t < ntau; ++t) {
+        total += (double)slow[t];
+        ctx->stats["sweep_slow_queries_" + std::to_string(t)] = (double)slow[t];
+    }
+    ctx->stats["search_slow_queries"] = total;
+    ctx->stats["sweep_fused_taus"] = (double)fused.size();
+    ctx->stats["sweep_stage1_passes"] = ngroups;
+    ctx->stats["sweep_emitted_per_query"] = ngroups ? ctx->stats["sweep_emitted"] / ((double)nq * ngroups) : 0.0;
+    return ASP_OK;
 }
 
 int64_t asp_hybrid_pool(int64_t n_total, int64_t topk, int64_t pool)

@@ -232,13 +232,20 @@ struct asp_tc_batch {                     // device buffers of one batch of quer
 enum { ASP_TC_ORDER_IDENTITY = 0, ASP_TC_ORDER_LAMBDA = 1, ASP_TC_ORDER_NORM = 2 };   // item order of the operand cache
 int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                   const double *qnorm_dev, double tau, int64_t topk, double score_floor, int force_terms, int capb_override,
-                  float *dump_dev, asp_tc_batch *b, bool l2 = false, const uint32_t *allowed_dev = nullptr);
+                  float *dump_dev, asp_tc_batch *b, bool l2 = false, const uint32_t *allowed_dev = nullptr,
+                  const double *sweep_taus = nullptr, int ntau = 1);
 int asp_device_max(asp_ctx *ctx, const double *v_dev, int64_t n, double *out);   // max(0, max v), synchronises
 // wide: topk up to 128 on the tensor-core route (wide stage 2 from 32 on); otherwise topk <= 32 as the graph-topk entry points use
 bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, double tau, bool wide = false);
 int asp_search_tc_impl(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                        const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
                        float *dump_dev, const uint32_t *allowed_dev = nullptr, bool wide = false);
+// Tau sweep: ONE candidate pass for ntau = 2 .. asp_sweep::NT_MAX taus (topk <= 16, each tau asp_search_tc_supported), then
+// per tau the search's stage 2 and remedies.  out_idx_dev[u] / out_score_dev[u]: [nq][topk] of tau u; slow_out[u]: the
+// queries of tau u that took the exact scan.
+int asp_search_tc_sweep(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
+                        const double *qnorm_dev, const double *taus, int ntau, int64_t topk, int64_t *const *out_idx_dev,
+                        double *const *out_score_dev, const uint32_t *allowed_dev, int64_t *slow_out);
 void asp_free_tc_cache(asp_space *s);
 int asp_launch_reciprocal(asp_ctx *ctx, const double *x, int64_t n, double *out);
 int asp_search_slow_path(const asp_space *s, const double *q_dev, int32_t qpitch, const double *lambda_q_dev,

@@ -56,6 +56,7 @@
 #include "warp_sort.cuh"
 #include "l2_bound.cuh"
 #include "large_k.cuh"
+#include "sweep_bound.cuh"
 
 #include <cuda_fp16.h>
 #include <algorithm>
@@ -439,6 +440,12 @@ struct TcParams {
     int32_t *emit_cnt;
     float *dump;                  // DUMP mode: approximate cosines [nq][n_local], local item order
     const uint32_t *vbits;        // FILTER: item mask in visiting order, zero beyond n_local (whole tiles)
+    // NT > 1 (tau sweep): ntau (2 .. NT) taus from one pass; tau t reads plane t of delta_q / theta_glob ([nq] each) and
+    // writes plane t of emit_sc (`plane` floats each) and of emit_cnt ([nq][nchunks] each); slots t >= ntau hold tau 1, beta 0
+// and are never read
+    int ntau;
+    float taus[asp_sweep::NT_MAX], betas[asp_sweep::NT_MAX], inv_taus[asp_sweep::NT_MAX];
+    size_t plane;
 };
 
 // ARES (1-term mode, <= 7 k blocks): the query operand (128 x kp fp16, <= 112 KB) is loaded ONCE and stays resident in
@@ -454,7 +461,8 @@ struct TcParams {
 // L2 (score kind of the Euclidean item graph): the score is -d^2~ (l2_bound.cuh) instead of tau cos~ + beta prox; lam_x /
 // lam_q / tile_lo / tile_hi then hold the f32 norms (items in norm order) and the per-(row, tile) raw-accumulator threshold
 // comes from asp_l2::threshold instead of the proximity bound.  The MMAs and the pipeline are the same.
-template <bool DUMP, int VARIANT, bool ARES, bool PAIR, int LISTN, bool L2 = false, bool FILTER = false>   // LISTN (>= topk): the four column-quarter threads of a query row keep LISTN / 4 scores each; VARIANT (profiling only): 0 normal, 2 epilogue does no work, 3 no MMA issued, 4 epilogue loads TMEM only
+// NT > 1: a tau sweep (search only, LISTN 16): the epilogue serves p.ntau <= NT taus from the one set of accumulators.
+template <bool DUMP, int VARIANT, bool ARES, bool PAIR, int LISTN, bool L2 = false, bool FILTER = false, int NT = 1>   // LISTN (>= topk): the four column-quarter threads of a query row keep LISTN / 4 scores each; VARIANT (profiling only): 0 normal, 2 epilogue does no work, 3 no MMA issued, 4 epilogue loads TMEM only
 __global__ void __launch_bounds__(TC_THREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_constant__ CUtensorMap map_q_lo,
                const __grid_constant__ CUtensorMap map_x_hi, const __grid_constant__ CUtensorMap map_x_lo,
@@ -463,6 +471,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
     static_assert(!PAIR || ARES, "the CTA-pair kernel keeps the query operand resident");
     static_assert(!L2 || (!DUMP && VARIANT == 0), "the l2 score kind has no dump or profiling variants");
     static_assert(!FILTER || (!L2 && !DUMP && VARIANT == 0), "only the search is filtered");
+    static_assert(NT == 1 || (!L2 && !DUMP && VARIANT == 0 && LISTN == 16 && NT <= asp_sweep::NT_MAX), "the tau sweep is a search of k <= 16");
     extern __shared__ __align__(1024) unsigned char smem_raw[];
     // SWIZZLE_128B tiles must start on 1024-byte boundaries
     constexpr int NST = PAIR ? 6 : ARES ? 3 : TC_STAGES;                         // ring depth
@@ -473,9 +482,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
     float *s_const = reinterpret_cast<float *>(stages + NST * STB);              // [2][TN]: item lambdas per accumulator
     __shared__ __align__(8) uint64_t full_bar[MAXST], empty_bar[MAXST], tmem_full[2], tmem_empty[2], a_full;
     __shared__ uint32_t s_tmem_base;
-    __shared__ uint32_t s_theta[TQ];          // per query row: best k-th score seen by its threads / other CTAs (ordered bits)
+    __shared__ uint32_t s_theta[NT * TQ];     // per query row: best k-th score seen by its threads / other CTAs (ordered bits)
     __shared__ int s_cnt[TQ];                 // per query row: emission cursor shared by its column-quarter threads
-    __shared__ float s_part[TQ * 4];          // per query row and column quarter: that quarter's ceil(topk/4)-th best score
+    __shared__ float s_part[NT * TQ * 4];     // per query row and column quarter: that quarter's ceil(topk/4)-th best score
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int qb = blockIdx.x, chunk = blockIdx.y;
@@ -503,8 +512,14 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
         for (int a = 0; a < 2; ++a) { asp::mbar_init(&tmem_full[a], 1); asp::mbar_init(&tmem_empty[a], PAIR ? 2 * EPI_WARPS : EPI_WARPS); }
         asp::fence_barrier_init();
     }
-    if (threadIdx.x < TQ) { s_theta[threadIdx.x] = 0u; s_cnt[threadIdx.x] = 0; }
-    if (threadIdx.x < TQ * 4) s_part[threadIdx.x] = -INFINITY;
+    if constexpr (NT == 1) {
+        if (threadIdx.x < TQ) { s_theta[threadIdx.x] = 0u; s_cnt[threadIdx.x] = 0; }
+        if (threadIdx.x < TQ * 4) s_part[threadIdx.x] = -INFINITY;
+    } else {                                                                     // one s_theta / s_part slot per tau
+        if (threadIdx.x < TQ) s_cnt[threadIdx.x] = 0;
+        for (int i = threadIdx.x; i < NT * TQ; i += TC_THREADS) s_theta[i] = 0u;
+        for (int i = threadIdx.x; i < NT * TQ * 4; i += TC_THREADS) s_part[i] = -INFINITY;
+    }
     if (warp == 1) { if (PAIR) asp::tmem_alloc_pair(&s_tmem_base, 512); else asp::tmem_alloc(&s_tmem_base, 512); }
     asp::tc_fence_before();
     __syncthreads();
@@ -603,6 +618,168 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap map_q_hi, const __grid_consta
                     if (++s == NST) { s = 0; ph ^= 1u; }
                 }
             }
+        }
+    } else if constexpr (NT > 1) {
+        // ===================== tau-sweep epilogue: warps 2..17, thread <-> (query row, column quarter) =====================
+        // Per tau u, the state of the single-tau epilogue below (running list, theta_k, theta_emit, beta_ub, its s_theta /
+        // s_part / theta_glob slot), every update as there.  The common path compares the max tree against the SMALLEST of
+        // the taus' raw-accumulator thresholds (sweep_bound.cuh); a column that passes gets its score at every tau, is emitted
+        // once if it reaches some tau's theta_emit (index in emit_ix, score u in plane u of emit_sc) and enters every tau's
+        // list it beats.  Slots u >= p.ntau start at +inf and never move.  DESIGN §2 item 8.
+        const int lg = warp & 3;
+        const int part = (warp - 2) >> 2;
+        const int row = lg * 32 + lane;
+        const int64_t gq = (int64_t)qb * TQ + row;
+        const bool qvalid = gq < p.nq;
+        const float lq = qvalid ? p.lam_q[gq] : 0.f;
+        const int et = threadIdx.x - 64;
+        constexpr int PL = LISTN / 4;
+        const int rr = (p.topk + 3) >> 2;
+        __shared__ float s_delta2[NT * TQ];                                    // 2 x the row's band per tau (needed when theta_k moves)
+        __shared__ int s_lost[TQ];                                             // per row: bit u = a record tau u admitted found the buffer full
+        if (part == 0) s_lost[row] = 0;
+        float theta_k[NT], theta_emit[NT], lst[NT][PL];
+        uint32_t nx_go[NT];
+#pragma unroll
+        for (int u = 0; u < NT; ++u) {
+            const bool used = u < p.ntau;
+            if (part == 0) s_delta2[u * TQ + row] = (qvalid && used) ? 2.0f * p.delta_q[u * p.nq + gq] : 0.f;
+            theta_k[u] = used ? -INFINITY : INFINITY;
+            theta_emit[u] = theta_k[u];
+            nx_go[u] = 0u;
+#pragma unroll
+            for (int i = 0; i < PL; ++i) lst[u][i] = (!used || i < PL - rr) ? INFINITY : -INFINITY;
+        }
+        const size_t ebase = ((size_t)gq * p.nchunks + chunk) * (size_t)p.capb;
+        float nx_lam = 0.f, nx_tl = 0.f, nx_th = 0.f;
+        auto prefetch = [&](int t) {
+            if (t >= ntiles) return;
+            const int tile = tile_of(t);
+            if (et < TN) { const int64_t n = (int64_t)tile * TN + et; nx_lam = (n < p.n_local) ? p.lam_x[n] : 0.f; }
+            nx_tl = p.tile_lo[tile];
+            nx_th = p.tile_hi[tile];
+            if (part == 0 && qvalid) {
+#pragma unroll
+                for (int u = 0; u < NT; ++u)
+                    if (u < p.ntau) nx_go[u] = p.theta_glob[u * p.nq + gq];
+            }
+        };
+        prefetch(0);
+        for (int t = 0; t < ntiles; ++t) {
+            const int acc = (int)(t & 1);
+            const int tile = tile_of(t);
+            const int64_t item0 = (int64_t)tile * TN;
+            float *c_lam = s_const + acc * TN;
+            if (et < TN) c_lam[et] = nx_lam;
+            const float tl = nx_tl, th = nx_th;
+            if (part == 0 && qvalid) {
+#pragma unroll
+                for (int u = 0; u < NT; ++u)
+                    if (nx_go[u] > s_theta[u * TQ + row]) atomicMax(&s_theta[u * TQ + row], nx_go[u]);
+            }
+            asm volatile("bar.sync 1, %0;\n" ::"n"(EPI_WARPS * 32) : "memory");    // epilogue warps only
+            prefetch(t + 1);
+            float theta_acc = INFINITY;
+            const float pb = asp_sweep::prox_bound(lq, tl, th);
+            if (qvalid) {
+#pragma unroll
+                for (int u = 0; u < NT; ++u) {
+                    const uint32_t so = s_theta[u * TQ + row];
+                    if (so != 0u) {
+                        const float sh = o2f(so);
+                        if (sh > theta_k[u]) { theta_k[u] = sh; theta_emit[u] = theta_k[u] - s_delta2[u * TQ + row]; }
+                    }
+                }
+                theta_acc = asp_sweep::combined_threshold(theta_emit, p.betas, p.inv_taus, pb, NT);
+            }
+            asp::mbar_wait_suspend(&tmem_full[acc], (uint32_t)((t >> 1) & 1), 8000);
+            asp::tc_fence_after();
+#pragma unroll 1
+            for (int c = 0; c < EPI_COLS / 32; ++c) {
+                const int col0 = part * EPI_COLS + c * 32;
+                uint32_t r[32];
+                asp::tmem_ld_32x32(tmem_base + ((uint32_t)(lg * 32) << 16) + (uint32_t)(acc * TN + col0), r);
+                asp::tmem_ld_wait();
+                float m[16];                                                     // common path: a max tree and one compare
+#pragma unroll
+                for (int j = 0; j < 16; ++j) m[j] = fmaxf(__uint_as_float(r[2 * j]), __uint_as_float(r[2 * j + 1]));
+#pragma unroll
+                for (int w = 8; w > 0; w >>= 1)
+#pragma unroll
+                    for (int j = 0; j < w; ++j) m[j] = fmaxf(m[j], m[j + w]);
+                if (m[0] < theta_acc) continue;
+                uint32_t mask = 0;
+#pragma unroll
+                for (int j = 0; j < 32; ++j) mask |= (__uint_as_float(r[j]) >= theta_acc) ? (1u << j) : 0u;
+                if constexpr (FILTER) mask &= p.vbits[(item0 + col0) >> 5];
+                while (mask) {
+                    const int j = __ffs(mask) - 1;
+                    mask &= mask - 1;
+                    const float a = pick32(r, j);
+                    if (a < theta_acc) continue;                                 // the threshold rose inside this loop
+                    const int col = col0 + j;
+                    const int64_t n = item0 + col;
+                    if (n >= p.n_local) continue;
+                    const float px = asp_sweep::prox(lq, c_lam[col]);
+                    float sc[NT];
+                    uint32_t adm = 0;                                            // the taus whose threshold admits the column
+#pragma unroll
+                    for (int u = 0; u < NT; ++u) {
+                        sc[u] = asp_sweep::score(p.taus[u], p.betas[u], px, a);
+                        adm |= (sc[u] >= theta_emit[u]) ? (1u << u) : 0u;
+                    }
+                    if (!adm) continue;
+                    const int pos = atomicAdd(&s_cnt[row], 1);
+                    if (pos < p.capb) {
+                        p.emit_ix[ebase + pos] = p.perm[n];
+#pragma unroll
+                        for (int u = 0; u < NT; ++u)
+                            if (u < p.ntau) p.emit_sc[u * p.plane + ebase + pos] = sc[u];
+                    } else {
+                        atomicOr(&s_lost[row], (int)adm);
+                    }
+                    bool raised = false;
+#pragma unroll
+                    for (int u = 0; u < NT; ++u) {
+                        if (!(sc[u] > lst[u][PL - 1])) continue;
+                        float v = sc[u];                                         // sorted insertion
+#pragma unroll
+                        for (int i = 0; i < PL; ++i) {
+                            const float o = lst[u][i];
+                            const bool sw = v > o;
+                            lst[u][i] = sw ? v : o;
+                            v = sw ? o : v;
+                        }
+                        volatile float *my_part = s_part + (u * TQ + row) * 4;
+                        my_part[part] = lst[u][PL - 1];                          // a stale (lower) value read by the others is still valid
+                        const float kth = fminf(fminf(my_part[0], my_part[1]), fminf(my_part[2], my_part[3]));
+                        if (kth > theta_k[u]) {
+                            theta_k[u] = kth;
+                            theta_emit[u] = theta_k[u] - s_delta2[u * TQ + row];
+                            raised = true;
+                            const uint32_t ko = f2o(kth);
+                            atomicMax(&s_theta[u * TQ + row], ko);
+                            atomicMax(&p.theta_glob[u * p.nq + gq], ko);
+                        }
+                    }
+                    if (raised) theta_acc = asp_sweep::combined_threshold(theta_emit, p.betas, p.inv_taus, pb, NT);
+                }
+            }
+            asp::tc_fence_before();
+            __syncwarp();
+            if (lane == 0) {
+                if (PAIR) asp::mbar_arrive_cluster(asp::mapa_shared(asp::smem_u32(&tmem_empty[acc]), 0));   // the leader's MMA thread waits
+                else asp::mbar_arrive(&tmem_empty[acc]);
+            }
+        }
+        asm volatile("bar.sync 1, %0;\n" ::"n"(EPI_WARPS * 32) : "memory");
+        if (qvalid && part == 0) {
+            // one count plane per tau: the overflow (count > capb) only for a tau that lost a record it admitted; the other
+            // taus keep every record their own thresholds asked for, and stage 2 reads the capb that were written
+            const int cnt = s_cnt[row], lost = s_lost[row];
+#pragma unroll
+            for (int u = 0; u < NT; ++u)
+                if (u < p.ntau) p.emit_cnt[(u * p.nq + gq) * p.nchunks + chunk] = ((lost >> u) & 1) ? cnt : min(cnt, p.capb);
         }
     } else {
         // ===================== epilogue: warps 2..17, thread <-> (query row, column quarter) =====================
@@ -1342,10 +1519,12 @@ bool asp_search_tc_supported(const asp_space *s, int64_t nq, int64_t topk, doubl
 // leaves the emission lists in `b` for the caller's stage 2 (search: tc_rescore_kernel; item graph: knn.cu).
 // lambda_q_dev == nullptr: no lambda term (cosine kNN): identity query order.  dump_dev != nullptr: approximate cosines
 // [nq][n_local] f32 (tests), no emission.  l2 (Euclidean item graph): score -d^2~, items in norm order, queries visited in
-// the order of their norms (qnorm_dev is the key; lambda_q_dev and tau are unused).
+// the order of their norms (qnorm_dev is the key; lambda_q_dev and tau are unused).  ntau > 1 (tau sweep, search of
+// topk <= 16): the pass serves sweep_taus[0 .. ntau), `tau` is unused, and delta_q, theta_glob and emit_sc hold one plane
+// per tau ([nq] / [nq] / [nq][nsub][capb]), and so does emit_cnt ([nq][nsub]).
 int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
                   const double *qnorm_dev, double tau, int64_t topk, double score_floor, int force_terms, int capb_override,
-                  float *dump_dev, asp_tc_batch *b, bool l2, const uint32_t *allowed_dev)
+                  float *dump_dev, asp_tc_batch *b, bool l2, const uint32_t *allowed_dev, const double *sweep_taus, int ntau)
 {
     asp_ctx *ctx = s->ctx;
     cudaStream_t st = ctx->stream;
@@ -1353,6 +1532,10 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     asp_tc_cache *c = nullptr;
     if (l2 && dump_dev) ASP_FAIL(ASP_ERR_ARG, "asp_tc_stage1: no dump of the l2 score");
     if (allowed_dev && (l2 || dump_dev)) ASP_FAIL(ASP_ERR_ARG, "asp_tc_stage1: only the search is filtered");
+    const bool sweep = ntau > 1;
+    if (sweep && (l2 || dump_dev || topk > 16 || ntau > asp_sweep::NT_MAX || score_floor > -1e300))
+        ASP_FAIL(ASP_ERR_ARG, "asp_tc_stage1: a tau sweep is a search of k <= 16 over at most %d taus", asp_sweep::NT_MAX);
+    const int planes = sweep ? ntau : 1;
     ASP_CHECK(ensure_tc_cache(s, l2, &c));
     if (l2) { lambda_q_dev = qnorm_dev; tau = 1.0; }
     const int kp = c->kp;
@@ -1368,7 +1551,7 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     ASP_CHECK(b->mem.get(&b->lam_q32, (size_t)nq));
     ASP_CHECK(b->mem.get(&b->inv_nq, (size_t)nq));
     ASP_CHECK(b->mem.get(&b->rho_q, (size_t)nq));
-    ASP_CHECK(b->mem.get(&b->delta_q, (size_t)nq));
+    ASP_CHECK(b->mem.get(&b->delta_q, (size_t)nq * planes));
     ASP_CHECK(asp_launch_reciprocal(ctx, qnorm_dev, nq, b->inv_nq));
     const bool by_lambda = !dump_dev && lambda_q_dev && c->order != ASP_TC_ORDER_IDENTITY;   // (l2: by the query norms)
     if (by_lambda) {
@@ -1398,7 +1581,13 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     if (nterms == 3) ASP_CHECK(ensure_tc_lo(s, c));
     const double c_main = (nterms == 1) ? c_main1 : c_main3;
     if (l2) row_delta_l2_kernel<<<64, 256, 0, st>>>(b->rho_q, qnorm_dev, b->qperm, nq, c_main, c_fixed, c->norm_max, b->delta_q);
-    else row_delta_kernel<<<64, 256, 0, st>>>(b->rho_q, nq, c_main, c_fixed, fabs(tau), (fabs(tau) + fabs(1.0 - tau)) * 2e-6, b->delta_q);
+    else
+        for (int u = 0; u < planes; ++u) {
+            const double tu = sweep ? sweep_taus[u] : tau;
+            row_delta_kernel<<<64, 256, 0, st>>>(b->rho_q, nq, c_main, c_fixed, fabs(tu), (fabs(tu) + fabs(1.0 - tu)) * 2e-6,
+                                                 b->delta_q + (size_t)u * nq);
+            if (u + 1 < planes) { ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx); }
+        }
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
     b->nterms = nterms;
     b->delta_cos_max = rho_q_max * c_main + c_fixed;
@@ -1459,6 +1648,11 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
     p.nw_hi = c->nw;
     p.lam_x = c->lam32; p.lam_q = b->lam_q32; p.tile_lo = c->tile_lo; p.tile_hi = c->tile_hi; p.perm = c->perm; p.center = b->center;
     p.theta_glob = nullptr; p.emit_sc = nullptr; p.emit_ix = nullptr; p.emit_cnt = nullptr; p.dump = dump_dev; p.vbits = nullptr;
+    p.ntau = planes; p.plane = (size_t)nq * nchunks * capb;
+    for (int u = 0; u < asp_sweep::NT_MAX; ++u) {                 // unused slots: tau 1, beta 0 (never read)
+        const float tu = (sweep && u < ntau) ? (float)sweep_taus[u] : 1.0f;
+        p.taus[u] = tu; p.betas[u] = (sweep && u < ntau) ? (float)(1.0 - sweep_taus[u]) : 0.0f; p.inv_taus[u] = 1.0f / tu;
+    }
     if (allowed_dev) {                                            // from the cache's current order (it may have been rebuilt)
         const int64_t nwords = tiles_total * (TN / 32);
         ASP_CHECK(b->mem.get(&b->vbits, (size_t)nwords));
@@ -1468,11 +1662,11 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
         p.vbits = b->vbits;
     }
     if (!dump_dev) {
-        ASP_CHECK(b->mem.get(&b->emit_sc, (size_t)nq * nchunks * capb));
+        ASP_CHECK(b->mem.get(&b->emit_sc, (size_t)nq * nchunks * capb * planes));
         ASP_CHECK(b->mem.get(&b->emit_ix, (size_t)nq * nchunks * capb));
-        ASP_CHECK(b->mem.get(&b->emit_cnt, (size_t)nq * nchunks));
-        ASP_CHECK(b->mem.get(&b->theta_glob, (size_t)nq));
-        ASP_CUDA(cudaMemsetAsync(b->theta_glob, 0, sizeof(uint32_t) * (size_t)nq, st));
+        ASP_CHECK(b->mem.get(&b->emit_cnt, (size_t)nq * nchunks * planes));
+        ASP_CHECK(b->mem.get(&b->theta_glob, (size_t)nq * planes));
+        ASP_CUDA(cudaMemsetAsync(b->theta_glob, 0, sizeof(uint32_t) * (size_t)nq * planes, st));
         p.emit_sc = b->emit_sc; p.emit_ix = b->emit_ix; p.emit_cnt = b->emit_cnt; p.theta_glob = b->theta_glob;
     }
 
@@ -1527,6 +1721,12 @@ int asp_tc_stage1(const asp_space *s, const double *q_dev, int64_t nq, int32_t q
                          : tc_gemm_kernel<false, 0, false, false, 32, true>)
                  : (pair ? tc_gemm_kernel<false, 0, true, true, 16, true> : ares ? tc_gemm_kernel<false, 0, true, false, 16, true>
                          : tc_gemm_kernel<false, 0, false, false, 16, true>);
+    constexpr int NTS = asp_sweep::NT_MAX;
+    if (sweep)
+        k = allowed_dev ? (pair ? tc_gemm_kernel<false, 0, true, true, 16, false, true, NTS> : ares ? tc_gemm_kernel<false, 0, true, false, 16, false, true, NTS>
+                                : tc_gemm_kernel<false, 0, false, false, 16, false, true, NTS>)
+                        : (pair ? tc_gemm_kernel<false, 0, true, true, 16, false, false, NTS> : ares ? tc_gemm_kernel<false, 0, true, false, 16, false, false, NTS>
+                                : tc_gemm_kernel<false, 0, false, false, 16, false, false, NTS>);
     ASP_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     ASP_CUDA(cudaEventRecord(ctx->ev0, st));
     if (pair) {
@@ -1570,6 +1770,39 @@ __global__ void scatter_results_kernel(const int64_t *__restrict__ idx2, const d
 }
 }  // namespace
 
+// f64 band of stage 2's fast re-score at tau
+static double stage2_eps_fast(const asp_space *s, double tau)
+{
+    const double u = 1.1102230246251565e-16;
+    return (4.0 * s->f + 64.0) * u * (fabs(tau) + fabs(1.0 - tau) + 1.0);
+}
+
+// Stage 2 of topk <= 32 (tc_rescore_kernel) on the emission lists of b, with the scores, counts and bands of one tau (emit_sc,
+// emit_cnt, delta_q: b's own, or one plane of a tau sweep).
+static int launch_stage2(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
+                         const double *qnorm_dev, double tau, int64_t topk, const asp_tc_batch &b, const float *delta_q,
+                         const float *emit_sc, const int32_t *emit_cnt, int64_t *out_idx_dev, double *out_score_dev, int32_t *slow_list,
+                         int32_t *slow_count, unsigned long long *counters)
+{
+    cudaStream_t st = s->ctx->stream;
+    const double eps_fast = stage2_eps_fast(s, tau);
+    // small batches (the reference's one query per call, latency bound): a whole CTA per query
+    const int wpq = (nq <= 64) ? 32 : (nq <= 1024) ? 8 : 1;
+    auto launch_rescore = [&](auto kern, int nwarps, int qcopies, unsigned grid) -> int {
+        const size_t rsmem = (size_t)qcopies * s->fp * 8 + (size_t)nwarps * TR_QUEUE * 4 + (size_t)nwarps * 32 * 16;
+        ASP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rsmem));
+        kern<<<grid, nwarps * 32, rsmem, st>>>(
+            q_dev, qpitch, nq, s->items, s->n_local, s->f, s->fp, s->row0, s->norms, s->lambdas, qnorm_dev, lambda_q_dev, tau,
+            (int)topk, b.nsub, b.capb, delta_q, eps_fast, emit_sc, b.emit_ix, emit_cnt, b.theta_glob, b.qperm, out_idx_dev,
+            out_score_dev, slow_list, slow_count, counters, counters + 1);
+        return ASP_OK;
+    };
+    if (wpq == 32) return launch_rescore(tc_rescore_kernel<32>, 32, 1, (unsigned)nq);
+    if (wpq == 8) return launch_rescore(tc_rescore_kernel<8>, 8, 1, (unsigned)nq);
+    if (getenv("ASP_TC_RESCORE_OCC6")) return launch_rescore(tc_rescore_kernel<1>, TR_WARPS, TR_WARPS, (unsigned)asp_ceil_div(nq, TR_WARPS));
+    return launch_rescore(tc_rescore_kernel<1, TR_MIN_CTAS>, TR_WARPS, TR_WARPS, (unsigned)asp_ceil_div(nq, TR_WARPS));
+}
+
 // One attempt with a given number of MMA terms.  The search always tries ONE fp16 term first: its band is wide when the
 // residual norms are large (mean-zero embeddings: 2e-3 in cosine against 2e-5 for the three-term split), but a wide band only
 // costs survivors in stage 2 -- measured on the mean-zero C4 regime: 22.9 survivors per query instead of 10.1, 37 ms per 64k
@@ -1579,6 +1812,44 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
                              const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
                              float *dump_dev, int force_terms, bool may_retry, const uint32_t *allowed_dev, bool wide);
 
+// The retry of the slow queries (slow_list, device) of a single-term attempt with the three-term split; their results are
+// scattered into the caller's rows.  Synchronises the stream.
+static int retry_three_terms(const asp_space *s, const double *q_dev, int32_t qpitch, const double *lambda_q_dev,
+                             const double *qnorm_dev, double tau, int64_t topk, const int32_t *slow_list, int nslow,
+                             int64_t *out_idx_dev, double *out_score_dev, const uint32_t *allowed_dev, bool wide)
+{
+    asp_ctx *ctx = s->ctx;
+    cudaStream_t st = ctx->stream;
+    asp_scratch retry(st);
+    double *q2 = nullptr, *lam2 = nullptr, *nrm2 = nullptr, *sc2 = nullptr;
+    int64_t *idx2 = nullptr;
+    ASP_CHECK(retry.get(&q2, (size_t)nslow * qpitch));
+    ASP_CHECK(retry.get(&lam2, (size_t)nslow));
+    ASP_CHECK(retry.get(&nrm2, (size_t)nslow));
+    ASP_CHECK(retry.get(&idx2, (size_t)nslow * topk));
+    ASP_CHECK(retry.get(&sc2, (size_t)nslow * topk));
+    gather_queries_kernel<<<(unsigned)nslow, 128, 0, st>>>(q_dev, qpitch, lambda_q_dev, qnorm_dev, slow_list, nslow, q2, lam2, nrm2);
+    ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
+    int rc = search_tc_attempt(s, q2, nslow, qpitch, lam2, nrm2, tau, topk, idx2, sc2, nullptr, 3, false, allowed_dev, wide);
+    if (rc == ASP_OK) {
+        scatter_results_kernel<<<(unsigned)nslow, 32, 0, st>>>(idx2, sc2, slow_list, nslow, (int)topk, out_idx_dev, out_score_dev);
+        ASP_LAUNCHED(ctx);
+        if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) { asp_set_error("search retry: scatter failed"); rc = ASP_ERR_CUDA; }
+    }
+    return rc;
+}
+
+// MMA terms of a search's first attempt, and whether its slow queries may be retried with three
+static int first_terms(bool *may_retry)
+{
+    const char *e = getenv("ASP_TC_FIRST_TERMS");                  // A/B knob: "auto" = the band rule decides (the earlier behaviour)
+    int first = (e && e[0] == 'a') ? 0 : 1;
+    if (const char *t = getenv("ASP_TC_TERMS")) { const int v = atoi(t); if (v == 1 || v == 3) first = v; }   // test knob: that mode, no retry
+    const bool pinned = getenv("ASP_TC_TERMS") != nullptr;
+    *may_retry = first == 1 && !pinned;
+    return first;
+}
+
 // dump == nullptr: full search.  dump != nullptr: approximate cosines [nq][n_local] f32 (tests).  allowed_dev: item mask
 // (local item order, packed) or nullptr.  wide: topk = 32 .. 128 takes the wide stage 2 (tc_rescore_wide_kernel) instead of
 // the 32-per-warp one, whose lists cannot hold a candidate beyond the 32nd (the _k entry points only).
@@ -1586,12 +1857,10 @@ int asp_search_tc_impl(const asp_space *s, const double *q_dev, int64_t nq, int3
                        const double *qnorm_dev, double tau, int64_t topk, int64_t *out_idx_dev, double *out_score_dev,
                        float *dump_dev, const uint32_t *allowed_dev, bool wide)
 {
-    const char *e = getenv("ASP_TC_FIRST_TERMS");                  // A/B knob: "auto" = the band rule decides (the earlier behaviour)
-    int first = dump_dev ? 0 : (e && e[0] == 'a') ? 0 : 1;
-    if (const char *t = getenv("ASP_TC_TERMS")) { const int v = atoi(t); if (v == 1 || v == 3) first = v; }   // test knob: that mode, no retry
-    const bool pinned = getenv("ASP_TC_TERMS") != nullptr;
+    bool may_retry = false;
+    const int first = dump_dev ? 0 : first_terms(&may_retry);
     return search_tc_attempt(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, out_idx_dev, out_score_dev, dump_dev, first,
-                             first == 1 && !pinned, allowed_dev, wide);
+                             may_retry, allowed_dev, wide);
 }
 
 static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
@@ -1625,19 +1894,7 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
     ASP_CHECK(sc.get(&counters, 2));
     ASP_CUDA(cudaMemsetAsync(slow_count, 0, sizeof(int32_t), st));
     ASP_CUDA(cudaMemsetAsync(counters, 0, 2 * sizeof(unsigned long long), st));
-    const double u = 1.1102230246251565e-16;
-    const double eps_fast = (4.0 * s->f + 64.0) * u * (fabs(tau) + fabs(1.0 - tau) + 1.0);
-    // small batches (the reference's one query per call, latency bound): a whole CTA per query
-    const int wpq = (nq <= 64) ? 32 : (nq <= 1024) ? 8 : 1;
-    auto launch_rescore = [&](auto kern, int nwarps, int qcopies, unsigned grid) -> int {
-        const size_t rsmem = (size_t)qcopies * s->fp * 8 + (size_t)nwarps * TR_QUEUE * 4 + (size_t)nwarps * 32 * 16;
-        ASP_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rsmem));
-        kern<<<grid, nwarps * 32, rsmem, st>>>(
-            q_dev, qpitch, nq, s->items, s->n_local, s->f, s->fp, s->row0, s->norms, s->lambdas, qnorm_dev, lambda_q_dev, tau,
-            (int)topk, b.nsub, b.capb, b.delta_q, eps_fast, b.emit_sc, b.emit_ix, b.emit_cnt, b.theta_glob, b.qperm, out_idx_dev,
-            out_score_dev, slow_list, slow_count, counters, counters + 1);
-        return ASP_OK;
-    };
+    const double eps_fast = stage2_eps_fast(s, tau);
     if (wide2) {
         const size_t wsmem = (size_t)s->fp * 8 + (size_t)asp_lk::SURV_CAP * (sizeof(uint64_t) + sizeof(int32_t));
         ASP_CUDA(cudaFuncSetAttribute(tc_rescore_wide_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
@@ -1645,10 +1902,8 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
             q_dev, qpitch, s->items, s->n_local, s->f, s->fp, s->row0, s->norms, s->lambdas, qnorm_dev, lambda_q_dev, tau, (int)topk,
             b.nsub, b.capb, b.delta_q, eps_fast, b.emit_sc, b.emit_ix, b.emit_cnt, b.qperm, out_idx_dev, out_score_dev, slow_list,
             slow_count, counters, counters + 1);
-    } else if (wpq == 32) ASP_CHECK(launch_rescore(tc_rescore_kernel<32>, 32, 1, (unsigned)nq));
-    else if (wpq == 8) ASP_CHECK(launch_rescore(tc_rescore_kernel<8>, 8, 1, (unsigned)nq));
-    else if (getenv("ASP_TC_RESCORE_OCC6")) ASP_CHECK(launch_rescore(tc_rescore_kernel<1>, TR_WARPS, TR_WARPS, (unsigned)asp_ceil_div(nq, TR_WARPS)));
-    else ASP_CHECK(launch_rescore(tc_rescore_kernel<1, TR_MIN_CTAS>, TR_WARPS, TR_WARPS, (unsigned)asp_ceil_div(nq, TR_WARPS)));
+    } else ASP_CHECK(launch_stage2(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, tau, topk, b, b.delta_q, b.emit_sc, b.emit_cnt,
+                                   out_idx_dev, out_score_dev, slow_list, slow_count, counters));
     ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
     ASP_CUDA(cudaEventRecord(ctx->ev2, st));
     int32_t nslow = 0;
@@ -1670,23 +1925,9 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
     const bool wide_band = b.nterms == 1 && b.delta_cos_max > 2.5e-4;   // the three-term split has a much tighter band to offer
     if (nslow > 0 && may_retry && wide_band) {
         const std::map<std::string, double> first_stats = ctx->stats;
-        asp_scratch retry(st);
-        double *q2 = nullptr, *lam2 = nullptr, *nrm2 = nullptr, *sc2 = nullptr;
-        int64_t *idx2 = nullptr;
-        ASP_CHECK(retry.get(&q2, (size_t)nslow * qpitch));
-        ASP_CHECK(retry.get(&lam2, (size_t)nslow));
-        ASP_CHECK(retry.get(&nrm2, (size_t)nslow));
-        ASP_CHECK(retry.get(&idx2, (size_t)nslow * topk));
-        ASP_CHECK(retry.get(&sc2, (size_t)nslow * topk));
-        gather_queries_kernel<<<(unsigned)nslow, 128, 0, st>>>(q_dev, qpitch, lambda_q_dev, qnorm_dev, slow_list, nslow, q2, lam2, nrm2);
-        ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
         b.mem.release();                                              // the retry allocates its own emission buffers
-        rc = search_tc_attempt(s, q2, nslow, qpitch, lam2, nrm2, tau, topk, idx2, sc2, nullptr, 3, false, allowed_dev, wide);
-        if (rc == ASP_OK) {
-            scatter_results_kernel<<<(unsigned)nslow, 32, 0, st>>>(idx2, sc2, slow_list, nslow, (int)topk, out_idx_dev, out_score_dev);
-            ASP_LAUNCHED(ctx);
-            if (cudaGetLastError() != cudaSuccess || cudaStreamSynchronize(st) != cudaSuccess) { asp_set_error("search retry: scatter failed"); rc = ASP_ERR_CUDA; }
-        }
+        rc = retry_three_terms(s, q_dev, qpitch, lambda_q_dev, qnorm_dev, tau, topk, slow_list, nslow, out_idx_dev, out_score_dev,
+                               allowed_dev, wide);
         const double retry_slow = ctx->stats["search_slow_queries"], retry_ms = ctx->stats["search_stage1_ms"] + ctx->stats["search_stage2_ms"];
         ctx->stats = first_stats;                                     // the batch's figures stay those of the first attempt
         ctx->stats["search_retry_queries"] = nslow;
@@ -1697,4 +1938,69 @@ static int search_tc_attempt(const asp_space *s, const double *q_dev, int64_t nq
                                   allowed_dev);
     }
     return rc;
+}
+
+// Tau sweep (DESIGN §2 item 8): one candidate pass for all ntau taus, then per tau the stage 2 above on that tau's score
+// plane, and today's remedies for its slow queries (the three-term retry when the single-term band is wide, else the exact
+// scan).  The stage-2 kernels of all taus run back to back; the emission buffers are released before the remedies.
+int asp_search_tc_sweep(const asp_space *s, const double *q_dev, int64_t nq, int32_t qpitch, const double *lambda_q_dev,
+                        const double *qnorm_dev, const double *taus, int ntau, int64_t topk, int64_t *const *out_idx_dev,
+                        double *const *out_score_dev, const uint32_t *allowed_dev, int64_t *slow_out)
+{
+    asp_ctx *ctx = s->ctx;
+    cudaStream_t st = ctx->stream;
+    bool may_retry = false;
+    const int first = first_terms(&may_retry);
+    asp_tc_batch b;
+    // the records of ntau taus share each (query, chunk) buffer: ntau times the single-tau capacity, so that one tau's
+    // records (tau = 1 on near duplicates) do not crowd out the others' and send their queries to the remedies
+    ASP_CHECK(asp_tc_stage1(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, taus[0], topk, -INFINITY, first, 1024 * ntau, nullptr, &b,
+                            false, allowed_dev, taus, ntau));
+    asp_scratch sc(st);
+    int32_t *slow_list = nullptr, *slow_count = nullptr;
+    unsigned long long *counters = nullptr;
+    ASP_CHECK(sc.get(&slow_list, (size_t)ntau * (nq + 1)));
+    ASP_CHECK(sc.get(&slow_count, (size_t)ntau));
+    ASP_CHECK(sc.get(&counters, 2 * (size_t)ntau));
+    ASP_CUDA(cudaMemsetAsync(slow_count, 0, sizeof(int32_t) * ntau, st));
+    ASP_CUDA(cudaMemsetAsync(counters, 0, 2 * sizeof(unsigned long long) * ntau, st));
+    const size_t plane = (size_t)nq * b.nsub * b.capb;
+    for (int u = 0; u < ntau; ++u) {
+        ASP_CHECK(launch_stage2(s, q_dev, nq, qpitch, lambda_q_dev, qnorm_dev, taus[u], topk, b, b.delta_q + (size_t)u * nq,
+                                b.emit_sc + u * plane, b.emit_cnt + (size_t)u * nq * b.nsub, out_idx_dev[u], out_score_dev[u],
+                                slow_list + (size_t)u * (nq + 1),
+                                slow_count + u, counters + 2 * u));
+        ASP_CUDA(cudaGetLastError()); ASP_LAUNCHED(ctx);
+    }
+    ASP_CUDA(cudaEventRecord(ctx->ev2, st));
+    std::vector<int32_t> nslow(ntau), cnt((size_t)nq * b.nsub);
+    ASP_CUDA(cudaMemcpyAsync(nslow.data(), slow_count, sizeof(int32_t) * ntau, cudaMemcpyDeviceToHost, st));
+    ASP_CUDA(cudaMemcpyAsync(cnt.data(), b.emit_cnt, sizeof(int32_t) * cnt.size(), cudaMemcpyDeviceToHost, st));
+    ASP_CUDA(cudaStreamSynchronize(st));
+    float ms = 0.f, ms2 = 0.f;
+    cudaEventElapsedTime(&ms, ctx->ev0, ctx->ev1);
+    cudaEventElapsedTime(&ms2, ctx->ev1, ctx->ev2);
+    double emitted = 0.0;                                         // records written (an overflowing buffer counts its capacity)
+    for (int32_t c : cnt) emitted += std::min(c, b.capb);
+    const bool wide_band = b.nterms == 1 && b.delta_cos_max > 2.5e-4;
+    const int nterms = b.nterms;
+    b.mem.release();                                              // the remedies allocate their own buffers
+    for (int u = 0; u < ntau; ++u) {
+        slow_out[u] = nslow[u];
+        if (nslow[u] == 0) continue;
+        const int32_t *list = slow_list + (size_t)u * (nq + 1);
+        if (may_retry && wide_band) {
+            ASP_CHECK(retry_three_terms(s, q_dev, qpitch, lambda_q_dev, qnorm_dev, taus[u], topk, list, nslow[u], out_idx_dev[u],
+                                        out_score_dev[u], allowed_dev, false));
+            slow_out[u] = (int64_t)ctx->stats["search_slow_queries"];   // what finally took the exact scan
+        } else {
+            ASP_CHECK(asp_search_slow_path(s, q_dev, qpitch, lambda_q_dev, qnorm_dev, taus[u], topk, list, nslow[u], out_idx_dev[u],
+                                           out_score_dev[u], allowed_dev));
+        }
+    }
+    ctx->stats["sweep_stage1_ms"] += ms;
+    ctx->stats["sweep_stage2_ms"] += ms2;
+    ctx->stats["sweep_emitted"] += emitted;
+    ctx->stats["search_terms"] = nterms;
+    return ASP_OK;
 }
